@@ -15,6 +15,7 @@ strong-scaling leg splits rank 0's candidate set over the ranks and checks the N
     python bench.py --gpus 1 --steps 5 --warmup 3
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference      # the reference's own C++ evaluator on the host cores
+    python bench.py --dump-outputs DIR    # also write what the last timed step computed, DIR/<name>.npy
 
 torch is used only for the multi-process rendezvous (gloo) -- never for device work.
 """
@@ -153,6 +154,24 @@ def fp64_peak_crosscheck(clocks):
     except Exception:
         pass
     return out
+
+
+DUMP_MAX_SCORES = 1 << 21      # 16 MB of scores and 16 MB of their indices: a dump stays below 64 MB at any candidate count
+
+
+def dump_outputs(dirname, arrays):
+    """--dump-outputs: every array as DIR/<name>.npy in float64"""
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(dirname, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
+def score_sample(scores):
+    """all the scores of a step, or a fixed seeded sample of DUMP_MAX_SCORES of them beside their candidate indices"""
+    if len(scores) <= DUMP_MAX_SCORES:
+        return {"ei": scores}
+    idx = np.sort(np.random.RandomState(0).choice(len(scores), DUMP_MAX_SCORES, replace=False))
+    return {"ei": scores[idx], "ei_index": idx}
 
 
 def flops_per_candidate_k2(N):
@@ -557,12 +576,14 @@ def run_direct_workload(args, rank, world, device, dist):
     t0 = time.perf_counter()
     samples = 0
     for q in range(nq):
-        query(False, my_xi[q])
+        last = query(False, my_xi[q])
         samples += cdirectGP.last["nsamples"]
     sync_all()
     t_tp = time.perf_counter() - t0
     launches = L.ibo_launch_count() - launches0
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"opt": [last[0]], "optx": last[1]})
     # ---- latency of one query: unsharded on this GPU, and sharded over all GPUs ----
     t0 = time.perf_counter()
     opt1, optx1 = query(False)
@@ -623,7 +644,16 @@ def main():
     ap.add_argument("--fp64", action="store_true",
                     help="make the FP64 DMMA kernels (IBO_FLAG_FP64) the main arm instead of the library default (INT8 tensor-core path for wide batches)")
     ap.add_argument("--suite", action="store_true", help="extra measurements (maximizeEI wall ms, model build, configs #1/#4/#5)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed on rank 0 as DIR/<name>.npy (float64): best = [EI, "
+                         "global candidate index] of the step's argmax, ei = the EI of every candidate (above %d candidates a fixed "
+                         "seeded sample, their indices in ei_index); --workload 5: opt and optx of the last query.  The copy of the "
+                         "scores to the host is part of the last timed step; the JSON line says so under dump_outputs" % DUMP_MAX_SCORES)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.suite or args.impl != "ours"):
+        ap.error("--dump-outputs writes the outputs of the timed GPU steps: not with --suite or --impl reference")
     if args.suite:
         return run_suite(args)
     args.warmup = max(args.warmup, 3) if (args.impl == "ours" and args.workload == 2) else max(args.warmup, 1 if args.impl == "ours" else 0)
@@ -671,8 +701,8 @@ def main():
     flags = _lib.FLAG_MODE_CPP | (0 if use_i8 else _lib.FLAG_FP64)
     other_flags = _lib.FLAG_MODE_CPP | (_lib.FLAG_FP64 if use_i8 else _lib.FLAG_INT8)
 
-    def step_resident():
-        best, bidx, ms = cands.score(_lib.ACQ_EI, ymax, XI, flags)
+    def step_resident(scores_out=None):
+        best, bidx, ms = cands.score(_lib.ACQ_EI, ymax, XI, flags, scores_out=scores_out)
         gidx = ctypes.c_long(rank * M + bidx)
         sc = c_double(best)
         if world > 1:
@@ -686,14 +716,18 @@ def main():
 
     for _ in range(args.warmup):
         step_resident()
+    # --dump-outputs: the last timed step also copies its scores to the host, into a pinned buffer to keep that copy short
+    last_scores = np.empty(M) if (args.dump_outputs and rank == 0) else None
+    if last_scores is not None:
+        _lib.check(L.ibo_host_register(last_scores.ctypes.data_as(ctypes.c_void_p), last_scores.nbytes))
     sampler = ClockSampler(device, rank, world)
     sync_all()
     sampler.start()
     launches0 = L.ibo_launch_count()
     _lib.check(L.ibo_stream_mark(model.handle, 0))
     tw0 = time.perf_counter()
-    for _ in range(args.steps):
-        best = step_resident()
+    for s in range(args.steps):
+        best = step_resident(last_scores if s == args.steps - 1 else None)
     _lib.check(L.ibo_stream_mark(model.handle, 1))
     sync_all()
     tw1 = time.perf_counter()
@@ -701,6 +735,9 @@ def main():
     msf = c_float(0)
     _lib.check(L.ibo_stream_elapsed_ms(model.handle, ctypes.byref(msf)))
     clocks = sampler.stop()
+    if last_scores is not None:
+        _lib.check(L.ibo_host_unregister(last_scores.ctypes.data_as(ctypes.c_void_p)))
+        dump_outputs(args.dump_outputs, dict(best=[best[0], best[1]], **score_sample(last_scores)))
     t_dev = msf.value * 1e-3
     t_wall = tw1 - tw0
 
@@ -866,6 +903,10 @@ def main():
                                 "frac_of_fp64_dmma_peak": (M * F_step / t_step / 1e12 / peak.value) if peak.value else None}
     line["config"]["arithmetic"] += ("; sigma^2 through the INT8 tensor-core emulation of the FP64 GEMM (library default for wide batches), "
                                      "mu as k*.alpha in FP64" if use_i8 else "; FP64 DMMA kernels (IBO_FLAG_FP64)")
+    if last_scores is not None:
+        line["dump_outputs"] = {"dir": args.dump_outputs, "timed_d2h_bytes": int(last_scores.nbytes),
+                                "note": "the last timed step also copied its scores to the host (pinned buffer): that copy is inside "
+                                        "the timed region and lowers `value` slightly; runs without --dump-outputs do not copy them"}
     if other_arm is not None:
         line["fp64_dmma_arm" if use_i8 else "int8_arm"] = other_arm
     if argmax_ok is not None:
