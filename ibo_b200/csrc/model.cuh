@@ -36,11 +36,10 @@ struct ibo_model {
     double* dY = nullptr;       // [Np]
     int* dInfo = nullptr;
     bool from_inverse = false;        // built from a caller-supplied inverse (legacy acqmaxGP): sigma^2 >= noise is not guaranteed
-    // INT8 path of wide batches (score_i8.cuh), built on first use: base-256 digits of W -- digits 5..7 packed for shared memory
-    // (dWi8s), digits 1..4 for the TMEM loaders (dWi8t) --, per-row scales ([Np] slicing scale, [Np] 2 scale sf2, [Np] shift
-    // constant), alpha = W^T W Y and W^T W 1
-    double* dWi8s = nullptr; double* dWi8t = nullptr; double* dRowScale = nullptr; double* dAlphaY = nullptr; double* dAlpha1 = nullptr;
-    bool i8Valid = false; int i8Ntm = -1;
+    // INT8 path of wide batches (score_i8.cuh), built on first use: the seven base-256 digits of W packed for shared memory
+    // (dWi8s), per-row scales ([Np] slicing scale, [Np] 2 scale sf2, [Np] shift constant), alpha = W^T W Y and W^T W 1
+    double* dWi8s = nullptr; double* dRowScale = nullptr; double* dAlphaY = nullptr; double* dAlpha1 = nullptr;
+    bool i8Valid = false;
     cudaEvent_t evI8[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};   // K1 done [2], K2+K3 done [2], fork
     cudaEvent_t evCopy[5] = {nullptr, nullptr, nullptr, nullptr, nullptr}; // host candidates: chunk copy done [4], fork
     // guard pass of the INT8 path: per-candidate flags + block counts; index list, gathered candidates and their re-scored values

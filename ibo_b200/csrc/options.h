@@ -21,11 +21,8 @@ enum {
     OPT_I8_GUARD,        // 1 (default): candidates with sigma^2 < 2^-10 on the INT8 path are re-scored by the DMMA kernels
     OPT_I8_MIN_BATCH,    // batches of at least this many candidates (and at most narrow_max) also take the INT8 path (-1: measured break-even rule, 0: only wide batches)
     OPT_I8_RB_PER_CTA,   // row-blocks a CTA of the INT8 K2 sweeps (G = nb / this many CTAs share a candidate tile); 0: four groups whatever the size
-    OPT_I8_NTM,          // 0 (default): every operand of the INT8 K2 in shared memory; 1: W digits 1..4 reach the tensor core through TMEM
-                         // (measured 6-13 % slower under the power cap: profiles/r02_int8_k2.md)
     OPT_CHOL_PAIR,       // model build: block columns in pairs (256-deep trailing updates); -1 = from 48 block columns on, 0 / 1 forced
     OPT_TINY_SERVER,     // DIRECT on a one-row-block model: resident kernel fed through a mailbox in mapped host memory (1) or one launch per batch (0)
-    OPT_I8_DBG,          // timing experiments on the INT8 K2: honoured only by the debug build (EXTRA=-DIBO_I8_TRACE), ignored otherwise
     OPT_COUNT
 };
 long get_option(int id);

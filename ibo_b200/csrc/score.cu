@@ -885,9 +885,7 @@ constexpr int FLAG_I8_ANY_SIZE = 0x20000000;    // internal (sharded DIRECT): th
                                                 // arithmetic of a candidate is chosen from the size of the FULL batch on every rank
 
 static cudaError_t set_i8_attrs() {
-    cudaError_t e = cudaFuncSetAttribute(trigemm_i8_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, I8Cfg<4>::SMEM);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(trigemm_i8_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, I8Cfg<0>::SMEM);
-    return e;
+    return cudaFuncSetAttribute(trigemm_i8_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, I8_SMEM);
 }
 
 // Which arithmetic scores this batch.  Wide batches (more than `narrow_max` candidates) of a plain model go through the INT8
@@ -1328,14 +1326,6 @@ extern "C" int ibo_i8_peak(int device, double* tops) {
     if (!tops) { set_error("bad argument"); return IBO_E_BADARG; }
     return ibo_i8_peak2(device, 0.0, tops, nullptr);
 }
-
-#ifdef IBO_I8_TRACE
-extern "C" int ibo_debug_i8_trace(long long* out, int n) {
-    IBO_CUDA_TRY(cudaDeviceSynchronize());
-    IBO_CUDA_TRY(cudaMemcpyFromSymbol(out, ibo::g_i8_trace, sizeof(long long) * (n < 4096 ? n : 4096)));
-    return IBO_OK;
-}
-#endif
 
 // test hook: K1's exp_nonpos next to libdevice exp for n arguments <= 0 (host arrays)
 extern "C" int ibo_debug_exp(int device, const double* x, long n, double* out_fast, double* out_ref) {

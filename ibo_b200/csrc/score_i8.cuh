@@ -14,13 +14,12 @@
 // K-major operand, so A_t x [B_u0 .. B_u0+n-1] is ONE 128 x 64n x 32 instruction whose 64-column output blocks land on the
 // accumulators of groups t+u0 .. t+u0+n-1: 10 instructions per 32-deep k-step instead of 28.
 //
-// Operand feed.  With every operand in shared memory a k-step moves 138 KiB through the SM's 128 B/clk shared-memory pipe
-// (10 A reads of 4 KiB, 28 B reads of 2 KiB, 42 KiB of bulk-copy fill) against 896 clk of tensor work: the round-1 kernel
-// measured 0.75 of the INT8 peak with that pipe 92 % busy (profiles/r01_s5_summary.md).  Here the four most significant
-// W digits -- the operands of 7 of the 10 instructions -- never touch shared memory: four loader warps read them from
-// L2 straight into registers and write them with tcgen05.st into the 64 TMEM columns the accumulators leave free (two
-// buffers of 4 digits x 8 columns), and the MMAs take them as the TMEM A operand.  What is left on the shared-memory pipe is
-// 94 KiB per k-step (752 clk): the tensor pipe is the bound again.
+// Operand feed.  Every operand is in shared memory: per 32-deep k-step the producer issues two contiguous bulk copies into a
+// 4-stage ring, the seven W digits of the row-block (28 KiB) and the seven K* digits of the candidate tile (14 KiB), and the ten
+// MMAs read both through shared-memory descriptors.  A k-step moves 138 KiB through the SM's 128 B/clk shared-memory pipe (10 A
+// reads of 4 KiB, 28 B reads of 2 KiB, 42 KiB of bulk-copy fill) against 896 clk of tensor work, but under the 1 kW power cap
+// the lowered SM clock bounds the kernel (0.93 of the sustained INT8 peak).  A TMEM feed for W digits 1..4 was built, measured
+// 6-13 % slower under the power cap, and removed (profiles/r02_int8_k2.md).
 //
 // sigma^2 only needs sum_r V_r^2 per candidate; the posterior mean is k* . alpha (alpha = W^T W Y, plain FP64 dot products
 // inside K1, written to the partial-sum planes K2 would fill with V . beta), so K3 is the DMMA path's.
@@ -29,26 +28,18 @@
 namespace ibo {
 
 constexpr int I8_S = 7;                          // digits per operand
-// NTM: W digits 1..NTM go through TMEM, the rest through shared memory.  NTM = 4 is the design described above; NTM = 0 keeps every
-// operand in shared memory (option i8_ntm: the A/B switch between the two feeds).
 constexpr int I8_NT = 64;                        // candidates per tile
 constexpr int I8_A_SLICE = 128 * 32;             // bytes of one W digit of a k-step: 128 rows x 32 k
 constexpr int I8_B_SLICE = I8_NT * 32;           // bytes of one K* digit of a k-step: 64 candidates x 32 k
+constexpr int I8_A_STAGE = I8_S * I8_A_SLICE;                // 28672
 constexpr int I8_B_STAGE = I8_S * I8_B_SLICE;                // 14336
-template <int NTM> struct I8Cfg {
-    static constexpr int AS_STAGE = (I8_S - NTM) * I8_A_SLICE;   // shared-memory digits of W per k-step (12288 / 28672)
-    static constexpr int AT_STEP = NTM * I8_A_SLICE;             // TMEM digits of W per k-step (16384 / 0)
-    static constexpr int STAGES = NTM ? 6 : 4;                   // even: the loader sets step through the stages two at a time
-    static constexpr int SMEM = STAGES * (AS_STAGE + I8_B_STAGE) + 4 * 64 * 8 + 32 * 8;
-    static constexpr int FULL_ARRIVALS = NTM ? 5 : 1;            // producer (+ the four loader warps of the k-step)
-    static constexpr int THREADS = NTM ? 576 : 320;              // without a TMEM feed there are no loader warps: 10 warps, 31 K registers,
-                                                                 // which leaves room for two K1 CTAs of the next chunk beside a resident K2 CTA
-};
-constexpr int I8_ACC_COLS = 64 * I8_S;                       // 448 accumulator columns; the A buffers follow
+constexpr int I8_STAGES = 4;
+constexpr int I8_SMEM = I8_STAGES * (I8_A_STAGE + I8_B_STAGE) + 4 * 64 * 8 + 32 * 8;
+constexpr int I8_THREADS = 320;                  // 10 warps, 31 K registers: leaves room for two K1 CTAs of the next chunk beside a
+                                                 // resident K2 CTA
 // warp 0: bulk-copy producer, warp 1: TMEM owner + MMA issuer, warps 2-9: epilogue (warp w drains TMEM lanes 32 (w % 4) .. + 31
-// for candidates 32 ((w - 2) / 4) .. + 31 of the tile), warps 10-17: TMEM A loaders (two sets of four: set 0 feeds buffer 0 with
-// the even k-steps, set 1 buffer 1 with the odd ones)
-constexpr int I8_EPI_WARP0 = 2, I8_LOAD_WARP0 = 10;
+// for candidates 32 ((w - 2) / 4) .. + 31 of the tile)
+constexpr int I8_EPI_WARP0 = 2;
 // sigma^2 below this value is not taken from the integer path: the candidate is re-scored by the DMMA kernels in the same
 // call (score.cu: guard pass).  The scheme's absolute error on sum v^2 is ~1e-14 (1 + noise), so above the threshold its
 // relative effect on sigma^2 stays below 1e-11; a model with noise >= 2^-10 never gets there (sigma^2 >= noise).
@@ -71,11 +62,6 @@ __device__ __forceinline__ void umma_i8(uint32_t tmem_d, uint64_t da, uint64_t d
     asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\ttcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n\t}"
                  :: "r"(tmem_d), "l"(da), "l"(db), "r"(idesc), "r"(accumulate) : "memory");
 }
-// A operand in TMEM: lane = row, 8 columns = the row's 32 k bytes
-__device__ __forceinline__ void umma_i8_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t db, uint32_t idesc, uint32_t accumulate) {
-    asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\ttcgen05.mma.cta_group::1.kind::i8 [%0], [%1], %2, %3, p;\n\t}"
-                 :: "r"(tmem_d), "r"(tmem_a), "l"(db), "r"(idesc), "r"(accumulate) : "memory");
-}
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {               // arrives on `bar` once every MMA issued so far has completed
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" :: "r"(smem_u32(bar)) : "memory");
 }
@@ -90,11 +76,6 @@ __device__ __forceinline__ void tmem_ld4_nowait(uint32_t taddr, uint32_t* v) {
                  : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]) : "r"(taddr));
 }
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
-__device__ __forceinline__ void tmem_st8(uint32_t taddr, const uint4& a, const uint4& b) {
-    asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};"
-                 :: "r"(taddr), "r"(a.x), "r"(a.y), "r"(a.z), "r"(a.w), "r"(b.x), "r"(b.y), "r"(b.z), "r"(b.w) : "memory");
-}
-__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 // One lane of a converged warp (CUTLASS's elect_one_sync).  tcgen05.mma / tcgen05.commit / bulk copies run on the warp-uniform
 // datapath: under a plain `lane == 0` test the compiler cannot prove that a single thread is active and wraps EVERY such
 // instruction in an elect / vote loop (~150 issue slots per k-step: the MMA issuer, not the tensor pipe, was the bound of the
@@ -104,35 +85,6 @@ __device__ __forceinline__ bool elect_one() {
     asm volatile("{\n\t.reg .pred p;\n\telect.sync _|p, 0xffffffff;\n\tselp.u32 %0, 1, 0, p;\n\t}" : "=r"(pred));
     return pred != 0;
 }
-__device__ __forceinline__ uint4 ldg_nc16(const void* p) {
-    uint4 v;
-    asm volatile("ld.global.nc.L1::no_allocate.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p));
-    return v;
-}
-
-#ifdef IBO_I8_TRACE
-// debug build only (make EXTRA=-DIBO_I8_TRACE): clock64 stamps of one CTA, read back with ibo_debug_i8_trace
-__device__ long long g_i8_trace[4096];
-#define I8_STAMP(slot) do { if (traceCta && (slot) < 4096) g_i8_trace[slot] = clock64(); } while (0)
-#else
-#define I8_STAMP(slot) do { } while (0)
-#endif
-
-// The sequence of k-steps a CTA of row-block group g walks: row-blocks dealt to the G groups in snake order (work ~ i + 1),
-// largest first; every role of the K2 CTA iterates it in lock step.
-struct I8Seq {
-    int nb, G, g, rounds, r, i, j, nk;
-    bool valid;
-    __device__ void open_round() {
-        valid = false;
-        for (; r < rounds; r++) {
-            const int idx = r * G + ((r & 1) ? (G - 1 - g) : g);
-            if (idx < nb) { i = nb - 1 - idx; nk = (i + 1) * 4; j = 0; valid = true; return; }
-        }
-    }
-    __device__ I8Seq(int nb_, int G_, int g_) : nb(nb_), G(G_), g(g_), rounds((nb_ + G_ - 1) / G_), r(0), i(0), j(0), nk(0), valid(false) { open_round(); }
-    __device__ void next() { if (++j == nk) { r++; open_round(); } }
-};
 
 // ---------------------------------------------------------------------------------------------
 // model side: per-row power-of-two scale of W and its seven digits
@@ -159,11 +111,9 @@ __global__ void __launch_bounds__(256) i8_rowscale_kernel(const double* __restri
     }
 }
 
-// digits 1..NTM -> Wt: per k-step [digit][16-byte k chunk][row][16 B] (a loader warp's 16-byte loads are contiguous);
-// digits NTM+1..7 -> Ws: per k-step [digit][canonical 128 x 32 tile] (one contiguous bulk copy per stage)
-template <int NTM>
+// digits 1..7 -> Ws: per k-step [digit][canonical 128 x 32 tile] (one contiguous bulk copy per stage)
 __global__ void __launch_bounds__(256) i8_slice_w_kernel(const double* __restrict__ W, const double* __restrict__ rowScale, int Np,
-                                                         uint8_t* __restrict__ Ws, uint8_t* __restrict__ Wt) {
+                                                         uint8_t* __restrict__ Ws) {
     const int j = blockIdx.x, i = blockIdx.y;                 // k-step, row-block
     if (j >= (i + 1) * 4) return;
     const int r = threadIdx.x & 127, c16 = threadIdx.x >> 7;  // row of the block, 16-byte k chunk of the step
@@ -194,8 +144,7 @@ __global__ void __launch_bounds__(256) i8_slice_w_kernel(const double* __restric
             }
             w4[v] = word;
         }
-        uint8_t* dst = t <= NTM ? Wt + step * I8Cfg<NTM>::AT_STEP + ((size_t)(((t - 1) * 2 + c16) * 128 + r) << 4)
-                                : Ws + step * I8Cfg<NTM>::AS_STAGE + (size_t)(t - 1 - NTM) * I8_A_SLICE + i8_canon(r, c16 * 16);
+        uint8_t* dst = Ws + step * I8_A_STAGE + (size_t)(t - 1) * I8_A_SLICE + i8_canon(r, c16 * 16);
         *reinterpret_cast<uint4*>(dst) = make_uint4(w4[0], w4[1], w4[2], w4[3]);
     }
 }
@@ -296,25 +245,15 @@ __global__ void __launch_bounds__(256, (DMAX <= 8 ? 4 : (DMAX <= 16 ? 3 : 2))) k
 // into the seven group accumulators, then the epilogue warps assemble V in FP64 and reduce sum_r V_r^2 per candidate in a
 // fixed order.
 // ---------------------------------------------------------------------------------------------
-template <int NTM>
-__global__ void __launch_bounds__(I8Cfg<NTM>::THREADS, (NTM ? 1 : 2)) trigemm_i8_kernel(const uint8_t* __restrict__ Ws, const uint8_t* __restrict__ Wt,
-                                                                    const uint8_t* __restrict__ Ki8, const double* __restrict__ rowScaleSf,
-                                                                    double* __restrict__ part, int nb, long Mpad, int dbg_in) {
-    // dbg: timing experiments of the debug build only (make EXTRA=-DIBO_I8_TRACE; results are wrong when != 0): 1 loaders skip the
-    // L2 loads, 4 no MMAs from shared-memory A digits, 8 no MMAs from TMEM A digits, 16 no K* copy, 32 no W copy.  The shipped
-    // build compiles every switch out.
-#ifdef IBO_I8_TRACE
-    const int dbg = dbg_in;
-#else
-    constexpr int dbg = 0;
-    (void)dbg_in;
-#endif
+__global__ void __launch_bounds__(I8_THREADS, 2) trigemm_i8_kernel(const uint8_t* __restrict__ Ws, const uint8_t* __restrict__ Ki8,
+                                                                   const double* __restrict__ rowScaleSf, double* __restrict__ part,
+                                                                   int nb, long Mpad) {
     // rowScaleSf[row]: the factor that turns the assembled integer sum into v; rowScaleSf[Np + row]: the additive constant
-    constexpr int STAGES = I8Cfg<NTM>::STAGES, AS_STAGE = I8Cfg<NTM>::AS_STAGE, AT_STEP = I8Cfg<NTM>::AT_STEP;
+    constexpr int STAGES = I8_STAGES;
     extern __shared__ __align__(1024) uint8_t smem[];
-    uint8_t* sA = smem;                                          // [stage][3][128 x 32]   W digits 5..7
-    uint8_t* sB = smem + STAGES * AS_STAGE;                // [stage][7][64 x 32]    K* digits 1..7
-    double* red = reinterpret_cast<double*>(smem + STAGES * (AS_STAGE + I8_B_STAGE));     // [4][64]
+    uint8_t* sA = smem;                                          // [stage][7][128 x 32]   W digits 1..7
+    uint8_t* sB = smem + STAGES * I8_A_STAGE;                    // [stage][7][64 x 32]    K* digits 1..7
+    double* red = reinterpret_cast<double*>(smem + STAGES * (I8_A_STAGE + I8_B_STAGE));     // [4][64]
     uint64_t* full = reinterpret_cast<uint64_t*>(red + 4 * 64);
     uint64_t* empty = full + STAGES;
     uint64_t* tfull = empty + STAGES;
@@ -322,21 +261,17 @@ __global__ void __launch_bounds__(I8Cfg<NTM>::THREADS, (NTM ? 1 : 2)) trigemm_i8
     uint32_t* tbase = reinterpret_cast<uint32_t*>(tempty + 1);
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int g = blockIdx.x, G = gridDim.x, T = blockIdx.y;
-#ifdef IBO_I8_TRACE
-    const bool traceCta = blockIdx.x == 1 && blockIdx.y == 300;
-    if (tid == 0) I8_STAMP(0);
-#endif
     if (tid == 0) {
-        // full[s]: the producer's expect-tx arrival (+ the bytes of its two bulk copies) and the four loader warps that wrote this
-        // k-step's W digits 1..4 into TMEM; empty[s]: one tcgen05.commit -- the MMAs of the k-step have read the stage and the
-        // TMEM A buffer, which releases both the producer (stage s) and the loader set (buffer n & 1)
-        for (int s = 0; s < STAGES; s++) { mbar_init(&full[s], I8Cfg<NTM>::FULL_ARRIVALS); mbar_init(&empty[s], 1); }
+        // full[s]: the producer's expect-tx arrival (+ the bytes of its two bulk copies); empty[s]: one tcgen05.commit -- the MMAs
+        // of the k-step have read the stage
+        for (int s = 0; s < STAGES; s++) { mbar_init(&full[s], 1); mbar_init(&empty[s], 1); }
         mbar_init(tfull, 1);
         mbar_init(tempty, 8);
         fence_barrier_init();
         fence_proxy_async();
     }
     if (warp == 1) {
+        // 512 columns: the smallest allocation that holds the 448 accumulator columns
         asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" :: "r"(smem_u32(tbase)), "r"(512u) : "memory");
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
     }
@@ -355,42 +290,35 @@ __global__ void __launch_bounds__(I8Cfg<NTM>::THREADS, (NTM ? 1 : 2)) trigemm_i8
                 const int idx = r * G + ((r & 1) ? (G - 1 - g) : g);
                 if (idx >= nb) continue;
                 const int i = nb - 1 - idx, nk = (i + 1) * 4;
-                const uint8_t* Ab = Ws + i8_steps_before(i) * AS_STAGE;
+                const uint8_t* Ab = Ws + i8_steps_before(i) * I8_A_STAGE;
                 for (int j = 0; j < nk; j++) {
                     mbar_wait(&empty[s], ph ^ 1);
-                    mbar_arrive_expect_tx(&full[s], ((dbg & 32) ? 0 : AS_STAGE) + ((dbg & 16) ? 0 : I8_B_STAGE));
-                    if (!(dbg & 32)) bulk_g2s(sA + s * AS_STAGE, Ab + (size_t)j * AS_STAGE, AS_STAGE, &full[s]);
-                    if (!(dbg & 16)) bulk_g2s(sB + s * I8_B_STAGE, Bb + (size_t)j * I8_B_STAGE, I8_B_STAGE, &full[s]);
+                    mbar_arrive_expect_tx(&full[s], I8_A_STAGE + I8_B_STAGE);
+                    bulk_g2s(sA + s * I8_A_STAGE, Ab + (size_t)j * I8_A_STAGE, I8_A_STAGE, &full[s]);
+                    bulk_g2s(sB + s * I8_B_STAGE, Bb + (size_t)j * I8_B_STAGE, I8_B_STAGE, &full[s]);
                     if (++s == STAGES) { s = 0; ph ^= 1; }
                 }
             }
         }
     } else if (warp == 1) {
-        // ---------------- MMA issuer (one elected lane): the loop is its whole critical path -- one barrier test per operand
-        // source, ten MMAs, two commits per k-step and nothing else ----------------
+        // ---------------- MMA issuer (one elected lane): the loop is its whole critical path -- one barrier wait, ten MMAs and
+        // one commit per k-step and nothing else ----------------
         if (elect_one()) {
-            int s = 0; uint32_t ph = 0, n = 0; int rb = 0;
+            int s = 0; uint32_t ph = 0; int rb = 0;
             for (int r = 0; r < rounds; r++) {
                 const int idx = r * G + ((r & 1) ? (G - 1 - g) : g);
                 if (idx >= nb) continue;
                 const int nk = (nb - idx) * 4;
                 mbar_wait(tempty, (uint32_t)(rb & 1) ^ 1);          // the epilogue has drained the previous row-block's accumulators
-                for (int j = 0; j < nk; j++, n++) {
-                    const uint32_t ab = n & 1;
-                    I8_STAMP(16 + 4 * n);
+                for (int j = 0; j < nk; j++) {
                     mbar_wait(&full[s], ph);
                     tc_fence_after();
-                    I8_STAMP(16 + 4 * n + 1);
-                    const uint32_t at = tb + I8_ACC_COLS + 32u * ab;
-                    const uint64_t da = umma_smem_desc(smem_u32(sA + s * AS_STAGE)), db = umma_smem_desc(smem_u32(sB + s * I8_B_STAGE));
+                    const uint64_t da = umma_smem_desc(smem_u32(sA + s * I8_A_STAGE)), db = umma_smem_desc(smem_u32(sB + s * I8_B_STAGE));
                     const uint32_t first = j == 0 ? 0u : 1u;
                     // digit t of W against K* digits u0 .. u0+n-1: accumulator columns 64 (t + u0 - 2), N = 64 n
                     // (descriptor + (bytes >> 4): the start-address field counts 16-byte units and cannot carry here)
-#define I8_MMA_T(t, u0, n, acc) umma_i8_ts(tb + 64u * ((t) + (u0) - 2), at + 8u * ((t) - 1), \
-                                           db + (uint64_t)((((u0) - 1) * I8_B_SLICE) >> 4), umma_idesc_i8(128, 64 * (n)), acc)
-#define I8_MMA_S(t, u0, n, acc) umma_i8(tb + 64u * ((t) + (u0) - 2), da + (uint64_t)((((t) - 1 - NTM) * I8_A_SLICE) >> 4), \
-                                        db + (uint64_t)((((u0) - 1) * I8_B_SLICE) >> 4), umma_idesc_i8(128, 64 * (n)), acc)
-#define I8_MMA(t, u0, n, acc) do { if ((t) <= NTM) I8_MMA_T(t, u0, n, acc); else I8_MMA_S(t, u0, n, acc); } while (0)
+#define I8_MMA(t, u0, n, acc) umma_i8(tb + 64u * ((t) + (u0) - 2), da + (uint64_t)((((t) - 1) * I8_A_SLICE) >> 4), \
+                                      db + (uint64_t)((((u0) - 1) * I8_B_SLICE) >> 4), umma_idesc_i8(128, 64 * (n)), acc)
                     I8_MMA(1, 1, 4, first); I8_MMA(1, 5, 3, first);          // the two t = 1 instructions touch groups 2..8 first
                     I8_MMA(2, 1, 4, 1u);    I8_MMA(2, 5, 2, 1u);
                     I8_MMA(3, 1, 4, 1u);    I8_MMA(3, 5, 1, 1u);
@@ -399,66 +327,12 @@ __global__ void __launch_bounds__(I8Cfg<NTM>::THREADS, (NTM ? 1 : 2)) trigemm_i8
                     I8_MMA(6, 1, 2, 1u);
                     I8_MMA(7, 1, 1, 1u);
 #undef I8_MMA
-#undef I8_MMA_T
-#undef I8_MMA_S
-                    I8_STAMP(16 + 4 * n + 2);
-                    umma_commit(&empty[s]);                          // the stage and the A buffer are free once these MMAs have read them
-                    I8_STAMP(16 + 4 * n + 3);
+                    umma_commit(&empty[s]);                          // the stage is free once these MMAs have read it
                     if (++s == STAGES) { s = 0; ph ^= 1; }
                 }
                 umma_commit(tfull);                                  // accumulators of this row-block complete
                 rb++;
             }
-        }
-    } else if (warp >= I8_LOAD_WARP0) {
-        if constexpr (NTM > 0) {
-        // ---------------- TMEM A loaders: warp w owns TMEM lanes 32 (w % 4) .. + 31 = rows of the block ----------------
-        // Set `ab` = (w - 6) / 4 handles the k-steps n = ab (mod 2) and TMEM buffer ab.  Each thread keeps two k-steps of its set in
-        // flight in registers, so the L2 loads of k-step n are issued while the MMAs of k-step n - 4 run (the L2 round trip under
-        // this kernel's load is longer than one k-step of tensor work).
-        const uint32_t ab = (uint32_t)(warp - I8_LOAD_WARP0) >> 2;
-        const int row = (warp & 3) * 32 + lane;
-        const uint32_t tl = tb + ((uint32_t)((warp & 3) * 32) << 16) + I8_ACC_COLS + 32u * ab;
-        I8Seq pre(nb, G, g);
-        if (ab && pre.valid) pre.next();
-        uint4 b0[2 * NTM], b1[2 * NTM];
-        auto fetch = [&](uint4* buf) {
-            const uint8_t* src = Wt + (i8_steps_before(pre.i) + pre.j) * AT_STEP + ((size_t)row << 4);
-#pragma unroll
-            for (int x = 0; x < 2 * NTM; x++) buf[x] = (dbg & 1) ? make_uint4(x, x, x, x) : ldg_nc16(src + x * 2048);
-            pre.next();
-            if (pre.valid) pre.next();
-        };
-        // k-step n = 2 use + ab: its TMEM buffer was last read by the MMAs of k-step n - 2, whose commit completes phase
-        // (n - 2) / STAGES of empty[(n - 2) % STAGES]; the k-step itself is announced on full[n % STAGES]
-        uint32_t sPrev = (uint32_t)((ab + STAGES - 2) % STAGES), phPrev = 1;    // n - 2 < 0: passes at once on a fresh barrier
-        uint32_t sCur = ab;
-        uint32_t use = 0;
-        auto put = [&](const uint4* buf) {
-            if (warp == I8_LOAD_WARP0 && lane == 0) I8_STAMP(1024 + 4 * use);
-            mbar_wait_warp(&empty[sPrev], phPrev);
-            tc_fence_after();
-            if (warp == I8_LOAD_WARP0 && lane == 0) I8_STAMP(1024 + 4 * use + 1);
-#pragma unroll
-            for (int t = 0; t < NTM; t++) tmem_st8(tl + 8u * t, buf[2 * t], buf[2 * t + 1]);
-            tmem_st_wait();
-            tc_fence_before();
-            __syncwarp();
-            if (warp == I8_LOAD_WARP0 && lane == 0) I8_STAMP(1024 + 4 * use + 2);
-            if (lane == 0) mbar_arrive(&full[sCur]);
-            use++;
-            sPrev += 2; if (sPrev >= STAGES) { sPrev -= STAGES; phPrev ^= 1; }
-            sCur += 2; if (sCur >= STAGES) sCur -= STAGES;
-        };
-        bool v0 = pre.valid; if (v0) fetch(b0);
-        bool v1 = pre.valid; if (v1) fetch(b1);
-        while (v0) {
-            put(b0);
-            v0 = pre.valid; if (v0) fetch(b0);
-            if (!v1) break;
-            put(b1);
-            v1 = pre.valid; if (v1) fetch(b1);
-        }
         }
     } else {
         // ---------------- epilogue: warp w drains TMEM lanes 32 (w % 4) .. + 31 (rows) x candidates 32 h .. + 31, h = (w - 2) / 4 ----------------
@@ -473,7 +347,6 @@ __global__ void __launch_bounds__(I8Cfg<NTM>::THREADS, (NTM ? 1 : 2)) trigemm_i8
             const double rc = rowScaleSf[(size_t)nb * 128 + i * 128 + qd * 32 + lane];
             mbar_wait_warp(tfull, (uint32_t)(rb & 1));
             tc_fence_after();
-            if (et == 0) I8_STAMP(2 + 2 * rb);
 #pragma unroll 1
             for (int c16 = 0; c16 < 2; c16++) {
                 double sq[16];
@@ -514,7 +387,6 @@ __global__ void __launch_bounds__(I8Cfg<NTM>::THREADS, (NTM ? 1 : 2)) trigemm_i8
                 if (!(lane & 1)) red[qd * 64 + hf * 32 + c16 * 16 + (lane >> 1)] = sq[0];
             }
             tc_fence_before();
-            if (et == 0) I8_STAMP(3 + 2 * rb);
             __syncwarp();
             if (lane == 0) mbar_arrive(tempty);                      // 8 arrivals: the accumulators may be overwritten
             named_bar_sync(1, 256);
@@ -528,7 +400,6 @@ __global__ void __launch_bounds__(I8Cfg<NTM>::THREADS, (NTM ? 1 : 2)) trigemm_i8
     }
     tc_fence_before();
     __syncthreads();
-    if (tid == 0) I8_STAMP(1);
     if (warp == 1) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(tb), "r"(512u) : "memory");
 }
 
@@ -536,26 +407,20 @@ __global__ void __launch_bounds__(I8Cfg<NTM>::THREADS, (NTM ? 1 : 2)) trigemm_i8
 // host side
 // ---------------------------------------------------------------------------------------------
 // builds (once per model state) the packed digits of W, the row scales / constants and alpha
-static int i8_ntm() { return get_option(OPT_I8_NTM) != 0 ? 4 : 0; }
-
 static int ensure_i8(ibo_model* m) {
+    if (m->i8Valid) return IBO_OK;
     const int Np = m->Np, nb = m->nb;
     cudaStream_t st = m->stream;
-    const int ntm = i8_ntm();
-    if (m->i8Valid && m->i8Ntm == ntm) return IBO_OK;
-    m->i8Ntm = ntm;
-    for (double** p : {&m->dAlphaY, &m->dAlpha1, &m->dWi8s, &m->dWi8t, &m->dRowScale}) if (*p) { pool_free(*p); *p = nullptr; }
+    for (double** p : {&m->dAlphaY, &m->dAlpha1, &m->dWi8s, &m->dRowScale}) if (*p) { pool_free(*p); *p = nullptr; }
     IBO_CUDA_TRY(pool_malloc((void**)&m->dAlphaY, sizeof(double) * Np));
     IBO_CUDA_TRY(pool_malloc((void**)&m->dAlpha1, sizeof(double) * Np));
     launch_tri_matvec_t(m->dW, m->dBetaY, m->dAlphaY, Np, Np, st);       // alpha = W^T (W Y)
     launch_tri_matvec_t(m->dW, m->dBeta1, m->dAlpha1, Np, Np, st);
     for (auto& e : m->evI8) if (!e) IBO_CUDA_TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    IBO_CUDA_TRY(pool_malloc((void**)&m->dWi8s, i8_steps_before(nb) * (size_t)(I8_S - ntm) * I8_A_SLICE));
-    IBO_CUDA_TRY(pool_malloc((void**)&m->dWi8t, i8_steps_before(nb) * (size_t)std::max(ntm, 1) * I8_A_SLICE));
+    IBO_CUDA_TRY(pool_malloc((void**)&m->dWi8s, i8_steps_before(nb) * (size_t)I8_A_STAGE));
     IBO_CUDA_TRY(pool_malloc((void**)&m->dRowScale, sizeof(double) * 3 * Np));
     i8_rowscale_kernel<<<(Np + 7) / 8, 256, 0, st>>>(m->dW, Np, m->N, m->sf2, m->dRowScale);
-    if (ntm) i8_slice_w_kernel<4><<<dim3(nb * 4, nb), 256, 0, st>>>(m->dW, m->dRowScale, Np, reinterpret_cast<uint8_t*>(m->dWi8s), reinterpret_cast<uint8_t*>(m->dWi8t));
-    else i8_slice_w_kernel<0><<<dim3(nb * 4, nb), 256, 0, st>>>(m->dW, m->dRowScale, Np, reinterpret_cast<uint8_t*>(m->dWi8s), reinterpret_cast<uint8_t*>(m->dWi8t));
+    i8_slice_w_kernel<<<dim3(nb * 4, nb), 256, 0, st>>>(m->dW, m->dRowScale, Np, reinterpret_cast<uint8_t*>(m->dWi8s));
     g_launches += 4;
     IBO_CUDA_TRY(cudaGetLastError());
     m->i8Valid = true;
@@ -600,10 +465,7 @@ static void launch_trigemm_i8(ibo_model* m, long tiles, long Mpad, const uint8_t
     int G = per > 0 ? (int)std::max<long>(1, m->nb / per) : std::min(m->nb, 4);
     if (tiles * 2 * G < sms) G = (int)std::min<long>(m->nb, (sms + tiles * 2 - 1) / (tiles * 2));
     const dim3 grid(G, (unsigned)(tiles * 2));
-    if (m->i8Ntm) trigemm_i8_kernel<4><<<grid, I8Cfg<4>::THREADS, I8Cfg<4>::SMEM, st>>>(reinterpret_cast<const uint8_t*>(m->dWi8s), reinterpret_cast<const uint8_t*>(m->dWi8t),
-                                                         Ki8, m->dRowScale + m->Np, part, m->nb, Mpad, (int)get_option(OPT_I8_DBG));
-    else trigemm_i8_kernel<0><<<grid, I8Cfg<0>::THREADS, I8Cfg<0>::SMEM, st>>>(reinterpret_cast<const uint8_t*>(m->dWi8s), reinterpret_cast<const uint8_t*>(m->dWi8t),
-                                                         Ki8, m->dRowScale + m->Np, part, m->nb, Mpad, (int)get_option(OPT_I8_DBG));
+    trigemm_i8_kernel<<<grid, I8_THREADS, I8_SMEM, st>>>(reinterpret_cast<const uint8_t*>(m->dWi8s), Ki8, m->dRowScale + m->Np, part, m->nb, Mpad);
 }
 
 // ---- live INT8 tensor peak (bench.py): back-to-back 128 x 256 x 32 MMAs from resident operands, one CTA per SM -------------

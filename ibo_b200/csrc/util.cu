@@ -45,7 +45,7 @@ cudaError_t ensure_attrs(int device, int family, cudaError_t (*setter)()) {
 struct OptDef { const char* name; long def; };
 static const OptDef g_optdef[OPT_COUNT] = {
     {"int8", 1}, {"i8_pipe", 1}, {"chunk_tiles", 0}, {"narrow_max", 2048}, {"narrow_mt", 0}, {"k2_deep", -1}, {"pdl", 1},
-    {"kstar_direct", 0}, {"debug_plan", 0}, {"tiny", -1}, {"direct_timing", 0}, {"shard_min", 0}, {"i8_guard", 1}, {"i8_min_batch", -1}, {"i8_rb_per_cta", 0}, {"i8_ntm", 0}, {"chol_pair", -1}, {"tiny_server", 1}, {"i8_dbg", 0}};
+    {"kstar_direct", 0}, {"debug_plan", 0}, {"tiny", -1}, {"direct_timing", 0}, {"shard_min", 0}, {"i8_guard", 1}, {"i8_min_batch", -1}, {"i8_rb_per_cta", 0}, {"chol_pair", -1}, {"tiny_server", 1}};
 static long g_opt[OPT_COUNT];
 static std::once_flag g_opt_once;
 static void init_options() {

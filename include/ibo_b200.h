@@ -217,8 +217,7 @@ int ibo_debug_exp(int device, const double* x, long n, double* out_fast, double*
  *                     4096 / 8192), 0: wide batches only
  *   i8_guard (1)      INT8 path: re-score candidates with sigma^2 < 2^-10 on the DMMA path
  *   i8_pipe (1)       INT8 path: cross-covariance of chunk c+1 on a low-priority stream under the GEMM of chunk c
- *   i8_rb_per_cta (0), i8_ntm (0)   INT8 GEMM: row-blocks per CTA (0: four row-block groups whatever the size), W digits fed through
- *                     TMEM (0: all operands from shared memory -- faster under the power cap)
+ *   i8_rb_per_cta (0) INT8 GEMM: row-blocks per CTA (0: four row-block groups whatever the size)
  *   chunk_tiles (0)   128-candidate tiles per chunk (0: 2 x number of SMs)
  *   narrow_max (2048) batches up to this size use the latency shapes of the FP64 GEMM
  *   narrow_mt (0), k2_deep (-1), pdl (1), kstar_direct (0), tiny (-1)   shape / launch switches of the small-batch path

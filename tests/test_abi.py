@@ -70,13 +70,16 @@ def documented_options():
     return {n: int(v) for n, v in re.findall(r"\b([a-z][a-z0-9_]+) \((-?\d+)\)", sec)}
 
 
-def test_options_are_what_the_header_says():
-    """every option the header documents exists with the documented default (read in a fresh process: other tests change options),
-    unknown names are rejected, values round-trip, and IBO_<NAME> presets an option when the library is loaded"""
+def test_options_are_exactly_what_the_header_says():
+    """the header documents exactly the library's options, each exists with the documented default (read in a fresh process: other
+    tests change options), unknown and removed names are rejected, values round-trip, and IBO_<NAME> presets an option when the
+    library is loaded"""
     import subprocess
     import sys
     opts = documented_options()
-    assert len(opts) >= 18 and opts["int8"] == 1 and opts["i8_min_batch"] == -1 and opts["tiny_server"] == 1
+    assert set(opts) == {"int8", "i8_min_batch", "i8_guard", "i8_pipe", "i8_rb_per_cta", "chunk_tiles", "narrow_max", "narrow_mt",
+                         "k2_deep", "pdl", "kstar_direct", "tiny", "debug_plan", "direct_timing", "shard_min", "tiny_server", "chol_pair"}
+    assert opts["int8"] == 1 and opts["i8_min_batch"] == -1 and opts["tiny_server"] == 1
     code = ("import sys; sys.path.insert(0, %r)\nfrom ibo_b200 import _lib\n"
             "print(' '.join('%%s=%%d' %% (n, _lib.get_option(n)) for n in %r))" % (ROOT, sorted(opts)))
     env = {k: v for k, v in os.environ.items() if not k.startswith("IBO_")}
@@ -88,7 +91,8 @@ def test_options_are_what_the_header_says():
     assert got["int8"] == 0 and got["chol_pair"] == 1 and got["i8_guard"] == 1
     L = _lib.lib()
     v = ctypes.c_long(0)
-    assert L.ibo_set_option(b"no_such_option", 1) == _lib.E_BADARG and L.ibo_get_option(b"no_such_option", ctypes.byref(v)) == _lib.E_BADARG
+    for name in (b"no_such_option", b"i8_ntm", b"i8_dbg"):
+        assert L.ibo_set_option(name, 1) == _lib.E_BADARG and L.ibo_get_option(name, ctypes.byref(v)) == _lib.E_BADARG
     old = _lib.get_option("narrow_mt")
     try:
         _lib.set_option("narrow_mt", 4)

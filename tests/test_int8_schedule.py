@@ -1,8 +1,8 @@
 """CPU check of the MMA schedule of trigemm_i8_kernel (ibo_b200/csrc/score_i8.cuh), parsed from the source: every k-step issues
-A_t x [B_u0 .. B_u0+n-1] instructions whose 64-column output blocks land on TMEM columns 64 (t + u - 2) (the macro takes W digit t from the TMEM
-A buffers when t <= NTM, from shared memory otherwise).  Emulated on an accumulator array pre-filled with
-garbage, the schedule must leave exactly D_g = sum_k sum_{t+u=g} A_t B_u^T in every group -- in particular the first k-step must
-overwrite every group exactly once before anything accumulates into it -- and must stay clear of the TMEM A buffers."""
+A_t x [B_u0 .. B_u0+n-1] instructions whose 64-column output blocks land on TMEM columns 64 (t + u - 2).  Emulated on an accumulator
+array pre-filled with garbage, the schedule must leave exactly D_g = sum_k sum_{t+u=g} A_t B_u^T in every group -- in particular the
+first k-step must overwrite every group exactly once before anything accumulates into it -- and must stay within the 448 accumulator
+columns."""
 import os
 import re
 
@@ -33,7 +33,7 @@ def test_mma_schedule_builds_the_group_sums():
             assert 1 <= t <= S and u0 >= 1 and u0 + n - 1 <= S and t + u0 + n - 1 <= gmax
             assert n * 64 in (64, 128, 192, 256)                                   # legal UMMA N for M = 128
             col = (t + u0 - 2) * NC
-            assert col + n * NC <= 7 * NC                                          # 448 accumulator columns; 448..511 hold the A buffers
+            assert col + n * NC <= 7 * NC                                          # 448 accumulator columns
             prod = np.concatenate([A[j, t - 1] @ B[j, u - 1].T for u in range(u0, u0 + n)], axis=1)
             if first and j == 0:
                 tmem[:, col:col + n * NC] = prod

@@ -49,10 +49,3 @@ print("K2 int8: %.2f TOP/s; burst peak %.2f (frac %.3f), sustained peak with ran
 a, b = res["fp64"][0], res["int8"][0]
 print("max |dEI| / max(|EI|, 1e-5) = %.3g   same argmax %s   speed-up %.2fx"
       % (np.max(np.abs(a - b) / np.maximum(np.abs(a), 1e-5)), res["fp64"][1][1] == res["int8"][1][1], res["fp64"][2] / res["int8"][2]))
-for ntm in (0, 1):
-    _lib.set_option("i8_ntm", ntm)
-    c.score(_lib.ACQ_EI, ymax, 0.01, _lib.FLAG_MODE_CPP)
-    ts = [c.score(_lib.ACQ_EI, ymax, 0.01, _lib.FLAG_MODE_CPP)[2] for _ in range(4)]
-    c.score(_lib.ACQ_EI, ymax, 0.01, _lib.FLAG_MODE_CPP | _lib.FLAG_PROFILE)
-    p = m.profile()
-    print("i8_ntm=%d: step %.3f ms (median of 4: %.3f)  K1 %.2f K2 %.2f ms" % (ntm, min(ts), float(np.median(ts)), p["k1_ms"], p["k2_ms"]))
