@@ -19,7 +19,7 @@ EXPORTED = [
     "ibo_model_create", "ibo_model_create_pref", "ibo_model_create_laplace", "ibo_model_create_from_inverse", "ibo_model_append", "ibo_model_destroy", "ibo_model_n", "ibo_model_dim",
     "ibo_model_get_matrix", "ibo_model_set_variance_model", "ibo_pref_fit",
     "ibo_nlml", "ibo_kernel_matrix",
-    "ibo_posterior_batch", "ibo_score_batch",
+    "ibo_posterior_batch", "ibo_score_batch", "ibo_posterior_cov", "ibo_posterior_sample",
     "ibo_cands_create", "ibo_cands_destroy", "ibo_score_resident", "ibo_get_profile", "ibo_launch_count",
     "ibo_fp64_peak", "ibo_i8_peak", "ibo_i8_peak2", "ibo_host_register", "ibo_host_unregister", "ibo_stream_mark", "ibo_stream_elapsed_ms",
     "ibo_device_synchronize", "ibo_debug_exp",
@@ -100,6 +100,8 @@ def lib():
     L.ibo_kernel_matrix.argtypes = [c_int, c_int, pd, c_int, pd, c_int, c_int, c_int, c_int, pd]
     L.ibo_posterior_batch.argtypes = [c_void_p, pd, c_long, c_int, pd, pd]
     L.ibo_score_batch.argtypes = [c_void_p, pd, c_long, c_int, c_double, c_double, c_int, pd, pd, pd, pd, pl]
+    L.ibo_posterior_cov.argtypes = [c_void_p, pd, c_long, pd, pd]
+    L.ibo_posterior_sample.argtypes = [c_void_p, pd, c_long, pd, c_int, c_double, pd, pl, pi]
     L.ibo_cands_create.argtypes = [c_void_p, pd, c_long, POINTER(c_void_p)]
     L.ibo_cands_destroy.argtypes = [c_void_p]
     L.ibo_score_resident.argtypes = [c_void_p, c_void_p, c_int, c_double, c_double, c_int, pd, pd, pl, POINTER(c_float)]
@@ -291,6 +293,36 @@ class Model(object):
         mu, s2 = np.empty(M), np.empty(M)
         check(lib().ibo_posterior_batch(self._h, dptr(Xs), M, flags, dptr(mu), dptr(s2)))
         return mu, s2
+
+    def _candidates(self, Xs):
+        Xs = as_f64(Xs, 2)
+        if Xs.shape[1] != self.d:
+            raise ValueError("candidates have %d columns, the model %d" % (Xs.shape[1], self.d))
+        return Xs
+
+    def posterior_cov(self, Xs):
+        """joint posterior over the candidates (ibo_posterior_cov) -> (mu[M], cov[M, M]); diag(cov) is the unclipped sigma^2"""
+        Xs = self._candidates(Xs)
+        M = Xs.shape[0]
+        mu, cov = np.empty(M), np.empty((M, M))
+        check(lib().ibo_posterior_cov(self._h, dptr(Xs), M, dptr(mu), dptr(cov)))
+        return mu, cov
+
+    def posterior_sample(self, Xs, Z, jitter=0.0, want_F=True):
+        """joint posterior samples F = mu + chol(cov + jitter I) Z for standard normals Z[M, S] (ibo_posterior_sample)
+        -> (F[M, S] or None, argmax[S]); raises NotPositiveDefinite (pivot = 1-based candidate) when cov + jitter I is not SPD"""
+        Xs = self._candidates(Xs)
+        Z = as_f64(Z, 2)
+        M, S = Xs.shape[0], Z.shape[1]
+        if Z.shape[0] != M:
+            raise ValueError("Z has %d rows for %d candidates" % (Z.shape[0], M))
+        F = np.empty((M, S)) if want_F else None
+        am = np.empty(S, dtype=np.int64)
+        info = c_int(0)
+        rc = lib().ibo_posterior_sample(self._h, dptr(Xs), M, dptr(Z), S, float(jitter), dptr(F) if want_F else None,
+                                        am.ctypes.data_as(POINTER(c_long)), ctypes.byref(info))
+        check(rc, info.value)
+        return F, am
 
     def score(self, Xs, acq, ymax, parm, flags=FLAG_MODE_PY, want_scores=True, want_posterior=False, out=None):
         """`out` (optional, float64[M]) receives the scores in place (lets callers reuse a pinned buffer)."""

@@ -128,6 +128,24 @@ def cdirectGP(model, bounds, maxiter, maxtime, maxsample, acqfunc=None, xi=-1, b
     return opt, optx
 
 
+def thompsonBatch(GP, bounds, q, samples=2048, candidates=None, seed=None, jitter=0.0):
+    """Thompson sampling of a batch of q points to evaluate in parallel: q joint posterior draws over a candidate set, each
+    draw's maximiser is one point of the batch.
+
+    Candidates are `samples` Latin-hypercube points within `bounds` (lhcSample with `seed`) unless given as an array.  The
+    draws are mu + chol(cov + jitter I) Z with Z = numpy.random.default_rng(seed).standard_normal((M, q)); only the q
+    argmax indices leave the device.  Two draws can pick the same candidate, so a point may appear more than once in the
+    batch.  Returns (points[q, d], indices[q])."""
+    if len(GP.X) == 0:
+        raise ValueError("Thompson sampling over a GP without data")
+    if candidates is None:
+        candidates = lhcSample(bounds, samples, seed=seed)
+    C = np.array(candidates, dtype=float, ndmin=2)
+    Z = np.random.default_rng(seed).standard_normal((C.shape[0], q))
+    _, idx = GP.model.posterior_sample(C, Z, jitter, want_F=False)
+    return C[idx], idx
+
+
 def _python_direct(obj, bounds, **kw):
     """useCDIRECT=False route: the same DIRECT driver over the Python-path objective (batched)."""
     opt, optx = direct(obj.negf, bounds, batch_objective=lambda P: -obj.f_batch(P), pure=True, **kw)

@@ -49,8 +49,8 @@ extern long g_launches;   // kernels launched by this library (bench.py's gpu_la
 // per-device state and tuning options (util.cu)
 // ---------------------------------------------------------------------------------------------
 // cudaFuncSetAttribute is per device: every kernel family records, per device ordinal, that its attributes are set.
-enum { ATTR_MODEL = 0, ATTR_SCORE, ATTR_TINY, ATTR_I8, ATTR_GRAM, ATTR_COUNT };
-struct DevInfo { int sms = 148; bool known = false; bool attrs[ATTR_COUNT] = {false, false, false, false, false}; };
+enum { ATTR_MODEL = 0, ATTR_SCORE, ATTR_TINY, ATTR_I8, ATTR_GRAM, ATTR_JOINT, ATTR_COUNT };
+struct DevInfo { int sms = 148; bool known = false; bool attrs[ATTR_COUNT] = {false, false, false, false, false, false}; };
 DevInfo& dev_info(int device);            // SM count filled on first use
 // Runs `setter` once per (device, family) with `device` current; returns the CUDA error of the first failing call.
 cudaError_t ensure_attrs(int device, int family, cudaError_t (*setter)());

@@ -242,7 +242,7 @@ extern "C" int ibo_pref_fit(ibo_model* m, int P, const int* v, const int* u, con
         if ((rc = launch_syrk_identity(B->dA, G, Np, K, st))) return rc;
         neg_sum_kernel<<<gn, 256, 0, st>>>(ltg, a, B->dY, N, Np);
         g_launches++;
-        if ((rc = launch_factorize(B, false, false))) return rc;       // B->dW = inv(chol(B)), B->dBetaY = dW * rhs
+        if ((rc = launch_factorize(B, false, false, true))) return rc;       // B->dW = inv(chol(B)), B->dBetaY = dW * rhs
         TRYS(cudaMemsetAsync(da, 0, sizeof(double) * Np, st));
         launch_tri_matvec_t(B->dW, B->dBetaY, da, Np, Np, st);         // da = dW^T dW rhs
         // backtracking on S (convex: the full step is accepted except far from the optimum)

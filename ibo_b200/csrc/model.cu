@@ -762,7 +762,7 @@ static int set_kernel_attrs() {
 
 // Factorise m->dA in place, produce dW, dD, dWpack, dBetaY, dBeta1.
 // from_inverse_reversed: dA holds J invR J; W' = reverse-transpose of its Cholesky factor.
-int launch_factorize(ibo_model* m, bool from_inverse_reversed, bool pack) {
+int launch_factorize(ibo_model* m, bool from_inverse_reversed, bool pack, bool invert) {
     int rc = set_kernel_attrs();
     if (rc) return rc;
     cudaStream_t st = m->stream;
@@ -784,7 +784,7 @@ int launch_factorize(ibo_model* m, bool from_inverse_reversed, bool pack) {
     // near stream, all later rows on the far stream (after evScale; near(k) waits for far(k-w) through evFar).
     cudaStream_t s2 = from_inverse_reversed ? st : m->stream2;
     cudaStream_t s4 = m->stream4;
-    const bool trtri = !from_inverse_reversed;
+    const bool trtri = invert && !from_inverse_reversed;
     if (trtri) {
         IBO_CUDA_TRY(cudaEventRecord(m->evStep, st));            // orders s2 / s4 after whatever produced dA / dD users
         IBO_CUDA_TRY(cudaStreamWaitEvent(s2, m->evStep, 0));
@@ -896,6 +896,10 @@ int launch_factorize(ibo_model* m, bool from_inverse_reversed, bool pack) {
 #endif
     IBO_CUDA_TRY(cudaEventRecord(m->evRest, sb));
     IBO_CUDA_TRY(cudaStreamWaitEvent(st, m->evRest, 0));
+    if (!invert) {
+        IBO_CUDA_TRY(cudaGetLastError());
+        return IBO_OK;
+    }
     if (from_inverse_reversed) {
         reverse_transpose_kernel<<<g2, 256, 0, st>>>(m->dW, m->dA, m->N, Np);
         g_launches++;
@@ -968,6 +972,7 @@ static void free_model(ibo_model* m) {
     if (m->stream3) cudaStreamSynchronize(m->stream3);
     if (m->stream4) cudaStreamSynchronize(m->stream4);
     if (m->stream) cudaStreamSynchronize(m->stream);   // blocks go back to the pool: nothing may still be using them
+    free_joint(m);
     double** ptrs[] = {&m->dXt, &m->dInvTheta, &m->dCenter, &m->dA, &m->dAorig, &m->dW, &m->dD, &m->dWpack, &m->dBetaY, &m->dBeta1, &m->dY,
                        &m->dPmeans, &m->dPbeta, &m->dPlb, &m->dPwidth, &m->dCand, &m->dSlab, &m->dPart, &m->dOut, &m->dBlkBest, &m->dBest, &m->dAppend,
                        &m->dWi8s, &m->dRowScale, &m->dAlphaY, &m->dAlpha1, &m->dGuard, &m->dGuardList, &m->dCinv};
@@ -1125,7 +1130,7 @@ static int create_common(int device, int kind, const double* hyper, int nhyper, 
                 pref_build_C_kernel<<<(Np + 127) / 128, 128, 0, st>>>(m->dA, N, Np, pref->P, dPairs, dPairs + pref->P, dWts, pref->cdiag);
             }
             g_launches++;
-            rc = launch_factorize(m, false, false);
+            rc = launch_factorize(m, false, false, true);
             int cinfo = 0;
             if (!rc) {
                 TRYM(cudaMemcpyAsync(&cinfo, m->dInfo, sizeof(int), cudaMemcpyDeviceToHost, st));
@@ -1152,7 +1157,7 @@ static int create_common(int device, int kind, const double* hyper, int nhyper, 
         TRYM(pool_malloc((void**)&m->dAorig, sizeof(double) * (size_t)Np * Np));
         TRYM(cudaMemcpyAsync(m->dAorig, m->dA, sizeof(double) * (size_t)Np * Np, cudaMemcpyDeviceToDevice, st));
     }
-    rc = launch_factorize(m, invR != nullptr, true);
+    rc = launch_factorize(m, invR != nullptr, true, true);
     if (rc) { if (dTmp) pool_free(dTmp); return fail(rc); }
     // beta1 = W 1 (prior-mean correction term)
     TRYM(cudaMemcpyAsync(m->dBeta1, ones.data(), sizeof(double) * Np, cudaMemcpyHostToDevice, st));

@@ -6,6 +6,8 @@
 #include <utility>
 #include <vector>
 
+namespace ibo { struct JointWork; }
+
 struct ibo_model {
     int device = 0;
     cudaStream_t stream = nullptr;
@@ -71,6 +73,8 @@ struct ibo_model {
     // profile of the last call
     double prof[6] = {0, 0, 0, 0, 0, 0};
     cudaEvent_t ev[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+    // joint posterior (joint.cu): covariance, samples and their Cholesky factor, built on first use
+    ibo::JointWork* joint = nullptr;
 };
 
 struct ibo_cands {
@@ -94,7 +98,8 @@ void pool_free(void* p);
 cudaError_t pinned_get(double** p);
 void pinned_put(double* p);
 // launches (all on m->stream)
-int launch_factorize(ibo_model* m, bool from_inverse_reversed, bool pack);
+// invert = false: the Cholesky factor only (no W = inv(L), no beta = W Y); dW, dWpack and the beta vectors are not touched
+int launch_factorize(ibo_model* m, bool from_inverse_reversed, bool pack, bool invert);
 void launch_tri_matvec(const double* T, const double* v, double* out, int Np, cudaStream_t st);              // out = T v, T lower [Np][Np]
 void launch_tri_matvec_t(const double* T, const double* v, double* out, int n, int Np, cudaStream_t st);     // out = T^T v over the leading n x n
 int launch_syrk_identity(double* C, const double* G, int Np, int K, cudaStream_t st);                        // C = I + G G^T (lower tiles)
@@ -103,4 +108,8 @@ int create_model_with_diag(int device, int kind, const double* hyper, int nhyper
                            double noise, double diag, ibo_model** out, int* info);
 int launch_gram_wtw(double* C, const ibo_model* m, cudaStream_t st);      // hyper.cu: C (lower tiles) = W^T W = inv(A)
 const char* get_error();
+// score.cu: mu of M device-resident candidates on the FP64 path (what ibo_posterior_batch returns with IBO_FLAG_FP64) at out + M;
+// out holds 3 M + 2 doubles
+int posterior_mean_device(ibo_model* m, const double* dCand, long M, double* out);
+void free_joint(ibo_model* m);           // joint.cu: the model's joint-posterior workspace
 }  // namespace ibo

@@ -1194,6 +1194,13 @@ int batch_uses_i8(ibo_model* m, long n, int flags) {
     if (n > narrow_threshold()) return i8_eligible(m, flags) ? 1 : 0;
     return i8_for_small_batch(m, n, flags) ? 1 : 0;
 }
+// mu of the joint posterior (joint.cu): the FP64 kernels of ibo_posterior_batch(..., IBO_FLAG_FP64) on device-resident candidates,
+// so that mu is that call's mu bit for bit
+int posterior_mean_device(ibo_model* m, const double* dCand, long M, double* out) {
+    ScoreReq rq{-1, 0.0, 0.0, IBO_FLAG_FP64, false, true, false};
+    return score_device(m, dCand, M, rq, out);
+}
+
 int eval_neg_acq(ibo_model* m, const double* Xs, long n, int acq, double ymax, double parm, int flags, double* y) {
     ScoreReq rq{acq, ymax, parm, flags, true, false, false};
     rq.want_argmax = false;      // DIRECT consumes every value; the argmax kernels would be wasted launches

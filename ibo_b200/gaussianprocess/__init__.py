@@ -157,6 +157,25 @@ class GaussianProcess(object):
             return m, np.ones(len(X))
         return self.model.posterior(X, _lib.FLAG_MODE_PY)
 
+    def _candidates(self, X):
+        if len(self.X) == 0:
+            raise ValueError("joint posterior of a GP without data")
+        X = np.asarray(X, dtype=float)
+        return X.reshape(-1, 1) if X.ndim == 1 else X
+
+    def posterior_cov(self, X):
+        """joint posterior over the points in X -> (mu[M], cov[M, M]).  mu is what `posteriors` returns; diag(cov) is its
+        sigma^2 before clipping (the variance of an observation: 1 + noise - v.v)."""
+        return self.model.posterior_cov(self._candidates(X))
+
+    def sample_posterior(self, X, n_samples=1, seed=None, jitter=0.0):
+        """joint draws of the posterior at the points in X -> F[M, n_samples] = mu + chol(cov + jitter I) Z, with
+        Z = numpy.random.default_rng(seed).standard_normal((M, n_samples)): a seed reproduces the draws exactly.
+        Raises NotPositiveDefinite when cov + jitter I is not positive definite (near-duplicate points); a small jitter helps."""
+        X = self._candidates(X)
+        Z = np.random.default_rng(seed).standard_normal((X.shape[0], n_samples))
+        return self.model.posterior_sample(X, Z, jitter)[0]
+
     def score_batch(self, Xs, acq='ei', xi=0.01, parm=None, mode='py', want_posterior=False, out=None, int8=None):
         """Acquisition values for a candidate array (batched EI.negf / PI.negf / UCB.negf, negated).
 

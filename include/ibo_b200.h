@@ -176,6 +176,22 @@ int ibo_posterior_batch(ibo_model* m, const double* Xs, long M, int flags, doubl
 int ibo_score_batch(ibo_model* m, const double* Xs, long M, int acq, double ymax, double parm, int flags,
                     double* scores, double* mu, double* s2, double* best_score, long* best_idx);
 
+/* ---- joint posterior over a candidate set --------------------------------------------------------
+ * Xs: M x d row-major candidates (original coordinates), 1 <= M <= 16384, d <= 64.  With R the model's correlation function
+ * (k off the diagonal, 1 + noise on it) and W = inv(L) of the model (of its variance model when one is attached):
+ *     V = W R(X, Xs),  Sigma = R(Xs, Xs) - V^T V     (diag(Sigma) = the unclipped sigma^2 of ibo_posterior_batch)
+ * mu = the posterior mean exactly as ibo_posterior_batch returns it with IBO_FLAG_FP64.  GEMMs and the Cholesky on the FP64
+ * tensor pipe; workspace stays with the model (M x M and N x M doubles).
+ * mu[M] (may be NULL) and cov[M x M] row-major, full symmetric; 1 <= M <= 16384, d <= 64 */
+int ibo_posterior_cov(ibo_model* m, const double* Xs, long M, double* mu, double* cov);
+/* F[M x S] row-major = mu + chol(Sigma + jitter I) Z for caller-supplied standard normals Z[M x S] (row-major);
+ * argmax[S] = per-sample argmax over the M candidates (a Thompson batch).  F or argmax may be NULL.
+ * IBO_E_NOTSPD with *info = 1-based failing pivot when Sigma + jitter I is not positive definite.
+ * jitter is added for the factorisation only.  Ties go to the lowest index, NaN never wins.  IBO_E_BADARG for a NULL model,
+ * Xs or Z, M outside [1, 16384], S < 1, or jitter < 0 or NaN. */
+int ibo_posterior_sample(ibo_model* m, const double* Xs, long M, const double* Z, int S, double jitter,
+                         double* F, long* argmax, int* info);
+
 /* Candidates kept resident in HBM (the bench's device-resident leg; also used for sharded sets). */
 int ibo_cands_create(ibo_model* m, const double* Xs, long M, ibo_cands** out);
 int ibo_cands_destroy(ibo_cands* c);
