@@ -20,6 +20,7 @@ EXPORTED = [
     "ibo_model_get_matrix", "ibo_model_set_variance_model", "ibo_pref_fit",
     "ibo_nlml", "ibo_kernel_matrix",
     "ibo_posterior_batch", "ibo_score_batch", "ibo_posterior_cov", "ibo_posterior_sample",
+    "ibo_posterior_grad", "ibo_score_grad",
     "ibo_cands_create", "ibo_cands_destroy", "ibo_score_resident", "ibo_get_profile", "ibo_launch_count",
     "ibo_fp64_peak", "ibo_i8_peak", "ibo_i8_peak2", "ibo_host_register", "ibo_host_unregister", "ibo_stream_mark", "ibo_stream_elapsed_ms",
     "ibo_device_synchronize", "ibo_debug_exp",
@@ -102,6 +103,8 @@ def lib():
     L.ibo_score_batch.argtypes = [c_void_p, pd, c_long, c_int, c_double, c_double, c_int, pd, pd, pd, pd, pl]
     L.ibo_posterior_cov.argtypes = [c_void_p, pd, c_long, pd, pd]
     L.ibo_posterior_sample.argtypes = [c_void_p, pd, c_long, pd, c_int, c_double, pd, pl, pi]
+    L.ibo_posterior_grad.argtypes = [c_void_p, pd, c_long, c_int, pd, pd, pd, pd]
+    L.ibo_score_grad.argtypes = [c_void_p, pd, c_long, c_int, c_double, c_double, c_int, pd, pd]
     L.ibo_cands_create.argtypes = [c_void_p, pd, c_long, POINTER(c_void_p)]
     L.ibo_cands_destroy.argtypes = [c_void_p]
     L.ibo_score_resident.argtypes = [c_void_p, c_void_p, c_int, c_double, c_double, c_int, pd, pd, pl, POINTER(c_float)]
@@ -323,6 +326,24 @@ class Model(object):
                                         am.ctypes.data_as(POINTER(c_long)), ctypes.byref(info))
         check(rc, info.value)
         return F, am
+
+    def posterior_grad(self, Xs, flags=FLAG_MODE_PY):
+        """posterior and its gradient with respect to the candidate (ibo_posterior_grad) -> (mu[M], s2[M], dmu[M, d], ds2[M, d]);
+        values are ibo_posterior_batch's with FLAG_FP64, ds2 = 0 where s2 is clipped"""
+        Xs = self._candidates(Xs)
+        M = Xs.shape[0]
+        mu, s2, dmu, ds2 = np.empty(M), np.empty(M), np.empty((M, self.d)), np.empty((M, self.d))
+        check(lib().ibo_posterior_grad(self._h, dptr(Xs), M, flags, dptr(mu), dptr(s2), dptr(dmu), dptr(ds2)))
+        return mu, s2, dmu, ds2
+
+    def score_grad(self, Xs, acq, ymax, parm, flags=FLAG_MODE_PY):
+        """acquisition values and their gradient with respect to the candidate (ibo_score_grad) -> (scores[M], dscores[M, d]);
+        scores are ibo_score_batch's with FLAG_FP64"""
+        Xs = self._candidates(Xs)
+        M = Xs.shape[0]
+        sc, dsc = np.empty(M), np.empty((M, self.d))
+        check(lib().ibo_score_grad(self._h, dptr(Xs), M, acq, float(ymax), float(parm), flags, dptr(sc), dptr(dsc)))
+        return sc, dsc
 
     def score(self, Xs, acq, ymax, parm, flags=FLAG_MODE_PY, want_scores=True, want_posterior=False, out=None):
         """`out` (optional, float64[M]) receives the scores in place (lets callers reuse a pinned buffer)."""

@@ -97,13 +97,20 @@ class EI(_Acquisition):
         return self.ymax
 
 
-def cdirectGP(model, bounds, maxiter, maxtime, maxsample, acqfunc=None, xi=-1, beta=-1, scale=-1, delta=-1, **kwargs):
+def cdirectGP(model, bounds, maxiter, maxtime, maxsample, acqfunc=None, xi=-1, beta=-1, scale=-1, delta=-1, polish=0, **kwargs):
     """DIRECT over the GPU acquisition (replaces the ctypes marshalling into libego.acqmaxGP, :307-447).
 
     Same arguments and return value (opt, optx).  The arithmetic is libego's: libm erf, sigma^2 floor
     1e-8, and the UCB multiplier of :317-319.  No explicit inverse of R is formed (the reference does
     linalg.inv(R) / inv(R + inv(C)) per call, :385-388): the model's device-resident factor is reused.
+
+    polish = k > 0 refines DIRECT's answer by gradient ascent (polishAcquisition) from k starts: DIRECT's optx and the best
+    k - 1 of 1024 seeded Latin-hypercube points.  The best polished point is returned, with its FP64 value, only when that
+    value beats DIRECT's optx re-scored in the same call; otherwise DIRECT's (opt, optx) come back unchanged.
+    cdirectGP.last['polish'] gives the objective evaluations and whether the point moved.
     """
+    if polish and kwargs.get('shard'):
+        raise ValueError("polish is not supported with shard")
     if acqfunc == 'ei':
         acquisition, parm = _lib.ACQ_EI, xi
     elif acqfunc == 'pi':
@@ -125,7 +132,82 @@ def cdirectGP(model, bounds, maxiter, maxtime, maxsample, acqfunc=None, xi=-1, b
     opt, optx, nsamples, iters = model.model.acqmax(lower, upper, acquisition, np.max(model.Y), parm, flags,
                                                    maxiter=maxiter, maxtime=maxtime, maxsample=maxsample)
     cdirectGP.last = dict(nsamples=nsamples, iterations=iters)
+    if polish > 0:
+        fp64 = _lib.FLAG_MODE_CPP | _lib.FLAG_FP64
+        P = np.array(lhcSample(bounds, 1024, seed=_POLISH_SEED), dtype=float)
+        sc = model.model.score(P, acquisition, np.max(model.Y), parm, fp64)[0]
+        starts = np.r_[np.asarray(optx, dtype=float)[None, :], P[np.argsort(-sc, kind='stable')[:polish - 1]]]
+        acq = {_lib.ACQ_EI: 'ei', _lib.ACQ_PI: 'pi', _lib.ACQ_UCB: 'ucb'}[acquisition]
+        vals, X, v0, nfev = _polish_model(model, bounds, starts, acq, parm, 'cpp', 100)
+        b = int(np.argmax(vals))
+        moved = bool(vals[b] > v0[0])
+        cdirectGP.last['polish'] = dict(evaluations=nfev, moved=moved)
+        if moved:
+            return float(vals[b]), X[b]
     return opt, optx
+
+
+_POLISH_SEED = 0
+
+
+def _polish(fg, bounds, X0, maxiter=100):
+    """Maximise a separable sum of S acquisitions from the starts X0[S, d] with L-BFGS-B.  fg(X[S, d]) -> (values[S],
+    gradients[S, d]) is called once per objective evaluation for all starts.  Dimensions with equal bounds stay at that
+    bound; the others are clipped into the box.  One final call scores the starts and the results together, and each row keeps
+    whichever is better.  Returns (values[S], X[S, d], values of the starts[S], evaluations)."""
+    from scipy.optimize import minimize
+    b = np.array(bounds, dtype=float).reshape(-1, 2)
+    lo, hi = b[:, 0], b[:, 1]
+    X0 = np.clip(np.array(X0, dtype=float, ndmin=2), lo, hi)
+    S = X0.shape[0]
+    free = lo < hi
+    nf = int(free.sum())
+    state = dict(n=0, scale=None)
+
+    def X_of(z):
+        X = X0.copy()
+        X[:, free] = np.clip(z.reshape(S, nf), lo[free], hi[free])
+        return X
+
+    def obj(z):
+        v, g = fg(X_of(z))
+        state['n'] += 1
+        if state['scale'] is None:       # the first evaluation is at the starts: a fixed scale keeps EI of any size well conditioned
+            m = np.max(np.abs(v[np.isfinite(v)])) if np.any(np.isfinite(v)) else 0.0
+            state['scale'] = 1.0 / m if m > 0 else 1.0
+        f = -state['scale'] * np.sum(v)
+        gr = -state['scale'] * g[:, free].ravel()
+        if not np.isfinite(f) or not np.all(np.isfinite(gr)):
+            return np.inf, np.zeros_like(gr)
+        return f, gr
+
+    X = X0
+    if nf > 0:
+        res = minimize(obj, X0[:, free].ravel(), jac=True, method='L-BFGS-B', bounds=list(zip(np.tile(lo[free], S), np.tile(hi[free], S))),
+                       options=dict(maxiter=maxiter, ftol=1e-15, gtol=1e-12))
+        X = X_of(res.x)
+    v, _ = fg(np.r_[X0, X])
+    state['n'] += 1
+    v0, v1 = v[:S], v[S:]
+    better = v1 > v0
+    return np.where(better, v1, v0), np.where(better[:, None], X, X0), v0, state['n']
+
+
+def _polish_model(GP, bounds, X0, acq, parm, mode, maxiter):
+    flags = _lib.FLAG_MODE_PY if mode == 'py' else _lib.FLAG_MODE_CPP
+    acq_id = {'ei': _lib.ACQ_EI, 'pi': _lib.ACQ_PI, 'ucb': _lib.ACQ_UCB}[acq]
+    ymax = np.max(GP.Y)
+    return _polish(lambda X: GP.model.score_grad(X, acq_id, ymax, parm, flags), bounds, X0, maxiter)
+
+
+def polishAcquisition(GP, bounds, X0, acq='ei', xi=0.01, parm=None, mode='cpp', maxiter=100):
+    """Gradient refinement of acquisition maximisers: L-BFGS-B from each start in X0[S, d] within `bounds`, all starts in one
+    batched value-and-gradient call (GaussianProcess.score_grad) per evaluation.  Dimensions with equal bounds stay fixed.  Each
+    returned row is at least as good as its start (FP64 values).  Returns (values[S], X[S, d])."""
+    if len(GP.X) == 0:
+        raise ValueError("acquisition over a GP without data")
+    vals, X, _, _ = _polish_model(GP, bounds, X0, acq, xi if parm is None else parm, mode, maxiter)
+    return vals, X
 
 
 def thompsonBatch(GP, bounds, q, samples=2048, candidates=None, seed=None, jitter=0.0):

@@ -9,6 +9,7 @@
 // library's sigma^2 before clipping.  With a variance model attached (PrefGaussianProcess.addObservationPoint) Sigma comes
 // from that model's X and W, as sigma^2 does; mu always comes from the scoring path (score.cu) on the FP64 kernels.
 // Both GEMMs and the Cholesky of Sigma run on the FP64 tensor pipe (tile_gemm_core, launch_factorize).
+// The candidate scaling, R(X, X*) and the two W GEMMs are also what grad.cu builds the gradient of sigma^2 from.
 #include "model.cuh"
 #include "scoremath.cuh"
 #include "tilegemm.cuh"
@@ -101,6 +102,30 @@ __global__ void __launch_bounds__(256, 1) trimm_kernel(double* __restrict__ C, i
         }
 }
 
+// The transposed twin of trimm_kernel: C[I][J] = sum_{k >= I} T_kI^T B_kJ, T as there (the transposed-A tile path).  K = (nbr - I) 128,
+// so row block 0 is the heaviest and is scheduled first.  With T = W (identity padding rows) and B zero in its padding rows, C is
+// zero in its padding rows.
+__global__ void __launch_bounds__(256, 1) trimm_t_kernel(double* __restrict__ C, int ldc, const double* __restrict__ T, int ldt,
+                                                         const double* __restrict__ B, int ldb, int nbr) {
+    extern __shared__ double sm[];
+    const int I = blockIdx.y, J = blockIdx.x;
+    double acc[8][4][2];
+#pragma unroll
+    for (int a = 0; a < 8; a++)
+#pragma unroll
+        for (int b = 0; b < 4; b++) acc[a][b][0] = acc[a][b][1] = 0.0;
+    tile_gemm_core<false, true>(T + (size_t)I * 128 * ldt + (size_t)I * 128, ldt, B + (size_t)I * 128 * ldb + (size_t)J * 128, ldb,
+                                (nbr - I) * 128, acc, sm);
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, wm = warp >> 2, wn = warp & 3;
+#pragma unroll
+    for (int mt = 0; mt < 8; mt++)
+#pragma unroll
+        for (int nt = 0; nt < 4; nt++) {
+            const int row = I * 128 + wm * 64 + mt * 8 + (lane >> 2), c = wn * 32 + nt * 8 + 2 * (lane & 3);
+            *reinterpret_cast<double2*>(C + (size_t)row * ldc + (size_t)J * 128 + c) = make_double2(acc[mt][nt][0], acc[mt][nt][1]);
+        }
+}
+
 // Sigma tile (I, J), J <= I, in place over R(X*, X*): S_IJ -= sum_k V_kI^T V_kJ (the transposed-A path of gram_wtw_kernel), + jitter on
 // the diagonal of the real candidates
 __global__ void __launch_bounds__(256, 1) sigma_kernel(double* __restrict__ S, const double* __restrict__ V, int Mp, int K, int M, double jitter) {
@@ -171,6 +196,7 @@ __global__ void __launch_bounds__(256) sample_argmax_kernel(const double* __rest
 cudaError_t set_joint_attrs() {
     cudaError_t e = cudaFuncSetAttribute(trimm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TILE_SMEM_DOUBLES * 8);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(sigma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TILE_SMEM_DOUBLES * 8);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(trimm_t_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TILE_SMEM_DOUBLES * 8);
     return e;
 }
 
@@ -232,6 +258,25 @@ void free_joint(ibo_model* m) {
     if (w->chol.dInfo) cudaFree(w->chol.dInfo);
     delete w;
     m->joint = nullptr;
+}
+
+// launch wrappers for grad.cu
+void launch_scale_cands(double* Cs, const double* X, const ibo_model* g, long M, long Mp, cudaStream_t st) {
+    scale_cands_kernel<<<(unsigned)((Mp * g->d + 255) / 256), 256, 0, st>>>(Cs, X, g->dInvTheta, g->dCenter, M, Mp, g->d);
+    g_launches++;
+}
+void launch_cross_cov(double* Kc, const ibo_model* g, const double* Cs, int M, int Mp, cudaStream_t st) {
+    cross_cov_kernel<<<dim3((Mp + 255) / 256, g->Np), 256, 0, st>>>(Kc, g->dXt, Cs, g->N, M, Mp, g->d, g->kind, g->sf2);
+    g_launches++;
+}
+int launch_w_gemms(double* Z, double* V, const ibo_model* g, const double* Kc, int Mp, cudaStream_t st) {
+    cudaError_t ae = ensure_attrs(g->device, ATTR_JOINT, set_joint_attrs);
+    if (ae != cudaSuccess) { set_error(std::string("cudaFuncSetAttribute: ") + cudaGetErrorString(ae)); return IBO_E_CUDA; }
+    const dim3 grid(Mp / 128, g->nb);
+    trimm_kernel<<<grid, 256, TILE_SMEM_DOUBLES * 8, st>>>(V, Mp, g->dW, g->Np, Kc, Mp, g->nb, nullptr, 0);
+    trimm_t_kernel<<<grid, 256, TILE_SMEM_DOUBLES * 8, st>>>(Z, Mp, g->dW, g->Np, V, Mp, g->nb);
+    g_launches += 2;
+    return IBO_OK;
 }
 
 }  // namespace ibo

@@ -6,7 +6,7 @@
 #include <utility>
 #include <vector>
 
-namespace ibo { struct JointWork; }
+namespace ibo { struct JointWork; struct GradWork; }
 
 struct ibo_model {
     int device = 0;
@@ -75,6 +75,8 @@ struct ibo_model {
     cudaEvent_t ev[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
     // joint posterior (joint.cu): covariance, samples and their Cholesky factor, built on first use
     ibo::JointWork* joint = nullptr;
+    // gradients with respect to the candidate (grad.cu), built on first use
+    ibo::GradWork* grad = nullptr;
 };
 
 struct ibo_cands {
@@ -111,5 +113,14 @@ const char* get_error();
 // score.cu: mu of M device-resident candidates on the FP64 path (what ibo_posterior_batch returns with IBO_FLAG_FP64) at out + M;
 // out holds 3 M + 2 doubles
 int posterior_mean_device(ibo_model* m, const double* dCand, long M, double* out);
+// score.cu: [score | mu | s2] of M device-resident candidates at out, what ibo_score_batch (acq >= 0) or ibo_posterior_batch
+// (acq < 0) returns with flags; out holds 3 M + 2 doubles
+int posterior_score_device(ibo_model* m, const double* dCand, long M, int acq, double ymax, double parm, int flags, double* out);
 void free_joint(ibo_model* m);           // joint.cu: the model's joint-posterior workspace
+// joint.cu, on st: candidates scaled and centred like g's training inputs ([Mp][d], zero padded); R(X_g, X*) with exact
+// zeros in the padding ([Np][Mp]); V = W_g Kc and Z = W_g^T V ([Np][Mp] each, Z may overwrite Kc)
+void launch_scale_cands(double* Cs, const double* X, const ibo_model* g, long M, long Mp, cudaStream_t st);
+void launch_cross_cov(double* Kc, const ibo_model* g, const double* Cs, int M, int Mp, cudaStream_t st);
+int launch_w_gemms(double* Z, double* V, const ibo_model* g, const double* Kc, int Mp, cudaStream_t st);
+void free_grad(ibo_model* m);            // grad.cu: the model's gradient workspace
 }  // namespace ibo

@@ -1200,6 +1200,13 @@ int posterior_mean_device(ibo_model* m, const double* dCand, long M, double* out
     ScoreReq rq{-1, 0.0, 0.0, IBO_FLAG_FP64, false, true, false};
     return score_device(m, dCand, M, rq, out);
 }
+// values of the candidate gradients (grad.cu): the scoring path's own kernels, so that they are ibo_score_batch's /
+// ibo_posterior_batch's bit for bit
+int posterior_score_device(ibo_model* m, const double* dCand, long M, int acq, double ymax, double parm, int flags, double* out) {
+    ScoreReq rq{acq, ymax, parm, flags, acq >= 0, true, true};
+    rq.want_argmax = false;
+    return score_device(m, dCand, M, rq, out);
+}
 
 int eval_neg_acq(ibo_model* m, const double* Xs, long n, int acq, double ymax, double parm, int flags, double* y) {
     ScoreReq rq{acq, ymax, parm, flags, true, false, false};

@@ -17,6 +17,22 @@ __device__ __forceinline__ double cov_r2(int kind, double sf2, double r2) {
     return sf2 * (1.0 + z + 5.0 * r2 / 3.0) * exp(-z);
 }
 
+// dk/dx_t = -(1 / theta_t) h(r) (s_t - s_i,t) in the scaled coordinates s = x / theta - centre: h = k for SE,
+// 3 sf2 e^(-sqrt3 r) for Matern-3/2, (5/3) sf2 (1 + sqrt5 r) e^(-sqrt5 r) for Matern-5/2 -- finite at r = 0 for all of them.
+// *k receives k(r) (cov_r2's formulas).
+__device__ __forceinline__ double cov_grad_h(int kind, double sf2, double r2, double* k) {
+    if (kind <= IBO_KERNEL_SE_ISO) { *k = sf2 * exp(-0.5 * r2); return *k; }
+    const double r = sqrt(r2);
+    if (kind == IBO_KERNEL_MATERN3) {
+        const double z = 1.7320508075688772 * r, e = sf2 * exp(-z);
+        *k = (1.0 + z) * e;
+        return 3.0 * e;
+    }
+    const double z = 2.23606797749979 * r, e = sf2 * exp(-z);
+    *k = (1.0 + z + 5.0 * r2 / 3.0) * e;
+    return (5.0 / 3.0) * (1.0 + z) * e;
+}
+
 // exp(x) for x <= 0 with the coefficients in the constant bank.  K1 is issue bound (ncu: 78 % of the issue slots, FP64 pipe
 // 39 %), and libdevice's exp materialises its eleven 64-bit polynomial constants with two uniform moves each per call
 // (UMOV = 26 % of all executed instructions of K1): here every coefficient is a constant-bank operand of its DFMA.
@@ -74,6 +90,51 @@ __device__ __forceinline__ double erf_nr(double z) {
     p = 1.00002368 + t * p;
     double ans = 1 - t * exp(-z * z - 1.26551223 + t * p);
     return z >= 0.0 ? ans : -ans;
+}
+
+// d erf_nr / dz: erf_nr(z) = sign(z) g(|z|), g(u) = 1 - t e^E, t = 1 / (1 + u / 2), E = -u^2 - 1.26551223 + t p(t), so the
+// derivative is g'(|z|) = -e^E (t' + t E') with t' = -t^2 / 2 and E' = -2 u + t' (p + t p').  The derivative of the formula
+// erf_nr evaluates (same constants, Horner order), not of the exact erf.
+__device__ __forceinline__ double erf_nr_deriv(double z) {
+    const double u = fabs(z);
+    const double t = 1.0 / (1.0 + 0.5 * u);
+    double p = 0.17087277, dp = 0.0;
+    dp = p + t * dp; p = -0.82215223 + t * p;
+    dp = p + t * dp; p = 1.48851587 + t * p;
+    dp = p + t * dp; p = -1.13520398 + t * p;
+    dp = p + t * dp; p = 0.27886807 + t * p;
+    dp = p + t * dp; p = -0.18628806 + t * p;
+    dp = p + t * dp; p = 0.09678418 + t * p;
+    dp = p + t * dp; p = 0.37409196 + t * p;
+    dp = p + t * dp; p = 1.00002368 + t * p;
+    const double e = exp(-u * u - 1.26551223 + t * p);
+    const double dt = -0.5 * t * t;
+    const double dE = -2.0 * u + dt * (p + t * dp);
+    return -e * (dt + t * dE);
+}
+
+// partial derivatives of acq_value with respect to mu and s = sqrt(s2), in the same arithmetic: libm mode through the exact
+// pair (Phi, phi); Python mode through the derivative of its own formula (erf_nr, 0.707106, 0.398942)
+__device__ __forceinline__ void acq_partials(int acq, int mode_py, double mu, double s2, double ymax, double parm, double* dmu,
+                                             double* ds) {
+    const double s = sqrt(s2);
+    if (acq == IBO_ACQ_UCB) { *dmu = 1.0; *ds = parm; return; }
+    const double Z = (acq == IBO_ACQ_EI ? mu - ymax - parm : mu - (ymax + parm)) / s;
+    if (mode_py) {
+        const double cdf = 0.5 * (1 + erf_nr(Z * 0.707106));
+        const double dcdf = 0.5 * 0.707106 * erf_nr_deriv(Z * 0.707106);
+        if (acq == IBO_ACQ_PI) { *dmu = dcdf / s; *ds = -Z * dcdf / s; return; }
+        const double pdf = exp(-(Z * Z / 2)) * 0.398942;
+        const double dpdf = -Z * pdf;
+        // v = ydiff cdf(Z) + s pdf(Z), ydiff = s Z
+        *dmu = cdf + Z * dcdf + dpdf;
+        *ds = pdf - Z * Z * dcdf - Z * dpdf;
+        return;
+    }
+    const double pdf = exp(-(Z * Z / 2.)) / 2.5066282746310002;
+    if (acq == IBO_ACQ_PI) { *dmu = pdf / s; *ds = -Z * pdf / s; return; }
+    *dmu = 0.5 * (1. + erf(Z / 1.4142135623730951));
+    *ds = pdf;
 }
 
 __device__ __forceinline__ double acq_value(int acq, int mode_py, double mu, double s2, double ymax, double parm) {

@@ -191,6 +191,19 @@ class GaussianProcess(object):
             return sc, best, bidx, mu, s2
         return sc, best, bidx
 
+    def posterior_grad(self, X, mode='py'):
+        """posterior at the points in X and its gradient with respect to the point -> (mu[M], s2[M], dmu[M, d], ds2[M, d]).
+        Values are those of the FP64 kernels; ds2 = 0 where s2 is clipped (floor by mode, ceiling 10)."""
+        flags = _lib.FLAG_MODE_PY if mode == 'py' else _lib.FLAG_MODE_CPP
+        return self.model.posterior_grad(self._candidates(X), flags)
+
+    def score_grad(self, Xs, acq='ei', xi=0.01, parm=None, mode='py'):
+        """acquisition values at the points in Xs and their gradient with respect to the point -> (scores[M], dscores[M, d]),
+        with score_batch's incumbent and defaults; the values are score_batch's with int8=False."""
+        acq_id = {'ei': _lib.ACQ_EI, 'pi': _lib.ACQ_PI, 'ucb': _lib.ACQ_UCB}[acq]
+        flags = _lib.FLAG_MODE_PY if mode == 'py' else _lib.FLAG_MODE_CPP
+        return self.model.score_grad(self._candidates(Xs), acq_id, np.max(self.Y), xi if parm is None else parm, flags)
+
     def mu(self, x):
         return self.posterior(x, getvar=False)
 

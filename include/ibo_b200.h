@@ -192,6 +192,21 @@ int ibo_posterior_cov(ibo_model* m, const double* Xs, long M, double* mu, double
 int ibo_posterior_sample(ibo_model* m, const double* Xs, long M, const double* Z, int S, double jitter,
                          double* F, long* argmax, int* info);
 
+/* ---- gradients with respect to the candidate ----------------------------------------------------
+ * Xs: M x d row-major candidates (original coordinates), M >= 1, d <= 64.  flags: 0 (IBO_FLAG_MODE_CPP) or IBO_FLAG_MODE_PY.
+ * Values (mu, s2, scores) are those of the FP64 kernels (IBO_FLAG_FP64) bit for bit.  With s = x / theta - centre,
+ *     dk_i / dx_t = -(1 / theta_t) h(r_i) (s_t - s_i,t),   d mu = d m0 (1 - k^T b) + sum_i (a_i - m0 b_i) dk_i,
+ *     d s2 = -2 sum_i z_i dk_i,  z = R^-1 k         (a = R^-1 Y, b = R^-1 1; R of the variance model for s2 when one is attached)
+ * z comes from two DMMA triangular GEMMs (W K*, W^T V) per chunk of candidates; workspace stays with the model.
+ * dmu, ds2: M x d row-major; ds2 = 0 where sigma^2 is clipped (floor by mode, ceiling 10).  Any output may be NULL.
+ * IBO_E_BADARG for a NULL model or Xs, M < 1, d > 64, acq outside 0..2, or a flag bit other than IBO_FLAG_MODE_PY. */
+int ibo_posterior_grad(ibo_model* m, const double* Xs, long M, int flags, double* mu, double* s2, double* dmu, double* ds2);
+/* scores[M] as ibo_score_batch returns them with IBO_FLAG_FP64; dscores[M x d] row-major = the chain rule through (mu, sqrt(s2)):
+ * EI d/dmu = Phi(Z), d/ds = phi(Z); PI phi(Z) / s, -Z phi(Z) / s; UCB 1, parm.  In IBO_FLAG_MODE_PY Phi and phi are the derivatives
+ * of that mode's own formula (the Chebyshev erf with 0.707106 / 0.398942), so that dscores match finite differences of its values. */
+int ibo_score_grad(ibo_model* m, const double* Xs, long M, int acq, double ymax, double parm, int flags,
+                   double* scores, double* dscores);
+
 /* Candidates kept resident in HBM (the bench's device-resident leg; also used for sharded sets). */
 int ibo_cands_create(ibo_model* m, const double* Xs, long M, ibo_cands** out);
 int ibo_cands_destroy(ibo_cands* c);
