@@ -20,7 +20,7 @@ EXPORTED = [
     "ibo_model_get_matrix", "ibo_model_set_variance_model", "ibo_pref_fit",
     "ibo_nlml", "ibo_kernel_matrix",
     "ibo_posterior_batch", "ibo_score_batch", "ibo_posterior_cov", "ibo_posterior_sample",
-    "ibo_posterior_grad", "ibo_score_grad",
+    "ibo_posterior_grad", "ibo_score_grad", "ibo_qei",
     "ibo_cands_create", "ibo_cands_destroy", "ibo_score_resident", "ibo_get_profile", "ibo_launch_count",
     "ibo_fp64_peak", "ibo_i8_peak", "ibo_i8_peak2", "ibo_host_register", "ibo_host_unregister", "ibo_stream_mark", "ibo_stream_elapsed_ms",
     "ibo_device_synchronize", "ibo_debug_exp",
@@ -105,6 +105,7 @@ def lib():
     L.ibo_posterior_sample.argtypes = [c_void_p, pd, c_long, pd, c_int, c_double, pd, pl, pi]
     L.ibo_posterior_grad.argtypes = [c_void_p, pd, c_long, c_int, pd, pd, pd, pd]
     L.ibo_score_grad.argtypes = [c_void_p, pd, c_long, c_int, c_double, c_double, c_int, pd, pd]
+    L.ibo_qei.argtypes = [c_void_p, pd, c_long, c_int, pd, c_int, c_double, c_double, c_double, pd, pd, pi]
     L.ibo_cands_create.argtypes = [c_void_p, pd, c_long, POINTER(c_void_p)]
     L.ibo_cands_destroy.argtypes = [c_void_p]
     L.ibo_score_resident.argtypes = [c_void_p, c_void_p, c_int, c_double, c_double, c_int, pd, pd, pl, POINTER(c_float)]
@@ -344,6 +345,23 @@ class Model(object):
         sc, dsc = np.empty(M), np.empty((M, self.d))
         check(lib().ibo_score_grad(self._h, dptr(Xs), M, acq, float(ymax), float(parm), flags, dptr(sc), dptr(dsc)))
         return sc, dsc
+
+    def qei(self, Xb, Z, ymax, xi, jitter=0.0, want_grad=True):
+        """batch expected improvement of B batches of q points Xb[B, q, d] for standard normals Z[q, S] (ibo_qei) ->
+        (values[B], dvalues[B, q, d] or None, number of batches whose covariance + jitter I is not positive definite: NaN rows)"""
+        Xb = as_f64(Xb, 3)
+        Z = as_f64(Z, 2)
+        B, q, d = Xb.shape
+        if d != self.d:
+            raise ValueError("points have %d columns, the model %d" % (d, self.d))
+        if Z.shape[0] != q:
+            raise ValueError("Z has %d rows for batches of %d points" % (Z.shape[0], q))
+        vals = np.empty(B)
+        dv = np.empty((B, q, d)) if want_grad else None
+        nbad = c_int(0)
+        check(lib().ibo_qei(self._h, dptr(Xb), B, q, dptr(Z), Z.shape[1], float(ymax), float(xi), float(jitter), dptr(vals),
+                            dptr(dv) if want_grad else None, ctypes.byref(nbad)))
+        return vals, dv, nbad.value
 
     def score(self, Xs, acq, ymax, parm, flags=FLAG_MODE_PY, want_scores=True, want_posterior=False, out=None):
         """`out` (optional, float64[M]) receives the scores in place (lets callers reuse a pinned buffer)."""

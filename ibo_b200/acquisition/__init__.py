@@ -228,6 +228,50 @@ def thompsonBatch(GP, bounds, q, samples=2048, candidates=None, seed=None, jitte
     return C[idx], idx
 
 
+def _polish_batches(fg, bounds, starts, pending=None, maxiter=100):
+    """L-BFGS-B over whole batches: fg(X[S, n, d]) -> (values[S], gradients[S, n, d]) for S batches of n = q + p points, starts[S, q, d],
+    pending[p, d] appended to every batch and held fixed (lo = hi bounds).  Returns (best value, its q free points[q, d], the values
+    of the starts[S], evaluations)."""
+    b = np.array(bounds, dtype=float).reshape(-1, 2)
+    starts = np.array(starts, dtype=float, ndmin=3)
+    S, q, d = starts.shape
+    P = np.zeros((0, d)) if pending is None else np.array(pending, dtype=float, ndmin=2).reshape(-1, d)
+    n = q + P.shape[0]
+    X0 = np.concatenate([starts, np.broadcast_to(P, (S,) + P.shape)], axis=1).reshape(S, n * d)
+    tb = np.r_[np.tile(b, (q, 1)), np.repeat(P.reshape(-1, 1), 2, axis=1)]
+
+    def flat(X):
+        v, g = fg(X.reshape(-1, n, d))
+        return v, g.reshape(-1, n * d)
+    vals, X, v0, nfev = _polish(flat, tb, X0, maxiter)
+    vs = np.where(np.isnan(vals), -np.inf, vals)
+    k = int(np.argmax(vs))
+    return float(vals[k]), X[k].reshape(n, d)[:q], v0, nfev
+
+
+def maximizeQEI(GP, bounds, q, samples=512, seed=0, xi=0.01, starts=8, pending=None, jitter=0.0, maxiter=100):
+    """Choose q points to evaluate in parallel by maximising their Monte-Carlo batch expected improvement (GaussianProcess.qEI) with
+    L-BFGS-B on its exact gradient.  Z is drawn once (numpy.random.default_rng(seed), q + p rows, `samples` columns), so every
+    evaluation uses the same common random numbers and the objective is deterministic.  The starts are
+    thompsonBatch(GP, bounds, q, seed=seed + k) for k < starts; all of them are polished together, one ibo_qei call per evaluation.
+    pending[p, d] are points already under evaluation: they join every batch, held fixed, so the q new points improve on them too.
+    Returns (value, batch[q, d]); the value is at least the best start's.  maximizeQEI.last records the evaluations and the values
+    of the starts."""
+    if len(GP.X) == 0:
+        raise ValueError("q-EI over a GP without data")
+    p = 0 if pending is None else np.array(pending, dtype=float, ndmin=2).shape[0]
+    Z = np.random.default_rng(seed).standard_normal((q + p, samples))
+    ymax = np.max(GP.Y)
+    X0 = np.array([thompsonBatch(GP, bounds, q, seed=seed + k, jitter=jitter)[0] for k in range(starts)])
+
+    def fg(X):
+        v, g, _ = GP.model.qei(X, Z, ymax, xi, jitter)
+        return v, g
+    val, batch, v0, nfev = _polish_batches(fg, bounds, X0, pending, maxiter)
+    maximizeQEI.last = dict(evaluations=nfev, start_values=v0)
+    return val, batch
+
+
 def _python_direct(obj, bounds, **kw):
     """useCDIRECT=False route: the same DIRECT driver over the Python-path objective (batched)."""
     opt, optx = direct(obj.negf, bounds, batch_objective=lambda P: -obj.f_batch(P), pure=True, **kw)

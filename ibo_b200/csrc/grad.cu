@@ -161,6 +161,9 @@ __global__ void __launch_bounds__(256) grad_epilogue_kernel(GradEpi P) {
     }
 }
 
+}  // namespace
+
+// launch wrappers, also for qei.cu
 template <bool DZ, bool DA, bool DB>
 void launch_reduce(const ibo_model* src, const double* Cs, int Mc, const double* Z, int ldz, const double* a, const double* b,
                    double* G, size_t plane, double* kb, cudaStream_t st) {
@@ -169,6 +172,28 @@ void launch_reduce(const ibo_model* src, const double* Cs, int Mc, const double*
                                                           a, b, G, plane, kb);
     g_launches++;
 }
+template void launch_reduce<true, false, false>(const ibo_model*, const double*, int, const double*, int, const double*, const double*,
+                                                double*, size_t, double*, cudaStream_t);
+template void launch_reduce<false, true, false>(const ibo_model*, const double*, int, const double*, int, const double*, const double*,
+                                                double*, size_t, double*, cudaStream_t);
+template void launch_reduce<false, true, true>(const ibo_model*, const double*, int, const double*, int, const double*, const double*,
+                                               double*, size_t, double*, cudaStream_t);
+template void launch_reduce<true, true, false>(const ibo_model*, const double*, int, const double*, int, const double*, const double*,
+                                               double*, size_t, double*, cudaStream_t);
+template void launch_reduce<true, true, true>(const ibo_model*, const double*, int, const double*, int, const double*, const double*,
+                                              double*, size_t, double*, cudaStream_t);
+
+void launch_grad_prior(const ibo_model* m, const double* cand, long M, const double* kb, double* G, cudaStream_t st) {
+    GradEpi P{};
+    P.M = M; P.d = m->d; P.npb = m->npb; P.ptheta = m->ptheta;
+    P.cand = cand; P.kb = kb;
+    P.pmeans = m->dPmeans; P.pbeta = m->dPbeta; P.plb = m->dPlb; P.pwidth = m->dPwidth;
+    P.G = G;
+    grad_prior_kernel<<<(unsigned)((M + 255) / 256), 256, 0, st>>>(P);
+    g_launches++;
+}
+
+namespace {
 
 inline long round128(long x) { return (x + 127) / 128 * 128; }
 
@@ -217,7 +242,7 @@ int grad_device(ibo_model* m, const double* Xs, long M, int acq, double ymax, do
         double* kb = prior ? w->dKb + c0 : nullptr;
         launch_scale_cands(w->dScaled, raw, g, Mc, Mcp, st);
         launch_cross_cov(w->dKc, g, w->dScaled, Mc, Mcp, st);
-        if ((rc = launch_w_gemms(w->dKc, w->dV, g, w->dKc, Mcp, st))) return rc;
+        if ((rc = launch_w_gemm_v(w->dV, g, w->dKc, Mcp, st)) || (rc = launch_w_gemm_z(w->dKc, g, w->dV, Mcp, st))) return rc;
         if (vm) {
             launch_reduce<true, false, false>(g, w->dScaled, Mc, w->dKc, Mcp, nullptr, nullptr, G, plane, nullptr, st);
             launch_scale_cands(w->dScaledM, raw, m, Mc, Mcp, st);
@@ -229,15 +254,13 @@ int grad_device(ibo_model* m, const double* Xs, long M, int acq, double ymax, do
             launch_reduce<true, true, false>(m, w->dScaled, Mc, w->dKc, Mcp, dA, nullptr, G, plane, nullptr, st);
         }
     }
-    GradEpi P;
+    GradEpi P{};
     P.M = M; P.d = d; P.acq = acq; P.mode_py = (flags & IBO_FLAG_MODE_PY) ? 1 : 0; P.npb = m->npb;
-    P.ymax = ymax; P.parm = parm; P.ptheta = m->ptheta;
-    P.vals = w->dVals; P.cand = w->dRaw; P.kb = w->dKb;
-    P.pmeans = m->dPmeans; P.pbeta = m->dPbeta; P.plb = m->dPlb; P.pwidth = m->dPwidth;
+    P.ymax = ymax; P.parm = parm;
+    P.vals = w->dVals;
     P.G = w->dG;
-    const unsigned nblk = (unsigned)((M + 255) / 256);
-    if (prior) { grad_prior_kernel<<<nblk, 256, 0, st>>>(P); g_launches++; }
-    grad_epilogue_kernel<<<nblk, 256, 0, st>>>(P);
+    if (prior) launch_grad_prior(m, w->dRaw, M, w->dKb, w->dG, st);
+    grad_epilogue_kernel<<<(unsigned)((M + 255) / 256), 256, 0, st>>>(P);
     g_launches++;
     IBO_CUDA_TRY(cudaGetLastError());
     return IBO_OK;

@@ -260,7 +260,7 @@ void free_joint(ibo_model* m) {
     m->joint = nullptr;
 }
 
-// launch wrappers for grad.cu
+// launch wrappers for grad.cu and qei.cu
 void launch_scale_cands(double* Cs, const double* X, const ibo_model* g, long M, long Mp, cudaStream_t st) {
     scale_cands_kernel<<<(unsigned)((Mp * g->d + 255) / 256), 256, 0, st>>>(Cs, X, g->dInvTheta, g->dCenter, M, Mp, g->d);
     g_launches++;
@@ -269,13 +269,18 @@ void launch_cross_cov(double* Kc, const ibo_model* g, const double* Cs, int M, i
     cross_cov_kernel<<<dim3((Mp + 255) / 256, g->Np), 256, 0, st>>>(Kc, g->dXt, Cs, g->N, M, Mp, g->d, g->kind, g->sf2);
     g_launches++;
 }
-int launch_w_gemms(double* Z, double* V, const ibo_model* g, const double* Kc, int Mp, cudaStream_t st) {
+int launch_w_gemm_v(double* V, const ibo_model* g, const double* Kc, int Mp, cudaStream_t st) {
     cudaError_t ae = ensure_attrs(g->device, ATTR_JOINT, set_joint_attrs);
     if (ae != cudaSuccess) { set_error(std::string("cudaFuncSetAttribute: ") + cudaGetErrorString(ae)); return IBO_E_CUDA; }
-    const dim3 grid(Mp / 128, g->nb);
-    trimm_kernel<<<grid, 256, TILE_SMEM_DOUBLES * 8, st>>>(V, Mp, g->dW, g->Np, Kc, Mp, g->nb, nullptr, 0);
-    trimm_t_kernel<<<grid, 256, TILE_SMEM_DOUBLES * 8, st>>>(Z, Mp, g->dW, g->Np, V, Mp, g->nb);
-    g_launches += 2;
+    trimm_kernel<<<dim3(Mp / 128, g->nb), 256, TILE_SMEM_DOUBLES * 8, st>>>(V, Mp, g->dW, g->Np, Kc, Mp, g->nb, nullptr, 0);
+    g_launches++;
+    return IBO_OK;
+}
+int launch_w_gemm_z(double* Z, const ibo_model* g, const double* V, int Mp, cudaStream_t st) {
+    cudaError_t ae = ensure_attrs(g->device, ATTR_JOINT, set_joint_attrs);
+    if (ae != cudaSuccess) { set_error(std::string("cudaFuncSetAttribute: ") + cudaGetErrorString(ae)); return IBO_E_CUDA; }
+    trimm_t_kernel<<<dim3(Mp / 128, g->nb), 256, TILE_SMEM_DOUBLES * 8, st>>>(Z, Mp, g->dW, g->Np, V, Mp, g->nb);
+    g_launches++;
     return IBO_OK;
 }
 

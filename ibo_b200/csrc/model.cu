@@ -974,6 +974,7 @@ static void free_model(ibo_model* m) {
     if (m->stream) cudaStreamSynchronize(m->stream);   // blocks go back to the pool: nothing may still be using them
     free_joint(m);
     free_grad(m);
+    free_qei(m);
     double** ptrs[] = {&m->dXt, &m->dInvTheta, &m->dCenter, &m->dA, &m->dAorig, &m->dW, &m->dD, &m->dWpack, &m->dBetaY, &m->dBeta1, &m->dY,
                        &m->dPmeans, &m->dPbeta, &m->dPlb, &m->dPwidth, &m->dCand, &m->dSlab, &m->dPart, &m->dOut, &m->dBlkBest, &m->dBest, &m->dAppend,
                        &m->dWi8s, &m->dRowScale, &m->dAlphaY, &m->dAlpha1, &m->dGuard, &m->dGuardList, &m->dCinv};

@@ -6,7 +6,7 @@
 #include <utility>
 #include <vector>
 
-namespace ibo { struct JointWork; struct GradWork; }
+namespace ibo { struct JointWork; struct GradWork; struct QeiWork; }
 
 struct ibo_model {
     int device = 0;
@@ -77,6 +77,8 @@ struct ibo_model {
     ibo::JointWork* joint = nullptr;
     // gradients with respect to the candidate (grad.cu), built on first use
     ibo::GradWork* grad = nullptr;
+    // batch expected improvement (qei.cu), built on first use
+    ibo::QeiWork* qei = nullptr;
 };
 
 struct ibo_cands {
@@ -121,6 +123,15 @@ void free_joint(ibo_model* m);           // joint.cu: the model's joint-posterio
 // zeros in the padding ([Np][Mp]); V = W_g Kc and Z = W_g^T V ([Np][Mp] each, Z may overwrite Kc)
 void launch_scale_cands(double* Cs, const double* X, const ibo_model* g, long M, long Mp, cudaStream_t st);
 void launch_cross_cov(double* Kc, const ibo_model* g, const double* Cs, int M, int Mp, cudaStream_t st);
-int launch_w_gemms(double* Z, double* V, const ibo_model* g, const double* Kc, int Mp, cudaStream_t st);
+int launch_w_gemm_v(double* V, const ibo_model* g, const double* Kc, int Mp, cudaStream_t st);
+int launch_w_gemm_z(double* Z, const ibo_model* g, const double* V, int Mp, cudaStream_t st);
 void free_grad(ibo_model* m);            // grad.cu: the model's gradient workspace
+// grad.cu, on st: G[q][j][t] = sum_i w_q,i dk_i(x*_j) / dx_t over src's training points for the weights enabled (w_0 = Z[:, j],
+// w_1 = a, w_2 = b; planes `plane` doubles apart), kb[j] = sum_i b_i k_i; Cs scaled like src's training inputs
+template <bool DZ, bool DA, bool DB>
+void launch_reduce(const ibo_model* src, const double* Cs, int Mc, const double* Z, int ldz, const double* a, const double* b,
+                   double* G, size_t plane, double* kb, cudaStream_t st);
+// grad.cu, on st: the prior's share of dmu in place over plane 2 of G ([3][M][d]) for the M candidates `cand` (original coordinates)
+void launch_grad_prior(const ibo_model* m, const double* cand, long M, const double* kb, double* G, cudaStream_t st);
+void free_qei(ibo_model* m);             // qei.cu: the model's q-EI workspace
 }  // namespace ibo

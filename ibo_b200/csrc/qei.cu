@@ -1,0 +1,448 @@
+// Batch expected improvement (q-EI) of B batches of q points and its gradient with respect to the points, by Monte Carlo with
+// caller-supplied standard normals Z[q][S] (Ginsbourger et al. 2010; reparameterisation gradients, Wilson et al. 2018):
+//
+//   qEI(b) = (1 / S) sum_s max(0, max_j (mu_b + L_b z_s)_j - ymax - xi),   L_b = chol(Sigma_b + jitter I)
+//
+// mu is the posterior mean sum_i a_i k_i (a = R^-1 Y; with the prior's terms), summed in a fixed order per point: the scoring path's
+// FP64 mean groups its sums by the size of the call, which would make a batch's value depend on the other batches.
+// Sigma_b = R(X*_b, X*_b) - V_b^T V_b is ibo_posterior_cov's (of the variance model when one is attached).  Reverse mode with Z
+// fixed: per sample with positive improvement and argmax j* (lowest index wins), mubar_j* += 1 / S and Lbar_j*,k += z_k,s / S
+// (k <= j*); the reverse Cholesky (Murray 2016) turns Lbar into the symmetric Gbar = d qEI / d Sigma (sum over all ordered pairs), and
+//
+//   d qEI / dx_j = mubar_j dmu(x_j) + 2 sum_l Gbar_jl d1 k(x_j, x_l) - 2 sum_i y_j,i dk_i(x_j) / dx_j,   y_j = sum_l Gbar_jl z_l
+//
+// with z_l = R_g^-1 k(X_g, x_l) = column l of W_g^T W_g K*.  Per chunk of whole batches: K* and V = W_g K* on the DMMA tile GEMM
+// (joint.cu), the q x q blocks of Sigma on CUDA cores, one CTA per batch for the Cholesky, the sample loop and the reverse
+// pass; with gradients Z = W_g^T V, y into V's buffer, and grad.cu's reduction with y in place of z.  Every sum runs in a fixed
+// order without atomics and touches one batch only, so a batch's value and gradient do not depend on the other batches.
+#include "model.cuh"
+#include "scoremath.cuh"
+#include <algorithm>
+#include <cmath>
+
+namespace ibo {
+
+// Workspace of ibo_qei, kept with the model that owns the call and grown on demand.
+struct QeiWork {
+    double* dRaw = nullptr;    size_t rawCap = 0;     // points as given [M][d], M = B q
+    double* dZ = nullptr;      size_t zCap = 0;       // standard normals [q][S]
+    double* dMu = nullptr;     size_t muCap = 0;      // mu [M]
+    double* dVal = nullptr;    size_t valCap = 0;     // values [B]
+    double* dMubar = nullptr;  size_t mubarCap = 0;   // d qEI / d mu [M]
+    double* dG = nullptr;      size_t gCap = 0;       // three [M][d] planes: sums with y, a, b -> the gradient in plane 0
+    double* dKb = nullptr;     size_t kbCap = 0;      // k^T b [M] (prior only)
+    double* dSig = nullptr;    size_t sigCap = 0;     // Sigma of the chunk's batches [Bc][q][q]
+    double* dGbar = nullptr;   size_t gbarCap = 0;    // Gbar of the chunk's batches [Bc][q][q]
+    double* dScaled = nullptr; size_t scaledCap = 0;  // chunk scaled like g's training inputs [Mcp][d]
+    double* dScaledM = nullptr; size_t scaledMCap = 0;// chunk scaled like the model's (variance model attached) [Mcp][d]
+    double* dKc = nullptr;     size_t kcCap = 0;      // K*, then Z [Np][Mcp]
+    double* dV = nullptr;      size_t vCap = 0;       // V, then y [Np][Mcp]
+    double* dAB = nullptr;     size_t abCap = 0;      // a | b [2][Np]
+};
+
+namespace {
+
+constexpr int QEI_MAX_Q = 32;
+constexpr int SIG_SLICES = 8;                                        // training points i = s, s + 8, ... per partial sum
+constexpr int SIG_ROWS = 32;                                         // rows of V staged per step (a multiple of SIG_SLICES)
+constexpr int SIG_ITEMS = QEI_MAX_Q * (QEI_MAX_Q + 1) / 2 * SIG_SLICES;
+constexpr int SIG_PER_THREAD = (SIG_ITEMS + 255) / 256;
+constexpr int QW = 4;                                                // warps of the per-batch kernel
+
+// One CTA per batch: Sigma_b[j][l] = k(x_j, x_l) (diag on the diagonal) - sum_i V_ij V_il over the batch's q columns of V.  Item
+// (pair p, slice s) sums the rows i = s (mod 8) in ascending order and the eight slices are added in slice order, so the order of
+// every entry is the same whatever q is: a batch's Sigma_00 is that of its first point alone.
+__global__ void __launch_bounds__(256) qei_sigma_kernel(double* __restrict__ Sig, const double* __restrict__ V, int ldv,
+                                                        const double* __restrict__ Cs, int N, int q, int d, int kind, double sf2,
+                                                        double diag) {
+    __shared__ double tile[SIG_ROWS][QEI_MAX_Q + 1];
+    __shared__ double part[SIG_ITEMS];
+    const int b = blockIdx.x, c0 = b * q, np = q * (q + 1) / 2, items = np * SIG_SLICES;
+    int pj[SIG_PER_THREAD], pl[SIG_PER_THREAD];
+    double acc[SIG_PER_THREAD];
+#pragma unroll
+    for (int u = 0; u < SIG_PER_THREAD; u++) {
+        const int p = (threadIdx.x + 256 * u) / SIG_SLICES;
+        int j = 0;
+        while ((j + 1) * (j + 2) / 2 <= p) j++;                      // p = j (j + 1) / 2 + l, l <= j
+        pj[u] = j; pl[u] = p - j * (j + 1) / 2; acc[u] = 0.0;
+    }
+    for (int i0 = 0; i0 < N; i0 += SIG_ROWS) {
+        __syncthreads();
+        for (int idx = threadIdx.x; idx < SIG_ROWS * q; idx += 256) {
+            const int r = idx / q, c = idx - r * q;
+            tile[r][c] = i0 + r < N ? V[(size_t)(i0 + r) * ldv + c0 + c] : 0.0;
+        }
+        __syncthreads();
+#pragma unroll
+        for (int u = 0; u < SIG_PER_THREAD; u++) {
+            const int it = threadIdx.x + 256 * u;
+            if (it < items)
+                for (int r = it % SIG_SLICES; r < SIG_ROWS; r += SIG_SLICES) acc[u] = fma(tile[r][pj[u]], tile[r][pl[u]], acc[u]);
+        }
+    }
+#pragma unroll
+    for (int u = 0; u < SIG_PER_THREAD; u++) {
+        const int it = threadIdx.x + 256 * u;
+        if (it < items) part[it] = acc[u];
+    }
+    __syncthreads();
+    for (int p = threadIdx.x; p < np; p += 256) {
+        int j = 0;
+        while ((j + 1) * (j + 2) / 2 <= p) j++;
+        const int l = p - j * (j + 1) / 2;
+        double s = part[p * SIG_SLICES];
+        for (int k = 1; k < SIG_SLICES; k++) s += part[p * SIG_SLICES + k];
+        double v = diag;
+        if (j != l) {
+            const double* xa = Cs + (size_t)(c0 + l) * d;
+            const double* xb = Cs + (size_t)(c0 + j) * d;
+            double r2 = 0;
+            for (int t = 0; t < d; t++) { const double df = xa[t] - xb[t]; r2 = fma(df, df, r2); }
+            v = cov_r2(kind, sf2, r2);
+        }
+        v -= s;
+        Sig[(size_t)b * q * q + j * q + l] = v;
+        Sig[(size_t)b * q * q + l * q + j] = v;
+    }
+}
+
+// One CTA of four warps per batch.  Warp 0 factorises Sigma_b + jitter I (lane = row); warp w takes the samples s = w, w + 4, ...
+// (lane j computes (mu + L z_s)_j, a butterfly finds the maximum and its lowest index) and the four warps' sums are added in warp
+// order.  GRAD: per warp, lane k adds z_k,s to Lbar[j*][k]; the warps' Lbar are added in warp order, and warp 0 runs the reverse
+// Cholesky Gbar = sym(L^-T Phi(L^T Lbar) L^-1) (Phi: lower triangle, halved diagonal).  The value path is the same code with
+// and without GRAD.  A batch whose factorisation fails gets NaN for its value, mubar and Gbar.
+template <bool GRAD>
+__global__ void __launch_bounds__(QW * 32) qei_batch_kernel(const double* __restrict__ Sig, const double* __restrict__ mu,
+                                                            const double* __restrict__ Z, int S, int q, double ymax, double xi,
+                                                            double jitter, double* __restrict__ val, double* __restrict__ mubar,
+                                                            double* __restrict__ Gbar) {
+    __shared__ double L[QEI_MAX_Q][QEI_MAX_Q + 1];
+    __shared__ double Lb[GRAD ? QW : 1][QEI_MAX_Q][QEI_MAX_Q + 1];
+    __shared__ double wacc[QW];
+    __shared__ int cnt[QW][QEI_MAX_Q];
+    __shared__ int bad;
+    const int b = blockIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const double* A = Sig + (size_t)b * q * q;
+    for (int idx = threadIdx.x; idx < q * q; idx += QW * 32) {
+        const int r = idx / q, c = idx - r * q;
+        L[r][c] = r == c ? A[idx] + jitter : A[idx];
+    }
+    if (GRAD)
+        for (int idx = threadIdx.x; idx < QW * QEI_MAX_Q * (QEI_MAX_Q + 1); idx += QW * 32) (&Lb[0][0][0])[idx] = 0.0;
+    __syncthreads();
+    if (warp == 0) {
+        int ok = 1;
+        for (int k = 0; k < q && ok; k++) {
+            double s = lane >= k && lane < q ? L[lane][k] : 0.0;
+            if (lane >= k && lane < q)
+                for (int i = 0; i < k; i++) s = fma(-L[lane][i], L[k][i], s);
+            const double dk = __shfl_sync(0xffffffffu, s, k);
+            ok = dk > 0.0;                                           // NaN fails too
+            if (ok) {
+                const double lkk = sqrt(dk);
+                if (lane == k) L[k][k] = lkk;
+                else if (lane > k && lane < q) L[lane][k] = s / lkk;
+            }
+            __syncwarp();
+        }
+        if (lane == 0) bad = !ok;
+    }
+    __syncthreads();
+    if (bad) {
+        if (threadIdx.x == 0) val[b] = NAN;
+        if (GRAD) {
+            for (int j = threadIdx.x; j < q; j += QW * 32) mubar[(size_t)b * q + j] = NAN;
+            for (int j = threadIdx.x; j < q * q; j += QW * 32) Gbar[(size_t)b * q * q + j] = NAN;
+        }
+        return;
+    }
+    const bool live = lane < q;
+    const double muj = live ? mu[(size_t)b * q + lane] : 0.0;
+    double acc = 0.0;
+    int c = 0;
+    for (int s = warp; s < S; s += QW) {
+        const double zk = live ? Z[(size_t)lane * S + s] : 0.0;
+        double f = muj;
+        for (int k = 0; k < q; k++) {
+            const double zz = __shfl_sync(0xffffffffu, zk, k);
+            if (k <= lane && live) f = fma(L[lane][k], zz, f);
+        }
+        double v = live ? f : -INFINITY;
+        int ix = lane;
+#pragma unroll
+        for (int off = 16; off > 0; off >>= 1) {
+            const double ov = __shfl_xor_sync(0xffffffffu, v, off);
+            const int oi = __shfl_xor_sync(0xffffffffu, ix, off);
+            if (ov > v || (ov == v && oi < ix)) { v = ov; ix = oi; }
+        }
+        const double imp = __dsub_rn(__dsub_rn(v, ymax), xi);
+        acc = __dadd_rn(acc, imp > 0.0 ? imp : 0.0);
+        if (GRAD && imp > 0.0) {
+            if (lane <= ix) Lb[warp][ix][lane] += zk;
+            if (lane == ix) c++;
+        }
+    }
+    if (lane == 0) wacc[warp] = acc;
+    if (GRAD && live) cnt[warp][lane] = c;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double t = wacc[0];
+        for (int w = 1; w < QW; w++) t = __dadd_rn(t, wacc[w]);
+        val[b] = t / S;
+    }
+    if (!GRAD) return;
+    if (threadIdx.x < q) {
+        int n = 0;
+        for (int w = 0; w < QW; w++) n += cnt[w][threadIdx.x];
+        mubar[(size_t)b * q + threadIdx.x] = (double)n / S;
+    }
+    for (int idx = threadIdx.x; idx < q * q; idx += QW * 32) {        // Lbar into Lb[0]
+        const int r = idx / q, k = idx - r * q;
+        double t = Lb[0][r][k];
+        for (int w = 1; w < QW; w++) t += Lb[w][r][k];
+        Lb[0][r][k] = k <= r ? t / S : 0.0;
+    }
+    __syncthreads();
+    if (warp != 0) return;
+    double (*Lbar)[QEI_MAX_Q + 1] = Lb[0];
+    double (*P)[QEI_MAX_Q + 1] = Lb[1];
+    double (*X)[QEI_MAX_Q + 1] = Lb[2];
+    double (*Sm)[QEI_MAX_Q + 1] = Lb[3];
+    if (live) {                                                       // P = Phi(L^T Lbar), lane = column
+        for (int k = 0; k < q; k++) {
+            double s = 0.0;
+            for (int i = max(k, lane); i < q; i++) s = fma(L[i][k], Lbar[i][lane], s);
+            P[k][lane] = k > lane ? s : (k == lane ? 0.5 * s : 0.0);
+        }
+    }
+    __syncwarp();
+    if (live) {                                                       // X = L^-T P, lane = column
+        for (int k = q - 1; k >= 0; k--) {
+            double s = P[k][lane];
+            for (int i = k + 1; i < q; i++) s = fma(-L[i][k], X[i][lane], s);
+            X[k][lane] = s / L[k][k];
+        }
+    }
+    __syncwarp();
+    if (live) {                                                       // S = X L^-1, lane = row: L^T S[r]^T = X[r]^T
+        for (int k = q - 1; k >= 0; k--) {
+            double s = X[lane][k];
+            for (int i = k + 1; i < q; i++) s = fma(-L[i][k], Sm[lane][i], s);
+            Sm[lane][k] = s / L[k][k];
+        }
+    }
+    __syncwarp();
+    if (live)
+        for (int l = 0; l < q; l++) Gbar[(size_t)b * q * q + lane * q + l] = 0.5 * (Sm[lane][l] + Sm[l][lane]);
+}
+
+// mu of the chunk's points over the model's training points, mu = sum_i a_i k_i (a = R^-1 Y), with a prior m0 + sum_i a_i k_i -
+// m0 sum_i b_i k_i (b = R^-1 1).  One CTA: 32 points (lane = point) x 8 warps striding the training points i = w, w + 8, ...; the
+// warps' partial sums are added in warp order, so a point's mu does not depend on the other points of the call.
+__global__ void __launch_bounds__(256) qei_mean_kernel(double* __restrict__ mu, const double* __restrict__ Xt, int N,
+                                                       const double* __restrict__ Cs, const double* __restrict__ raw, int Mc, int d,
+                                                       int kind, double sf2, const double* __restrict__ a, const double* __restrict__ b,
+                                                       int npb, const double* __restrict__ pmeans, const double* __restrict__ pbeta,
+                                                       double ptheta, const double* __restrict__ plb, const double* __restrict__ pwidth) {
+    __shared__ double sh[32 * 65];
+    __shared__ double pa[8][32], pb[8][32];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, j0 = blockIdx.x * 32, j = j0 + lane, ldc = d | 1;
+    for (int idx = threadIdx.x; idx < 32 * d; idx += 256) {
+        const int c = idx / d, t = idx - c * d;
+        sh[c * ldc + t] = j0 + c < Mc ? Cs[(size_t)(j0 + c) * d + t] : 0.0;
+    }
+    __syncthreads();
+    const double* cj = sh + lane * ldc;
+    double sa = 0.0, sb = 0.0;
+    for (int i = warp; i < N && j < Mc; i += 8) {
+        const double* xi = Xt + (size_t)i * d;
+        double r2 = 0;
+        for (int t = 0; t < d; t++) { const double df = xi[t] - cj[t]; r2 = fma(df, df, r2); }
+        const double k = cov_r2(kind, sf2, r2);
+        sa = fma(a[i], k, sa);
+        if (npb > 0) sb = fma(b[i], k, sb);
+    }
+    pa[warp][lane] = sa;
+    pb[warp][lane] = sb;
+    __syncthreads();
+    if (warp != 0 || j >= Mc) return;
+    double A = pa[0][lane], Bs = pb[0][lane];
+    for (int w = 1; w < 8; w++) { A += pa[w][lane]; Bs += pb[w][lane]; }
+    if (npb > 0) {
+        const double m0 = prior_mean(raw + (size_t)j * d, d, npb, pmeans, pbeta, ptheta, plb, pwidth);
+        A = m0 + A - m0 * Bs;
+    }
+    mu[j] = A;
+}
+
+// y[i][j] = sum_l Zm[i][b q + l] Gbar_b[j - b q][l] for the training points i < N and the chunk's points j (b = j / q)
+__global__ void __launch_bounds__(256) qei_y_kernel(double* __restrict__ Y, const double* __restrict__ Zm, int ld,
+                                                    const double* __restrict__ Gbar, int Mc, int q) {
+    const int j = blockIdx.x * 256 + threadIdx.x, i = blockIdx.y;
+    if (j >= Mc) return;
+    const int b = j / q, jj = j - b * q;
+    const double* z = Zm + (size_t)i * ld + (size_t)b * q;
+    const double* g = Gbar + (size_t)b * q * q + (size_t)jj * q;
+    double s = 0.0;
+    for (int l = 0; l < q; l++) s = fma(z[l], g[l], s);
+    Y[(size_t)i * ld + j] = s;
+}
+
+// One thread per point of the chunk, in place over its row of plane 0 (sum_i y_i dk_i): -2 (that) + 2 sum_{l != j} Gbar_jl d1 k(x_j, x_l)
+// with d1 k(x_j, x_l) / dx_t = -(1 / theta_t) h(r) (s_j,t - s_l,t) in g's scaled coordinates Cs
+__global__ void __launch_bounds__(256) qei_pair_kernel(double* __restrict__ G, const double* __restrict__ Cs, const double* __restrict__ Gbar,
+                                                       int Mc, int q, int d, int kind, double sf2, const double* __restrict__ inv_theta) {
+    const int j = blockIdx.x * 256 + threadIdx.x;
+    if (j >= Mc) return;
+    const int b = j / q, jj = j - b * q;
+    double* g = G + (size_t)j * d;
+    const double* xj = Cs + (size_t)j * d;
+    for (int t = 0; t < d; t++) g[t] *= -2.0;
+    for (int l = 0; l < q; l++) {
+        if (l == jj) continue;
+        const double* xl = Cs + (size_t)(b * q + l) * d;
+        double r2 = 0;
+        for (int t = 0; t < d; t++) { const double df = xj[t] - xl[t]; r2 = fma(df, df, r2); }
+        double k;
+        const double w = 2.0 * Gbar[(size_t)b * q * q + (size_t)jj * q + l] * cov_grad_h(kind, sf2, r2, &k);
+        for (int t = 0; t < d; t++) g[t] = fma(-inv_theta[t] * w, xj[t] - xl[t], g[t]);
+    }
+}
+
+// One thread per point: plane 0 += mubar dmu, dmu = plane 1 (+ plane 2 with a prior)
+__global__ void __launch_bounds__(256) qei_epilogue_kernel(double* __restrict__ G, long M, int d, const double* __restrict__ mubar, int prior) {
+    const long m = blockIdx.x * 256L + threadIdx.x;
+    if (m >= M) return;
+    const size_t plane = (size_t)M * d;
+    double* g = G + (size_t)m * d;
+    for (int t = 0; t < d; t++) {
+        const double dmu = prior ? g[plane + t] + g[2 * plane + t] : g[plane + t];
+        g[t] = fma(mubar[m], dmu, g[t]);
+    }
+}
+
+inline long round128(long x) { return (x + 127) / 128 * 128; }
+
+// Enqueues everything on m->stream and leaves the values in w->dVal and, with wantGrad, the gradient [M][d] in w->dG.
+int qei_device(ibo_model* m, const double* Xs, long B, int q, const double* Z, int S, double ymax, double xi, double jitter, bool wantGrad) {
+    if (!m->qei) m->qei = new QeiWork();
+    QeiWork* w = m->qei;
+    ibo_model* vm = m->var_model;
+    ibo_model* g = vm ? vm : m;                          // the model Sigma comes from
+    cudaStream_t st = m->stream;
+    const int d = m->d;
+    const bool prior = m->npb > 0;
+    const long M = B * q;
+    // chunk: as many whole batches as fit in grad.cu's bound (the largest multiple of 128 points whose K* / Z and V fit in 512 MiB)
+    const long chunkPts = std::max(128L, (long)((512L << 20) / (2L * 8 * g->Np)) / 128 * 128);
+    const long Bc = chunkPts / q;
+    const long Bcap = std::min(B, Bc), Mcap = round128(Bcap * q);
+    int rc;
+    if ((rc = grow(&w->dRaw, &w->rawCap, (size_t)M * d))) return rc;
+    if ((rc = grow(&w->dZ, &w->zCap, (size_t)q * S))) return rc;
+    if ((rc = grow(&w->dMu, &w->muCap, (size_t)M))) return rc;
+    if ((rc = grow(&w->dAB, &w->abCap, (size_t)2 * m->Np))) return rc;
+    if (vm && (rc = grow(&w->dScaledM, &w->scaledMCap, (size_t)Mcap * d))) return rc;
+    if ((rc = grow(&w->dVal, &w->valCap, (size_t)B))) return rc;
+    if ((rc = grow(&w->dSig, &w->sigCap, (size_t)Bcap * q * q))) return rc;
+    if ((rc = grow(&w->dScaled, &w->scaledCap, (size_t)Mcap * d))) return rc;
+    if ((rc = grow(&w->dKc, &w->kcCap, (size_t)g->Np * Mcap))) return rc;
+    if ((rc = grow(&w->dV, &w->vCap, (size_t)g->Np * Mcap))) return rc;
+    if (wantGrad) {
+        if ((rc = grow(&w->dMubar, &w->mubarCap, (size_t)M))) return rc;
+        if ((rc = grow(&w->dG, &w->gCap, (size_t)3 * M * d))) return rc;
+        if ((rc = grow(&w->dGbar, &w->gbarCap, (size_t)Bcap * q * q))) return rc;
+        if (prior && (rc = grow(&w->dKb, &w->kbCap, (size_t)M))) return rc;
+    }
+    IBO_CUDA_TRY(cudaMemcpyAsync(w->dRaw, Xs, sizeof(double) * (size_t)M * d, cudaMemcpyHostToDevice, st));
+    IBO_CUDA_TRY(cudaMemcpyAsync(w->dZ, Z, sizeof(double) * (size_t)q * S, cudaMemcpyHostToDevice, st));
+    const double* mu = w->dMu;
+    double* const dA = w->dAB;
+    double* const dB = prior ? w->dAB + m->Np : nullptr;
+    launch_tri_matvec_t(m->dW, m->dBetaY, dA, m->N, m->Np, st);     // a = W^T (W Y), b = W^T (W 1) of the model, as grad.cu
+    if (prior) launch_tri_matvec_t(m->dW, m->dBeta1, dB, m->N, m->Np, st);
+    const size_t plane = (size_t)M * d;
+    for (long b0 = 0; b0 < B; b0 += Bc) {
+        const int nbt = (int)std::min(Bc, B - b0), Mc = nbt * q, Mcp = (int)round128(Mc);
+        const long c0 = b0 * q;
+        const double* raw = w->dRaw + (size_t)c0 * d;
+        launch_scale_cands(w->dScaled, raw, g, Mc, Mcp, st);
+        if (vm) launch_scale_cands(w->dScaledM, raw, m, Mc, Mcp, st);
+        const double* Cm = vm ? w->dScaledM : w->dScaled;          // the chunk scaled like the model's training inputs
+        qei_mean_kernel<<<(Mc + 31) / 32, 256, 0, st>>>(w->dMu + c0, m->dXt, m->N, Cm, raw, Mc, d, m->kind, m->sf2, dA, dB, m->npb,
+                                                        m->dPmeans, m->dPbeta, m->ptheta, m->dPlb, m->dPwidth);
+        g_launches++;
+        launch_cross_cov(w->dKc, g, w->dScaled, Mc, Mcp, st);
+        if ((rc = launch_w_gemm_v(w->dV, g, w->dKc, Mcp, st))) return rc;
+        qei_sigma_kernel<<<nbt, 256, 0, st>>>(w->dSig, w->dV, Mcp, w->dScaled, g->N, q, d, g->kind, g->sf2, 1.0 + g->noise);
+        g_launches += 2;
+        if (!wantGrad) {
+            qei_batch_kernel<false><<<nbt, QW * 32, 0, st>>>(w->dSig, mu + c0, w->dZ, S, q, ymax, xi, jitter, w->dVal + b0, nullptr, nullptr);
+            continue;
+        }
+        qei_batch_kernel<true><<<nbt, QW * 32, 0, st>>>(w->dSig, mu + c0, w->dZ, S, q, ymax, xi, jitter, w->dVal + b0, w->dMubar + c0, w->dGbar);
+        if ((rc = launch_w_gemm_z(w->dKc, g, w->dV, Mcp, st))) return rc;
+        qei_y_kernel<<<dim3((Mc + 255) / 256, g->N), 256, 0, st>>>(w->dV, w->dKc, Mcp, w->dGbar, Mc, q);
+        g_launches += 2;
+        double* G = w->dG + (size_t)c0 * d;
+        double* kb = prior ? w->dKb + c0 : nullptr;
+        if (vm) {
+            launch_reduce<true, false, false>(g, w->dScaled, Mc, w->dV, Mcp, nullptr, nullptr, G, plane, nullptr, st);
+            if (prior) launch_reduce<false, true, true>(m, w->dScaledM, Mc, nullptr, 0, dA, dB, G, plane, kb, st);
+            else launch_reduce<false, true, false>(m, w->dScaledM, Mc, nullptr, 0, dA, nullptr, G, plane, nullptr, st);
+        } else if (prior) {
+            launch_reduce<true, true, true>(m, w->dScaled, Mc, w->dV, Mcp, dA, dB, G, plane, kb, st);
+        } else {
+            launch_reduce<true, true, false>(m, w->dScaled, Mc, w->dV, Mcp, dA, nullptr, G, plane, nullptr, st);
+        }
+        qei_pair_kernel<<<(Mc + 255) / 256, 256, 0, st>>>(G, w->dScaled, w->dGbar, Mc, q, d, g->kind, g->sf2, g->dInvTheta);
+        g_launches++;
+    }
+    if (wantGrad) {
+        if (prior) launch_grad_prior(m, w->dRaw, M, w->dKb, w->dG, st);
+        qei_epilogue_kernel<<<(unsigned)((M + 255) / 256), 256, 0, st>>>(w->dG, M, d, w->dMubar, prior ? 1 : 0);
+        g_launches++;
+    }
+    IBO_CUDA_TRY(cudaGetLastError());
+    return IBO_OK;
+}
+
+}  // namespace
+
+void free_qei(ibo_model* m) {
+    QeiWork* w = m->qei;
+    if (!w) return;
+    double** ptrs[] = {&w->dRaw, &w->dZ, &w->dMu, &w->dVal, &w->dMubar, &w->dG, &w->dKb, &w->dSig, &w->dGbar, &w->dScaled,
+                       &w->dScaledM, &w->dKc, &w->dV, &w->dAB};
+    for (auto p : ptrs) if (*p) pool_free(*p);
+    delete w;
+    m->qei = nullptr;
+}
+
+}  // namespace ibo
+
+using namespace ibo;
+
+extern "C" int ibo_qei(ibo_model* m, const double* Xs, long B, int q, const double* Z, int S, double ymax, double xi, double jitter,
+                       double* values, double* dvalues, int* nbad) {
+    if (nbad) *nbad = 0;
+    // every scalar check comes before the model is read; NaN jitter fails the comparison
+    if (!m || !Xs || !Z || !values || B < 1 || q < 1 || q > QEI_MAX_Q || S < 1 || S > 65536 || !(jitter >= 0.0)) {
+        set_error("bad argument");
+        return IBO_E_BADARG;
+    }
+    if (m->d > 64) { set_error("d > 64 not supported"); return IBO_E_BADARG; }
+    IBO_CUDA_TRY(cudaSetDevice(m->device));
+    int rc = qei_device(m, Xs, B, q, Z, S, ymax, xi, jitter, dvalues != nullptr);
+    if (rc) return rc;
+    QeiWork* w = m->qei;
+    cudaStream_t st = m->stream;
+    IBO_CUDA_TRY(cudaMemcpyAsync(values, w->dVal, sizeof(double) * B, cudaMemcpyDeviceToHost, st));
+    if (dvalues) IBO_CUDA_TRY(cudaMemcpyAsync(dvalues, w->dG, sizeof(double) * (size_t)B * q * m->d, cudaMemcpyDeviceToHost, st));
+    IBO_CUDA_TRY(cudaStreamSynchronize(st));
+    IBO_CUDA_TRY(cudaGetLastError());
+    if (nbad)
+        for (long b = 0; b < B; b++) *nbad += std::isnan(values[b]) ? 1 : 0;
+    return IBO_OK;
+}

@@ -204,6 +204,25 @@ class GaussianProcess(object):
         flags = _lib.FLAG_MODE_PY if mode == 'py' else _lib.FLAG_MODE_CPP
         return self.model.score_grad(self._candidates(Xs), acq_id, np.max(self.Y), xi if parm is None else parm, flags)
 
+    def qEI(self, batches, samples=512, seed=None, xi=0.01, jitter=0.0, Z=None, grad=False):
+        """Monte-Carlo expected improvement of batches of points evaluated together (q-EI) over the incumbent max(Y):
+        batches[B, q, d] (or one batch [q, d]) -> values[B] (a float for one batch), and with grad=True also the gradient with
+        respect to the points [B, q, d] (or [q, d]).  The draws are mu + chol(cov + jitter I) Z with
+        Z = numpy.random.default_rng(seed).standard_normal((q, samples)) unless Z[q, S] is given: the same Z makes every call
+        score with the same common random numbers.  A batch whose cov + jitter I is not positive definite (e.g. a repeated point
+        without noise) gets NaN."""
+        if len(self.X) == 0:
+            raise ValueError("q-EI of a GP without data")
+        Xb = np.asarray(batches, dtype=float)
+        one = Xb.ndim == 2
+        Xb = Xb[None] if one else Xb
+        if Z is None:
+            Z = np.random.default_rng(seed).standard_normal((Xb.shape[1], samples))
+        vals, dv, _ = self.model.qei(Xb, Z, np.max(self.Y), xi, jitter, want_grad=grad)
+        if one:
+            vals, dv = float(vals[0]), (dv[0] if grad else None)
+        return (vals, dv) if grad else vals
+
     def mu(self, x):
         return self.posterior(x, getvar=False)
 

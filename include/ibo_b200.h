@@ -207,6 +207,25 @@ int ibo_posterior_grad(ibo_model* m, const double* Xs, long M, int flags, double
 int ibo_score_grad(ibo_model* m, const double* Xs, long M, int acq, double ymax, double parm, int flags,
                    double* scores, double* dscores);
 
+/* ---- batch expected improvement (q-EI) -----------------------------------------------------------
+ * Xs: B x q x d row-major, batch b = (x_b1 .. x_bq) contiguous (original coordinates).  With mu_b, Sigma_b the joint posterior of
+ * batch b as ibo_posterior_cov defines it (Sigma = R(Xs, Xs) - V^T V, 1 + noise on the diagonal, unclipped; from the variance model
+ * when one is attached; mu = the posterior mean, summed in a fixed order per point, so it agrees with ibo_posterior_batch's to
+ * rounding but does not depend on the other points of the call), L_b = chol(Sigma_b + jitter I) and caller-supplied standard
+ * normals Z[q x S] (row-major, the layout of ibo_posterior_sample):
+ *     values[b] = (1 / S) sum_s max(0, max_j (mu_b + L_b z_s)_j - ymax - xi)
+ * (at q = 1 the Monte-Carlo estimate of EI in libm arithmetic with the unclipped sigma^2).  dvalues[B x q x d] (may be NULL) is its
+ * exact gradient with respect to the points for the fixed Z: per sample with positive improvement and argmax j* (lowest index wins
+ * ties) mubar_j* += 1 / S, Lbar_j*,k += z_k,s / S (k <= j*); Gbar = d qEI / d Sigma by the reverse Cholesky (Murray 2016), summed
+ * over all ordered pairs; then
+ *     d qEI / dx_j = mubar_j dmu(x_j) + 2 sum_l Gbar_jl d1 k(x_j, x_l) - 2 sum_i y_j,i dk_i(x_j) / dx_j,   y_j = sum_l Gbar_jl R^-1 k(X, x_l)
+ * Without dvalues the gradient work is skipped; the values are the same bits either way, and a batch's value and gradient do not
+ * depend on the other batches of the call.  A batch whose Sigma_b + jitter I is not positive definite gets NaN for its value and
+ * its gradient rows; *nbad (may be NULL) receives the number of such batches and the call still returns IBO_OK.
+ * IBO_E_BADARG for a NULL model, Xs, Z or values, B < 1, q outside [1, 32], S outside [1, 65536], d > 64, or jitter < 0 or NaN. */
+int ibo_qei(ibo_model* m, const double* Xs, long B, int q, const double* Z, int S,
+            double ymax, double xi, double jitter, double* values, double* dvalues, int* nbad);
+
 /* Candidates kept resident in HBM (the bench's device-resident leg; also used for sharded sets). */
 int ibo_cands_create(ibo_model* m, const double* Xs, long M, ibo_cands** out);
 int ibo_cands_destroy(ibo_cands* c);
