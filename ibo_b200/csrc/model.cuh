@@ -69,7 +69,7 @@ struct ibo_model {
     double* hServer = nullptr; unsigned long long* dSrvCount = nullptr; bool srvRunning = false; long long srvSeq = 0;
     int srvAcq = 0, srvFlags = 0, srvCtas = 0; double srvYmax = 0, srvParm = 0;
     std::map<long, std::pair<int*, int>> unitTables;              // K2 work tables (device), keyed by shape and group count
-    std::map<long, std::pair<int, int>> planCache;                // K2 launch plan (MT, G) per number of 32-candidate CTA tiles
+    std::map<std::pair<long, int>, std::pair<int, int>> planCache;   // K2 launch plan (MT, G) per (32-candidate CTA tiles, option narrow_mt)
     // profile of the last call
     double prof[6] = {0, 0, 0, 0, 0, 0};
     cudaEvent_t ev[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};

@@ -14,7 +14,7 @@ enum {
     OPT_K2_DEEP,         // -1 auto, 0 never, 1 always: deep-pipeline variant of the latency shapes
     OPT_PDL,             // programmatic dependent launch for small batches
     OPT_KSTAR_DIRECT,    // 1: K1 from direct differences instead of the DMMA expansion
-    OPT_DEBUG_PLAN,      // print the latency-shape plan
+    OPT_DEBUG_PLAN,      // print the latency-shape plan and the instance of every FP64 K2 launch
     OPT_TINY,            // -1 auto, 0 never, 1 force: fused small-model kernel
     OPT_DIRECT_TIMING,   // print the host/GPU split of a DIRECT query
     OPT_SHARD_MIN,       // sharded DIRECT: batches below this many points stay on every rank (0: 64 x ranks)

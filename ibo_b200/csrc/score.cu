@@ -96,6 +96,13 @@ __global__ void __launch_bounds__(256) kstar_kernel(const double* __restrict__ X
 // ---------------------------------------------------------------------------------------------
 constexpr double EXPAND_LIMIT = 256.0;    // => relative error of k below ~2e-13
 
+// dynamic shared memory of kstar_mma_kernel<DP4, *>: from DP4 = 6 (d > 20) on it is above the 48 KiB a launch gets without the opt-in
+template <int DP4> constexpr size_t kstar_mma_smem() {
+    constexpr int DP = 4 * DP4;
+    constexpr int S = (DP % 16 == 4 || DP % 16 == 12) ? DP : DP + 4;
+    return (2 * 128 * S + 256) * 8;
+}
+
 template <int DP4, int KC>   // DP4: number of 4-wide dimension groups, d <= 4*DP4; KC: kernel class (cov_r2_t)
 __global__ void __launch_bounds__(256) kstar_mma_kernel(const double* __restrict__ Xt, const double* __restrict__ cand_dev,
                                                         const double* __restrict__ inv_theta, const double* __restrict__ center,
@@ -642,9 +649,18 @@ static cudaError_t set_k2_attr() {
     }
     return e;
 }
+template <int DP4>
+static cudaError_t set_kstar_mma_attr() {
+    cudaError_t e = cudaFuncSetAttribute(kstar_mma_kernel<DP4, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kstar_mma_smem<DP4>());
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(kstar_mma_kernel<DP4, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kstar_mma_smem<DP4>());
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(kstar_mma_kernel<DP4, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kstar_mma_smem<DP4>());
+    if constexpr (DP4 > 1) { if (e == cudaSuccess) e = set_kstar_mma_attr<DP4 - 1>(); }
+    return e;
+}
 // dynamic shared-memory opt-ins of the scoring kernels; cudaFuncSetAttribute is per device (ensure_attrs runs this once per device)
 static cudaError_t set_score_attrs() {
-    cudaError_t e = set_k2_attr<4, 8>();
+    cudaError_t e = set_kstar_mma_attr<8>();
+    if (e == cudaSuccess) e = set_k2_attr<4, 8>();
     if (e == cudaSuccess) e = set_k2_attr<1, 8>();
     if (e == cudaSuccess) e = set_k2_attr<1, 4>();
     if (e == cudaSuccess) e = set_k2_attr<1, 2>();
@@ -744,12 +760,15 @@ static K2Plan plan_narrow(int nb, long ctaTiles, int g_num_sms) {
     return best;
 }
 
+// keyed on the forced shape too: option narrow_mt is a run-time switch and must take effect on a model that has already scored
+// a batch of this size
 static K2Plan plan_narrow_cached(ibo_model* m, long ctaTiles) {
-    auto it = m->planCache.find(ctaTiles);
+    const std::pair<long, int> key(ctaTiles, (int)get_option(OPT_NARROW_MT));
+    auto it = m->planCache.find(key);
     if (it == m->planCache.end()) {
         K2Plan pl = plan_narrow(m->nb, ctaTiles, dev_info(m->device).sms);
         if (get_option(OPT_DEBUG_PLAN)) fprintf(stderr, "[plan_narrow] nb=%d ctaTiles=%ld -> MT=%d G=%d (%ld CTAs)\n", m->nb, ctaTiles, pl.MT, pl.G, ctaTiles * pl.G);
-        it = m->planCache.emplace(ctaTiles, std::make_pair(pl.MT, pl.G)).first;
+        it = m->planCache.emplace(key, std::make_pair(pl.MT, pl.G)).first;
     }
     return K2Plan{it->second.first, it->second.second};
 }
@@ -799,9 +818,12 @@ static int deep_mode() { return (int)get_option(OPT_K2_DEEP); }
 template <int NT, int MT>
 static void launch_k2_shape(const ibo_model* m, bool p1, dim3 grid, const int* dUnits, const int* dStart, long Mpad, long Mvalid, cudaStream_t st) {
     const bool pdl = (NT == 1) && pdl_enabled();     // small batches only: the throughput shape must not sit on SMs K1 is using
+    const int dm = deep_mode();
+    const bool deep = NT == 1 && (dm == 1 || (dm < 0 && (long)grid.x * grid.y <= dev_info(m->device).sms));
+    if (get_option(OPT_DEBUG_PLAN))
+        fprintf(stderr, "[k2] nb=%d NT=%d MT=%d P1=%d DEEP=%d PDL=%d grid=%ux%u\n", m->nb, NT, MT, p1 ? 1 : 0, deep ? 1 : 0, pdl ? 1 : 0, grid.x, grid.y);
     if constexpr (NT == 1) {
-        const int dm = deep_mode();
-        if (dm == 1 || (dm < 0 && (long)grid.x * grid.y <= dev_info(m->device).sms)) {
+        if (deep) {
             if (p1) launch_ex(trigemm_kernel<NT, MT, true, NT == 1>, grid, dim3(K2_THREADS), K2Cfg<NT, MT, NT == 1>::SMEM, st, pdl,
                               m->dWpack, m->dSlab, m->dBetaY, m->dBeta1, m->dPart, dUnits, dStart, m->nb, Mpad, Mvalid);
             else launch_ex(trigemm_kernel<NT, MT, false, NT == 1>, grid, dim3(K2_THREADS), K2Cfg<NT, MT, NT == 1>::SMEM, st, pdl,
@@ -832,9 +854,7 @@ static int launch_trigemm(ibo_model* m, bool narrow, K2Plan pl, bool p1, long yt
 template <int DP4>
 static void launch_kstar_mma(dim3 grid, cudaStream_t st, const ibo_model* m, const double* dCand, double* slab, long M, long m0,
                              const CandInline& inl) {
-    constexpr int DP = 4 * DP4;
-    constexpr int S = (DP % 16 == 4 || DP % 16 == 12) ? DP : DP + 4;
-    const size_t smem = (2 * 128 * S + 256) * 8;
+    const size_t smem = kstar_mma_smem<DP4>();
     if (m->kind <= IBO_KERNEL_SE_ISO)
         kstar_mma_kernel<DP4, 0><<<grid, 256, smem, st>>>(m->dXt, dCand, m->dInvTheta, m->dCenter, slab, m->N, m->d, m->nb, M, m0, m->kind, m->sf2, inl);
     else if (m->kind == IBO_KERNEL_MATERN3)

@@ -49,7 +49,9 @@ extern "C" {
 /* flag word of the scoring entry points */
 #define IBO_FLAG_MODE_CPP      0x0  /* libm erf, exact constants, sigma^2 floor 1e-8  (cpp/optimizeGP.cpp:150-215) */
 #define IBO_FLAG_MODE_PY       0x1  /* Chebyshev erf, 0.707106/0.398942, floor 10e-8  (gaussianprocess/__init__.py:55-77,224) */
-#define IBO_FLAG_KSTAR_EXPAND  0x2  /* cross-covariance through |x|^2+|y|^2-2x.y on the DMMA pipe (default: direct differences) */
+#define IBO_FLAG_KSTAR_EXPAND  0x2  /* no effect, value kept for ABI compatibility: the cross-covariance of the FP64 kernels always goes
+                                       through |x|^2+|y|^2-2x.y on the DMMA pipe for d <= 32 (pairs with large scaled norms are
+                                       recomputed from direct differences); option "kstar_direct" = 1 selects direct differences */
 #define IBO_FLAG_DIRECT_SEQ    0x4  /* DIRECT: evaluate rectangle by rectangle in the reference's call order */
 #define IBO_FLAG_PROFILE       0x8  /* record per-kernel CUDA-event times (ibo_get_profile) */
 #define IBO_FLAG_SHARD         0x20 /* ibo_acqmax: cut every DIRECT batch into one slice per rank of the communicator
@@ -271,7 +273,8 @@ int ibo_debug_exp(int device, const double* x, long n, double* out_fast, double*
  *   chunk_tiles (0)   128-candidate tiles per chunk (0: 2 x number of SMs)
  *   narrow_max (2048) batches up to this size use the latency shapes of the FP64 GEMM
  *   narrow_mt (0), k2_deep (-1), pdl (1), kstar_direct (0), tiny (-1)   shape / launch switches of the small-batch path
- *   debug_plan (0), direct_timing (0)   diagnostics on stderr
+ *   debug_plan (0), direct_timing (0)   diagnostics on stderr (debug_plan: each new latency-shape plan, "[plan_narrow] ...",
+ *                     and the instance of every FP64 GEMM launch, "[k2] ... MT=.. P1=.. DEEP=..")
  *   shard_min (0)     sharded DIRECT: batches below this many points are not sharded (0: 64 x ranks)
  *   tiny_server (1)   DIRECT on a model of <= 128 observations: the fused kernel stays resident for the query and takes its batches
  *                     from a mailbox in mapped host memory (0: one launch per batch)
