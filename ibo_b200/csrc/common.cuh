@@ -30,6 +30,9 @@ __host__ __device__ inline int blob_offset(int r, int k) {
 // first blob of row-block i in the packed W array (row-block i owns (i+1)*8 blobs)
 __host__ __device__ inline size_t wpack_base(int i) { return (size_t)KB_PER_BLOCK * ((size_t)i * (i + 1) / 2); }
 
+// x rounded up to whole 128-wide tiles
+inline long round128(long x) { return (x + 127) / 128 * 128; }
+
 // ---------------------------------------------------------------------------------------------
 // error handling
 // ---------------------------------------------------------------------------------------------

@@ -17,22 +17,8 @@
 
 namespace ibo {
 
-// Workspace of the gradient entry points, kept with the model that owns the call and grown on demand.
-struct GradWork {
-    double* dRaw = nullptr;    size_t rawCap = 0;     // candidates as given [M][d]
-    double* dVals = nullptr;   size_t valsCap = 0;    // [score | mu | s2] of the scoring path, 3 M + 2
-    double* dG = nullptr;      size_t gCap = 0;       // three [M][d] planes: sums with z, a, b -> ds2, dmu, dscore in place
-    double* dKb = nullptr;     size_t kbCap = 0;      // k^T b [M] (prior only)
-    double* dScaled = nullptr; size_t scaledCap = 0;  // chunk scaled like g's training inputs [Mcp][d]
-    double* dScaledM = nullptr; size_t scaledMCap = 0;// chunk scaled like the model's (variance model attached) [Mcp][d]
-    double* dKc = nullptr;     size_t kcCap = 0;      // K*, then Z [Np][Mcp]
-    double* dV = nullptr;      size_t vCap = 0;       // V [Np][Mcp]
-    double* dAB = nullptr;     size_t abCap = 0;      // a | b [2][Np]
-};
-
 namespace {
 
-constexpr int GRAD_MAX_D = 64;
 constexpr int RC = 32;    // candidates per CTA (lane = candidate)
 constexpr int RW = 8;     // warps per CTA: warp w takes the training points i = w, w + 8, ...
 constexpr int RDS = 16;   // dimensions per CTA (grid.y slices d)
@@ -161,9 +147,6 @@ __global__ void __launch_bounds__(256) grad_epilogue_kernel(GradEpi P) {
     }
 }
 
-}  // namespace
-
-// launch wrappers, also for qei.cu
 template <bool DZ, bool DA, bool DB>
 void launch_reduce(const ibo_model* src, const double* Cs, int Mc, const double* Z, int ldz, const double* a, const double* b,
                    double* G, size_t plane, double* kb, cudaStream_t st) {
@@ -172,16 +155,31 @@ void launch_reduce(const ibo_model* src, const double* Cs, int Mc, const double*
                                                           a, b, G, plane, kb);
     g_launches++;
 }
-template void launch_reduce<true, false, false>(const ibo_model*, const double*, int, const double*, int, const double*, const double*,
-                                                double*, size_t, double*, cudaStream_t);
-template void launch_reduce<false, true, false>(const ibo_model*, const double*, int, const double*, int, const double*, const double*,
-                                                double*, size_t, double*, cudaStream_t);
-template void launch_reduce<false, true, true>(const ibo_model*, const double*, int, const double*, int, const double*, const double*,
-                                               double*, size_t, double*, cudaStream_t);
-template void launch_reduce<true, true, false>(const ibo_model*, const double*, int, const double*, int, const double*, const double*,
-                                               double*, size_t, double*, cudaStream_t);
-template void launch_reduce<true, true, true>(const ibo_model*, const double*, int, const double*, int, const double*, const double*,
-                                              double*, size_t, double*, cudaStream_t);
+
+}  // namespace
+
+long cand_chunk(const ibo_model* g) { return std::max(128L, (long)((512L << 20) / (2L * 8 * g->Np)) / 128 * 128); }
+
+double* launch_ab(const ibo_model* m, double* ab, cudaStream_t st) {
+    launch_tri_matvec_t(m->dW, m->dBetaY, ab, m->N, m->Np, st);
+    if (m->npb == 0) return nullptr;
+    launch_tri_matvec_t(m->dW, m->dBeta1, ab + m->Np, m->N, m->Np, st);
+    return ab + m->Np;
+}
+
+// with a variance model the weights of s2 and those of mu run over different training points: two launches
+void launch_grad_sums(const ibo_model* m, const double* Cs, const double* Cm, int Mc, const double* Zw, int ldz, const double* a,
+                      const double* b, double* G, size_t plane, double* kb, cudaStream_t st) {
+    if (const ibo_model* vm = m->var_model) {
+        launch_reduce<true, false, false>(vm, Cs, Mc, Zw, ldz, nullptr, nullptr, G, plane, nullptr, st);
+        if (b) launch_reduce<false, true, true>(m, Cm, Mc, nullptr, 0, a, b, G, plane, kb, st);
+        else launch_reduce<false, true, false>(m, Cm, Mc, nullptr, 0, a, nullptr, G, plane, nullptr, st);
+    } else if (b) {
+        launch_reduce<true, true, true>(m, Cs, Mc, Zw, ldz, a, b, G, plane, kb, st);
+    } else {
+        launch_reduce<true, true, false>(m, Cs, Mc, Zw, ldz, a, nullptr, G, plane, nullptr, st);
+    }
+}
 
 void launch_grad_prior(const ibo_model* m, const double* cand, long M, const double* kb, double* G, cudaStream_t st) {
     GradEpi P{};
@@ -195,69 +193,48 @@ void launch_grad_prior(const ibo_model* m, const double* cand, long M, const dou
 
 namespace {
 
-inline long round128(long x) { return (x + 127) / 128 * 128; }
-
-// every scalar check comes before the model is read
-int check_args(const ibo_model* m, const double* Xs, long M, int flags, bool extra_ok) {
-    if (!m || !Xs || M < 1 || (flags & ~IBO_FLAG_MODE_PY) != 0 || !extra_ok) { set_error("bad argument"); return IBO_E_BADARG; }
-    if (m->d > GRAD_MAX_D) { set_error("d > 64 not supported"); return IBO_E_BADARG; }
-    return IBO_OK;
-}
-
-// Enqueues everything on m->stream and leaves [score | mu | s2] in w->dVals and ds2, dmu, dscore ([M][d] each) in w->dG.
+// Enqueues everything on m->stream and leaves [score | mu | s2] in w->dPost and ds2, dmu, dscore ([M][d] each) in w->dG.
 int grad_device(ibo_model* m, const double* Xs, long M, int acq, double ymax, double parm, int flags, bool wantGrad) {
-    if (!m->grad) m->grad = new GradWork();
-    GradWork* w = m->grad;
+    int rc;
+    if ((rc = ensure_joint_attrs(m->device))) return rc;
+    CandWork* w = cand_work(m);
     ibo_model* vm = m->var_model;
     ibo_model* g = vm ? vm : m;                          // the model sigma^2 comes from
     cudaStream_t st = m->stream;
     const int d = m->d;
     const bool prior = m->npb > 0;
-    // chunk: the largest multiple of 128 candidates whose K* / Z and V (2 Np doubles per candidate) fit in 512 MiB
-    const long chunk = std::max(128L, (long)((512L << 20) / (2L * 8 * g->Np)) / 128 * 128);
-    const long Mcap = round128(std::min(M, chunk));
-    int rc;
+    const long chunk = cand_chunk(g), Mcap = round128(std::min(M, chunk));
     if ((rc = grow(&w->dRaw, &w->rawCap, (size_t)M * d))) return rc;
-    if ((rc = grow(&w->dVals, &w->valsCap, (size_t)3 * M + 2))) return rc;
+    if ((rc = grow(&w->dPost, &w->postCap, (size_t)3 * M + 2))) return rc;
+    if (wantGrad) {
+        if ((rc = grow(&w->dG, &w->gCap, (size_t)3 * M * d))) return rc;
+        if (prior && (rc = grow(&w->dKb, &w->kbCap, (size_t)M))) return rc;
+        if ((rc = grow(&w->dScaled, &w->scaledCap, (size_t)Mcap * d))) return rc;
+        if (vm && (rc = grow(&w->dScaledM, &w->scaledMCap, (size_t)Mcap * d))) return rc;
+        if ((rc = grow(&w->dKc, &w->kcCap, (size_t)g->Np * Mcap))) return rc;
+        if ((rc = grow(&w->dV, &w->vCap, (size_t)g->Np * Mcap))) return rc;
+        if ((rc = grow(&w->dAB, &w->abCap, (size_t)2 * m->Np))) return rc;
+    }
     IBO_CUDA_TRY(cudaMemcpyAsync(w->dRaw, Xs, sizeof(double) * (size_t)M * d, cudaMemcpyHostToDevice, st));
-    if ((rc = posterior_score_device(m, w->dRaw, M, acq, ymax, parm, IBO_FLAG_FP64 | flags, w->dVals))) return rc;
+    if ((rc = posterior_score_device(m, w->dRaw, M, acq, ymax, parm, IBO_FLAG_FP64 | flags, w->dPost))) return rc;
     if (!wantGrad) return IBO_OK;
-    if ((rc = grow(&w->dG, &w->gCap, (size_t)3 * M * d))) return rc;
-    if (prior && (rc = grow(&w->dKb, &w->kbCap, (size_t)M))) return rc;
-    if ((rc = grow(&w->dScaled, &w->scaledCap, (size_t)Mcap * d))) return rc;
-    if (vm && (rc = grow(&w->dScaledM, &w->scaledMCap, (size_t)Mcap * d))) return rc;
-    if ((rc = grow(&w->dKc, &w->kcCap, (size_t)g->Np * Mcap))) return rc;
-    if ((rc = grow(&w->dV, &w->vCap, (size_t)g->Np * Mcap))) return rc;
-    if ((rc = grow(&w->dAB, &w->abCap, (size_t)2 * m->Np))) return rc;
-    // a = W^T (W Y), b = W^T (W 1) of the model, recomputed every call (an appended model needs no invalidation)
     double* const dA = w->dAB;
-    double* const dB = prior ? w->dAB + m->Np : nullptr;
-    launch_tri_matvec_t(m->dW, m->dBetaY, dA, m->N, m->Np, st);
-    if (prior) launch_tri_matvec_t(m->dW, m->dBeta1, dB, m->N, m->Np, st);
+    double* const dB = launch_ab(m, w->dAB, st);
     const size_t plane = (size_t)M * d;
     for (long c0 = 0; c0 < M; c0 += chunk) {
         const int Mc = (int)std::min(chunk, M - c0), Mcp = (int)round128(Mc);
         const double* raw = w->dRaw + (size_t)c0 * d;
-        double* G = w->dG + (size_t)c0 * d;
-        double* kb = prior ? w->dKb + c0 : nullptr;
         launch_scale_cands(w->dScaled, raw, g, Mc, Mcp, st);
         launch_cross_cov(w->dKc, g, w->dScaled, Mc, Mcp, st);
-        if ((rc = launch_w_gemm_v(w->dV, g, w->dKc, Mcp, st)) || (rc = launch_w_gemm_z(w->dKc, g, w->dV, Mcp, st))) return rc;
-        if (vm) {
-            launch_reduce<true, false, false>(g, w->dScaled, Mc, w->dKc, Mcp, nullptr, nullptr, G, plane, nullptr, st);
-            launch_scale_cands(w->dScaledM, raw, m, Mc, Mcp, st);
-            if (prior) launch_reduce<false, true, true>(m, w->dScaledM, Mc, nullptr, 0, dA, dB, G, plane, kb, st);
-            else launch_reduce<false, true, false>(m, w->dScaledM, Mc, nullptr, 0, dA, nullptr, G, plane, nullptr, st);
-        } else if (prior) {
-            launch_reduce<true, true, true>(m, w->dScaled, Mc, w->dKc, Mcp, dA, dB, G, plane, kb, st);
-        } else {
-            launch_reduce<true, true, false>(m, w->dScaled, Mc, w->dKc, Mcp, dA, nullptr, G, plane, nullptr, st);
-        }
+        launch_w_gemm_v(w->dV, g, w->dKc, Mcp, st);
+        launch_w_gemm_z(w->dKc, g, w->dV, Mcp, st);
+        if (vm) launch_scale_cands(w->dScaledM, raw, m, Mc, Mcp, st);
+        launch_grad_sums(m, w->dScaled, w->dScaledM, Mc, w->dKc, Mcp, dA, dB, w->dG + (size_t)c0 * d, plane, prior ? w->dKb + c0 : nullptr, st);
     }
     GradEpi P{};
     P.M = M; P.d = d; P.acq = acq; P.mode_py = (flags & IBO_FLAG_MODE_PY) ? 1 : 0; P.npb = m->npb;
     P.ymax = ymax; P.parm = parm;
-    P.vals = w->dVals;
+    P.vals = w->dPost;
     P.G = w->dG;
     if (prior) launch_grad_prior(m, w->dRaw, M, w->dKb, w->dG, st);
     grad_epilogue_kernel<<<(unsigned)((M + 255) / 256), 256, 0, st>>>(P);
@@ -273,28 +250,19 @@ int copy_out(double* dst, const double* src, size_t n, cudaStream_t st) {
 
 }  // namespace
 
-void free_grad(ibo_model* m) {
-    GradWork* w = m->grad;
-    if (!w) return;
-    double** ptrs[] = {&w->dRaw, &w->dVals, &w->dG, &w->dKb, &w->dScaled, &w->dScaledM, &w->dKc, &w->dV, &w->dAB};
-    for (auto p : ptrs) if (*p) pool_free(*p);
-    delete w;
-    m->grad = nullptr;
-}
-
 }  // namespace ibo
 
 using namespace ibo;
 
 extern "C" int ibo_posterior_grad(ibo_model* m, const double* Xs, long M, int flags, double* mu, double* s2, double* dmu, double* ds2) {
-    int rc = check_args(m, Xs, M, flags, true);
+    int rc = check_cands(m, Xs, M, (flags & ~IBO_FLAG_MODE_PY) == 0);
     if (rc) return rc;
     IBO_CUDA_TRY(cudaSetDevice(m->device));
     if ((rc = grad_device(m, Xs, M, -1, 0.0, 0.0, flags, dmu || ds2))) return rc;
-    GradWork* w = m->grad;
+    CandWork* w = m->cand;
     cudaStream_t st = m->stream;
     const size_t plane = (size_t)M * m->d;
-    if ((rc = copy_out(mu, w->dVals + M, M, st)) || (rc = copy_out(s2, w->dVals + 2 * M, M, st)) ||
+    if ((rc = copy_out(mu, w->dPost + M, M, st)) || (rc = copy_out(s2, w->dPost + 2 * M, M, st)) ||
         (rc = copy_out(ds2, w->dG, plane, st)) || (rc = copy_out(dmu, w->dG + plane, plane, st)))
         return rc;
     IBO_CUDA_TRY(cudaStreamSynchronize(st));
@@ -304,13 +272,13 @@ extern "C" int ibo_posterior_grad(ibo_model* m, const double* Xs, long M, int fl
 
 extern "C" int ibo_score_grad(ibo_model* m, const double* Xs, long M, int acq, double ymax, double parm, int flags,
                               double* scores, double* dscores) {
-    int rc = check_args(m, Xs, M, flags, acq >= 0 && acq <= 2);
+    int rc = check_cands(m, Xs, M, (flags & ~IBO_FLAG_MODE_PY) == 0 && acq >= 0 && acq <= 2);
     if (rc) return rc;
     IBO_CUDA_TRY(cudaSetDevice(m->device));
     if ((rc = grad_device(m, Xs, M, acq, ymax, parm, flags, dscores != nullptr))) return rc;
-    GradWork* w = m->grad;
+    CandWork* w = m->cand;
     cudaStream_t st = m->stream;
-    if ((rc = copy_out(scores, w->dVals, M, st)) || (rc = copy_out(dscores, w->dG + 2 * (size_t)M * m->d, (size_t)M * m->d, st))) return rc;
+    if ((rc = copy_out(scores, w->dPost, M, st)) || (rc = copy_out(dscores, w->dG + 2 * (size_t)M * m->d, (size_t)M * m->d, st))) return rc;
     IBO_CUDA_TRY(cudaStreamSynchronize(st));
     IBO_CUDA_TRY(cudaGetLastError());
     return IBO_OK;

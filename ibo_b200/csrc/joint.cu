@@ -9,7 +9,7 @@
 // library's sigma^2 before clipping.  With a variance model attached (PrefGaussianProcess.addObservationPoint) Sigma comes
 // from that model's X and W, as sigma^2 does; mu always comes from the scoring path (score.cu) on the FP64 kernels.
 // Both GEMMs and the Cholesky of Sigma run on the FP64 tensor pipe (tile_gemm_core, launch_factorize).
-// The candidate scaling, R(X, X*) and the two W GEMMs are also what grad.cu builds the gradient of sigma^2 from.
+// The candidate scaling, R(X, X*) and the two W GEMMs are launched through wrappers that grad.cu and qei.cu use as well.
 #include "model.cuh"
 #include "scoremath.cuh"
 #include "tilegemm.cuh"
@@ -20,20 +20,6 @@
 namespace ibo {
 
 constexpr long JOINT_MAX_M = 16384;
-
-// Workspace of the joint entry points, kept with the model that owns the call and grown on demand.
-struct JointWork {
-    ibo_model chol;               // Sigma in chol.dA (Mp x Mp), factorised in place; its streams and events are the owner's
-    size_t aCap = 0, dCap = 0;    // chol.dA, chol.dD
-    double* dRaw = nullptr;    size_t rawCap = 0;     // candidates as given [M][d]
-    double* dScaled = nullptr; size_t scaledCap = 0;  // candidates scaled and centred like the training inputs, [Mp][d]
-    double* dKc = nullptr;     size_t kcCap = 0;      // R(X, X*) [Np][Mp]
-    double* dV = nullptr;      size_t vCap = 0;       // V = W R(X, X*) [Np][Mp]
-    double* dMu = nullptr;     size_t muCap = 0;      // [score | mu | s2] of the scoring path, mu at M
-    double* dZ = nullptr;      size_t zCap = 0;       // standard normals [Mp][Sp], zero padded
-    double* dF = nullptr;      size_t fCap = 0;       // samples [Mp][Sp]
-    double* dArg = nullptr;    size_t argCap = 0;     // per-sample argmax (long long)
-};
 
 namespace {
 
@@ -200,67 +186,62 @@ cudaError_t set_joint_attrs() {
     return e;
 }
 
-inline long round128(long x) { return (x + 127) / 128 * 128; }
-
-// Enqueues on m->stream: the candidates Xs (host, M x d) to the device, mu of the scoring path into w->dMu + M (when wantMu),
-// and Sigma + jitter I (lower tiles) into w->chol.dA.
-int joint_sigma(ibo_model* m, const double* Xs, long M, double jitter, bool wantMu) {
-    cudaError_t ae = ensure_attrs(m->device, ATTR_JOINT, set_joint_attrs);
-    if (ae != cudaSuccess) { set_error(std::string("cudaFuncSetAttribute: ") + cudaGetErrorString(ae)); return IBO_E_CUDA; }
-    if (!m->joint) {
-        m->joint = new JointWork();
-        ibo_model& c = m->joint->chol;
+// Enqueues on m->stream: the candidates Xs (host, M x d) to the device, mu of the scoring path into w->dPost + M (when wantMu),
+// and Sigma + jitter I (lower tiles) into w->chol.dA.  S > 0: also grows the buffers of S samples.
+int joint_sigma(ibo_model* m, const double* Xs, long M, double jitter, bool wantMu, int S) {
+    int rc;
+    if ((rc = ensure_joint_attrs(m->device))) return rc;
+    CandWork* w = cand_work(m);
+    ibo_model& c = w->chol;
+    if (!c.dInfo) {
         c.device = m->device;
         c.stream = m->stream; c.stream2 = m->stream2; c.stream3 = m->stream3; c.stream4 = m->stream4;
         c.evStep = m->evStep; c.evRest = m->evRest; c.evScale = m->evScale; c.evFar = m->evFar;
         IBO_CUDA_TRY(cudaMalloc(&c.dInfo, sizeof(int)));
     }
-    JointWork* w = m->joint;
     ibo_model* g = m->var_model ? m->var_model : m;      // the model sigma^2 comes from
     cudaStream_t st = m->stream;
     const int d = m->d, Np = g->Np, Mp = (int)round128(M), nbM = Mp / 128;
-    int rc;
+    const size_t Sp = (size_t)round128(S);
     if ((rc = grow(&w->dRaw, &w->rawCap, (size_t)M * d))) return rc;
     if ((rc = grow(&w->dScaled, &w->scaledCap, (size_t)Mp * d))) return rc;
     if ((rc = grow(&w->dKc, &w->kcCap, (size_t)Np * Mp))) return rc;
     if ((rc = grow(&w->dV, &w->vCap, (size_t)Np * Mp))) return rc;
-    if ((rc = grow(&w->dMu, &w->muCap, (size_t)3 * M + 2))) return rc;
-    if ((rc = grow(&w->chol.dA, &w->aCap, (size_t)Mp * Mp))) return rc;
-    if ((rc = grow(&w->chol.dD, &w->dCap, (size_t)nbM * 128 * 128))) return rc;
-    w->chol.N = (int)M; w->chol.Np = Mp; w->chol.nb = nbM; w->chol.d = d;
+    if ((rc = grow(&w->dPost, &w->postCap, (size_t)3 * M + 2))) return rc;
+    if ((rc = grow(&c.dA, &w->cholACap, (size_t)Mp * Mp))) return rc;
+    if ((rc = grow(&c.dD, &w->cholDCap, (size_t)nbM * 128 * 128))) return rc;
+    if (S > 0) {
+        if ((rc = grow(&w->dNormals, &w->normalsCap, (size_t)Mp * Sp))) return rc;
+        if ((rc = grow(&w->dF, &w->fCap, (size_t)Mp * Sp))) return rc;
+        if ((rc = grow(&w->dArg, &w->argCap, (size_t)S))) return rc;
+    }
+    c.N = (int)M; c.Np = Mp; c.nb = nbM; c.d = d;
     IBO_CUDA_TRY(cudaMemcpyAsync(w->dRaw, Xs, sizeof(double) * (size_t)M * d, cudaMemcpyHostToDevice, st));
-    if (wantMu && (rc = posterior_mean_device(m, w->dRaw, M, w->dMu))) return rc;
-    const long ns = (long)Mp * d;
-    scale_cands_kernel<<<(unsigned)((ns + 255) / 256), 256, 0, st>>>(w->dScaled, w->dRaw, g->dInvTheta, g->dCenter, M, Mp, d);
-    cross_cov_kernel<<<dim3((Mp + 255) / 256, Np), 256, 0, st>>>(w->dKc, g->dXt, w->dScaled, g->N, (int)M, Mp, d, g->kind, g->sf2);
-    trimm_kernel<<<dim3(nbM, g->nb), 256, TILE_SMEM_DOUBLES * 8, st>>>(w->dV, Mp, g->dW, Np, w->dKc, Mp, g->nb, nullptr, 0);
-    prior_cov_kernel<<<dim3((Mp + 255) / 256, Mp), 256, 0, st>>>(w->chol.dA, w->dScaled, (int)M, Mp, d, g->kind, g->sf2, 1.0 + g->noise);
-    sigma_kernel<<<dim3(nbM, nbM), 256, TILE_SMEM_DOUBLES * 8, st>>>(w->chol.dA, w->dV, Mp, Np, (int)M, jitter);
-    g_launches += 5;
+    if (wantMu && (rc = posterior_score_device(m, w->dRaw, M, -1, 0.0, 0.0, IBO_FLAG_FP64, w->dPost))) return rc;
+    launch_scale_cands(w->dScaled, w->dRaw, g, M, Mp, st);
+    launch_cross_cov(w->dKc, g, w->dScaled, (int)M, Mp, st);
+    launch_w_gemm_v(w->dV, g, w->dKc, Mp, st);
+    prior_cov_kernel<<<dim3((Mp + 255) / 256, Mp), 256, 0, st>>>(c.dA, w->dScaled, (int)M, Mp, d, g->kind, g->sf2, 1.0 + g->noise);
+    sigma_kernel<<<dim3(nbM, nbM), 256, TILE_SMEM_DOUBLES * 8, st>>>(c.dA, w->dV, Mp, Np, (int)M, jitter);
+    g_launches += 2;
     IBO_CUDA_TRY(cudaGetLastError());
-    return IBO_OK;
-}
-
-// every scalar check comes before the model is read
-int check_args(const ibo_model* m, const double* Xs, long M, bool extra_ok) {
-    if (!m || !Xs || M < 1 || M > JOINT_MAX_M || !extra_ok) { set_error("bad argument"); return IBO_E_BADARG; }
-    if (m->d > 64) { set_error("d > 64 not supported"); return IBO_E_BADARG; }
     return IBO_OK;
 }
 
 }  // namespace
 
-void free_joint(ibo_model* m) {
-    JointWork* w = m->joint;
-    if (!w) return;
-    double** ptrs[] = {&w->chol.dA, &w->chol.dD, &w->dRaw, &w->dScaled, &w->dKc, &w->dV, &w->dMu, &w->dZ, &w->dF, &w->dArg};
-    for (auto p : ptrs) if (*p) pool_free(*p);
-    if (w->chol.dInfo) cudaFree(w->chol.dInfo);
-    delete w;
-    m->joint = nullptr;
+int check_cands(const ibo_model* m, const double* Xs, long M, bool extra_ok) {
+    if (!m || !Xs || M < 1 || !extra_ok) { set_error("bad argument"); return IBO_E_BADARG; }
+    if (m->d > 64) { set_error("d > 64 not supported"); return IBO_E_BADARG; }
+    return IBO_OK;
 }
 
-// launch wrappers for grad.cu and qei.cu
+int ensure_joint_attrs(int device) {
+    cudaError_t ae = ensure_attrs(device, ATTR_JOINT, set_joint_attrs);
+    if (ae != cudaSuccess) { set_error(std::string("cudaFuncSetAttribute: ") + cudaGetErrorString(ae)); return IBO_E_CUDA; }
+    return IBO_OK;
+}
+
 void launch_scale_cands(double* Cs, const double* X, const ibo_model* g, long M, long Mp, cudaStream_t st) {
     scale_cands_kernel<<<(unsigned)((Mp * g->d + 255) / 256), 256, 0, st>>>(Cs, X, g->dInvTheta, g->dCenter, M, Mp, g->d);
     g_launches++;
@@ -269,19 +250,13 @@ void launch_cross_cov(double* Kc, const ibo_model* g, const double* Cs, int M, i
     cross_cov_kernel<<<dim3((Mp + 255) / 256, g->Np), 256, 0, st>>>(Kc, g->dXt, Cs, g->N, M, Mp, g->d, g->kind, g->sf2);
     g_launches++;
 }
-int launch_w_gemm_v(double* V, const ibo_model* g, const double* Kc, int Mp, cudaStream_t st) {
-    cudaError_t ae = ensure_attrs(g->device, ATTR_JOINT, set_joint_attrs);
-    if (ae != cudaSuccess) { set_error(std::string("cudaFuncSetAttribute: ") + cudaGetErrorString(ae)); return IBO_E_CUDA; }
+void launch_w_gemm_v(double* V, const ibo_model* g, const double* Kc, int Mp, cudaStream_t st) {
     trimm_kernel<<<dim3(Mp / 128, g->nb), 256, TILE_SMEM_DOUBLES * 8, st>>>(V, Mp, g->dW, g->Np, Kc, Mp, g->nb, nullptr, 0);
     g_launches++;
-    return IBO_OK;
 }
-int launch_w_gemm_z(double* Z, const ibo_model* g, const double* V, int Mp, cudaStream_t st) {
-    cudaError_t ae = ensure_attrs(g->device, ATTR_JOINT, set_joint_attrs);
-    if (ae != cudaSuccess) { set_error(std::string("cudaFuncSetAttribute: ") + cudaGetErrorString(ae)); return IBO_E_CUDA; }
+void launch_w_gemm_z(double* Z, const ibo_model* g, const double* V, int Mp, cudaStream_t st) {
     trimm_t_kernel<<<dim3(Mp / 128, g->nb), 256, TILE_SMEM_DOUBLES * 8, st>>>(Z, Mp, g->dW, g->Np, V, Mp, g->nb);
     g_launches++;
-    return IBO_OK;
 }
 
 }  // namespace ibo
@@ -289,14 +264,14 @@ int launch_w_gemm_z(double* Z, const ibo_model* g, const double* V, int Mp, cuda
 using namespace ibo;
 
 extern "C" int ibo_posterior_cov(ibo_model* m, const double* Xs, long M, double* mu, double* cov) {
-    int rc = check_args(m, Xs, M, cov != nullptr);
+    int rc = check_cands(m, Xs, M, M <= JOINT_MAX_M && cov != nullptr);
     if (rc) return rc;
     IBO_CUDA_TRY(cudaSetDevice(m->device));
-    if ((rc = joint_sigma(m, Xs, M, 0.0, mu != nullptr))) return rc;
-    JointWork* w = m->joint;
+    if ((rc = joint_sigma(m, Xs, M, 0.0, mu != nullptr, 0))) return rc;
+    CandWork* w = m->cand;
     cudaStream_t st = m->stream;
     const size_t Mp = (size_t)round128(M);
-    if (mu) IBO_CUDA_TRY(cudaMemcpyAsync(mu, w->dMu + M, sizeof(double) * M, cudaMemcpyDeviceToHost, st));
+    if (mu) IBO_CUDA_TRY(cudaMemcpyAsync(mu, w->dPost + M, sizeof(double) * M, cudaMemcpyDeviceToHost, st));
     IBO_CUDA_TRY(cudaMemcpy2DAsync(cov, sizeof(double) * M, w->chol.dA, sizeof(double) * Mp, sizeof(double) * M, M, cudaMemcpyDeviceToHost, st));
     IBO_CUDA_TRY(cudaStreamSynchronize(st));
     IBO_CUDA_TRY(cudaGetLastError());
@@ -313,11 +288,11 @@ extern "C" int ibo_posterior_cov(ibo_model* m, const double* Xs, long M, double*
 extern "C" int ibo_posterior_sample(ibo_model* m, const double* Xs, long M, const double* Z, int S, double jitter,
                                     double* F, long* argmax, int* info) {
     if (info) *info = 0;
-    int rc = check_args(m, Xs, M, Z && S >= 1 && jitter >= 0.0);      // NaN jitter fails the comparison
+    int rc = check_cands(m, Xs, M, M <= JOINT_MAX_M && Z && S >= 1 && jitter >= 0.0);      // NaN jitter fails the comparison
     if (rc) return rc;
     IBO_CUDA_TRY(cudaSetDevice(m->device));
-    if ((rc = joint_sigma(m, Xs, M, jitter, true))) return rc;
-    JointWork* w = m->joint;
+    if ((rc = joint_sigma(m, Xs, M, jitter, true, S))) return rc;
+    CandWork* w = m->cand;
     cudaStream_t st = m->stream;
     const int Mp = (int)round128(M), nbM = Mp / 128, Sp = (int)round128(S);
     if ((rc = launch_factorize(&w->chol, false, false, false))) return rc;
@@ -329,13 +304,10 @@ extern "C" int ibo_posterior_sample(ibo_model* m, const double* Xs, long M, cons
         set_error("posterior covariance + jitter I is not positive definite (pivot " + std::to_string(hinfo) + ")");
         return IBO_E_NOTSPD;
     }
-    if ((rc = grow(&w->dZ, &w->zCap, (size_t)Mp * Sp))) return rc;
-    if ((rc = grow(&w->dF, &w->fCap, (size_t)Mp * Sp))) return rc;
-    if ((rc = grow(&w->dArg, &w->argCap, (size_t)S))) return rc;
     zero_diag_upper_kernel<<<nbM, 256, 0, st>>>(w->chol.dA, Mp);
-    IBO_CUDA_TRY(cudaMemsetAsync(w->dZ, 0, sizeof(double) * (size_t)Mp * Sp, st));
-    IBO_CUDA_TRY(cudaMemcpy2DAsync(w->dZ, sizeof(double) * Sp, Z, sizeof(double) * S, sizeof(double) * S, M, cudaMemcpyHostToDevice, st));
-    trimm_kernel<<<dim3(Sp / 128, nbM), 256, TILE_SMEM_DOUBLES * 8, st>>>(w->dF, Sp, w->chol.dA, Mp, w->dZ, Sp, nbM, w->dMu + M, (int)M);
+    IBO_CUDA_TRY(cudaMemsetAsync(w->dNormals, 0, sizeof(double) * (size_t)Mp * Sp, st));
+    IBO_CUDA_TRY(cudaMemcpy2DAsync(w->dNormals, sizeof(double) * Sp, Z, sizeof(double) * S, sizeof(double) * S, M, cudaMemcpyHostToDevice, st));
+    trimm_kernel<<<dim3(Sp / 128, nbM), 256, TILE_SMEM_DOUBLES * 8, st>>>(w->dF, Sp, w->chol.dA, Mp, w->dNormals, Sp, nbM, w->dPost + M, (int)M);
     g_launches += 2;
     long long* dArg = reinterpret_cast<long long*>(w->dArg);
     std::vector<long long> harg(argmax ? S : 0);

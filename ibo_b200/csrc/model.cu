@@ -957,6 +957,22 @@ static std::set<ibo_model*> g_live;
 
 static void register_model(ibo_model* m) { std::lock_guard<std::mutex> lk(g_live_mu); g_live.insert(m); }
 
+CandWork* ibo::cand_work(ibo_model* m) {
+    if (!m->cand) m->cand = new CandWork();
+    return m->cand;
+}
+
+static void free_cand_work(ibo_model* m) {
+    CandWork* w = m->cand;
+    if (!w) return;
+    double** ptrs[] = {&w->dRaw, &w->dScaled, &w->dScaledM, &w->dKc, &w->dV, &w->dAB, &w->dKb, &w->dG, &w->dNormals, &w->dPost,
+                       &w->chol.dA, &w->chol.dD, &w->dF, &w->dArg, &w->dQei, &w->dMubar, &w->dSig, &w->dGbar};
+    for (auto p : ptrs) if (*p) pool_free(*p);
+    if (w->chol.dInfo) cudaFree(w->chol.dInfo);
+    delete w;
+    m->cand = nullptr;
+}
+
 static void free_model(ibo_model* m) {
     if (!m) return;
     {
@@ -972,9 +988,7 @@ static void free_model(ibo_model* m) {
     if (m->stream3) cudaStreamSynchronize(m->stream3);
     if (m->stream4) cudaStreamSynchronize(m->stream4);
     if (m->stream) cudaStreamSynchronize(m->stream);   // blocks go back to the pool: nothing may still be using them
-    free_joint(m);
-    free_grad(m);
-    free_qei(m);
+    free_cand_work(m);
     double** ptrs[] = {&m->dXt, &m->dInvTheta, &m->dCenter, &m->dA, &m->dAorig, &m->dW, &m->dD, &m->dWpack, &m->dBetaY, &m->dBeta1, &m->dY,
                        &m->dPmeans, &m->dPbeta, &m->dPlb, &m->dPwidth, &m->dCand, &m->dSlab, &m->dPart, &m->dOut, &m->dBlkBest, &m->dBest, &m->dAppend,
                        &m->dWi8s, &m->dRowScale, &m->dAlphaY, &m->dAlpha1, &m->dGuard, &m->dGuardList, &m->dCinv};

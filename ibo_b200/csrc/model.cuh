@@ -6,7 +6,7 @@
 #include <utility>
 #include <vector>
 
-namespace ibo { struct JointWork; struct GradWork; struct QeiWork; }
+namespace ibo { struct CandWork; }
 
 struct ibo_model {
     int device = 0;
@@ -73,13 +73,39 @@ struct ibo_model {
     // profile of the last call
     double prof[6] = {0, 0, 0, 0, 0, 0};
     cudaEvent_t ev[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
-    // joint posterior (joint.cu): covariance, samples and their Cholesky factor, built on first use
-    ibo::JointWork* joint = nullptr;
-    // gradients with respect to the candidate (grad.cu), built on first use
-    ibo::GradWork* grad = nullptr;
-    // batch expected improvement (qei.cu), built on first use
-    ibo::QeiWork* qei = nullptr;
+    // workspace of the joint posterior, the candidate gradients and q-EI (joint.cu, grad.cu, qei.cu), built on first use
+    ibo::CandWork* cand = nullptr;
 };
+
+namespace ibo {
+// Workspace of the candidate-side entry points (joint.cu, grad.cu, qei.cu), kept with the model that owns the call and grown on
+// demand.  One call at a time runs on a model, so the three share one set of buffers, one per role; g is the variance model when
+// one is attached and the model otherwise.  Within a call no two live roles share a buffer: Z overwrites K* and y overwrites V
+// once K* and V are dead.  A call grows every buffer it uses before it takes a pointer into the workspace.
+struct CandWork {
+    double* dRaw = nullptr;     size_t rawCap = 0;     // candidates as given [M][d]
+    double* dScaled = nullptr;  size_t scaledCap = 0;  // candidates (of the chunk) scaled and centred like g's training inputs [Mcp][d]
+    double* dScaledM = nullptr; size_t scaledMCap = 0; // the same scaled like the model's (variance model attached) [Mcp][d]
+    double* dKc = nullptr;      size_t kcCap = 0;      // K* = R(X_g, X*), then Z = W_g^T V [Np][Mcp]
+    double* dV = nullptr;       size_t vCap = 0;       // V = W_g K*, then y (q-EI) [Np][Mcp]
+    double* dAB = nullptr;      size_t abCap = 0;      // a | b [2][Np]
+    double* dKb = nullptr;      size_t kbCap = 0;      // k^T b [M] (prior only)
+    double* dG = nullptr;       size_t gCap = 0;       // three [M][d] gradient planes
+    double* dNormals = nullptr; size_t normalsCap = 0; // standard normals: [Mp][Sp] zero padded (samples), [q][S] (q-EI)
+    double* dPost = nullptr;    size_t postCap = 0;    // [score | mu | s2] of the scoring path, 3 M + 2 (joint, gradients); mu [M] (q-EI)
+    // joint posterior only
+    ibo_model chol;                                    // Sigma in chol.dA (Mp x Mp), factorised in place; its streams and events are the owner's
+    size_t cholACap = 0, cholDCap = 0;                 // chol.dA, chol.dD
+    double* dF = nullptr;       size_t fCap = 0;       // samples [Mp][Sp]
+    double* dArg = nullptr;     size_t argCap = 0;     // per-sample argmax (long long)
+    // q-EI only
+    double* dQei = nullptr;     size_t qeiCap = 0;     // values [B]
+    double* dMubar = nullptr;   size_t mubarCap = 0;   // d qEI / d mu [M]
+    double* dSig = nullptr;     size_t sigCap = 0;     // Sigma of the chunk's batches [Bc][q][q]
+    double* dGbar = nullptr;    size_t gbarCap = 0;    // Gbar of the chunk's batches [Bc][q][q]
+};
+CandWork* cand_work(ibo_model* m);                     // model.cu: the model's workspace, created empty on first use
+}  // namespace ibo
 
 struct ibo_cands {
     ibo_model* owner = nullptr;
@@ -112,26 +138,31 @@ int create_model_with_diag(int device, int kind, const double* hyper, int nhyper
                            double noise, double diag, ibo_model** out, int* info);
 int launch_gram_wtw(double* C, const ibo_model* m, cudaStream_t st);      // hyper.cu: C (lower tiles) = W^T W = inv(A)
 const char* get_error();
-// score.cu: mu of M device-resident candidates on the FP64 path (what ibo_posterior_batch returns with IBO_FLAG_FP64) at out + M;
-// out holds 3 M + 2 doubles
-int posterior_mean_device(ibo_model* m, const double* dCand, long M, double* out);
 // score.cu: [score | mu | s2] of M device-resident candidates at out, what ibo_score_batch (acq >= 0) or ibo_posterior_batch
 // (acq < 0) returns with flags; out holds 3 M + 2 doubles
 int posterior_score_device(ibo_model* m, const double* dCand, long M, int acq, double ymax, double parm, int flags, double* out);
-void free_joint(ibo_model* m);           // joint.cu: the model's joint-posterior workspace
+// joint.cu: the argument checks of the candidate-side entry points (Xs, M >= 1, d <= 64); extra_ok carries the entry point's own
+// bounds, computed before the model is read
+int check_cands(const ibo_model* m, const double* Xs, long M, bool extra_ok);
+// joint.cu: the dynamic shared memory of the W GEMMs below, once per call before them
+int ensure_joint_attrs(int device);
 // joint.cu, on st: candidates scaled and centred like g's training inputs ([Mp][d], zero padded); R(X_g, X*) with exact
 // zeros in the padding ([Np][Mp]); V = W_g Kc and Z = W_g^T V ([Np][Mp] each, Z may overwrite Kc)
 void launch_scale_cands(double* Cs, const double* X, const ibo_model* g, long M, long Mp, cudaStream_t st);
 void launch_cross_cov(double* Kc, const ibo_model* g, const double* Cs, int M, int Mp, cudaStream_t st);
-int launch_w_gemm_v(double* V, const ibo_model* g, const double* Kc, int Mp, cudaStream_t st);
-int launch_w_gemm_z(double* Z, const ibo_model* g, const double* V, int Mp, cudaStream_t st);
-void free_grad(ibo_model* m);            // grad.cu: the model's gradient workspace
-// grad.cu, on st: G[q][j][t] = sum_i w_q,i dk_i(x*_j) / dx_t over src's training points for the weights enabled (w_0 = Z[:, j],
-// w_1 = a, w_2 = b; planes `plane` doubles apart), kb[j] = sum_i b_i k_i; Cs scaled like src's training inputs
-template <bool DZ, bool DA, bool DB>
-void launch_reduce(const ibo_model* src, const double* Cs, int Mc, const double* Z, int ldz, const double* a, const double* b,
-                   double* G, size_t plane, double* kb, cudaStream_t st);
+void launch_w_gemm_v(double* V, const ibo_model* g, const double* Kc, int Mp, cudaStream_t st);
+void launch_w_gemm_z(double* Z, const ibo_model* g, const double* V, int Mp, cudaStream_t st);
+// grad.cu: candidates per chunk of the gradient and q-EI paths, the largest multiple of 128 whose K* / Z and V over g's training
+// points (2 Np doubles per candidate) fit in 512 MiB
+long cand_chunk(const ibo_model* g);
+// grad.cu, on st: a = W^T (W Y) and, with a prior, b = W^T (W 1) of the model into ab ([2][Np]), recomputed every call (an appended
+// model needs no invalidation); returns b, or nullptr without a prior
+double* launch_ab(const ibo_model* m, double* ab, cudaStream_t st);
+// grad.cu, on st: G[q][j][t] = sum_i w_q,i dk_i(x*_j) / dx_t for the Mc candidates of a chunk (planes `plane` doubles apart): w_0 =
+// Zw[:, j] (leading dimension ldz) over g's training points with Cs scaled like them, w_1 = a and w_2 = b over the model's with Cm
+// scaled like them (Cm is read with a variance model attached only); b and kb[j] = sum_i b_i k_i with a prior only (b non-null)
+void launch_grad_sums(const ibo_model* m, const double* Cs, const double* Cm, int Mc, const double* Zw, int ldz, const double* a,
+                      const double* b, double* G, size_t plane, double* kb, cudaStream_t st);
 // grad.cu, on st: the prior's share of dmu in place over plane 2 of G ([3][M][d]) for the M candidates `cand` (original coordinates)
 void launch_grad_prior(const ibo_model* m, const double* cand, long M, const double* kb, double* G, cudaStream_t st);
-void free_qei(ibo_model* m);             // qei.cu: the model's q-EI workspace
 }  // namespace ibo

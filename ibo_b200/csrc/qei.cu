@@ -22,24 +22,6 @@
 
 namespace ibo {
 
-// Workspace of ibo_qei, kept with the model that owns the call and grown on demand.
-struct QeiWork {
-    double* dRaw = nullptr;    size_t rawCap = 0;     // points as given [M][d], M = B q
-    double* dZ = nullptr;      size_t zCap = 0;       // standard normals [q][S]
-    double* dMu = nullptr;     size_t muCap = 0;      // mu [M]
-    double* dVal = nullptr;    size_t valCap = 0;     // values [B]
-    double* dMubar = nullptr;  size_t mubarCap = 0;   // d qEI / d mu [M]
-    double* dG = nullptr;      size_t gCap = 0;       // three [M][d] planes: sums with y, a, b -> the gradient in plane 0
-    double* dKb = nullptr;     size_t kbCap = 0;      // k^T b [M] (prior only)
-    double* dSig = nullptr;    size_t sigCap = 0;     // Sigma of the chunk's batches [Bc][q][q]
-    double* dGbar = nullptr;   size_t gbarCap = 0;    // Gbar of the chunk's batches [Bc][q][q]
-    double* dScaled = nullptr; size_t scaledCap = 0;  // chunk scaled like g's training inputs [Mcp][d]
-    double* dScaledM = nullptr; size_t scaledMCap = 0;// chunk scaled like the model's (variance model attached) [Mcp][d]
-    double* dKc = nullptr;     size_t kcCap = 0;      // K*, then Z [Np][Mcp]
-    double* dV = nullptr;      size_t vCap = 0;       // V, then y [Np][Mcp]
-    double* dAB = nullptr;     size_t abCap = 0;      // a | b [2][Np]
-};
-
 namespace {
 
 constexpr int QEI_MAX_Q = 32;
@@ -322,29 +304,25 @@ __global__ void __launch_bounds__(256) qei_epilogue_kernel(double* __restrict__ 
     }
 }
 
-inline long round128(long x) { return (x + 127) / 128 * 128; }
-
-// Enqueues everything on m->stream and leaves the values in w->dVal and, with wantGrad, the gradient [M][d] in w->dG.
+// Enqueues everything on m->stream and leaves the values in w->dQei and, with wantGrad, the gradient [M][d] in w->dG.
 int qei_device(ibo_model* m, const double* Xs, long B, int q, const double* Z, int S, double ymax, double xi, double jitter, bool wantGrad) {
-    if (!m->qei) m->qei = new QeiWork();
-    QeiWork* w = m->qei;
+    int rc;
+    if ((rc = ensure_joint_attrs(m->device))) return rc;
+    CandWork* w = cand_work(m);
     ibo_model* vm = m->var_model;
     ibo_model* g = vm ? vm : m;                          // the model Sigma comes from
     cudaStream_t st = m->stream;
     const int d = m->d;
     const bool prior = m->npb > 0;
     const long M = B * q;
-    // chunk: as many whole batches as fit in grad.cu's bound (the largest multiple of 128 points whose K* / Z and V fit in 512 MiB)
-    const long chunkPts = std::max(128L, (long)((512L << 20) / (2L * 8 * g->Np)) / 128 * 128);
-    const long Bc = chunkPts / q;
+    const long Bc = cand_chunk(g) / q;                   // whole batches per chunk
     const long Bcap = std::min(B, Bc), Mcap = round128(Bcap * q);
-    int rc;
     if ((rc = grow(&w->dRaw, &w->rawCap, (size_t)M * d))) return rc;
-    if ((rc = grow(&w->dZ, &w->zCap, (size_t)q * S))) return rc;
-    if ((rc = grow(&w->dMu, &w->muCap, (size_t)M))) return rc;
+    if ((rc = grow(&w->dNormals, &w->normalsCap, (size_t)q * S))) return rc;
+    if ((rc = grow(&w->dPost, &w->postCap, (size_t)M))) return rc;
     if ((rc = grow(&w->dAB, &w->abCap, (size_t)2 * m->Np))) return rc;
     if (vm && (rc = grow(&w->dScaledM, &w->scaledMCap, (size_t)Mcap * d))) return rc;
-    if ((rc = grow(&w->dVal, &w->valCap, (size_t)B))) return rc;
+    if ((rc = grow(&w->dQei, &w->qeiCap, (size_t)B))) return rc;
     if ((rc = grow(&w->dSig, &w->sigCap, (size_t)Bcap * q * q))) return rc;
     if ((rc = grow(&w->dScaled, &w->scaledCap, (size_t)Mcap * d))) return rc;
     if ((rc = grow(&w->dKc, &w->kcCap, (size_t)g->Np * Mcap))) return rc;
@@ -356,12 +334,10 @@ int qei_device(ibo_model* m, const double* Xs, long B, int q, const double* Z, i
         if (prior && (rc = grow(&w->dKb, &w->kbCap, (size_t)M))) return rc;
     }
     IBO_CUDA_TRY(cudaMemcpyAsync(w->dRaw, Xs, sizeof(double) * (size_t)M * d, cudaMemcpyHostToDevice, st));
-    IBO_CUDA_TRY(cudaMemcpyAsync(w->dZ, Z, sizeof(double) * (size_t)q * S, cudaMemcpyHostToDevice, st));
-    const double* mu = w->dMu;
+    IBO_CUDA_TRY(cudaMemcpyAsync(w->dNormals, Z, sizeof(double) * (size_t)q * S, cudaMemcpyHostToDevice, st));
+    double* const mu = w->dPost;
     double* const dA = w->dAB;
-    double* const dB = prior ? w->dAB + m->Np : nullptr;
-    launch_tri_matvec_t(m->dW, m->dBetaY, dA, m->N, m->Np, st);     // a = W^T (W Y), b = W^T (W 1) of the model, as grad.cu
-    if (prior) launch_tri_matvec_t(m->dW, m->dBeta1, dB, m->N, m->Np, st);
+    double* const dB = launch_ab(m, w->dAB, st);
     const size_t plane = (size_t)M * d;
     for (long b0 = 0; b0 < B; b0 += Bc) {
         const int nbt = (int)std::min(Bc, B - b0), Mc = nbt * q, Mcp = (int)round128(Mc);
@@ -370,32 +346,23 @@ int qei_device(ibo_model* m, const double* Xs, long B, int q, const double* Z, i
         launch_scale_cands(w->dScaled, raw, g, Mc, Mcp, st);
         if (vm) launch_scale_cands(w->dScaledM, raw, m, Mc, Mcp, st);
         const double* Cm = vm ? w->dScaledM : w->dScaled;          // the chunk scaled like the model's training inputs
-        qei_mean_kernel<<<(Mc + 31) / 32, 256, 0, st>>>(w->dMu + c0, m->dXt, m->N, Cm, raw, Mc, d, m->kind, m->sf2, dA, dB, m->npb,
+        qei_mean_kernel<<<(Mc + 31) / 32, 256, 0, st>>>(mu + c0, m->dXt, m->N, Cm, raw, Mc, d, m->kind, m->sf2, dA, dB, m->npb,
                                                         m->dPmeans, m->dPbeta, m->ptheta, m->dPlb, m->dPwidth);
         g_launches++;
         launch_cross_cov(w->dKc, g, w->dScaled, Mc, Mcp, st);
-        if ((rc = launch_w_gemm_v(w->dV, g, w->dKc, Mcp, st))) return rc;
+        launch_w_gemm_v(w->dV, g, w->dKc, Mcp, st);
         qei_sigma_kernel<<<nbt, 256, 0, st>>>(w->dSig, w->dV, Mcp, w->dScaled, g->N, q, d, g->kind, g->sf2, 1.0 + g->noise);
         g_launches += 2;
         if (!wantGrad) {
-            qei_batch_kernel<false><<<nbt, QW * 32, 0, st>>>(w->dSig, mu + c0, w->dZ, S, q, ymax, xi, jitter, w->dVal + b0, nullptr, nullptr);
+            qei_batch_kernel<false><<<nbt, QW * 32, 0, st>>>(w->dSig, mu + c0, w->dNormals, S, q, ymax, xi, jitter, w->dQei + b0, nullptr, nullptr);
             continue;
         }
-        qei_batch_kernel<true><<<nbt, QW * 32, 0, st>>>(w->dSig, mu + c0, w->dZ, S, q, ymax, xi, jitter, w->dVal + b0, w->dMubar + c0, w->dGbar);
-        if ((rc = launch_w_gemm_z(w->dKc, g, w->dV, Mcp, st))) return rc;
+        qei_batch_kernel<true><<<nbt, QW * 32, 0, st>>>(w->dSig, mu + c0, w->dNormals, S, q, ymax, xi, jitter, w->dQei + b0, w->dMubar + c0, w->dGbar);
+        launch_w_gemm_z(w->dKc, g, w->dV, Mcp, st);
         qei_y_kernel<<<dim3((Mc + 255) / 256, g->N), 256, 0, st>>>(w->dV, w->dKc, Mcp, w->dGbar, Mc, q);
         g_launches += 2;
         double* G = w->dG + (size_t)c0 * d;
-        double* kb = prior ? w->dKb + c0 : nullptr;
-        if (vm) {
-            launch_reduce<true, false, false>(g, w->dScaled, Mc, w->dV, Mcp, nullptr, nullptr, G, plane, nullptr, st);
-            if (prior) launch_reduce<false, true, true>(m, w->dScaledM, Mc, nullptr, 0, dA, dB, G, plane, kb, st);
-            else launch_reduce<false, true, false>(m, w->dScaledM, Mc, nullptr, 0, dA, nullptr, G, plane, nullptr, st);
-        } else if (prior) {
-            launch_reduce<true, true, true>(m, w->dScaled, Mc, w->dV, Mcp, dA, dB, G, plane, kb, st);
-        } else {
-            launch_reduce<true, true, false>(m, w->dScaled, Mc, w->dV, Mcp, dA, nullptr, G, plane, nullptr, st);
-        }
+        launch_grad_sums(m, w->dScaled, w->dScaledM, Mc, w->dV, Mcp, dA, dB, G, plane, prior ? w->dKb + c0 : nullptr, st);
         qei_pair_kernel<<<(Mc + 255) / 256, 256, 0, st>>>(G, w->dScaled, w->dGbar, Mc, q, d, g->kind, g->sf2, g->dInvTheta);
         g_launches++;
     }
@@ -410,16 +377,6 @@ int qei_device(ibo_model* m, const double* Xs, long B, int q, const double* Z, i
 
 }  // namespace
 
-void free_qei(ibo_model* m) {
-    QeiWork* w = m->qei;
-    if (!w) return;
-    double** ptrs[] = {&w->dRaw, &w->dZ, &w->dMu, &w->dVal, &w->dMubar, &w->dG, &w->dKb, &w->dSig, &w->dGbar, &w->dScaled,
-                       &w->dScaledM, &w->dKc, &w->dV, &w->dAB};
-    for (auto p : ptrs) if (*p) pool_free(*p);
-    delete w;
-    m->qei = nullptr;
-}
-
 }  // namespace ibo
 
 using namespace ibo;
@@ -427,18 +384,14 @@ using namespace ibo;
 extern "C" int ibo_qei(ibo_model* m, const double* Xs, long B, int q, const double* Z, int S, double ymax, double xi, double jitter,
                        double* values, double* dvalues, int* nbad) {
     if (nbad) *nbad = 0;
-    // every scalar check comes before the model is read; NaN jitter fails the comparison
-    if (!m || !Xs || !Z || !values || B < 1 || q < 1 || q > QEI_MAX_Q || S < 1 || S > 65536 || !(jitter >= 0.0)) {
-        set_error("bad argument");
-        return IBO_E_BADARG;
-    }
-    if (m->d > 64) { set_error("d > 64 not supported"); return IBO_E_BADARG; }
-    IBO_CUDA_TRY(cudaSetDevice(m->device));
-    int rc = qei_device(m, Xs, B, q, Z, S, ymax, xi, jitter, dvalues != nullptr);
+    int rc = check_cands(m, Xs, B, Z && values && q >= 1 && q <= QEI_MAX_Q && S >= 1 && S <= 65536 && jitter >= 0.0);   // NaN jitter fails
     if (rc) return rc;
-    QeiWork* w = m->qei;
+    IBO_CUDA_TRY(cudaSetDevice(m->device));
+    rc = qei_device(m, Xs, B, q, Z, S, ymax, xi, jitter, dvalues != nullptr);
+    if (rc) return rc;
+    CandWork* w = m->cand;
     cudaStream_t st = m->stream;
-    IBO_CUDA_TRY(cudaMemcpyAsync(values, w->dVal, sizeof(double) * B, cudaMemcpyDeviceToHost, st));
+    IBO_CUDA_TRY(cudaMemcpyAsync(values, w->dQei, sizeof(double) * B, cudaMemcpyDeviceToHost, st));
     if (dvalues) IBO_CUDA_TRY(cudaMemcpyAsync(dvalues, w->dG, sizeof(double) * (size_t)B * q * m->d, cudaMemcpyDeviceToHost, st));
     IBO_CUDA_TRY(cudaStreamSynchronize(st));
     IBO_CUDA_TRY(cudaGetLastError());

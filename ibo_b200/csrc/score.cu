@@ -1214,14 +1214,8 @@ int batch_uses_i8(ibo_model* m, long n, int flags) {
     if (n > narrow_threshold()) return i8_eligible(m, flags) ? 1 : 0;
     return i8_for_small_batch(m, n, flags) ? 1 : 0;
 }
-// mu of the joint posterior (joint.cu): the FP64 kernels of ibo_posterior_batch(..., IBO_FLAG_FP64) on device-resident candidates,
-// so that mu is that call's mu bit for bit
-int posterior_mean_device(ibo_model* m, const double* dCand, long M, double* out) {
-    ScoreReq rq{-1, 0.0, 0.0, IBO_FLAG_FP64, false, true, false};
-    return score_device(m, dCand, M, rq, out);
-}
-// values of the candidate gradients (grad.cu): the scoring path's own kernels, so that they are ibo_score_batch's /
-// ibo_posterior_batch's bit for bit
+// values of the joint posterior (joint.cu) and of the candidate gradients (grad.cu): the scoring path's own kernels, so that they
+// are ibo_score_batch's / ibo_posterior_batch's bit for bit
 int posterior_score_device(ibo_model* m, const double* dCand, long M, int acq, double ymax, double parm, int flags, double* out) {
     ScoreReq rq{acq, ymax, parm, flags, acq >= 0, true, true};
     rq.want_argmax = false;
