@@ -98,3 +98,132 @@ def test_posterior_by_hand_and_against_the_fp64_oracle():
             assert mu.dtype == LD and s2.dtype == LD
             assert np.max(np.abs(mu - mu_o)) <= 1e-12 and np.max(np.abs(s2 - s2_o)) <= 1e-12
         assert bo.rel(bo.build_R(kern, X, 0.1), o.R) <= 1e-15
+
+
+# -- the candidate-side reference: joint posterior, gradients with respect to the candidate, reverse Cholesky, q-EI -----------------
+
+CAND_KINDS = [(orc.K_SE_ARD, [.3, .4, .5]), (orc.K_MATERN3, [.5, .9]), (orc.K_MATERN5_ARD, [.3, .4, .5, .95])]
+
+
+def _cand_problem(kind, hyper, seed, N=40, d=3, with_prior=False, with_aug=False, noise=0.1):
+    """(spec, X, Y, prior, aug, FP64 GPOracle with the same prior / variance factor) on [0, 1]^d"""
+    rs = np.random.RandomState(seed)
+    X = rs.rand(N, d)
+    Y = np.sin(3 * X).sum(axis=1)
+    spec = orc.KernelSpec(kind, hyper, d)
+    prior = orc.PriorSpec(rs.rand(4, d), 0.3 * rs.randn(4), 3.0, np.zeros(d), np.ones(d)) if with_prior else None
+    o = orc.GPOracle(spec, X, Y, noise, prior=prior)
+    aug = None
+    if with_aug:
+        augX = np.r_[X, rs.rand(3, d)]
+        A = rs.randn(N, N) * 0.05
+        pad = np.zeros((N + 3, N + 3))
+        pad[:N, :N] = np.linalg.inv(np.eye(N) * 5 + A.dot(A.T))
+        aug = (augX, bo.build_R(spec, augX, noise) + pad)
+        o.augX, o.augL = augX, np.linalg.cholesky(orc.build_R(spec, augX, noise) + pad)
+    return spec, X, Y, prior, aug, o, rs
+
+
+def _fd(f, x, h):
+    """central differences of the longdouble function f at the longdouble point x, one coordinate at a time -> [..., x.size]"""
+    x = np.asarray(x, dtype=LD)
+    out = []
+    for t in range(x.size):
+        e = np.zeros(x.size, dtype=LD)
+        e[t] = h
+        e = e.reshape(x.shape)
+        out.append((f(x + e) - f(x - e)) / (2 * h))
+    return np.stack(out, axis=-1)
+
+
+def _rel_max(a, b):
+    a, b = np.asarray(a, dtype=LD), np.asarray(b, dtype=LD)
+    return float(np.max(np.abs(a - b)) / np.max(np.abs(b)))
+
+
+@pytest.mark.parametrize("kind,hyper", CAND_KINDS)
+@pytest.mark.parametrize("extra", ["", "prior", "aug"])
+def test_posterior_gradient_agrees_with_longdouble_differences(kind, hyper, extra):
+    spec, X, Y, prior, aug, _, rs = _cand_problem(kind, hyper, 20 + kind, with_prior=extra == "prior", with_aug=extra == "aug")
+    Xs = rs.rand(4, 3).astype(LD)
+    model = bo._Model(spec, X, Y, 0.1, prior, aug)
+    mu, s2, dmu, ds2 = bo.posterior_grad(spec, X, Y, 0.1, Xs, model=model)
+    h = LD(1e-7)
+    for j in range(len(Xs)):
+        f = lambda x: np.array(bo.posterior_grad(spec, X, Y, 0.1, x[None], model=model)[:2])[:, 0]
+        g = _fd(f, Xs[j], h)
+        assert _rel_max(dmu[j], g[0]) <= 1e-10 and _rel_max(ds2[j], g[1]) <= 1e-10, (j, dmu[j], g[0], ds2[j], g[1])
+
+
+def test_chol_rev_agrees_with_longdouble_differences():
+    """f(Sigma) = <Lbar, chol(Sigma)>: df / dSigma_kl over the symmetric perturbation of (k, l) and (l, k) is 2 Gbar_kl off the
+    diagonal and Gbar_kk on it"""
+    A = _spd(6, 10.0, 4)
+    Lbar = np.tril(np.random.RandomState(5).randn(6, 6)).astype(LD)
+    G = bo.chol_rev(bo.cholesky(A), Lbar)
+    assert np.array_equal(G, G.T)
+    h = LD(1e-7)
+    for k in range(6):
+        for l in range(k + 1):
+            E = np.zeros((6, 6), dtype=LD)
+            E[k, l] = E[l, k] = h
+            fd = (np.sum(Lbar * bo.cholesky(A + E)) - np.sum(Lbar * bo.cholesky(A - E))) / (2 * h)
+            want = G[k, l] * (1 if k == l else 2)
+            assert abs(fd - want) <= 1e-10 * np.max(np.abs(G)), (k, l, fd, want)
+
+
+@pytest.mark.parametrize("extra", ["", "prior", "aug"])
+def test_qei_gradient_agrees_with_longdouble_differences(extra):
+    spec, X, Y, prior, aug, _, rs = _cand_problem(orc.K_MATERN5_ARD, [.3, .4, .5, .95], 31, with_prior=extra == "prior",
+                                                  with_aug=extra == "aug")
+    model = bo._Model(spec, X, Y, 0.1, prior, aug)
+    Z = np.random.default_rng(2).standard_normal((3, 64))
+    ymax, xi = Y.max() - 0.3, 0.01
+    Xb = rs.rand(12, 3, 3).astype(LD)
+    v, G, gap, imp = bo.qei(spec, X, Y, 0.1, Xb, Z, ymax, xi, 1e-8, model=model)
+    keep = [b for b in range(len(Xb)) if min(gap[b], imp[b]) > 1e-4 and v[b] > 0]
+    assert len(keep) >= 3
+    for b in keep[:3]:
+        f = lambda x: bo.qei(spec, X, Y, 0.1, x[None], Z, ymax, xi, 1e-8, model=model)[0][0]
+        g = _fd(f, Xb[b], LD(1e-7))
+        assert _rel_max(G[b].reshape(-1), g) <= 1e-9, (b, G[b], g)
+
+
+@pytest.mark.parametrize("kind,hyper", CAND_KINDS)
+@pytest.mark.parametrize("extra", ["", "prior", "aug"])
+def test_candidate_paths_agree_with_the_fp64_oracles(kind, hyper, extra):
+    """noise 0.1, d = 3: the longdouble joint posterior, gradients, scores' gradients and q-EI agree with joint_oracle, grad_oracle
+    and qei_oracle to about 1e-12"""
+    import grad_oracle as go
+    import joint_oracle as jo
+    import qei_oracle as qo
+    spec, X, Y, prior, aug, o, rs = _cand_problem(kind, hyper, 40 + kind, N=150, with_prior=extra == "prior", with_aug=extra == "aug")
+    Xs = rs.rand(30, 3)
+    Xs[:2] = X[:2]
+    model = bo._Model(spec, X, Y, 0.1, prior, aug)
+    close = lambda a, b: np.max(np.abs(np.asarray(a, dtype=float) - b)) <= 1e-12 * max(1.0, np.max(np.abs(b)))
+    mu, Sig = bo.posterior_joint(spec, X, Y, 0.1, Xs, model=model)
+    mu_o, Sig_o = jo.posterior_joint(o, Xs)
+    assert close(mu, mu_o) and close(Sig, Sig_o)
+    mu, s2, dmu, ds2 = bo.posterior_grad(spec, X, Y, 0.1, Xs, model=model)
+    _, _, dmu_o, ds2_o = go.posterior_grad(o, Xs, "cpp")
+    assert close(dmu, dmu_o) and close(ds2, ds2_o) and close(s2, np.diag(Sig_o))
+    Z = np.random.default_rng(3).standard_normal((4, 128))
+    Xb = rs.rand(5, 4, 3)
+    v, G, _, _ = bo.qei(spec, X, Y, 0.1, Xb, Z, Y.max() - 0.3, 0.01, 0.0, model=model)
+    v_o, G_o = qo.qei(o, Xb, Z, Y.max() - 0.3, 0.01)
+    assert np.any(v_o > 0) and close(v, v_o) and close(G, G_o)
+
+
+def test_joint_covariance_is_symmetric_and_bounded_below_by_the_noise():
+    """Sigma = K** + noise I - k*^T inv(R) k*, and the posterior covariance of f is positive semi-definite; near-duplicate and
+    on-data candidates make it singular up to the noise"""
+    for noise in (0.1, 1e-4):
+        spec, X, Y, _, _, _, rs = _cand_problem(orc.K_SE_ARD, [.6, .8, 1.0], 50, N=120, noise=noise)
+        Xs = rs.rand(40, 3)
+        Xs[:5] = X[:5]
+        Xs[5:10] = Xs[10:15] + 1e-5
+        _, Sig = bo.posterior_joint(spec, X, Y, noise, Xs)
+        assert np.array_equal(Sig, Sig.T)
+        ev = np.linalg.eigvalsh(np.asarray(Sig, dtype=float))
+        assert np.min(ev) >= noise - 100 * EPS and np.min(ev) <= noise * 1.01
