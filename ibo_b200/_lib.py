@@ -20,7 +20,7 @@ EXPORTED = [
     "ibo_model_get_matrix", "ibo_model_set_variance_model", "ibo_pref_fit",
     "ibo_nlml", "ibo_kernel_matrix",
     "ibo_posterior_batch", "ibo_score_batch", "ibo_posterior_cov", "ibo_posterior_sample",
-    "ibo_posterior_grad", "ibo_score_grad", "ibo_qei",
+    "ibo_posterior_grad", "ibo_score_grad", "ibo_qei", "ibo_max_value_gumbel", "ibo_mes",
     "ibo_cands_create", "ibo_cands_destroy", "ibo_score_resident", "ibo_get_profile", "ibo_launch_count",
     "ibo_fp64_peak", "ibo_i8_peak", "ibo_i8_peak2", "ibo_host_register", "ibo_host_unregister", "ibo_stream_mark", "ibo_stream_elapsed_ms",
     "ibo_device_synchronize", "ibo_debug_exp",
@@ -106,6 +106,8 @@ def lib():
     L.ibo_posterior_grad.argtypes = [c_void_p, pd, c_long, c_int, pd, pd, pd, pd]
     L.ibo_score_grad.argtypes = [c_void_p, pd, c_long, c_int, c_double, c_double, c_int, pd, pd]
     L.ibo_qei.argtypes = [c_void_p, pd, c_long, c_int, pd, c_int, c_double, c_double, c_double, pd, pd, pi]
+    L.ibo_max_value_gumbel.argtypes = [c_void_p, pd, c_long, c_int, pd, pd, pd]
+    L.ibo_mes.argtypes = [c_void_p, pd, c_long, pd, c_int, c_int, pd, pd, pd, pl]
     L.ibo_cands_create.argtypes = [c_void_p, pd, c_long, POINTER(c_void_p)]
     L.ibo_cands_destroy.argtypes = [c_void_p]
     L.ibo_score_resident.argtypes = [c_void_p, c_void_p, c_int, c_double, c_double, c_int, pd, pd, pl, POINTER(c_float)]
@@ -362,6 +364,28 @@ class Model(object):
         check(lib().ibo_qei(self._h, dptr(Xb), B, q, dptr(Z), Z.shape[1], float(ymax), float(xi), float(jitter), dptr(vals),
                             dptr(dv) if want_grad else None, ctypes.byref(nbad)))
         return vals, dv, nbad.value
+
+    def max_value_gumbel(self, Xs, flags=FLAG_MODE_CPP):
+        """Gumbel fit of the distribution of the maximum over the candidates (ibo_max_value_gumbel) -> (q[3], loc, scale): q solve
+        F(q) = 0.25, 0.5, 0.75 for F(y) = prod_i Phi((y - mu_i) / s_i) with mu, s2 as `posterior` returns them with `flags`"""
+        Xs = self._candidates(Xs)
+        q, loc, scale = np.empty(3), c_double(0), c_double(0)
+        check(lib().ibo_max_value_gumbel(self._h, dptr(Xs), Xs.shape[0], flags, dptr(q), ctypes.byref(loc), ctypes.byref(scale)))
+        return q, loc.value, scale.value
+
+    def mes(self, Xs, ystar, flags=FLAG_MODE_CPP, want_grad=False):
+        """max-value entropy search at the candidates for samples ystar[K] of the maximum (ibo_mes) -> (values[M],
+        dvalues[M, d] or None, best value, its index).  With want_grad, flags may carry FLAG_MODE_PY only and the values are
+        those of the FP64 kernels."""
+        Xs = self._candidates(Xs)
+        ystar = as_f64(ystar)
+        M = Xs.shape[0]
+        vals = np.empty(M)
+        dv = np.empty((M, self.d)) if want_grad else None
+        best, bidx = c_double(0), c_long(-1)
+        check(lib().ibo_mes(self._h, dptr(Xs), M, dptr(ystar), ystar.shape[0], flags, dptr(vals), dptr(dv) if want_grad else None,
+                            ctypes.byref(best), ctypes.byref(bidx)))
+        return vals, dv, best.value, bidx.value
 
     def score(self, Xs, acq, ymax, parm, flags=FLAG_MODE_PY, want_scores=True, want_posterior=False, out=None):
         """`out` (optional, float64[M]) receives the scores in place (lets callers reuse a pinned buffer)."""

@@ -12,7 +12,7 @@ import ctypes
 import numpy as np
 
 from .. import _lib
-from ..gaussianprocess import GaussianProcess, PrefGaussianProcess
+from ..gaussianprocess import GaussianProcess, PrefGaussianProcess, gumbel_draws
 from ..utils.optimize import direct, cdirect  # noqa: F401
 from ..utils.latinhypercube import lhcSample  # noqa: F401
 
@@ -95,6 +95,22 @@ class EI(_Acquisition):
 
     def _ymax(self):
         return self.ymax
+
+
+class MES(_Acquisition):
+    """max-value entropy search (Wang & Jegelka 2017) for samples ystar of the maximum: the mean over the samples of
+    h(g) = g psi(g) / 2 - log Phi(g), g = (y* - mu) / sigma, psi = phi / Phi (ibo_mes, Python-path arithmetic)"""
+
+    def __init__(self, GP, ystar, **kwargs):
+        super(MES, self).__init__(GP)
+        self.ystar = np.array(ystar, dtype=float, ndmin=1)
+        self.evaluations = 0
+
+    def f_batch(self, Xs):
+        if len(self.GP.X) == 0:
+            raise ValueError("acquisition over a GP without data")
+        self.evaluations += len(Xs)
+        return self.GP.model.mes(Xs, self.ystar, _lib.FLAG_MODE_PY)[0]
 
 
 def cdirectGP(model, bounds, maxiter, maxtime, maxsample, acqfunc=None, xi=-1, beta=-1, scale=-1, delta=-1, polish=0, **kwargs):
@@ -270,6 +286,42 @@ def maximizeQEI(GP, bounds, q, samples=512, seed=0, xi=0.01, starts=8, pending=N
     val, batch, v0, nfev = _polish_batches(fg, bounds, X0, pending, maxiter)
     maximizeQEI.last = dict(evaluations=nfev, start_values=v0)
     return val, batch
+
+
+def _polish_from(fg, bounds, opt, optx, C, cvals, k, maxiter=100):
+    """Gradient polish of a DIRECT answer: L-BFGS-B (_polish, fg(X) -> (values, gradients)) from DIRECT's optx and the k - 1
+    candidates C with the largest values cvals.  The best polished point replaces (opt, optx) only when its value beats optx
+    re-scored in the same call.  Returns (opt, optx, dict(evaluations, moved, starts))."""
+    starts = np.r_[np.asarray(optx, dtype=float)[None, :], np.asarray(C, dtype=float)[np.argsort(-np.asarray(cvals), kind='stable')[:k - 1]]]
+    vals, X, v0, nfev = _polish(fg, bounds, starts, maxiter)
+    b = int(np.argmax(vals))
+    moved = bool(vals[b] > v0[0])
+    rec = dict(evaluations=nfev, moved=moved, starts=starts)
+    return (float(vals[b]), X[b], rec) if moved else (opt, optx, rec)
+
+
+def maximizeMES(GP, bounds, n_samples=10, seed=0, candidates=None, samples=16384, floor=None, maxiter=50, maxtime=30,
+                maxsample=10000, polish=0):
+    """Maximise max-value entropy search (MES) with DIRECT.  The samples y* of the maximum come from the Gumbel fit over the
+    `candidates` or, by default, over `samples` Latin-hypercube points (lhcSample with `seed`), drawn with `seed` and raised to
+    `floor` (GaussianProcess.sample_max_values).  polish = k > 0 refines DIRECT's answer by L-BFGS-B on the gradient of MES from
+    DIRECT's optx and the k - 1 candidates of largest MES; the polished point (with its FP64 value) is returned only when it beats
+    DIRECT's optx re-scored in the same call.  Returns (opt, optx); maximizeMES.last records ystar, loc, scale, DIRECT's samples
+    and the polish evaluations."""
+    if len(GP.X) == 0:
+        raise ValueError("MES over a GP without data")
+    C = np.array(lhcSample(bounds, samples, seed=seed) if candidates is None else candidates, dtype=float, ndmin=2)
+    _, loc, scale = GP.model.max_value_gumbel(C, _lib.FLAG_MODE_PY)
+    ystar = np.maximum(gumbel_draws(loc, scale, n_samples, seed), np.max(GP.Y) if floor is None else floor)
+    obj = MES(GP, ystar)
+    opt, optx = _python_direct(obj, bounds, maxiter=maxiter, maxtime=maxtime, maxsample=maxsample)
+    maximizeMES.last = dict(ystar=ystar, loc=loc, scale=scale, samples=obj.evaluations, polish=None)
+    if polish > 0:
+        cvals = GP.model.mes(C, ystar, _lib.FLAG_MODE_PY)[0]
+        fg = lambda X: GP.model.mes(X, ystar, _lib.FLAG_MODE_PY, want_grad=True)[:2]        # noqa: E731
+        opt, optx, rec = _polish_from(fg, bounds, opt, optx, C, cvals, polish)
+        maximizeMES.last['polish'] = dict(evaluations=rec['evaluations'], moved=rec['moved'])
+    return opt, optx
 
 
 def _python_direct(obj, bounds, **kw):

@@ -191,8 +191,6 @@ void launch_grad_prior(const ibo_model* m, const double* cand, long M, const dou
     g_launches++;
 }
 
-namespace {
-
 // Enqueues everything on m->stream and leaves [score | mu | s2] in w->dPost and ds2, dmu, dscore ([M][d] each) in w->dG.
 int grad_device(ibo_model* m, const double* Xs, long M, int acq, double ymax, double parm, int flags, bool wantGrad) {
     int rc;
@@ -242,6 +240,8 @@ int grad_device(ibo_model* m, const double* Xs, long M, int acq, double ymax, do
     IBO_CUDA_TRY(cudaGetLastError());
     return IBO_OK;
 }
+
+namespace {
 
 int copy_out(double* dst, const double* src, size_t n, cudaStream_t st) {
     if (dst) IBO_CUDA_TRY(cudaMemcpyAsync(dst, src, sizeof(double) * n, cudaMemcpyDeviceToHost, st));

@@ -73,13 +73,13 @@ struct ibo_model {
     // profile of the last call
     double prof[6] = {0, 0, 0, 0, 0, 0};
     cudaEvent_t ev[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
-    // workspace of the joint posterior, the candidate gradients and q-EI (joint.cu, grad.cu, qei.cu), built on first use
+    // workspace of the joint posterior, the candidate gradients, q-EI and MES (joint.cu, grad.cu, qei.cu, mes.cu), built on first use
     ibo::CandWork* cand = nullptr;
 };
 
 namespace ibo {
-// Workspace of the candidate-side entry points (joint.cu, grad.cu, qei.cu), kept with the model that owns the call and grown on
-// demand.  One call at a time runs on a model, so the three share one set of buffers, one per role; g is the variance model when
+// Workspace of the candidate-side entry points (joint.cu, grad.cu, qei.cu, mes.cu), kept with the model that owns the call and grown
+// on demand.  One call at a time runs on a model, so the four share one set of buffers, one per role; g is the variance model when
 // one is attached and the model otherwise.  Within a call no two live roles share a buffer: Z overwrites K* and y overwrites V
 // once K* and V are dead.  A call grows every buffer it uses before it takes a pointer into the workspace.
 struct CandWork {
@@ -92,7 +92,8 @@ struct CandWork {
     double* dKb = nullptr;      size_t kbCap = 0;      // k^T b [M] (prior only)
     double* dG = nullptr;       size_t gCap = 0;       // three [M][d] gradient planes
     double* dNormals = nullptr; size_t normalsCap = 0; // standard normals: [Mp][Sp] zero padded (samples), [q][S] (q-EI)
-    double* dPost = nullptr;    size_t postCap = 0;    // [score | mu | s2] of the scoring path, 3 M + 2 (joint, gradients); mu [M] (q-EI)
+    double* dPost = nullptr;    size_t postCap = 0;    // [score | mu | s2] of the scoring path, 3 M + 2 (joint, gradients; MES values in
+                                                       // the score plane, best value and index at 3 M); mu [M] (q-EI)
     // joint posterior only
     ibo_model chol;                                    // Sigma in chol.dA (Mp x Mp), factorised in place; its streams and events are the owner's
     size_t cholACap = 0, cholDCap = 0;                 // chol.dA, chol.dD
@@ -103,6 +104,11 @@ struct CandWork {
     double* dMubar = nullptr;   size_t mubarCap = 0;   // d qEI / d mu [M]
     double* dSig = nullptr;     size_t sigCap = 0;     // Sigma of the chunk's batches [Bc][q][q]
     double* dGbar = nullptr;    size_t gbarCap = 0;    // Gbar of the chunk's batches [Bc][q][q]
+    // max-value entropy search only
+    double* dYstar = nullptr;   size_t ystarCap = 0;   // y* samples [K]
+    double* dMesD = nullptr;    size_t mesDCap = 0;    // d MES / d mu | d MES / d s [2][M]
+    double* dBlk = nullptr;     size_t blkCap = 0;     // per-block partials: argmax values | indices (long long) [2][nblk]; Gumbel fit:
+                                                       // bracket state lo[3] | hi[3], then trial sums [nblk][3 T] | bracket ends [nblk][2]
 };
 CandWork* cand_work(ibo_model* m);                     // model.cu: the model's workspace, created empty on first use
 }  // namespace ibo
@@ -165,4 +171,10 @@ void launch_grad_sums(const ibo_model* m, const double* Cs, const double* Cm, in
                       const double* b, double* G, size_t plane, double* kb, cudaStream_t st);
 // grad.cu, on st: the prior's share of dmu in place over plane 2 of G ([3][M][d]) for the M candidates `cand` (original coordinates)
 void launch_grad_prior(const ibo_model* m, const double* cand, long M, const double* kb, double* G, cudaStream_t st);
+// grad.cu: enqueues everything on m->stream and leaves [score | mu | s2] (the FP64 kernels' with flags) in the workspace's dPost and,
+// with wantGrad, ds2, dmu and dscore ([M][d] each; ds2 = 0 where s2 is clipped; dscore = 0 for acq < 0) in its dG
+int grad_device(ibo_model* m, const double* Xs, long M, int acq, double ymax, double parm, int flags, bool wantGrad);
+// score.cu, on st: the final argmax over nblk per-block (best, index) pairs of the scoring path's block argmax (lowest index wins
+// ties, NaN never wins)
+void launch_argmax_final(const double* blkBest, const long long* blkIdx, long nblk, double* best, long long* bestIdx, cudaStream_t st);
 }  // namespace ibo

@@ -560,6 +560,11 @@ __global__ void __launch_bounds__(256) argmax_final_kernel(const double* __restr
     }
 }
 
+void launch_argmax_final(const double* blkBest, const long long* blkIdx, long nblk, double* best, long long* bestIdx, cudaStream_t st) {
+    argmax_final_kernel<<<1, 256, 0, st>>>(blkBest, blkIdx, nblk, best, bestIdx);
+    g_launches++;
+}
+
 
 // ---------------------------------------------------------------------------------------------
 // Guard pass of the INT8 path: ordered compaction of the flagged candidates (ascending index, so that "lowest index wins" keeps

@@ -47,6 +47,13 @@ def PDF(x):
     return np.exp(-(x ** 2 / 2)) * 0.398942
 
 
+def gumbel_draws(loc, scale, n, seed=None):
+    """n draws loc - scale log(-log u) of a Gumbel distribution, u = k / 2^53 for k uniform in 1 .. 2^53 - 1 from
+    numpy.random.default_rng(seed): strictly inside (0, 1), so every draw is finite"""
+    u = np.random.default_rng(seed).integers(1, 2 ** 53, size=n) / 2.0 ** 53
+    return loc - scale * np.log(-np.log(u))
+
+
 class GaussianProcess(object):
 
     append_above = 256       # addData appends on the device when the resident model has at least this many points ...
@@ -221,6 +228,31 @@ class GaussianProcess(object):
         vals, dv, _ = self.model.qei(Xb, Z, np.max(self.Y), xi, jitter, want_grad=grad)
         if one:
             vals, dv = float(vals[0]), (dv[0] if grad else None)
+        return (vals, dv) if grad else vals
+
+    def sample_max_values(self, X, n_samples=10, seed=None, floor=None, method='gumbel', jitter=0.0):
+        """samples y*[n_samples] of the maximum of f over the points in X, for max-value entropy search (`mes`).
+        method='gumbel' (Wang & Jegelka 2017): the Gumbel fit of F(y) = prod_i Phi((y - mu_i) / s_i) over X
+        (ibo_max_value_gumbel), y* = loc - scale log(-log u) for u from numpy.random.default_rng(seed), strictly inside (0, 1).
+        method='joint': the maxima over X of joint posterior draws (sample_posterior with seed and jitter; at most 16384
+        points), which ignore no correlation.  Samples below `floor` (default max(Y)) are raised to it."""
+        X = self._candidates(X)
+        if method == 'gumbel':
+            _, loc, scale = self.model.max_value_gumbel(X, _lib.FLAG_MODE_PY)
+            ys = gumbel_draws(loc, scale, n_samples, seed)
+        elif method == 'joint':
+            ys = np.max(self.sample_posterior(X, n_samples, seed, jitter), axis=0)
+        else:
+            raise ValueError("unknown method %r" % (method,))
+        return np.maximum(ys, np.max(self.Y) if floor is None else floor)
+
+    def mes(self, Xs, ystar, grad=False, int8=None, mode='py'):
+        """max-value entropy search at the points in Xs for samples ystar of the maximum (sample_max_values): the mean over
+        the samples of h(g) = g psi(g) / 2 - log Phi(g), g = (y* - mu) / sigma, psi = phi / Phi -> values[M], and with grad=True
+        also their gradient with respect to the point [M, d] (values then those of the FP64 kernels).  `int8` and `mode` as in
+        score_batch; sigma^2 is the same clipped variance of a noisy observation."""
+        flags = (_lib.FLAG_MODE_PY if mode == 'py' else _lib.FLAG_MODE_CPP) | (0 if int8 is None else (_lib.FLAG_INT8 if int8 else _lib.FLAG_FP64))
+        vals, dv, _, _ = self.model.mes(self._candidates(Xs), ystar, flags, want_grad=grad)
         return (vals, dv) if grad else vals
 
     def mu(self, x):

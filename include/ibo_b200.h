@@ -228,6 +228,36 @@ int ibo_score_grad(ibo_model* m, const double* Xs, long M, int acq, double ymax,
 int ibo_qei(ibo_model* m, const double* Xs, long B, int q, const double* Z, int S,
             double ymax, double xi, double jitter, double* values, double* dvalues, int* nbad);
 
+/* ---- max-value entropy search (MES) -------------------------------------------------------------
+ * Xs: M x d row-major candidates (original coordinates), M >= 1, d <= 64.  mu and s2 are what ibo_posterior_batch returns with the
+ * same flags: s2 is the library's clipped variance (floor 1e-8, 1e-7 under IBO_FLAG_MODE_PY, ceiling 10), which like EI's carries
+ * the 1 + noise diagonal of R, so MES measures the information about max y of a noisy observation.  For samples y*[K] of the maximum
+ *     g_k = (y*_k - mu) / s,  s = sqrt(s2),  psi = phi / Phi,  h(g) = g psi(g) / 2 - log Phi(g) >= 0,  MES = (1 / K) sum_k h(g_k)
+ * summed in ascending k.  h'(g) = -(psi / 2)(1 + g (g + psi)) < 0: raising a y* lowers every value.  For g <= -1.5 sqrt2, h and h'
+ * come from the continued fraction of erfc, which does not cancel.  The gradient is the chain rule
+ *     d MES = d MES / d mu  d mu + d MES / d s  d s2 / (2 s),  d MES / d mu = -(1 / (K s)) sum h'(g_k),  d MES / d s = -(1 / (K s)) sum g_k h'(g_k)
+ * with d s2 = 0 where s2 is clipped (ibo_posterior_grad's).
+ *
+ * Gumbel fit of the distribution of max f over the candidate set Xs (M x d, M >= 1): with mu_i, s_i = sqrt(s2_i) as
+ * ibo_posterior_batch returns them with `flags` (0, IBO_FLAG_MODE_PY, IBO_FLAG_INT8, IBO_FLAG_FP64), q[0..2] solve
+ * sum_i log Phi((q - mu_i) / s_i) = log 0.25, log 0.5, log 0.75; scale = (q[2] - q[0]) / (log(-log .25) - log(-log .75)),
+ * loc = q[1] + scale log(-log .5).  Any output may be NULL.  Deterministic: the same set gives the same bits.
+ * Samples of the maximum are then y* = loc - scale log(-log u) for uniforms u in (0, 1) the caller draws.  The three roots are
+ * bracketed by max(mu_i - s_i) and max(mu_i + c s_i), c = sqrt(2 ln 5M), and found by 16 passes of multisection with 15 trial
+ * points per bracket (64 bits), each pass one kernel over all candidates and one that adds the blocks' sums in a fixed order: q[b]
+ * is the upper end of the final bracket.  The grid is a function of M alone.
+ * IBO_E_BADARG for a NULL model or Xs, M < 1, d > 64, or a flag bit other than those listed. */
+int ibo_max_value_gumbel(ibo_model* m, const double* Xs, long M, int flags, double* q, double* loc, double* scale);
+
+/* values[M] = (1/K) sum_k h((ystar[k] - mu) / s), h(g) = g psi(g) / 2 - log Phi(g), psi = phi / Phi; 1 <= K <= 1024, every ystar
+ * finite.  Without dvalues: mu, s2 as ibo_posterior_batch with `flags`.  With dvalues (M x d, d <= 64): flags 0 or IBO_FLAG_MODE_PY
+ * only, mu and s2 of the FP64 kernels (as ibo_score_grad), and values the same bits as the dvalues = NULL call with IBO_FLAG_FP64.
+ * best / best_idx: argmax, lowest index wins, NaN never wins; any output may be NULL.
+ * IBO_E_BADARG for a NULL model, Xs, ystar or values, M < 1, d > 64, K outside [1, 1024], a non-finite ystar, a flag bit other
+ * than IBO_FLAG_MODE_PY, IBO_FLAG_INT8 and IBO_FLAG_FP64, or dvalues with a flag other than IBO_FLAG_MODE_PY. */
+int ibo_mes(ibo_model* m, const double* Xs, long M, const double* ystar, int K, int flags,
+            double* values, double* dvalues, double* best, long* best_idx);
+
 /* Candidates kept resident in HBM (the bench's device-resident leg; also used for sharded sets). */
 int ibo_cands_create(ibo_model* m, const double* Xs, long M, ibo_cands** out);
 int ibo_cands_destroy(ibo_cands* c);
