@@ -21,6 +21,7 @@ EXPORTED = [
     "ibo_nlml", "ibo_kernel_matrix",
     "ibo_posterior_batch", "ibo_score_batch", "ibo_posterior_cov", "ibo_posterior_sample",
     "ibo_posterior_grad", "ibo_score_grad", "ibo_qei", "ibo_max_value_gumbel", "ibo_mes",
+    "ibo_paths_create", "ibo_paths_eval", "ibo_paths_grad", "ibo_paths_destroy",
     "ibo_cands_create", "ibo_cands_destroy", "ibo_score_resident", "ibo_get_profile", "ibo_launch_count",
     "ibo_fp64_peak", "ibo_i8_peak", "ibo_i8_peak2", "ibo_host_register", "ibo_host_unregister", "ibo_stream_mark", "ibo_stream_elapsed_ms",
     "ibo_device_synchronize", "ibo_debug_exp",
@@ -108,6 +109,10 @@ def lib():
     L.ibo_qei.argtypes = [c_void_p, pd, c_long, c_int, pd, c_int, c_double, c_double, c_double, pd, pd, pi]
     L.ibo_max_value_gumbel.argtypes = [c_void_p, pd, c_long, c_int, pd, pd, pd]
     L.ibo_mes.argtypes = [c_void_p, pd, c_long, pd, c_int, c_int, pd, pd, pd, pl]
+    L.ibo_paths_create.argtypes = [c_void_p, c_int, c_int, pd, pd, pd, pd, POINTER(c_void_p), pi]
+    L.ibo_paths_eval.argtypes = [c_void_p, pd, c_long, pd, pd, pl]
+    L.ibo_paths_grad.argtypes = [c_void_p, pd, c_long, pi, pd, pd]
+    L.ibo_paths_destroy.argtypes = [c_void_p]
     L.ibo_cands_create.argtypes = [c_void_p, pd, c_long, POINTER(c_void_p)]
     L.ibo_cands_destroy.argtypes = [c_void_p]
     L.ibo_score_resident.argtypes = [c_void_p, c_void_p, c_int, c_double, c_double, c_int, pd, pd, pl, POINTER(c_float)]
@@ -387,6 +392,12 @@ class Model(object):
                             ctypes.byref(best), ctypes.byref(bidx)))
         return vals, dv, best.value, bidx.value
 
+    def sample_paths(self, omega, phase, w, e):
+        """pathwise posterior samples for caller-supplied draws (ibo_paths_create): omega[F, d] spectral frequencies, phase[F],
+        w[F, S] and e[Ng, S] standard normals (Ng: the training points of the variance model when one is attached) -> Paths;
+        raises NotPositiveDefinite when inv(C) + (1 + noise - sf2) I of a Laplace model is not positive definite"""
+        return Paths(self, omega, phase, w, e)
+
     def score(self, Xs, acq, ymax, parm, flags=FLAG_MODE_PY, want_scores=True, want_posterior=False, out=None):
         """`out` (optional, float64[M]) receives the scores in place (lets callers reuse a pinned buffer)."""
         if not (isinstance(Xs, np.ndarray) and Xs.dtype == np.float64 and Xs.ndim == 2 and Xs.flags.c_contiguous):
@@ -417,6 +428,53 @@ class Model(object):
         out = np.zeros(6)
         check(lib().ibo_get_profile(self._h, dptr(out)))
         return dict(k1_ms=out[0], k2_ms=out[1], k3_ms=out[2], total_ms=out[3], launches=int(out[4]), k2_launches=int(out[5]))
+
+
+class Paths(object):
+    """Owner of an `ibo_paths*` handle: S posterior sample paths, a snapshot of the model they were drawn from"""
+
+    def __init__(self, model, omega, phase, w, e):
+        omega, phase, w, e = as_f64(omega, 2), as_f64(phase), as_f64(w, 2), as_f64(e, 2)
+        F, S = w.shape
+        ng = (model._var or model).N           # the training points Sigma comes from: the variance model's when one is attached
+        if omega.shape != (F, model.d) or phase.shape != (F,) or e.shape != (ng, S):
+            raise ValueError("draws have inconsistent shapes: omega %s, phase %s, w %s, e %s" % (omega.shape, phase.shape, w.shape, e.shape))
+        self.d, self.S, self.F = model.d, S, F
+        self._h = c_void_p()
+        info = c_int(0)
+        check(lib().ibo_paths_create(model.handle, F, S, dptr(omega), dptr(phase), dptr(w), dptr(e), ctypes.byref(self._h),
+                                     ctypes.byref(info)), info.value)
+
+    def _points(self, X):
+        X = as_f64(X, 2)
+        if X.shape[1] != self.d:
+            raise ValueError("points have %d columns, the paths %d" % (X.shape[1], self.d))
+        return X
+
+    def eval(self, X, want_values=True):
+        """(values[M, S] or None, best[S], argmax[S]) at the points X[M, d] (ibo_paths_eval)"""
+        X = self._points(X)
+        M = X.shape[0]
+        vals = np.empty((M, self.S)) if want_values else None
+        best, idx = np.empty(self.S), np.empty(self.S, dtype=np.int64)
+        check(lib().ibo_paths_eval(self._h, dptr(X), M, dptr(vals) if want_values else None, dptr(best), idx.ctypes.data_as(POINTER(c_long))))
+        return vals, best, idx
+
+    def grad(self, X, which):
+        """point j on path which[j] -> (values[M], gradients[M, d]) (ibo_paths_grad); values are eval's bits"""
+        X = self._points(X)
+        M = X.shape[0]
+        wh = np.ascontiguousarray(np.broadcast_to(np.asarray(which), (M,)), dtype=np.int32)
+        vals, g = np.empty(M), np.empty((M, self.d))
+        check(lib().ibo_paths_grad(self._h, dptr(X), M, wh.ctypes.data_as(POINTER(c_int)), dptr(vals), dptr(g)))
+        return vals, g
+
+    def close(self):
+        if getattr(self, "_h", None) is not None and self._h:
+            lib().ibo_paths_destroy(self._h)
+            self._h = None
+
+    __del__ = close
 
 
 def acqmax_many(models, lb, ub, acq, ymax, parm, flags=FLAG_MODE_CPP, maxiter=50, maxtime=30, maxsample=10000):

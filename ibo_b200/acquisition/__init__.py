@@ -226,22 +226,41 @@ def polishAcquisition(GP, bounds, X0, acq='ei', xi=0.01, parm=None, mode='cpp', 
     return vals, X
 
 
-def thompsonBatch(GP, bounds, q, samples=2048, candidates=None, seed=None, jitter=0.0):
-    """Thompson sampling of a batch of q points to evaluate in parallel: q joint posterior draws over a candidate set, each
-    draw's maximiser is one point of the batch.
+def thompsonBatch(GP, bounds, q, samples=2048, candidates=None, seed=None, jitter=0.0, method='joint', n_features=2048, polish=False):
+    """Thompson sampling of a batch of q points to evaluate in parallel: q posterior draws over a candidate set, each draw's
+    maximiser is one point of the batch.
 
-    Candidates are `samples` Latin-hypercube points within `bounds` (lhcSample with `seed`) unless given as an array.  The
-    draws are mu + chol(cov + jitter I) Z with Z = numpy.random.default_rng(seed).standard_normal((M, q)); only the q
-    argmax indices leave the device.  Two draws can pick the same candidate, so a point may appear more than once in the
-    batch.  Returns (points[q, d], indices[q])."""
+    Candidates are `samples` Latin-hypercube points within `bounds` (lhcSample with `seed`) unless given as an array.
+    method='joint': the draws are mu + chol(cov + jitter I) Z with Z = numpy.random.default_rng(seed).standard_normal((M, q))
+    (at most 16384 candidates).  method='paths': q sample paths (GaussianProcess.sample_paths with n_features and seed), with no
+    limit on the candidates; with polish=True each path's maximiser is then refined by L-BFGS-B on that path's gradient within
+    `bounds`, every path in one call per evaluation, and a point is kept only where its path value beats the start's.  Only the
+    q argmax indices leave the device.  Two draws can pick the same candidate, so a point may appear more than once in the
+    batch.  Returns (points[q, d], indices[q]); the indices name the starting candidates."""
     if len(GP.X) == 0:
         raise ValueError("Thompson sampling over a GP without data")
+    if method not in ('joint', 'paths'):
+        raise ValueError("unknown method %r" % (method,))
+    if polish and method != 'paths':
+        raise ValueError("polish=True needs method='paths'")
     if candidates is None:
         candidates = lhcSample(bounds, samples, seed=seed)
     C = np.array(candidates, dtype=float, ndmin=2)
-    Z = np.random.default_rng(seed).standard_normal((C.shape[0], q))
-    _, idx = GP.model.posterior_sample(C, Z, jitter, want_F=False)
-    return C[idx], idx
+    if method == 'joint':
+        Z = np.random.default_rng(seed).standard_normal((C.shape[0], q))
+        _, idx = GP.model.posterior_sample(C, Z, jitter, want_F=False)
+        return C[idx], idx
+    paths = GP.sample_paths(q, n_features, seed)
+    try:
+        _, idx = paths.argmax(C)
+        if np.any(idx < 0):
+            raise ValueError("a sample path is NaN at every candidate (NaN in the candidates?)")
+        X = C[idx]
+        if polish:
+            _, X, _, _ = _polish(lambda P: paths.grad(P, np.arange(len(P)) % q), bounds, X)
+    finally:
+        paths.close()
+    return X, idx
 
 
 def _polish_batches(fg, bounds, starts, pending=None, maxiter=100):

@@ -54,6 +54,67 @@ def gumbel_draws(loc, scale, n, seed=None):
     return loc - scale * np.log(-np.log(u))
 
 
+def spectral_draws(kind, rng, F, d):
+    """F frequencies [F, d] from the spectral density of kernel `kind` (_lib.KERNEL_*) in unit-length-scale coordinates: N(0, I)
+    for the squared exponential; for Matern-nu (nu = 3/2, 5/2) the multivariate Student-t with 2 nu degrees of freedom,
+    z sqrt(2 nu / u) with z ~ N(0, I) and one u ~ chi^2(2 nu) per frequency (z first, then u)"""
+    if kind in (_lib.KERNEL_SE_ARD, _lib.KERNEL_SE_ISO):
+        return rng.standard_normal((F, d))
+    if kind == _lib.KERNEL_MATERN3:
+        nu = 1.5
+    elif kind in (_lib.KERNEL_MATERN5, _lib.KERNEL_MATERN5_ARD):
+        nu = 2.5
+    else:
+        raise ValueError("unknown kernel kind %r" % (kind,))
+    z = rng.standard_normal((F, d))
+    u = rng.chisquare(2 * nu, size=F)
+    return z * np.sqrt(2 * nu / u)[:, None]
+
+
+def path_draws(kind, d, n_features, n_paths, n_train, seed=None):
+    """the draws of GaussianProcess.sample_paths, from numpy.random.default_rng(seed) in this order: omega = spectral_draws(kind,
+    rng, F, d), phase ~ U(0, 2 pi) [F], w ~ N(0, 1) [F, S], e ~ N(0, 1) [n_train, S]"""
+    if n_features < 1 or n_paths < 1:
+        raise ValueError("n_features and n_paths must be at least 1")
+    rng = np.random.default_rng(seed)
+    omega = spectral_draws(kind, rng, n_features, d)
+    phase = rng.uniform(0.0, 2 * np.pi, n_features)
+    w = rng.standard_normal((n_features, n_paths))
+    e = rng.standard_normal((n_train, n_paths))
+    return omega, phase, w, e
+
+
+class PosteriorPaths(object):
+    """S posterior sample paths f_s(x) = mu(x) + phi(x)^T w_s - k(x)^T c_s (GaussianProcess.sample_paths): deterministic functions,
+    evaluated on the device at any number of points.  They sample the latent function (no observation noise).  A snapshot: later
+    changes to the GP do not change them."""
+
+    def __init__(self, paths):
+        self._paths = paths
+        self.n_paths = paths.S
+
+    def __call__(self, X):
+        """values F[M, S] of every path at the points X"""
+        return self._paths.eval(_as_points(X), want_values=True)[0]
+
+    def argmax(self, X):
+        """per path the maximum over the points X and its index -> (best[S], idx[S]); lowest index wins ties"""
+        _, best, idx = self._paths.eval(_as_points(X), want_values=False)
+        return best, idx
+
+    def grad(self, X, which):
+        """point j on path which[j] -> (values[M], gradients[M, d])"""
+        return self._paths.grad(_as_points(X), which)
+
+    def close(self):
+        self._paths.close()
+
+
+def _as_points(X):
+    X = np.asarray(X, dtype=float)
+    return X.reshape(-1, 1) if X.ndim == 1 else X
+
+
 class GaussianProcess(object):
 
     append_above = 256       # addData appends on the device when the resident model has at least this many points ...
@@ -230,18 +291,34 @@ class GaussianProcess(object):
             vals, dv = float(vals[0]), (dv[0] if grad else None)
         return (vals, dv) if grad else vals
 
-    def sample_max_values(self, X, n_samples=10, seed=None, floor=None, method='gumbel', jitter=0.0):
+    def sample_paths(self, n_paths, n_features=2048, seed=None):
+        """n_paths posterior sample paths by pathwise conditioning (Matheron's rule) with n_features random Fourier features of the
+        prior -> PosteriorPaths.  The draws come from numpy.random.default_rng(seed) in the order of `path_draws` (frequencies,
+        phases, w, e): a seed reproduces the paths exactly.  Unlike sample_posterior there is no limit on the number of points."""
+        if len(self.X) == 0:
+            raise ValueError("sample paths of a GP without data")
+        kind, _ = self.kernel.spec(self.X.shape[1])
+        ng = len(self.augX) if self.augX is not None else len(self.X)
+        omega, phase, w, e = path_draws(kind, self.X.shape[1], n_features, n_paths, ng, seed)
+        return PosteriorPaths(self.model.sample_paths(omega, phase, w, e))
+
+    def sample_max_values(self, X, n_samples=10, seed=None, floor=None, method='gumbel', jitter=0.0, n_features=2048):
         """samples y*[n_samples] of the maximum of f over the points in X, for max-value entropy search (`mes`).
         method='gumbel' (Wang & Jegelka 2017): the Gumbel fit of F(y) = prod_i Phi((y - mu_i) / s_i) over X
         (ibo_max_value_gumbel), y* = loc - scale log(-log u) for u from numpy.random.default_rng(seed), strictly inside (0, 1).
         method='joint': the maxima over X of joint posterior draws (sample_posterior with seed and jitter; at most 16384
-        points), which ignore no correlation.  Samples below `floor` (default max(Y)) are raised to it."""
+        points), which ignore no correlation.  method='paths': the maxima over X of sample_paths(n_samples, n_features, seed), with
+        no limit on the number of points.  Samples below `floor` (default max(Y)) are raised to it."""
         X = self._candidates(X)
         if method == 'gumbel':
             _, loc, scale = self.model.max_value_gumbel(X, _lib.FLAG_MODE_PY)
             ys = gumbel_draws(loc, scale, n_samples, seed)
         elif method == 'joint':
             ys = np.max(self.sample_posterior(X, n_samples, seed, jitter), axis=0)
+        elif method == 'paths':
+            paths = self.sample_paths(n_samples, n_features, seed)
+            ys = paths.argmax(X)[0]
+            paths.close()
         else:
             raise ValueError("unknown method %r" % (method,))
         return np.maximum(ys, np.max(self.Y) if floor is None else floor)

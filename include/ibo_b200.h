@@ -258,6 +258,41 @@ int ibo_max_value_gumbel(ibo_model* m, const double* Xs, long M, int flags, doub
 int ibo_mes(ibo_model* m, const double* Xs, long M, const double* ystar, int K, int flags,
             double* values, double* dvalues, double* best, long* best_idx);
 
+/* ---- pathwise posterior samples (Matheron's rule, Wilson et al. 2020) -------------------------------
+ * S posterior sample paths drawn from one model, each a deterministic function of x that can be evaluated at any number of points.
+ * g is the model Sigma comes from: the attached variance model if there is one, otherwise m (ibo_posterior_cov's rule); Ng is g's N.
+ * The caller supplies every random number, so the same draws reproduce the same bits:
+ *   omega[F x d]  frequencies in unit-length-scale coordinates, drawn from the kernel's spectral density (SE: N(0, I); Matern-nu:
+ *                 multivariate Student-t with 2 nu degrees of freedom, z sqrt(2 nu / u), u ~ chi^2(2 nu));
+ *   phase[F]      b_j ~ U(0, 2 pi);   w[F x S], e[Ng x S]  standard normals (row-major).
+ * With s(x) = x / theta (g's length scales, no centring; g's centre is folded into the phases on the device):
+ *   phi_j(x) = sqrt(2 sf2 / F) cos(omega_j . s(x) + b_j)
+ *   mu(x)    = m0(x) + k_m(x)^T a - m0(x) k_m(x)^T b,  a = R_m^-1 Y, b = R_m^-1 1, m0 the prior mean as ibo_posterior_batch applies it
+ *              (the mean whose derivative ibo_posterior_grad uses; it agrees with ibo_posterior_batch's mu to rounding, not bit for bit)
+ *   f_s(x)   = mu(x) + phi(x)^T w_s - k_g(x)^T R_g^-1 (Phi_g w_s + E e_s),  Phi_g = phi at g's training points, with the training
+ *              noise E e_s = sqrt(1 + noise - sf2) e_s (plain, legacy or appended g) or chol(inv(C) + (1 + noise - sf2) I) e_s (g with a
+ *              Laplace term, R_g = R + inv(C); factorised on the device at create time: the noise that R_g implies, as k(x, x) = sf2)
+ * These are samples of the LATENT function: their covariance approximates Sigma - (1 + noise - sf2) I with Sigma from
+ * ibo_posterior_cov, whereas the draws of ibo_posterior_sample carry the 1 + noise diagonal of an observation.
+ * A paths object is a snapshot: it holds copies of everything it reads (scaled training inputs of m and g, a, b, c_s, the folded
+ * phases, w, omega, the prior) and gives the same bits after ibo_model_append or ibo_model_destroy on m.  It has its own stream on m's
+ * device and does not use the model's workspace.
+ * Limits: 1 <= F <= 65536, 1 <= S <= 1024, d <= 64, M >= 1.  IBO_E_BADARG for NULL pointers, sizes out of range, sf2 > 1 + noise, or
+ * a g with a host-supplied inv(C) (ibo_model_create with Cinv) of more than 4096 points, whose inv(C) the device no longer holds.
+ * IBO_E_NOTSPD with *info = 1-based pivot when inv(C) + (1 + noise - sf2) I is not positive definite. */
+typedef struct ibo_paths ibo_paths;
+int ibo_paths_create(ibo_model* m, int F, int S, const double* omega, const double* phase, const double* w, const double* e,
+                     ibo_paths** out, int* info);
+/* values[M x S] row-major (may be NULL) at the M x d points Xs (original coordinates); best[S] / best_idx[S] (may be NULL): per path the
+ * argmax over the M points, lowest index wins ties, NaN never wins.  Each value is one fixed-order sum over the rows, so a point's values
+ * do not depend on the other points of the call and two calls give the same bits. */
+int ibo_paths_eval(ibo_paths* p, const double* Xs, long M, double* values, double* best, long* best_idx);
+/* point j on path which[j] (0 <= which[j] < S): values[M] (the same bits as ibo_paths_eval's) and the exact gradient with respect to x,
+ * grad[M x d] = d mu - sqrt(2 sf2 / F) sum_j w_j,s sin(omega_j . s + b_j) omega_j / theta - sum_i c_i,s dk_i.  Meant for few points
+ * (one thread per point).  IBO_E_BADARG for NULL pointers, M < 1 or a which outside [0, S). */
+int ibo_paths_grad(ibo_paths* p, const double* Xs, long M, const int* which, double* values, double* grad);
+int ibo_paths_destroy(ibo_paths* p);
+
 /* Candidates kept resident in HBM (the bench's device-resident leg; also used for sharded sets). */
 int ibo_cands_create(ibo_model* m, const double* Xs, long M, ibo_cands** out);
 int ibo_cands_destroy(ibo_cands* c);
