@@ -180,6 +180,9 @@ extern "C" int ibo_pref_fit(ibo_model* m, int P, const int* v, const int* u, con
     TRYS(pool_malloc((void**)&B->dBetaY, sizeof(double) * Np));
     TRYS(pool_malloc((void**)&B->dY, sizeof(double) * Np));
     TRYS(cudaMalloc(&B->dInfo, sizeof(int)));
+    // cleared here as well as by each factorisation: a start that already meets gtol runs none, and the pivot read after the
+    // loop must not see what a recycled allocation held
+    TRYS(cudaMemsetAsync(B->dInfo, 0, sizeof(int), st));
     // ---- preference index arrays + CSR (point -> its preferences, in preference order) ----
     std::vector<int> rowptr(N + 1, 0), ent(2 * (size_t)P);
     for (int p = 0; p < P; p++) { rowptr[v[p] + 1]++; rowptr[u[p] + 1]++; }
