@@ -20,7 +20,7 @@ EXPORTED = [
     "ibo_model_get_matrix", "ibo_model_set_variance_model", "ibo_pref_fit",
     "ibo_nlml", "ibo_kernel_matrix",
     "ibo_posterior_batch", "ibo_score_batch", "ibo_posterior_cov", "ibo_posterior_sample",
-    "ibo_posterior_grad", "ibo_score_grad", "ibo_qei", "ibo_max_value_gumbel", "ibo_mes",
+    "ibo_posterior_grad", "ibo_score_grad", "ibo_qei", "ibo_qnei", "ibo_max_value_gumbel", "ibo_mes",
     "ibo_paths_create", "ibo_paths_eval", "ibo_paths_grad", "ibo_paths_destroy",
     "ibo_cands_create", "ibo_cands_destroy", "ibo_score_resident", "ibo_get_profile", "ibo_launch_count",
     "ibo_fp64_peak", "ibo_i8_peak", "ibo_i8_peak2", "ibo_host_register", "ibo_host_unregister", "ibo_stream_mark", "ibo_stream_elapsed_ms",
@@ -107,6 +107,7 @@ def lib():
     L.ibo_posterior_grad.argtypes = [c_void_p, pd, c_long, c_int, pd, pd, pd, pd]
     L.ibo_score_grad.argtypes = [c_void_p, pd, c_long, c_int, c_double, c_double, c_int, pd, pd]
     L.ibo_qei.argtypes = [c_void_p, pd, c_long, c_int, pd, c_int, c_double, c_double, c_double, pd, pd, pi]
+    L.ibo_qnei.argtypes = [c_void_p, pd, c_long, c_int, pd, c_long, pd, c_int, c_double, pd, pd, pd, pi, pi]
     L.ibo_max_value_gumbel.argtypes = [c_void_p, pd, c_long, c_int, pd, pd, pd]
     L.ibo_mes.argtypes = [c_void_p, pd, c_long, pd, c_int, c_int, pd, pd, pd, pl]
     L.ibo_paths_create.argtypes = [c_void_p, c_int, c_int, pd, pd, pd, pd, POINTER(c_void_p), pi]
@@ -369,6 +370,30 @@ class Model(object):
         check(lib().ibo_qei(self._h, dptr(Xb), B, q, dptr(Z), Z.shape[1], float(ymax), float(xi), float(jitter), dptr(vals),
                             dptr(dv) if want_grad else None, ctypes.byref(nbad)))
         return vals, dv, nbad.value
+
+    def qnei(self, Xb, Xbase, Z, jitter=0.0, want_grad=True):
+        """noisy batch expected improvement of B batches of q points Xb[B, q, d] over the baseline Xbase[P, d] for standard normals
+        Z[P + q, S], baseline rows first (ibo_qnei) -> (values[B], dvalues[B, q, d] or None, number of batches whose Schur
+        complement + jitter I is not positive definite: NaN rows, incumbent draws m[S]).  Raises NotPositiveDefinite with the
+        1-based pivot when the baseline's covariance + jitter I is not positive definite."""
+        Xb = as_f64(Xb, 3)
+        Xbase = as_f64(Xbase, 2)
+        Z = as_f64(Z, 2)
+        B, q, d = Xb.shape
+        if d != self.d or Xbase.shape[1] != self.d:
+            raise ValueError("points have %d and %d columns, the model %d" % (d, Xbase.shape[1], self.d))
+        P = Xbase.shape[0]
+        if Z.shape[0] != P + q:
+            raise ValueError("Z has %d rows for %d baseline points and batches of %d" % (Z.shape[0], P, q))
+        S = Z.shape[1]
+        vals = np.empty(B)
+        dv = np.empty((B, q, d)) if want_grad else None
+        inc = np.empty(S)
+        nbad, info = c_int(0), c_int(0)
+        rc = lib().ibo_qnei(self._h, dptr(Xb), B, q, dptr(Xbase), P, dptr(Z), S, float(jitter), dptr(vals),
+                            dptr(dv) if want_grad else None, dptr(inc), ctypes.byref(nbad), ctypes.byref(info))
+        check(rc, info.value)
+        return vals, dv, nbad.value, inc
 
     def max_value_gumbel(self, Xs, flags=FLAG_MODE_CPP):
         """Gumbel fit of the distribution of the maximum over the candidates (ibo_max_value_gumbel) -> (q[3], loc, scale): q solve

@@ -307,6 +307,28 @@ def maximizeQEI(GP, bounds, q, samples=512, seed=0, xi=0.01, starts=8, pending=N
     return val, batch
 
 
+def maximizeQNEI(GP, bounds, q, baseline=None, samples=512, seed=0, starts=8, pending=None, jitter=1e-8, maxiter=100):
+    """Choose q points to evaluate in parallel by maximising their Monte-Carlo noisy batch expected improvement
+    (GaussianProcess.qNEI): the incumbent is drawn jointly over the `baseline` points (default: the distinct rows of GP.X) instead
+    of the fixed max(Y).  maximizeQEI's driver: Z is drawn once (numpy.random.default_rng(seed), P + q + p rows, `samples`
+    columns, baseline rows first); the starts are thompsonBatch(GP, bounds, q, seed=seed + k) for k < starts, polished together
+    by L-BFGS-B, one ibo_qnei call per evaluation; pending[p, d] join every batch, held fixed.  Returns (value, batch[q, d]); the
+    value is at least the best start's.  maximizeQNEI.last records the evaluations, the values of the starts and the baseline."""
+    if len(GP.X) == 0:
+        raise ValueError("q-NEI over a GP without data")
+    base = GP.qnei_baseline() if baseline is None else np.array(baseline, dtype=float, ndmin=2)
+    p = 0 if pending is None else np.array(pending, dtype=float, ndmin=2).shape[0]
+    Z = np.random.default_rng(seed).standard_normal((base.shape[0] + q + p, samples))
+    X0 = np.array([thompsonBatch(GP, bounds, q, seed=seed + k, jitter=jitter)[0] for k in range(starts)])
+
+    def fg(X):
+        v, g, _, _ = GP.model.qnei(X, base, Z, jitter)
+        return v, g
+    val, batch, v0, nfev = _polish_batches(fg, bounds, X0, pending, maxiter)
+    maximizeQNEI.last = dict(evaluations=nfev, start_values=v0, baseline=base)
+    return val, batch
+
+
 def _polish_from(fg, bounds, opt, optx, C, cvals, k, maxiter=100):
     """Gradient polish of a DIRECT answer: L-BFGS-B (_polish, fg(X) -> (values, gradients)) from DIRECT's optx and the k - 1
     candidates C with the largest values cvals.  The best polished point replaces (opt, optx) only when its value beats optx

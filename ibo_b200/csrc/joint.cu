@@ -112,6 +112,39 @@ __global__ void __launch_bounds__(256, 1) trimm_t_kernel(double* __restrict__ C,
         }
 }
 
+// Dense tile GEMM C[I][J] = alpha op(A)_I B_J (+ C[I][J] when ACC), op(A) = A^T (A stored [K][rows]) with TRANSA, else A ([rows][K]);
+// B [K][cols].  K is the full depth for every tile (a multiple of 16), so a column of C does not depend on the other columns.
+// Padding rows and columns of C are zero when A and B are zero there (and C is, with ACC).
+template <bool TRANSA, bool ACC>
+__global__ void __launch_bounds__(256, 1) gemm_kernel(double* __restrict__ C, int ldc, const double* __restrict__ A, int lda,
+                                                      const double* __restrict__ B, int ldb, int K, double alpha) {
+    extern __shared__ double sm[];
+    const int I = blockIdx.y, J = blockIdx.x;
+    double acc[8][4][2];
+#pragma unroll
+    for (int a = 0; a < 8; a++)
+#pragma unroll
+        for (int b = 0; b < 4; b++) acc[a][b][0] = acc[a][b][1] = 0.0;
+    tile_gemm_core<false, TRANSA>(TRANSA ? A + (size_t)I * 128 : A + (size_t)I * 128 * lda, lda, B + (size_t)J * 128, ldb, K, acc, sm);
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, wm = warp >> 2, wn = warp & 3;
+#pragma unroll
+    for (int mt = 0; mt < 8; mt++)
+#pragma unroll
+        for (int nt = 0; nt < 4; nt++) {
+            const int row = I * 128 + wm * 64 + mt * 8 + (lane >> 2), c = wn * 32 + nt * 8 + 2 * (lane & 3);
+            double2* p = reinterpret_cast<double2*>(C + (size_t)row * ldc + (size_t)J * 128 + c);
+            double2 v;
+            if (ACC) {
+                v = *p;
+                v.x = fma(alpha, acc[mt][nt][0], v.x);
+                v.y = fma(alpha, acc[mt][nt][1], v.y);
+            } else {
+                v = make_double2(alpha * acc[mt][nt][0], alpha * acc[mt][nt][1]);
+            }
+            *p = v;
+        }
+}
+
 // Sigma tile (I, J), J <= I, in place over R(X*, X*): S_IJ -= sum_k V_kI^T V_kJ (the transposed-A path of gram_wtw_kernel), + jitter on
 // the diagonal of the real candidates
 __global__ void __launch_bounds__(256, 1) sigma_kernel(double* __restrict__ S, const double* __restrict__ V, int Mp, int K, int M, double jitter) {
@@ -159,7 +192,9 @@ __device__ __forceinline__ bool better(double v, long long i, double bv, long lo
     if (bi < 0) return true;
     return v > bv || (v == bv && i < bi);
 }
-__global__ void __launch_bounds__(256) sample_argmax_kernel(const double* __restrict__ F, int ldf, int M, int S, long long* __restrict__ arg) {
+// best (optional) receives the maximum itself (-inf when every value is NaN).
+__global__ void __launch_bounds__(256) sample_argmax_kernel(const double* __restrict__ F, int ldf, int M, int S, long long* __restrict__ arg,
+                                                            double* __restrict__ best) {
     __shared__ double sv[8][32];
     __shared__ long long si[8][32];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, s = blockIdx.x * 32 + lane;
@@ -176,6 +211,7 @@ __global__ void __launch_bounds__(256) sample_argmax_kernel(const double* __rest
         for (int w = 1; w < 8; w++)
             if (better(sv[w][lane], si[w][lane], bv, bi)) { bv = sv[w][lane]; bi = si[w][lane]; }
         arg[s] = bi;
+        if (best) best[s] = bv;
     }
 }
 
@@ -183,6 +219,10 @@ cudaError_t set_joint_attrs() {
     cudaError_t e = cudaFuncSetAttribute(trimm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TILE_SMEM_DOUBLES * 8);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(sigma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TILE_SMEM_DOUBLES * 8);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(trimm_t_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TILE_SMEM_DOUBLES * 8);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(gemm_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, TILE_SMEM_DOUBLES * 8);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(gemm_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TILE_SMEM_DOUBLES * 8);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(gemm_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, TILE_SMEM_DOUBLES * 8);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(gemm_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TILE_SMEM_DOUBLES * 8);
     return e;
 }
 
@@ -193,42 +233,72 @@ int joint_sigma(ibo_model* m, const double* Xs, long M, double jitter, bool want
     if ((rc = ensure_joint_attrs(m->device))) return rc;
     CandWork* w = cand_work(m);
     ibo_model& c = w->chol;
-    if (!c.dInfo) {
-        c.device = m->device;
-        c.stream = m->stream; c.stream2 = m->stream2; c.stream3 = m->stream3; c.stream4 = m->stream4;
-        c.evStep = m->evStep; c.evRest = m->evRest; c.evScale = m->evScale; c.evFar = m->evFar;
-        IBO_CUDA_TRY(cudaMalloc(&c.dInfo, sizeof(int)));
-    }
     ibo_model* g = m->var_model ? m->var_model : m;      // the model sigma^2 comes from
     cudaStream_t st = m->stream;
-    const int d = m->d, Np = g->Np, Mp = (int)round128(M), nbM = Mp / 128;
+    const int d = m->d, Np = g->Np, Mp = (int)round128(M);
     const size_t Sp = (size_t)round128(S);
     if ((rc = grow(&w->dRaw, &w->rawCap, (size_t)M * d))) return rc;
     if ((rc = grow(&w->dScaled, &w->scaledCap, (size_t)Mp * d))) return rc;
     if ((rc = grow(&w->dKc, &w->kcCap, (size_t)Np * Mp))) return rc;
     if ((rc = grow(&w->dV, &w->vCap, (size_t)Np * Mp))) return rc;
     if ((rc = grow(&w->dPost, &w->postCap, (size_t)3 * M + 2))) return rc;
-    if ((rc = grow(&c.dA, &w->cholACap, (size_t)Mp * Mp))) return rc;
-    if ((rc = grow(&c.dD, &w->cholDCap, (size_t)nbM * 128 * 128))) return rc;
+    if ((rc = chol_setup(m, M, false))) return rc;
     if (S > 0) {
         if ((rc = grow(&w->dNormals, &w->normalsCap, (size_t)Mp * Sp))) return rc;
         if ((rc = grow(&w->dF, &w->fCap, (size_t)Mp * Sp))) return rc;
         if ((rc = grow(&w->dArg, &w->argCap, (size_t)S))) return rc;
     }
-    c.N = (int)M; c.Np = Mp; c.nb = nbM; c.d = d;
     IBO_CUDA_TRY(cudaMemcpyAsync(w->dRaw, Xs, sizeof(double) * (size_t)M * d, cudaMemcpyHostToDevice, st));
     if (wantMu && (rc = posterior_score_device(m, w->dRaw, M, -1, 0.0, 0.0, IBO_FLAG_FP64, w->dPost))) return rc;
     launch_scale_cands(w->dScaled, w->dRaw, g, M, Mp, st);
     launch_cross_cov(w->dKc, g, w->dScaled, (int)M, Mp, st);
     launch_w_gemm_v(w->dV, g, w->dKc, Mp, st);
-    prior_cov_kernel<<<dim3((Mp + 255) / 256, Mp), 256, 0, st>>>(c.dA, w->dScaled, (int)M, Mp, d, g->kind, g->sf2, 1.0 + g->noise);
-    sigma_kernel<<<dim3(nbM, nbM), 256, TILE_SMEM_DOUBLES * 8, st>>>(c.dA, w->dV, Mp, Np, (int)M, jitter);
-    g_launches += 2;
+    launch_joint_sigma(&c, w->dScaled, w->dV, g, 1.0 + g->noise, jitter, st);
     IBO_CUDA_TRY(cudaGetLastError());
     return IBO_OK;
 }
 
 }  // namespace
+
+int chol_setup(ibo_model* m, long M, bool invert) {
+    int rc;
+    CandWork* w = cand_work(m);
+    ibo_model& c = w->chol;
+    if (!c.dInfo) {
+        c.device = m->device;
+        c.stream = m->stream; c.stream2 = m->stream2; c.stream3 = m->stream3; c.stream4 = m->stream4;
+        c.evStep = m->evStep; c.evRest = m->evRest; c.evScale = m->evScale; c.evFar = m->evFar;
+        IBO_CUDA_TRY(cudaMalloc(&c.dInfo, sizeof(int)));
+    }
+    const int Mp = (int)round128(M), nbM = Mp / 128;
+    if ((rc = grow(&c.dA, &w->cholACap, (size_t)Mp * Mp))) return rc;
+    if ((rc = grow(&c.dD, &w->cholDCap, (size_t)nbM * 128 * 128))) return rc;
+    if (invert) {
+        if ((rc = grow(&c.dW, &w->cholWCap, (size_t)Mp * Mp))) return rc;
+        if ((rc = grow(&c.dY, &w->cholYCap, (size_t)2 * Mp))) return rc;
+        c.dBetaY = c.dY + Mp;
+        IBO_CUDA_TRY(cudaMemsetAsync(c.dY, 0, sizeof(double) * Mp, m->stream));
+    }
+    c.N = (int)M; c.Np = Mp; c.nb = nbM; c.d = m->d;
+    return IBO_OK;
+}
+
+void launch_joint_sigma(ibo_model* c, const double* Cs, const double* V, const ibo_model* g, double diag, double jitter, cudaStream_t st) {
+    const int Mp = c->Np;
+    prior_cov_kernel<<<dim3((Mp + 255) / 256, Mp), 256, 0, st>>>(c->dA, Cs, c->N, Mp, g->d, g->kind, g->sf2, diag);
+    sigma_kernel<<<dim3(c->nb, c->nb), 256, TILE_SMEM_DOUBLES * 8, st>>>(c->dA, V, Mp, g->Np, c->N, jitter);
+    g_launches += 2;
+}
+
+void launch_clear_diag_upper(ibo_model* c, cudaStream_t st) {
+    zero_diag_upper_kernel<<<c->nb, 256, 0, st>>>(c->dA, c->Np);
+    g_launches++;
+}
+
+void launch_sample_max(const double* F, int ldf, int M, int S, long long* arg, double* best, cudaStream_t st) {
+    sample_argmax_kernel<<<(S + 31) / 32, 256, 0, st>>>(F, ldf, M, S, arg, best);
+    g_launches++;
+}
 
 int check_cands(const ibo_model* m, const double* Xs, long M, bool extra_ok) {
     if (!m || !Xs || M < 1 || !extra_ok) { set_error("bad argument"); return IBO_E_BADARG; }
@@ -256,6 +326,32 @@ void launch_w_gemm_v(double* V, const ibo_model* g, const double* Kc, int Mp, cu
 }
 void launch_w_gemm_z(double* Z, const ibo_model* g, const double* V, int Mp, cudaStream_t st) {
     trimm_t_kernel<<<dim3(Mp / 128, g->nb), 256, TILE_SMEM_DOUBLES * 8, st>>>(Z, Mp, g->dW, g->Np, V, Mp, g->nb);
+    g_launches++;
+}
+void launch_cross_cov_pts(double* Kc, const double* Xa, int Na, int Nap, const ibo_model* g, const double* Cs, int M, int Mp, cudaStream_t st) {
+    cross_cov_kernel<<<dim3((Mp + 255) / 256, Nap), 256, 0, st>>>(Kc, Xa, Cs, Na, M, Mp, g->d, g->kind, g->sf2);
+    g_launches++;
+}
+void launch_trimm(double* C, int ldc, const double* T, int ldt, const double* B, int ldb, int nbr, int cols, const double* bias, int nbias,
+                  cudaStream_t st) {
+    trimm_kernel<<<dim3(cols / 128, nbr), 256, TILE_SMEM_DOUBLES * 8, st>>>(C, ldc, T, ldt, B, ldb, nbr, bias, nbias);
+    g_launches++;
+}
+void launch_trimm_t(double* C, int ldc, const double* T, int ldt, const double* B, int ldb, int nbr, int cols, cudaStream_t st) {
+    trimm_t_kernel<<<dim3(cols / 128, nbr), 256, TILE_SMEM_DOUBLES * 8, st>>>(C, ldc, T, ldt, B, ldb, nbr);
+    g_launches++;
+}
+void launch_gemm(double* C, int ldc, const double* A, int lda, bool transA, const double* B, int ldb, int rows, int cols, int K,
+                 double alpha, bool acc, cudaStream_t st) {
+    const dim3 grid(cols / 128, rows / 128);
+    const int sm = TILE_SMEM_DOUBLES * 8;
+    if (transA) {
+        if (acc) gemm_kernel<true, true><<<grid, 256, sm, st>>>(C, ldc, A, lda, B, ldb, K, alpha);
+        else gemm_kernel<true, false><<<grid, 256, sm, st>>>(C, ldc, A, lda, B, ldb, K, alpha);
+    } else {
+        if (acc) gemm_kernel<false, true><<<grid, 256, sm, st>>>(C, ldc, A, lda, B, ldb, K, alpha);
+        else gemm_kernel<false, false><<<grid, 256, sm, st>>>(C, ldc, A, lda, B, ldb, K, alpha);
+    }
     g_launches++;
 }
 
@@ -304,16 +400,15 @@ extern "C" int ibo_posterior_sample(ibo_model* m, const double* Xs, long M, cons
         set_error("posterior covariance + jitter I is not positive definite (pivot " + std::to_string(hinfo) + ")");
         return IBO_E_NOTSPD;
     }
-    zero_diag_upper_kernel<<<nbM, 256, 0, st>>>(w->chol.dA, Mp);
+    launch_clear_diag_upper(&w->chol, st);
     IBO_CUDA_TRY(cudaMemsetAsync(w->dNormals, 0, sizeof(double) * (size_t)Mp * Sp, st));
     IBO_CUDA_TRY(cudaMemcpy2DAsync(w->dNormals, sizeof(double) * Sp, Z, sizeof(double) * S, sizeof(double) * S, M, cudaMemcpyHostToDevice, st));
     trimm_kernel<<<dim3(Sp / 128, nbM), 256, TILE_SMEM_DOUBLES * 8, st>>>(w->dF, Sp, w->chol.dA, Mp, w->dNormals, Sp, nbM, w->dPost + M, (int)M);
-    g_launches += 2;
+    g_launches++;
     long long* dArg = reinterpret_cast<long long*>(w->dArg);
     std::vector<long long> harg(argmax ? S : 0);
     if (argmax) {
-        sample_argmax_kernel<<<(S + 31) / 32, 256, 0, st>>>(w->dF, Sp, (int)M, S, dArg);
-        g_launches++;
+        launch_sample_max(w->dF, Sp, (int)M, S, dArg, nullptr, st);
         IBO_CUDA_TRY(cudaMemcpyAsync(harg.data(), dArg, sizeof(long long) * S, cudaMemcpyDeviceToHost, st));
     }
     if (F) IBO_CUDA_TRY(cudaMemcpy2DAsync(F, sizeof(double) * S, w->dF, sizeof(double) * Sp, sizeof(double) * S, M, cudaMemcpyDeviceToHost, st));

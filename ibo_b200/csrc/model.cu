@@ -966,7 +966,8 @@ static void free_cand_work(ibo_model* m) {
     CandWork* w = m->cand;
     if (!w) return;
     double** ptrs[] = {&w->dRaw, &w->dScaled, &w->dScaledM, &w->dKc, &w->dV, &w->dAB, &w->dKb, &w->dG, &w->dNormals, &w->dPost,
-                       &w->chol.dA, &w->chol.dD, &w->dF, &w->dArg, &w->dQei, &w->dMubar, &w->dSig, &w->dGbar, &w->dYstar, &w->dMesD, &w->dBlk};
+                       &w->chol.dA, &w->chol.dD, &w->dF, &w->dArg, &w->dQei, &w->dMubar, &w->dSig, &w->dGbar, &w->dYstar, &w->dMesD, &w->dBlk,
+                       &w->chol.dW, &w->chol.dY, &w->dBase, &w->dVb, &w->dZbase, &w->dZb, &w->dFb, &w->dCT, &w->dH};
     for (auto p : ptrs) if (*p) pool_free(*p);
     if (w->chol.dInfo) cudaFree(w->chol.dInfo);
     delete w;

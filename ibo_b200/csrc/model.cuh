@@ -96,7 +96,9 @@ struct CandWork {
                                                        // the score plane, best value and index at 3 M); mu [M] (q-EI)
     // joint posterior only
     ibo_model chol;                                    // Sigma in chol.dA (Mp x Mp), factorised in place; its streams and events are the owner's
+                                                       // (q-NEI: Sigma of the baseline, with W = inv(L) in chol.dW)
     size_t cholACap = 0, cholDCap = 0;                 // chol.dA, chol.dD
+    size_t cholWCap = 0, cholYCap = 0;                 // chol.dW; chol.dY (zeros) | chol.dBetaY [2][Mp], when inverted
     double* dF = nullptr;       size_t fCap = 0;       // samples [Mp][Sp]
     double* dArg = nullptr;     size_t argCap = 0;     // per-sample argmax (long long)
     // q-EI only
@@ -104,6 +106,14 @@ struct CandWork {
     double* dMubar = nullptr;   size_t mubarCap = 0;   // d qEI / d mu [M]
     double* dSig = nullptr;     size_t sigCap = 0;     // Sigma of the chunk's batches [Bc][q][q]
     double* dGbar = nullptr;    size_t gbarCap = 0;    // Gbar of the chunk's batches [Bc][q][q]
+    // q-NEI only (the per-batch buffers of q-EI above too; V grows to [Np + Pp][Mcp]: T below V, then Cbar in T's place)
+    double* dBase = nullptr;    size_t baseCap = 0;    // baseline raw [P][d] | scaled like g [Pp][d] | mu_b [Pp] | incumbent m [Sp]
+    double* dVb = nullptr;      size_t vbCap = 0;      // V_b = W_g K(X_g, X_b) [Np][Pp]
+    double* dZbase = nullptr;   size_t zbaseCap = 0;   // Z_b = W_g^T V_b [Np][Pp] (gradient only)
+    double* dZb = nullptr;      size_t zbCap = 0;      // baseline normals Z_b [Pp][Sp] zero padded
+    double* dFb = nullptr;      size_t fbCap = 0;      // baseline draws F_b [Pp][Sp]
+    double* dCT = nullptr;      size_t ctCap = 0;      // C = Sigma_bq, then Tbar [Pp][Mcp]
+    double* dH = nullptr;       size_t hCap = 0;       // H = Z_b^T T, then the winner indicator E [Sp][Mcp]
     // max-value entropy search only
     double* dYstar = nullptr;   size_t ystarCap = 0;   // y* samples [K]
     double* dMesD = nullptr;    size_t mesDCap = 0;    // d MES / d mu | d MES / d s [2][M]
@@ -158,6 +168,26 @@ void launch_scale_cands(double* Cs, const double* X, const ibo_model* g, long M,
 void launch_cross_cov(double* Kc, const ibo_model* g, const double* Cs, int M, int Mp, cudaStream_t st);
 void launch_w_gemm_v(double* V, const ibo_model* g, const double* Kc, int Mp, cudaStream_t st);
 void launch_w_gemm_z(double* Z, const ibo_model* g, const double* V, int Mp, cudaStream_t st);
+// joint.cu: the workspace's Cholesky model (chol) shaped for an M x M matrix, with the owner's streams and events; invert: also
+// chol.dW and the vectors launch_factorize(.., invert = true) reads and writes
+int chol_setup(ibo_model* m, long M, bool invert);
+// joint.cu, on st: chol.dA (lower tiles) = R(X*, X*) with `diag` on the diagonal, kernel of g elsewhere, - V^T V (K = g->Np) + jitter I
+void launch_joint_sigma(ibo_model* c, const double* Cs, const double* V, const ibo_model* g, double diag, double jitter, cudaStream_t st);
+// joint.cu, on st: zeros above the diagonal inside the diagonal blocks of a factorised chol.dA
+void launch_clear_diag_upper(ibo_model* c, cudaStream_t st);
+// joint.cu, on st: per column s < S of F ([M][ldf]) the argmax (lowest index wins, NaN never wins) and, when best is non-null, the max
+void launch_sample_max(const double* F, int ldf, int M, int S, long long* arg, double* best, cudaStream_t st);
+// joint.cu, on st: Kc[i][j] = k(xa_i, x*_j) with g's kernel for the Na points Xa scaled like g, exact zeros in the padding ([Nap][Mp])
+void launch_cross_cov_pts(double* Kc, const double* Xa, int Na, int Nap, const ibo_model* g, const double* Cs, int M, int Mp, cudaStream_t st);
+// joint.cu, on st: the DMMA triangular GEMMs with explicit operands: C = T B (T lower block-triangular, nbr block rows, + bias[row]
+// for rows < nbias) and C = T^T B; cols a multiple of 128
+void launch_trimm(double* C, int ldc, const double* T, int ldt, const double* B, int ldb, int nbr, int cols, const double* bias, int nbias,
+                  cudaStream_t st);
+void launch_trimm_t(double* C, int ldc, const double* T, int ldt, const double* B, int ldb, int nbr, int cols, cudaStream_t st);
+// joint.cu, on st: dense DMMA GEMM C = alpha op(A) B (+ C with acc), op(A) = A^T (A [K][rows]) with transA, else A [rows][K]; B [K][cols];
+// rows, cols multiples of 128, K of 16; every column of C runs over the full K in the same order
+void launch_gemm(double* C, int ldc, const double* A, int lda, bool transA, const double* B, int ldb, int rows, int cols, int K,
+                 double alpha, bool acc, cudaStream_t st);
 // grad.cu: candidates per chunk of the gradient and q-EI paths, the largest multiple of 128 whose K* / Z and V over g's training
 // points (2 Np doubles per candidate) fit in 512 MiB
 long cand_chunk(const ibo_model* g);

@@ -19,6 +19,7 @@
 #include "scoremath.cuh"
 #include <algorithm>
 #include <cmath>
+#include <string>
 
 namespace ibo {
 
@@ -94,11 +95,14 @@ __global__ void __launch_bounds__(256) qei_sigma_kernel(double* __restrict__ Sig
 // order.  GRAD: per warp, lane k adds z_k,s to Lbar[j*][k]; the warps' Lbar are added in warp order, and warp 0 runs the reverse
 // Cholesky Gbar = sym(L^-T Phi(L^T Lbar) L^-1) (Phi: lower triangle, halved diagonal).  The value path is the same code with
 // and without GRAD.  A batch whose factorisation fails gets NaN for its value, mubar and Gbar.
-template <bool GRAD>
+// NEI (q-NEI): F_s,j = (mu_j + H[s][b q + j]) + (L z_s)_j and the improvement is max_j F_s,j - mb[s]; GRAD then overwrites the batch's
+// columns of H with the winner indicator E[s][b q + j] = 1 / S (improving sample s, j = j*), else 0, rows S .. Sp - 1 included.
+template <bool GRAD, bool NEI = false>
 __global__ void __launch_bounds__(QW * 32) qei_batch_kernel(const double* __restrict__ Sig, const double* __restrict__ mu,
                                                             const double* __restrict__ Z, int S, int q, double ymax, double xi,
                                                             double jitter, double* __restrict__ val, double* __restrict__ mubar,
-                                                            double* __restrict__ Gbar) {
+                                                            double* __restrict__ Gbar, double* __restrict__ H = nullptr, int ldh = 0,
+                                                            const double* __restrict__ mb = nullptr, int Sp = 0) {
     __shared__ double L[QEI_MAX_Q][QEI_MAX_Q + 1];
     __shared__ double Lb[GRAD ? QW : 1][QEI_MAX_Q][QEI_MAX_Q + 1];
     __shared__ double wacc[QW];
@@ -146,6 +150,7 @@ __global__ void __launch_bounds__(QW * 32) qei_batch_kernel(const double* __rest
     for (int s = warp; s < S; s += QW) {
         const double zk = live ? Z[(size_t)lane * S + s] : 0.0;
         double f = muj;
+        if (NEI && live) f = muj + H[(size_t)s * ldh + (size_t)b * q + lane];
         for (int k = 0; k < q; k++) {
             const double zz = __shfl_sync(0xffffffffu, zk, k);
             if (k <= lane && live) f = fma(L[lane][k], zz, f);
@@ -158,13 +163,16 @@ __global__ void __launch_bounds__(QW * 32) qei_batch_kernel(const double* __rest
             const int oi = __shfl_xor_sync(0xffffffffu, ix, off);
             if (ov > v || (ov == v && oi < ix)) { v = ov; ix = oi; }
         }
-        const double imp = __dsub_rn(__dsub_rn(v, ymax), xi);
+        const double imp = NEI ? __dsub_rn(v, mb[s]) : __dsub_rn(__dsub_rn(v, ymax), xi);
         acc = __dadd_rn(acc, imp > 0.0 ? imp : 0.0);
+        if (GRAD && NEI && live) H[(size_t)s * ldh + (size_t)b * q + lane] = imp > 0.0 && lane == ix ? 1.0 / S : 0.0;
         if (GRAD && imp > 0.0) {
             if (lane <= ix) Lb[warp][ix][lane] += zk;
             if (lane == ix) c++;
         }
     }
+    if (GRAD && NEI && live)
+        for (int s = S + warp; s < Sp; s += QW) H[(size_t)s * ldh + (size_t)b * q + lane] = 0.0;
     if (lane == 0) wacc[warp] = acc;
     if (GRAD && live) cnt[warp][lane] = c;
     __syncthreads();
@@ -258,7 +266,9 @@ __global__ void __launch_bounds__(256) qei_mean_kernel(double* __restrict__ mu, 
     mu[j] = A;
 }
 
-// y[i][j] = sum_l Zm[i][b q + l] Gbar_b[j - b q][l] for the training points i < N and the chunk's points j (b = j / q)
+// y[i][j] = sum_l Zm[i][b q + l] Gbar_b[j - b q][l] for the rows i < gridDim.y and the chunk's points j (b = j / q); SUB2 (q-NEI's
+// Tbar): y[i][j] -= 2 (that) in place
+template <bool SUB2 = false>
 __global__ void __launch_bounds__(256) qei_y_kernel(double* __restrict__ Y, const double* __restrict__ Zm, int ld,
                                                     const double* __restrict__ Gbar, int Mc, int q) {
     const int j = blockIdx.x * 256 + threadIdx.x, i = blockIdx.y;
@@ -268,13 +278,18 @@ __global__ void __launch_bounds__(256) qei_y_kernel(double* __restrict__ Y, cons
     const double* g = Gbar + (size_t)b * q * q + (size_t)jj * q;
     double s = 0.0;
     for (int l = 0; l < q; l++) s = fma(z[l], g[l], s);
-    Y[(size_t)i * ld + j] = s;
+    if (SUB2) Y[(size_t)i * ld + j] = fma(-2.0, s, Y[(size_t)i * ld + j]);
+    else Y[(size_t)i * ld + j] = s;
 }
 
 // One thread per point of the chunk, in place over its row of plane 0 (sum_i y_i dk_i): -2 (that) + 2 sum_{l != j} Gbar_jl d1 k(x_j, x_l)
-// with d1 k(x_j, x_l) / dx_t = -(1 / theta_t) h(r) (s_j,t - s_l,t) in g's scaled coordinates Cs
+// with d1 k(x_j, x_l) / dx_t = -(1 / theta_t) h(r) (s_j,t - s_l,t) in g's scaled coordinates Cs.  BASE (q-NEI): then
+// + sum_{i < P} Cbar[i][j] d1 k(x_j, xb_i) over the baseline Cb, scaled like Cs
+template <bool BASE = false>
 __global__ void __launch_bounds__(256) qei_pair_kernel(double* __restrict__ G, const double* __restrict__ Cs, const double* __restrict__ Gbar,
-                                                       int Mc, int q, int d, int kind, double sf2, const double* __restrict__ inv_theta) {
+                                                       int Mc, int q, int d, int kind, double sf2, const double* __restrict__ inv_theta,
+                                                       const double* __restrict__ Cb = nullptr, const double* __restrict__ Cbar = nullptr,
+                                                       int ldcb = 0, int P = 0) {
     const int j = blockIdx.x * 256 + threadIdx.x;
     if (j >= Mc) return;
     const int b = j / q, jj = j - b * q;
@@ -290,6 +305,15 @@ __global__ void __launch_bounds__(256) qei_pair_kernel(double* __restrict__ G, c
         const double w = 2.0 * Gbar[(size_t)b * q * q + (size_t)jj * q + l] * cov_grad_h(kind, sf2, r2, &k);
         for (int t = 0; t < d; t++) g[t] = fma(-inv_theta[t] * w, xj[t] - xl[t], g[t]);
     }
+    if (BASE)
+        for (int i = 0; i < P; i++) {
+            const double* xb = Cb + (size_t)i * d;
+            double r2 = 0;
+            for (int t = 0; t < d; t++) { const double df = xj[t] - xb[t]; r2 = fma(df, df, r2); }
+            double k;
+            const double w = Cbar[(size_t)i * ldcb + j] * cov_grad_h(kind, sf2, r2, &k);
+            for (int t = 0; t < d; t++) g[t] = fma(-inv_theta[t] * w, xj[t] - xb[t], g[t]);
+        }
 }
 
 // One thread per point: plane 0 += mubar dmu, dmu = plane 1 (+ plane 2 with a prior)
@@ -375,6 +399,139 @@ int qei_device(ibo_model* m, const double* Xs, long B, int q, const double* Z, i
     return IBO_OK;
 }
 
+// q-NEI: points per chunk, the largest multiple of 128 whose K* and V (Np each), C and T (Pp each) and H (Sp) fit in 2^26 doubles
+long qnei_chunk(const ibo_model* g, long P, int S) {
+    return std::max(128L, (long)((1L << 26) / (2L * g->Np + 2 * round128(P) + round128(S))) / 128 * 128);
+}
+
+// Enqueues everything on m->stream and leaves the values in w->dQei, the incumbent draws m_s at the end of w->dBase and, with
+// wantGrad, the gradient [M][d] in w->dG.  The baseline's factorisation is checked on the host: IBO_E_NOTSPD with *info = its pivot.
+int qnei_device(ibo_model* m, const double* Xs, long B, int q, const double* Xbase, long P, const double* Z, int S, double jitter,
+                bool wantGrad, int* info) {
+    int rc;
+    if ((rc = ensure_joint_attrs(m->device))) return rc;
+    CandWork* w = cand_work(m);
+    ibo_model* vm = m->var_model;
+    ibo_model* g = vm ? vm : m;                          // the model Sigma comes from
+    cudaStream_t st = m->stream;
+    const int d = m->d, Np = g->Np, Pi = (int)P, Pp = (int)round128(P), Sp = (int)round128(S), nbP = Pp / 128;
+    const bool prior = m->npb > 0;
+    const long M = B * q;
+    const long Bc = qnei_chunk(g, P, S) / q;             // whole batches per chunk
+    const long Bcap = std::min(B, Bc), Mcap = round128(Bcap * q);
+    if ((rc = grow(&w->dRaw, &w->rawCap, (size_t)M * d))) return rc;
+    if ((rc = grow(&w->dNormals, &w->normalsCap, (size_t)q * S))) return rc;
+    if ((rc = grow(&w->dPost, &w->postCap, (size_t)M))) return rc;
+    if ((rc = grow(&w->dAB, &w->abCap, (size_t)2 * m->Np))) return rc;
+    if (vm && (rc = grow(&w->dScaledM, &w->scaledMCap, (size_t)std::max<long>(Mcap, Pp) * d))) return rc;
+    if ((rc = grow(&w->dQei, &w->qeiCap, (size_t)B))) return rc;
+    if ((rc = grow(&w->dSig, &w->sigCap, (size_t)Bcap * q * q))) return rc;
+    if ((rc = grow(&w->dScaled, &w->scaledCap, (size_t)Mcap * d))) return rc;
+    if ((rc = grow(&w->dKc, &w->kcCap, (size_t)Np * std::max<long>(Mcap, Pp)))) return rc;
+    if ((rc = grow(&w->dV, &w->vCap, (size_t)(Np + Pp) * Mcap))) return rc;
+    if ((rc = grow(&w->dBase, &w->baseCap, (size_t)P * d + (size_t)Pp * d + Pp + Sp))) return rc;
+    if ((rc = grow(&w->dVb, &w->vbCap, (size_t)Np * Pp))) return rc;
+    if ((rc = grow(&w->dZb, &w->zbCap, (size_t)Pp * Sp))) return rc;
+    if ((rc = grow(&w->dFb, &w->fbCap, (size_t)Pp * Sp))) return rc;
+    if ((rc = grow(&w->dCT, &w->ctCap, (size_t)Pp * Mcap))) return rc;
+    if ((rc = grow(&w->dH, &w->hCap, (size_t)Sp * Mcap))) return rc;
+    if ((rc = grow(&w->dArg, &w->argCap, (size_t)S))) return rc;
+    if (wantGrad) {
+        if ((rc = grow(&w->dZbase, &w->zbaseCap, (size_t)Np * Pp))) return rc;
+        if ((rc = grow(&w->dMubar, &w->mubarCap, (size_t)M))) return rc;
+        if ((rc = grow(&w->dG, &w->gCap, (size_t)3 * M * d))) return rc;
+        if ((rc = grow(&w->dGbar, &w->gbarCap, (size_t)Bcap * q * q))) return rc;
+        if (prior && (rc = grow(&w->dKb, &w->kbCap, (size_t)M))) return rc;
+    }
+    if ((rc = chol_setup(m, P, true))) return rc;
+    ibo_model* const c = &w->chol;
+    double* const baseRaw = w->dBase;
+    double* const baseS = baseRaw + (size_t)P * d;
+    double* const mub = baseS + (size_t)Pp * d;
+    double* const mmax = mub + Pp;
+    IBO_CUDA_TRY(cudaMemcpyAsync(w->dRaw, Xs, sizeof(double) * (size_t)M * d, cudaMemcpyHostToDevice, st));
+    IBO_CUDA_TRY(cudaMemcpyAsync(baseRaw, Xbase, sizeof(double) * (size_t)P * d, cudaMemcpyHostToDevice, st));
+    IBO_CUDA_TRY(cudaMemcpyAsync(w->dNormals, Z + (size_t)P * S, sizeof(double) * (size_t)q * S, cudaMemcpyHostToDevice, st));
+    IBO_CUDA_TRY(cudaMemsetAsync(w->dZb, 0, sizeof(double) * (size_t)Pp * Sp, st));
+    IBO_CUDA_TRY(cudaMemcpy2DAsync(w->dZb, sizeof(double) * Sp, Z, sizeof(double) * S, sizeof(double) * S, P, cudaMemcpyHostToDevice, st));
+    double* const mu = w->dPost;
+    double* const dA = w->dAB;
+    double* const dB = launch_ab(m, w->dAB, st);
+    // once per call: the baseline's mean, V_b, Sigma_bb = L_bb L_bb^T, W_bb = inv(L_bb), F_b = mu_b 1^T + L_bb Z_b and m_s
+    launch_scale_cands(baseS, baseRaw, g, P, Pp, st);
+    if (vm) launch_scale_cands(w->dScaledM, baseRaw, m, P, Pp, st);
+    qei_mean_kernel<<<(Pi + 31) / 32, 256, 0, st>>>(mub, m->dXt, m->N, vm ? w->dScaledM : baseS, baseRaw, Pi, d, m->kind, m->sf2, dA, dB,
+                                                    m->npb, m->dPmeans, m->dPbeta, m->ptheta, m->dPlb, m->dPwidth);
+    g_launches++;
+    launch_cross_cov(w->dKc, g, baseS, Pi, Pp, st);
+    launch_w_gemm_v(w->dVb, g, w->dKc, Pp, st);
+    if (wantGrad) launch_w_gemm_z(w->dZbase, g, w->dVb, Pp, st);                                 // R_g^-1 K(X_g, X_b)
+    launch_joint_sigma(c, baseS, w->dVb, g, g->sf2, jitter, st);
+    if ((rc = launch_factorize(c, false, false, true))) return rc;
+    int hinfo = 0;
+    IBO_CUDA_TRY(cudaMemcpyAsync(&hinfo, c->dInfo, sizeof(int), cudaMemcpyDeviceToHost, st));
+    IBO_CUDA_TRY(cudaStreamSynchronize(st));
+    if (hinfo != 0) {
+        if (info) *info = hinfo;
+        set_error("baseline covariance + jitter I is not positive definite (pivot " + std::to_string(hinfo) + ")");
+        return IBO_E_NOTSPD;
+    }
+    launch_clear_diag_upper(c, st);
+    launch_trimm(w->dFb, Sp, c->dA, Pp, w->dZb, Sp, nbP, Sp, mub, Pi, st);
+    launch_sample_max(w->dFb, Sp, Pi, S, reinterpret_cast<long long*>(w->dArg), mmax, st);
+    const size_t plane = (size_t)M * d;
+    for (long b0 = 0; b0 < B; b0 += Bc) {
+        const int nbt = (int)std::min(Bc, B - b0), Mc = nbt * q, Mcp = (int)round128(Mc);
+        const long c0 = b0 * q;
+        const double* raw = w->dRaw + (size_t)c0 * d;
+        double* const T = w->dV + (size_t)Np * Mcp;               // T = W_bb C below V_q, then Cbar
+        launch_scale_cands(w->dScaled, raw, g, Mc, Mcp, st);
+        if (vm) launch_scale_cands(w->dScaledM, raw, m, Mc, Mcp, st);
+        const double* Cm = vm ? w->dScaledM : w->dScaled;
+        qei_mean_kernel<<<(Mc + 31) / 32, 256, 0, st>>>(mu + c0, m->dXt, m->N, Cm, raw, Mc, d, m->kind, m->sf2, dA, dB, m->npb,
+                                                        m->dPmeans, m->dPbeta, m->ptheta, m->dPlb, m->dPwidth);
+        g_launches++;
+        launch_cross_cov(w->dKc, g, w->dScaled, Mc, Mcp, st);
+        launch_w_gemm_v(w->dV, g, w->dKc, Mcp, st);
+        launch_cross_cov_pts(w->dCT, baseS, Pi, Pp, g, w->dScaled, Mc, Mcp, st);                  // C = K(X_b, X_q) - V_b^T V_q
+        launch_gemm(w->dCT, Mcp, w->dVb, Pp, true, w->dV, Mcp, Pp, Mcp, Np, -1.0, true, st);
+        launch_trimm(T, Mcp, c->dW, Pp, w->dCT, Mcp, nbP, Mcp, nullptr, 0, st);                   // T = W_bb C
+        launch_gemm(w->dH, Mcp, w->dZb, Sp, true, T, Mcp, Sp, Mcp, Pp, 1.0, false, st);           // H = Z_b^T T
+        // Schur complements Sigma_qq - T^T T: the rows of [V_q; T] (V_q's padding rows are zero)
+        qei_sigma_kernel<<<nbt, 256, 0, st>>>(w->dSig, w->dV, Mcp, w->dScaled, Np + Pi, q, d, g->kind, g->sf2, g->sf2);
+        g_launches++;
+        if (!wantGrad) {
+            qei_batch_kernel<false, true><<<nbt, QW * 32, 0, st>>>(w->dSig, mu + c0, w->dNormals, S, q, 0.0, 0.0, jitter, w->dQei + b0,
+                                                                  nullptr, nullptr, w->dH, Mcp, mmax, Sp);
+            g_launches++;
+            continue;
+        }
+        qei_batch_kernel<true, true><<<nbt, QW * 32, 0, st>>>(w->dSig, mu + c0, w->dNormals, S, q, 0.0, 0.0, jitter, w->dQei + b0,
+                                                             w->dMubar + c0, w->dGbar, w->dH, Mcp, mmax, Sp);
+        g_launches++;
+        launch_gemm(w->dCT, Mcp, w->dZb, Sp, false, w->dH, Mcp, Pp, Mcp, Sp, 1.0, false, st);     // Tbar = Z_b E - 2 T Gbar
+        qei_y_kernel<true><<<dim3((Mc + 255) / 256, Pi), 256, 0, st>>>(w->dCT, T, Mcp, w->dGbar, Mc, q);
+        g_launches++;
+        launch_trimm_t(T, Mcp, c->dW, Pp, w->dCT, Mcp, nbP, Mcp, st);                             // Cbar = W_bb^T Tbar
+        launch_w_gemm_z(w->dKc, g, w->dV, Mcp, st);                                               // y = Z_q Gbar + Z_b Cbar / 2
+        qei_y_kernel<<<dim3((Mc + 255) / 256, g->N), 256, 0, st>>>(w->dV, w->dKc, Mcp, w->dGbar, Mc, q);
+        g_launches++;
+        launch_gemm(w->dV, Mcp, w->dZbase, Pp, false, T, Mcp, Np, Mcp, Pp, 0.5, true, st);
+        double* G = w->dG + (size_t)c0 * d;
+        launch_grad_sums(m, w->dScaled, w->dScaledM, Mc, w->dV, Mcp, dA, dB, G, plane, prior ? w->dKb + c0 : nullptr, st);
+        qei_pair_kernel<true><<<(Mc + 255) / 256, 256, 0, st>>>(G, w->dScaled, w->dGbar, Mc, q, d, g->kind, g->sf2, g->dInvTheta, baseS, T,
+                                                                Mcp, Pi);
+        g_launches++;
+    }
+    if (wantGrad) {
+        if (prior) launch_grad_prior(m, w->dRaw, M, w->dKb, w->dG, st);
+        qei_epilogue_kernel<<<(unsigned)((M + 255) / 256), 256, 0, st>>>(w->dG, M, d, w->dMubar, prior ? 1 : 0);
+        g_launches++;
+    }
+    IBO_CUDA_TRY(cudaGetLastError());
+    return IBO_OK;
+}
+
 }  // namespace
 
 }  // namespace ibo
@@ -393,6 +550,35 @@ extern "C" int ibo_qei(ibo_model* m, const double* Xs, long B, int q, const doub
     cudaStream_t st = m->stream;
     IBO_CUDA_TRY(cudaMemcpyAsync(values, w->dQei, sizeof(double) * B, cudaMemcpyDeviceToHost, st));
     if (dvalues) IBO_CUDA_TRY(cudaMemcpyAsync(dvalues, w->dG, sizeof(double) * (size_t)B * q * m->d, cudaMemcpyDeviceToHost, st));
+    IBO_CUDA_TRY(cudaStreamSynchronize(st));
+    IBO_CUDA_TRY(cudaGetLastError());
+    if (nbad)
+        for (long b = 0; b < B; b++) *nbad += std::isnan(values[b]) ? 1 : 0;
+    return IBO_OK;
+}
+
+extern "C" int ibo_qnei(ibo_model* m, const double* Xs, long B, int q, const double* Xbase, long P, const double* Z, int S, double jitter,
+                        double* values, double* dvalues, double* incumbent, int* nbad, int* info) {
+    if (nbad) *nbad = 0;
+    if (info) *info = 0;
+    bool ok = Xbase && Z && values && q >= 1 && q <= QEI_MAX_Q && P >= 1 && P <= 8192 && S >= 1 && S <= 8192 && jitter >= 0.0;   // NaN jitter fails
+    if (ok && m) {
+        const ibo_model* g = m->var_model ? m->var_model : m;
+        ok = g->sf2 <= 1.0 + g->noise;                   // the latent covariance is PSD only then
+    }
+    int rc = check_cands(m, Xs, B, ok);
+    if (rc) return rc;
+    IBO_CUDA_TRY(cudaSetDevice(m->device));
+    rc = qnei_device(m, Xs, B, q, Xbase, P, Z, S, jitter, dvalues != nullptr, info);
+    if (rc) return rc;
+    CandWork* w = m->cand;
+    cudaStream_t st = m->stream;
+    IBO_CUDA_TRY(cudaMemcpyAsync(values, w->dQei, sizeof(double) * B, cudaMemcpyDeviceToHost, st));
+    if (dvalues) IBO_CUDA_TRY(cudaMemcpyAsync(dvalues, w->dG, sizeof(double) * (size_t)B * q * m->d, cudaMemcpyDeviceToHost, st));
+    if (incumbent) {
+        const double* mmax = w->dBase + (size_t)P * m->d + (size_t)round128(P) * m->d + round128(P);
+        IBO_CUDA_TRY(cudaMemcpyAsync(incumbent, mmax, sizeof(double) * S, cudaMemcpyDeviceToHost, st));
+    }
     IBO_CUDA_TRY(cudaStreamSynchronize(st));
     IBO_CUDA_TRY(cudaGetLastError());
     if (nbad)

@@ -291,6 +291,33 @@ class GaussianProcess(object):
             vals, dv = float(vals[0]), (dv[0] if grad else None)
         return (vals, dv) if grad else vals
 
+    def qNEI(self, batches, baseline=None, samples=512, seed=None, jitter=1e-8, Z=None, grad=False):
+        """Monte-Carlo noisy expected improvement of batches of points evaluated together (q-NEI, Letham et al. 2019): the
+        incumbent is max_i f(x_i) over the `baseline` points (default: the distinct rows of X, in order of first appearance),
+        drawn jointly with the batch from the latent posterior, instead of the fixed number max(Y).  batches[B, q, d] (or one
+        batch [q, d]) -> values[B] (a float for one batch), and with grad=True also the gradient with respect to the points
+        [B, q, d] (or [q, d]).  Z = numpy.random.default_rng(seed).standard_normal((P + q, samples)) unless Z[P + q, S] is given
+        (baseline rows first).  Raises NotPositiveDefinite when the baseline's covariance + jitter I is not positive definite
+        (a repeated baseline point with jitter 0); a batch whose own factorisation fails gets NaN."""
+        if len(self.X) == 0:
+            raise ValueError("q-NEI of a GP without data")
+        Xb = np.asarray(batches, dtype=float)
+        one = Xb.ndim == 2
+        Xb = Xb[None] if one else Xb
+        base = self.qnei_baseline() if baseline is None else np.array(baseline, dtype=float, ndmin=2)
+        if Z is None:
+            Z = np.random.default_rng(seed).standard_normal((base.shape[0] + Xb.shape[1], samples))
+        vals, dv, _, _ = self.model.qnei(Xb, base, Z, jitter, want_grad=grad)
+        if one:
+            vals, dv = float(vals[0]), (dv[0] if grad else None)
+        return (vals, dv) if grad else vals
+
+    def qnei_baseline(self):
+        """the distinct rows of X in order of first appearance: q-NEI's default baseline"""
+        X = np.asarray(self.X, dtype=float)
+        _, idx = np.unique(X, axis=0, return_index=True)
+        return X[np.sort(idx)]
+
     def sample_paths(self, n_paths, n_features=2048, seed=None):
         """n_paths posterior sample paths by pathwise conditioning (Matheron's rule) with n_features random Fourier features of the
         prior -> PosteriorPaths.  The draws come from numpy.random.default_rng(seed) in the order of `path_draws` (frequencies,

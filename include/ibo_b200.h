@@ -228,6 +228,35 @@ int ibo_score_grad(ibo_model* m, const double* Xs, long M, int acq, double ymax,
 int ibo_qei(ibo_model* m, const double* Xs, long B, int q, const double* Z, int S,
             double ymax, double xi, double jitter, double* values, double* dvalues, int* nbad);
 
+/* ---- noisy batch expected improvement (q-NEI) ------------------------------------------------------
+ * Xs: B x q x d as for ibo_qei; Xbase: P x d row-major, the points already evaluated (original coordinates); Z[(P + q) x S]
+ * row-major standard normals, the P baseline rows first, then the q batch rows.  For each batch the LATENT joint posterior of the
+ * P + q points [Xbase; batch] is taken (Letham et al. 2019):
+ *     Sigma = K(., .) - V^T V,  V = W_g K(X_g, .)    (the kernel itself, sf2 on the diagonal; g the variance model when one is
+ *                                                     attached, else the model),
+ * mu the posterior mean of ibo_qei (fixed order per point), L = chol(Sigma + jitter I) and
+ *     F_s = mu + L z_s,   m_s = max_{i < P} F_s,i (the incumbent of sample s),
+ *     values[b] = (1 / S) sum_s max(0, max_{j >= P} F_s,j - m_s).
+ * The incumbent is the best true value among the evaluated points, drawn jointly with the batch: no observation noise is added
+ * to points already measured (the convention of ibo_paths_*), which needs sf2 <= 1 + noise.  L is formed blockwise with the
+ * baseline first: L_bb = chol(Sigma_bb + jitter I), m_s and W_bb = inv(L_bb) once per call, then per batch T = W_bb Sigma_bq,
+ * F_s,q = mu_q + T^T z_b + chol(Sigma_qq + jitter I - T^T T) z_q.  incumbent[S] (may be NULL) receives m_s.  dvalues[B x q x d]
+ * (may be NULL) is the exact gradient for the fixed Z in reverse mode (the baseline does not depend on the batch): per improving
+ * sample with winner j*, mubar_j* += 1 / S, Lbar_j*,k += z_q,k / S, Tbar[:, j*] += z_b / S; Gbar by the reverse Cholesky,
+ * Tbar -= 2 T Gbar, Cbar = W_bb^T Tbar, and
+ *     d qNEI / dx_j = mubar_j dmu(x_j) + 2 sum_l Gbar_jl d1 k(x_j, x_l) + sum_i Cbar_ij d1 k(x_j, xb_i) - 2 sum_i y_j,i dk_i(x_j) / dx_j,
+ *     y_j = R_g^-1 (K(X_g, X_q) Gbar + K(X_g, X_b) Cbar / 2)_j.
+ * Every sum runs in a fixed order without atomics: a batch's value and gradient do not depend on the other batches of the call,
+ * the values are the same bits with and without dvalues, and repeated calls give the same bits.  Points per chunk =
+ * max(128, floor(2^26 / (2 Np + 2 Pp + Sp) / 128) 128) (Np, Pp, Sp: g's training points, P and S rounded up to 128), whole
+ * batches per chunk.  If Sigma_bb + jitter I is not positive definite the call returns IBO_E_NOTSPD with *info (may be NULL) = the
+ * 1-based baseline pivot; a batch whose Schur complement is not gets NaN for its value and gradient rows and is counted in *nbad
+ * (may be NULL), and the call returns IBO_OK.
+ * IBO_E_BADARG, before the device is touched, for a NULL model, Xs, Xbase, Z or values, B < 1, q outside [1, 32], P outside
+ * [1, 8192], S outside [1, 8192], d > 64, jitter < 0 or NaN, or sf2 > 1 + noise (of g). */
+int ibo_qnei(ibo_model* m, const double* Xs, long B, int q, const double* Xbase, long P, const double* Z, int S, double jitter,
+             double* values, double* dvalues, double* incumbent, int* nbad, int* info);
+
 /* ---- max-value entropy search (MES) -------------------------------------------------------------
  * Xs: M x d row-major candidates (original coordinates), M >= 1, d <= 64.  mu and s2 are what ibo_posterior_batch returns with the
  * same flags: s2 is the library's clipped variance (floor 1e-8, 1e-7 under IBO_FLAG_MODE_PY, ceiling 10), which like EI's carries
