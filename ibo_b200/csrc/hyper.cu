@@ -12,6 +12,7 @@
 // matrices are recomputed on the fly from the scaled inputs inside one fused reduction over the lower triangle
 // (fixed summation order => deterministic).
 #include "model.cuh"
+#include "scoremath.cuh"
 #include "tilegemm.cuh"
 #include <cmath>
 #include <mutex>
@@ -28,17 +29,6 @@ struct KDesc {
     double sf2;
     double theta0; // isotropic kinds: the length scale (Matern-3/2 reference expression needs the unscaled distance)
 };
-
-__device__ __forceinline__ double kval_from_r2(int kind, double sf2, double r2) {   // same arithmetic as model.cu
-    if (kind <= IBO_KERNEL_SE_ISO) return sf2 * exp(-0.5 * r2);
-    double r = sqrt(r2);
-    if (kind == IBO_KERNEL_MATERN3) {
-        double z = 1.7320508075688772 * r;
-        return sf2 * (1.0 + z) * exp(-z);
-    }
-    double z = 2.23606797749979 * r;
-    return sf2 * (1.0 + z + 5.0 * r2 / 3.0) * exp(-z);
-}
 
 // dK_ij / d log hyper_h from the scaled squared distance r2, the scaled squared difference dh2 along dimension h
 // (ARD kinds) and K_ij itself.
@@ -75,7 +65,7 @@ __global__ void kernel_matrix_kernel(double* __restrict__ out, const double* __r
         r2 += df * df;
         if (t == which) dh2 = df * df;
     }
-    double kv = (i == j) ? kd.sf2 : kval_from_r2(kd.kind, kd.sf2, r2);
+    double kv = (i == j) ? kd.sf2 : cov_r2(kd.kind, kd.sf2, r2);
     out[(size_t)i * N + j] = which < 0 ? kv : dk_value(kd, which, r2, dh2, kv);
 }
 
@@ -140,7 +130,7 @@ __global__ void __launch_bounds__(256) grad_reduce_kernel(const double* __restri
         // (min, max) = (gj, gi) ordering of the difference as in build_A_kernel
         double r2 = 0;
         for (int t = 0; t < d; t++) { double df = Xj[c * d + t] - Xi[r * d + t]; r2 += df * df; }
-        const double kv = (gi == gj) ? kd.sf2 : kval_from_r2(kd.kind, kd.sf2, r2);
+        const double kv = (gi == gj) ? kd.sf2 : cov_r2(kd.kind, kd.sf2, r2);
         const double g = (Kinv[(size_t)gi * Np + gj] - alpha[gi] * aj) * (gi == gj ? 1.0 : 2.0);
 #pragma unroll
         for (int a = 0; a < GH; a++) {

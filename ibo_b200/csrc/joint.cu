@@ -232,7 +232,6 @@ int joint_sigma(ibo_model* m, const double* Xs, long M, double jitter, bool want
     int rc;
     if ((rc = ensure_joint_attrs(m->device))) return rc;
     CandWork* w = cand_work(m);
-    ibo_model& c = w->chol;
     ibo_model* g = m->var_model ? m->var_model : m;      // the model sigma^2 comes from
     cudaStream_t st = m->stream;
     const int d = m->d, Np = g->Np, Mp = (int)round128(M);
@@ -253,7 +252,7 @@ int joint_sigma(ibo_model* m, const double* Xs, long M, double jitter, bool want
     launch_scale_cands(w->dScaled, w->dRaw, g, M, Mp, st);
     launch_cross_cov(w->dKc, g, w->dScaled, (int)M, Mp, st);
     launch_w_gemm_v(w->dV, g, w->dKc, Mp, st);
-    launch_joint_sigma(&c, w->dScaled, w->dV, g, 1.0 + g->noise, jitter, st);
+    launch_joint_sigma(w->chol, w->dScaled, w->dV, g, 1.0 + g->noise, jitter, st);
     IBO_CUDA_TRY(cudaGetLastError());
     return IBO_OK;
 }
@@ -263,13 +262,8 @@ int joint_sigma(ibo_model* m, const double* Xs, long M, double jitter, bool want
 int chol_setup(ibo_model* m, long M, bool invert) {
     int rc;
     CandWork* w = cand_work(m);
-    ibo_model& c = w->chol;
-    if (!c.dInfo) {
-        c.device = m->device;
-        c.stream = m->stream; c.stream2 = m->stream2; c.stream3 = m->stream3; c.stream4 = m->stream4;
-        c.evStep = m->evStep; c.evRest = m->evRest; c.evScale = m->evScale; c.evFar = m->evFar;
-        IBO_CUDA_TRY(cudaMalloc(&c.dInfo, sizeof(int)));
-    }
+    Factor& c = w->chol;
+    if (!c.dInfo) IBO_CUDA_TRY(cudaMalloc(&c.dInfo, sizeof(int)));
     const int Mp = (int)round128(M), nbM = Mp / 128;
     if ((rc = grow(&c.dA, &w->cholACap, (size_t)Mp * Mp))) return rc;
     if ((rc = grow(&c.dD, &w->cholDCap, (size_t)nbM * 128 * 128))) return rc;
@@ -279,19 +273,19 @@ int chol_setup(ibo_model* m, long M, bool invert) {
         c.dBetaY = c.dY + Mp;
         IBO_CUDA_TRY(cudaMemsetAsync(c.dY, 0, sizeof(double) * Mp, m->stream));
     }
-    c.N = (int)M; c.Np = Mp; c.nb = nbM; c.d = m->d;
+    c.N = (int)M; c.Np = Mp; c.nb = nbM;
     return IBO_OK;
 }
 
-void launch_joint_sigma(ibo_model* c, const double* Cs, const double* V, const ibo_model* g, double diag, double jitter, cudaStream_t st) {
-    const int Mp = c->Np;
-    prior_cov_kernel<<<dim3((Mp + 255) / 256, Mp), 256, 0, st>>>(c->dA, Cs, c->N, Mp, g->d, g->kind, g->sf2, diag);
-    sigma_kernel<<<dim3(c->nb, c->nb), 256, TILE_SMEM_DOUBLES * 8, st>>>(c->dA, V, Mp, g->Np, c->N, jitter);
+void launch_joint_sigma(Factor& c, const double* Cs, const double* V, const ibo_model* g, double diag, double jitter, cudaStream_t st) {
+    const int Mp = c.Np;
+    prior_cov_kernel<<<dim3((Mp + 255) / 256, Mp), 256, 0, st>>>(c.dA, Cs, c.N, Mp, g->d, g->kind, g->sf2, diag);
+    sigma_kernel<<<dim3(c.nb, c.nb), 256, TILE_SMEM_DOUBLES * 8, st>>>(c.dA, V, Mp, g->Np, c.N, jitter);
     g_launches += 2;
 }
 
-void launch_clear_diag_upper(ibo_model* c, cudaStream_t st) {
-    zero_diag_upper_kernel<<<c->nb, 256, 0, st>>>(c->dA, c->Np);
+void launch_clear_diag_upper(Factor& c, cudaStream_t st) {
+    zero_diag_upper_kernel<<<c.nb, 256, 0, st>>>(c.dA, c.Np);
     g_launches++;
 }
 
@@ -391,7 +385,7 @@ extern "C" int ibo_posterior_sample(ibo_model* m, const double* Xs, long M, cons
     CandWork* w = m->cand;
     cudaStream_t st = m->stream;
     const int Mp = (int)round128(M), nbM = Mp / 128, Sp = (int)round128(S);
-    if ((rc = launch_factorize(&w->chol, false, false, false))) return rc;
+    if ((rc = launch_factorize(*m, w->chol, false, false, false))) return rc;
     int hinfo = 0;
     IBO_CUDA_TRY(cudaMemcpyAsync(&hinfo, w->chol.dInfo, sizeof(int), cudaMemcpyDeviceToHost, st));
     IBO_CUDA_TRY(cudaStreamSynchronize(st));
@@ -400,7 +394,7 @@ extern "C" int ibo_posterior_sample(ibo_model* m, const double* Xs, long M, cons
         set_error("posterior covariance + jitter I is not positive definite (pivot " + std::to_string(hinfo) + ")");
         return IBO_E_NOTSPD;
     }
-    launch_clear_diag_upper(&w->chol, st);
+    launch_clear_diag_upper(w->chol, st);
     IBO_CUDA_TRY(cudaMemsetAsync(w->dNormals, 0, sizeof(double) * (size_t)Mp * Sp, st));
     IBO_CUDA_TRY(cudaMemcpy2DAsync(w->dNormals, sizeof(double) * Sp, Z, sizeof(double) * S, sizeof(double) * S, M, cudaMemcpyHostToDevice, st));
     trimm_kernel<<<dim3(Sp / 128, nbM), 256, TILE_SMEM_DOUBLES * 8, st>>>(w->dF, Sp, w->chol.dA, Mp, w->dNormals, Sp, nbM, w->dPost + M, (int)M);

@@ -119,23 +119,9 @@ __global__ void axpy_kernel(const double* __restrict__ a, const double* __restri
 }
 
 struct Scratch {
-    ibo_model* B = nullptr;          // holds B = I + G G^T, its factor and inverse factor
     int *dV = nullptr, *dU = nullptr, *dRowptr = nullptr, *dEnt = nullptr;
     double* buf = nullptr;           // all double workspaces in one block
     ~Scratch() {
-        if (B) {
-            double** ptrs[] = {&B->dA, &B->dW, &B->dD, &B->dBetaY, &B->dY};
-            for (auto p : ptrs) if (*p) pool_free(*p);
-            if (B->dInfo) cudaFree(B->dInfo);
-            if (B->evStep) cudaEventDestroy(B->evStep);
-            if (B->evRest) cudaEventDestroy(B->evRest);
-            if (B->evScale) cudaEventDestroy(B->evScale);
-            if (B->evFar) cudaEventDestroy(B->evFar);
-            if (B->stream4) cudaStreamDestroy(B->stream4);
-            if (B->stream2) cudaStreamDestroy(B->stream2);
-            if (B->stream3) cudaStreamDestroy(B->stream3);
-            delete B;
-        }
         if (dV) cudaFree(dV);
         if (dU) cudaFree(dU);
         if (dRowptr) cudaFree(dRowptr);
@@ -153,7 +139,7 @@ extern "C" int ibo_pref_fit(ibo_model* m, int P, const int* v, const int* u, con
                             int maxit, double gtol, double* S_out, double* gnorm_out, int* iters_out) {
     if (!m || P < 1 || !v || !u || !deg || !y) { set_error("bad argument"); return IBO_E_BADARG; }
     if (m->cpp_prior || m->has_cinv) { set_error("ibo_pref_fit needs the plain R model of the preference points"); return IBO_E_BADARG; }
-    const int N = m->N, Np = m->Np, nb = m->nb;
+    const int N = m->N, Np = m->Np;
     for (int p = 0; p < P; p++)
         if (v[p] < 0 || v[p] >= N || u[p] < 0 || u[p] >= N) { set_error("preference index out of range"); return IBO_E_BADARG; }
     if (maxit <= 0) maxit = 100;
@@ -163,26 +149,13 @@ extern "C" int ibo_pref_fit(ibo_model* m, int P, const int* v, const int* u, con
     const int K = ((P + BK - 1) / BK) * BK;
     Scratch sc;
 #define TRYS(expr) do { cudaError_t e__ = (expr); if (e__ != cudaSuccess) { set_error(std::string(#expr) + ": " + cudaGetErrorString(e__)); cudaGetLastError(); return e__ == cudaErrorMemoryAllocation ? IBO_E_NOMEM : IBO_E_CUDA; } } while (0)
-    // ---- scratch factorisation state ----
-    sc.B = new ibo_model();
-    ibo_model* B = sc.B;
-    B->device = m->device; B->N = N; B->Np = Np; B->nb = nb; B->stream = st;
-    TRYS(cudaStreamCreateWithFlags(&B->stream2, cudaStreamNonBlocking));
-    TRYS(cudaStreamCreateWithFlags(&B->stream3, cudaStreamNonBlocking));
-    TRYS(cudaEventCreateWithFlags(&B->evStep, cudaEventDisableTiming));
-    TRYS(cudaEventCreateWithFlags(&B->evRest, cudaEventDisableTiming));
-    TRYS(cudaStreamCreateWithFlags(&B->stream4, cudaStreamNonBlocking));
-    TRYS(cudaEventCreateWithFlags(&B->evScale, cudaEventDisableTiming));
-    TRYS(cudaEventCreateWithFlags(&B->evFar, cudaEventDisableTiming));
-    TRYS(pool_malloc((void**)&B->dA, sizeof(double) * (size_t)Np * Np));
-    TRYS(pool_malloc((void**)&B->dW, sizeof(double) * (size_t)Np * Np));
-    TRYS(pool_malloc((void**)&B->dD, sizeof(double) * (size_t)nb * 128 * 128));
-    TRYS(pool_malloc((void**)&B->dBetaY, sizeof(double) * Np));
-    TRYS(pool_malloc((void**)&B->dY, sizeof(double) * Np));
-    TRYS(cudaMalloc(&B->dInfo, sizeof(int)));
+    // ---- B = I + G G^T, its factor and inverse factor: the model's scratch factor, factorised on the model's lanes ----
+    int rc = chol_setup(m, N, true);
+    if (rc) return rc;
+    Factor& B = cand_work(m)->chol;
     // cleared here as well as by each factorisation: a start that already meets gtol runs none, and the pivot read after the
-    // loop must not see what a recycled allocation held
-    TRYS(cudaMemsetAsync(B->dInfo, 0, sizeof(int), st));
+    // loop must see neither what a fresh allocation held nor the pivot an earlier failed factorisation on this model left there
+    TRYS(cudaMemsetAsync(B.dInfo, 0, sizeof(int), st));
     // ---- preference index arrays + CSR (point -> its preferences, in preference order) ----
     std::vector<int> rowptr(N + 1, 0), ent(2 * (size_t)P);
     for (int p = 0; p < P; p++) { rowptr[v[p] + 1]++; rowptr[u[p] + 1]++; }
@@ -234,20 +207,19 @@ extern "C" int ibo_pref_fit(ibo_model* m, int P, const int* v, const int* u, con
         TRYS(cudaStreamSynchronize(st));
         return IBO_OK;
     };
-    int rc = eval(a, true);
-    if (rc) return rc;
+    if ((rc = eval(a, true))) return rc;
     double S = hs[0], gn_inf = hs[1];
     int it = 0;
     for (; it < maxit && gn_inf > gtol; it++) {
         // B = I + G G^T, factorise, da = -inv(B) (L^T gl + a)
         build_G_kernel<<<dim3(gn, K), 256, 0, st>>>(m->dA, Np, N, sc.dV, sc.dU, w, P, K, G);
         g_launches++;
-        if ((rc = launch_syrk_identity(B->dA, G, Np, K, st))) return rc;
-        neg_sum_kernel<<<gn, 256, 0, st>>>(ltg, a, B->dY, N, Np);
+        if ((rc = launch_syrk_identity(B.dA, G, Np, K, st))) return rc;
+        neg_sum_kernel<<<gn, 256, 0, st>>>(ltg, a, B.dY, N, Np);
         g_launches++;
-        if ((rc = launch_factorize(B, false, false, true))) return rc;       // B->dW = inv(chol(B)), B->dBetaY = dW * rhs
+        if ((rc = launch_factorize(*m, B, false, false, true))) return rc;   // B.dW = inv(chol(B)), B.dBetaY = dW * rhs
         TRYS(cudaMemsetAsync(da, 0, sizeof(double) * Np, st));
-        launch_tri_matvec_t(B->dW, B->dBetaY, da, Np, Np, st);         // da = dW^T dW rhs
+        launch_tri_matvec_t(B.dW, B.dBetaY, da, Np, Np, st);           // da = dW^T dW rhs
         // backtracking on S (convex: the full step is accepted except far from the optimum)
         double t = 1.0;
         bool ok = false;
@@ -263,7 +235,7 @@ extern "C" int ibo_pref_fit(ibo_model* m, int P, const int* v, const int* u, con
         S = hs[0]; gn_inf = hs[1];
     }
     int hinfo = 0;
-    TRYS(cudaMemcpy(&hinfo, B->dInfo, sizeof(int), cudaMemcpyDeviceToHost));
+    TRYS(cudaMemcpy(&hinfo, B.dInfo, sizeof(int), cudaMemcpyDeviceToHost));
     // y = L a at the accepted point
     launch_tri_matvec(m->dA, a, ya, Np, st);
     TRYS(cudaMemcpyAsync(y, ya, sizeof(double) * N, cudaMemcpyDeviceToHost, st));

@@ -6,6 +6,7 @@
 // (ego/gaussianprocess/__init__.py:134-149,267-308), linalg.cholesky(R + inv(C)) (:487-498) and
 // the explicit linalg.inv(R) of cdirectGP (ego/acquisition/__init__.py:385-388).
 #include "model.cuh"
+#include "scoremath.cuh"
 #include "tilegemm.cuh"
 #include <cmath>
 #include <cstring>
@@ -102,21 +103,6 @@ int grow(double** p, size_t* cap, size_t need) {
     return IBO_OK;
 }
 
-// ---------------------------------------------------------------------------------------------
-// covariance function on the scaled squared distance r2 = sum_j ((x_j - y_j)/theta_j)^2
-//   (ego/gaussianprocess/kernel.py:87-89,147-149,207-210,246-248; cpp/optimizeGP.cpp:70-112)
-// ---------------------------------------------------------------------------------------------
-__device__ __forceinline__ double cov_from_r2(int kind, double sf2, double r2) {
-    if (kind <= IBO_KERNEL_SE_ISO) return sf2 * exp(-0.5 * r2);
-    double r = sqrt(r2);
-    if (kind == IBO_KERNEL_MATERN3) {
-        double z = 1.7320508075688772 * r;   // sqrt(3)
-        return sf2 * (1.0 + z) * exp(-z);
-    }
-    double z = 2.23606797749979 * r;         // sqrt(5)
-    return sf2 * (1.0 + z + 5.0 * r2 / 3.0) * exp(-z);
-}
-
 // A[i][j] = k(x_i, x_j) (i != j), `diag` (1 + noise for the GP's R) on the diagonal, + Cinv; identity in the padding.
 __global__ void build_A_kernel(double* __restrict__ A, const double* __restrict__ Xt, const double* __restrict__ Cinv,
                                int N, int Np, int d, int kind, double sf2, double diag) {
@@ -131,7 +117,7 @@ __global__ void build_A_kernel(double* __restrict__ A, const double* __restrict_
         int a = i < j ? i : j, b = i < j ? j : i;
         double r2 = 0;
         for (int t = 0; t < d; t++) { double df = Xt[(size_t)a * d + t] - Xt[(size_t)b * d + t]; r2 += df * df; }
-        v = cov_from_r2(kind, sf2, r2);
+        v = cov_r2(kind, sf2, r2);
     }
     if (Cinv && i < N && j < N) v += Cinv[(size_t)i * N + j];
     A[(size_t)i * Np + j] = v;
@@ -555,7 +541,7 @@ __global__ void __launch_bounds__(256) append_kvec_kernel(double* __restrict__ X
     if (c < p) {
         double r2 = 0;
         for (int t = 0; t < d; t++) { double df = Xt[(size_t)c * d + t] - xnew[t]; r2 += df * df; }   // (min, max) order as build_A_kernel
-        v = cov_from_r2(kind, sf2, r2);
+        v = cov_r2(kind, sf2, r2);
     }
     kvec[c] = v;
     if (Aorig) {
@@ -760,16 +746,16 @@ static int set_kernel_attrs() {
     return IBO_OK;
 }
 
-// Factorise m->dA in place, produce dW, dD, dWpack, dBetaY, dBeta1.
+// Factorise f.dA in place on the streams and events of ln, produce dW, dD, dWpack, dBetaY.
 // from_inverse_reversed: dA holds J invR J; W' = reverse-transpose of its Cholesky factor.
-int launch_factorize(ibo_model* m, bool from_inverse_reversed, bool pack, bool invert) {
+int launch_factorize(const Lanes& ln, Factor& f, bool from_inverse_reversed, bool pack, bool invert) {
     int rc = set_kernel_attrs();
     if (rc) return rc;
-    cudaStream_t st = m->stream;
-    const int Np = m->Np, nb = m->nb;
+    cudaStream_t st = ln.stream;
+    const int Np = f.Np, nb = f.nb;
     const int tile_smem = TILE_SMEM_DOUBLES * 8, half_smem = TileCfg<64>::SMEM_DOUBLES * 8;
     const int potrf_smem = POTRF_SMEM;
-    IBO_CUDA_TRY(cudaMemsetAsync(m->dInfo, 0, sizeof(int), st));
+    IBO_CUDA_TRY(cudaMemsetAsync(f.dInfo, 0, sizeof(int), st));
     dim3 g2((Np + 255) / 256, Np);
     // Block columns go in groups of w = 1 or 2.  With w = 2 everything behind the pair (k, k+1) is updated with both columns at
     // once: one pass with a 256-deep product instead of two 128-deep ones halves the read-modify-write traffic of the trailing
@@ -782,19 +768,19 @@ int launch_factorize(ibo_model* m, bool from_inverse_reversed, bool pack, bool i
     // The inversion W = inv(L) is a forward substitution on B = I that follows the factorisation group by group on its own pair
     // of streams, split the same way: rows k..k+w-1 are scaled by D (W_kj = D_k B_kj), the next group's rows are updated on the
     // near stream, all later rows on the far stream (after evScale; near(k) waits for far(k-w) through evFar).
-    cudaStream_t s2 = from_inverse_reversed ? st : m->stream2;
-    cudaStream_t s4 = m->stream4;
+    cudaStream_t s2 = from_inverse_reversed ? st : ln.stream2;
+    cudaStream_t s4 = ln.stream4;
     const bool trtri = invert && !from_inverse_reversed;
     if (trtri) {
-        IBO_CUDA_TRY(cudaEventRecord(m->evStep, st));            // orders s2 / s4 after whatever produced dA / dD users
-        IBO_CUDA_TRY(cudaStreamWaitEvent(s2, m->evStep, 0));
-        IBO_CUDA_TRY(cudaStreamWaitEvent(s4, m->evStep, 0));
-        set_identity_kernel<<<g2, 256, 0, s2>>>(m->dW, Np);
+        IBO_CUDA_TRY(cudaEventRecord(ln.evStep, st));            // orders s2 / s4 after whatever produced dA / dD users
+        IBO_CUDA_TRY(cudaStreamWaitEvent(s2, ln.evStep, 0));
+        IBO_CUDA_TRY(cudaStreamWaitEvent(s4, ln.evStep, 0));
+        set_identity_kernel<<<g2, 256, 0, s2>>>(f.dW, Np);
         g_launches++;
-        IBO_CUDA_TRY(cudaEventRecord(m->evFar, s2));
-        IBO_CUDA_TRY(cudaStreamWaitEvent(s4, m->evFar, 0));
+        IBO_CUDA_TRY(cudaEventRecord(ln.evFar, s2));
+        IBO_CUDA_TRY(cudaStreamWaitEvent(s4, ln.evFar, 0));
     }
-    cudaStream_t sb = m->stream3;
+    cudaStream_t sb = ln.stream3;
     const long pair_opt = get_option(OPT_CHOL_PAIR);
     const int w = (pair_opt < 0 ? nb >= 48 : pair_opt != 0) ? 2 : 1;
 #ifdef IBO_I8_TRACE
@@ -809,28 +795,28 @@ int launch_factorize(ibo_model* m, bool from_inverse_reversed, bool pack, bool i
 #else
 #define TL(s, k, tag) do { } while (0)
 #endif
-    IBO_CUDA_TRY(cudaEventRecord(m->evRest, st));
-    IBO_CUDA_TRY(cudaStreamWaitEvent(sb, m->evRest, 0));
+    IBO_CUDA_TRY(cudaEventRecord(ln.evRest, st));
+    IBO_CUDA_TRY(cudaStreamWaitEvent(sb, ln.evRest, 0));
     for (int k = 0; k < nb; k += w) {
         // ---- block column k
-        potrf_diag_kernel<<<1, 512, potrf_smem, st>>>(m->dA, Np, k, m->dD, m->dInfo);
+        potrf_diag_kernel<<<1, 512, potrf_smem, st>>>(f.dA, Np, k, f.dD, f.dInfo);
         g_launches++;
         TL(st, k, "potrf");
         int kl = k;                            // last block column of the group
         if (k + 1 < nb) {
-            block_step_kernel<MODE_CHOL_PANEL, 64><<<dim3(nb - 1 - k, 1, 2), 128, half_smem, st>>>(m->dA, nullptr, m->dD, Np, k);
+            block_step_kernel<MODE_CHOL_PANEL, 64><<<dim3(nb - 1 - k, 1, 2), 128, half_smem, st>>>(f.dA, nullptr, f.dD, Np, k);
             g_launches++;
             TL(st, k, "panel");
             if (w == 2) {
                 // ---- block column k+1: its update by column k, then the same two kernels
                 kl = k + 1;
-                block_step_kernel<MODE_CHOL_TRAIL, 64><<<dim3(1, nb - 1 - k, 2), 128, half_smem, st>>>(m->dA, nullptr, m->dD, Np, k, 0, k + 1, 128);
+                block_step_kernel<MODE_CHOL_TRAIL, 64><<<dim3(1, nb - 1 - k, 2), 128, half_smem, st>>>(f.dA, nullptr, f.dD, Np, k, 0, k + 1, 128);
                 TL(st, k, "first");
-                potrf_diag_kernel<<<1, 512, potrf_smem, st>>>(m->dA, Np, kl, m->dD, m->dInfo);
+                potrf_diag_kernel<<<1, 512, potrf_smem, st>>>(f.dA, Np, kl, f.dD, f.dInfo);
                 g_launches += 2;
                 TL(st, kl, "potrf");
                 if (kl + 1 < nb) {
-                    block_step_kernel<MODE_CHOL_PANEL, 64><<<dim3(nb - 1 - kl, 1, 2), 128, half_smem, st>>>(m->dA, nullptr, m->dD, Np, kl);
+                    block_step_kernel<MODE_CHOL_PANEL, 64><<<dim3(nb - 1 - kl, 1, 2), 128, half_smem, st>>>(f.dA, nullptr, f.dD, Np, kl);
                     g_launches++;
                     TL(st, kl, "panel");
                 }
@@ -839,45 +825,45 @@ int launch_factorize(ibo_model* m, bool from_inverse_reversed, bool pack, bool i
         const int gw = kl - k + 1;             // columns in this group (1 at the end of an odd count)
         const int nbehind = nb - 1 - kl;       // block rows / columns behind the group
         const int c0 = kl + 1, kspan = 128 * gw;
-        IBO_CUDA_TRY(cudaEventRecord(m->evStep, st));
+        IBO_CUDA_TRY(cudaEventRecord(ln.evStep, st));
         if (trtri) {
-            IBO_CUDA_TRY(cudaStreamWaitEvent(s2, m->evStep, 0));
-            block_step_kernel<MODE_TRTRI_SCALE><<<k + 1, 256, tile_smem, s2>>>(m->dA, m->dW, m->dD, Np, k);
+            IBO_CUDA_TRY(cudaStreamWaitEvent(s2, ln.evStep, 0));
+            block_step_kernel<MODE_TRTRI_SCALE><<<k + 1, 256, tile_smem, s2>>>(f.dA, f.dW, f.dD, Np, k);
             g_launches++;
             if (gw == 2) {
-                block_step_kernel<MODE_TRTRI_UPDATE, 64><<<dim3(k + 1, 1, 2), 128, half_smem, s2>>>(m->dA, m->dW, m->dD, Np, k, 0, k + 1, 128);
-                block_step_kernel<MODE_TRTRI_SCALE><<<kl + 1, 256, tile_smem, s2>>>(m->dA, m->dW, m->dD, Np, kl);
+                block_step_kernel<MODE_TRTRI_UPDATE, 64><<<dim3(k + 1, 1, 2), 128, half_smem, s2>>>(f.dA, f.dW, f.dD, Np, k, 0, k + 1, 128);
+                block_step_kernel<MODE_TRTRI_SCALE><<<kl + 1, 256, tile_smem, s2>>>(f.dA, f.dW, f.dD, Np, kl);
                 g_launches += 2;
             }
             if (nbehind > 0) {
                 // rows behind the group take all its block rows in one pass (the block W_(k),(k+1) above the diagonal is zero)
                 const int nnear = nbehind < w ? nbehind : w;
                 if (nbehind > nnear) {
-                    IBO_CUDA_TRY(cudaEventRecord(m->evScale, s2));
-                    IBO_CUDA_TRY(cudaStreamWaitEvent(s4, m->evScale, 0));
-                    block_step_kernel<MODE_TRTRI_UPDATE, 64><<<dim3(kl + 1, nbehind - nnear, 2), 128, half_smem, s4>>>(m->dA, m->dW, m->dD, Np, k, 0, c0 + nnear, kspan);
+                    IBO_CUDA_TRY(cudaEventRecord(ln.evScale, s2));
+                    IBO_CUDA_TRY(cudaStreamWaitEvent(s4, ln.evScale, 0));
+                    block_step_kernel<MODE_TRTRI_UPDATE, 64><<<dim3(kl + 1, nbehind - nnear, 2), 128, half_smem, s4>>>(f.dA, f.dW, f.dD, Np, k, 0, c0 + nnear, kspan);
                     g_launches++;
                     TL(s4, k, "far");
                 }
-                IBO_CUDA_TRY(cudaStreamWaitEvent(s2, m->evFar, 0));        // far(k-w) wrote the near rows of this group
-                block_step_kernel<MODE_TRTRI_UPDATE, 64><<<dim3(kl + 1, nnear, 2), 128, half_smem, s2>>>(m->dA, m->dW, m->dD, Np, k, 0, c0, kspan);
+                IBO_CUDA_TRY(cudaStreamWaitEvent(s2, ln.evFar, 0));        // far(k-w) wrote the near rows of this group
+                block_step_kernel<MODE_TRTRI_UPDATE, 64><<<dim3(kl + 1, nnear, 2), 128, half_smem, s2>>>(f.dA, f.dW, f.dD, Np, k, 0, c0, kspan);
                 g_launches++;
-                if (nbehind > nnear) IBO_CUDA_TRY(cudaEventRecord(m->evFar, s4));
+                if (nbehind > nnear) IBO_CUDA_TRY(cudaEventRecord(ln.evFar, s4));
             }
             TL(s2, k, "near");
         }
         if (nbehind > 0) {
             // look-ahead columns (they carry the bulk update of the previous group), then the rest in the background
-            if (k > 0) IBO_CUDA_TRY(cudaStreamWaitEvent(st, m->evRest, 0));
+            if (k > 0) IBO_CUDA_TRY(cudaStreamWaitEvent(st, ln.evRest, 0));
             const int nla = nbehind < w ? nbehind : w;
-            block_step_kernel<MODE_CHOL_TRAIL, 64><<<dim3(nla, nbehind, 2), 128, half_smem, st>>>(m->dA, nullptr, m->dD, Np, k, 0, c0, kspan);
+            block_step_kernel<MODE_CHOL_TRAIL, 64><<<dim3(nla, nbehind, 2), 128, half_smem, st>>>(f.dA, nullptr, f.dD, Np, k, 0, c0, kspan);
             g_launches++;
             TL(st, k, "ahead");
             if (nbehind > nla) {
-                IBO_CUDA_TRY(cudaStreamWaitEvent(sb, m->evStep, 0));
-                block_step_kernel<MODE_CHOL_TRAIL, 64><<<dim3(nbehind - nla, nbehind, 2), 128, half_smem, sb>>>(m->dA, nullptr, m->dD, Np, k, nla, c0, kspan);
+                IBO_CUDA_TRY(cudaStreamWaitEvent(sb, ln.evStep, 0));
+                block_step_kernel<MODE_CHOL_TRAIL, 64><<<dim3(nbehind - nla, nbehind, 2), 128, half_smem, sb>>>(f.dA, nullptr, f.dD, Np, k, nla, c0, kspan);
                 g_launches++;
-                IBO_CUDA_TRY(cudaEventRecord(m->evRest, sb));
+                IBO_CUDA_TRY(cudaEventRecord(ln.evRest, sb));
                 TL(sb, k, "bulk");
             }
         }
@@ -894,23 +880,23 @@ int launch_factorize(ibo_model* m, bool from_inverse_reversed, bool pack, bool i
 #else
 #undef TL
 #endif
-    IBO_CUDA_TRY(cudaEventRecord(m->evRest, sb));
-    IBO_CUDA_TRY(cudaStreamWaitEvent(st, m->evRest, 0));
+    IBO_CUDA_TRY(cudaEventRecord(ln.evRest, sb));
+    IBO_CUDA_TRY(cudaStreamWaitEvent(st, ln.evRest, 0));
     if (!invert) {
         IBO_CUDA_TRY(cudaGetLastError());
         return IBO_OK;
     }
     if (from_inverse_reversed) {
-        reverse_transpose_kernel<<<g2, 256, 0, st>>>(m->dW, m->dA, m->N, Np);
+        reverse_transpose_kernel<<<g2, 256, 0, st>>>(f.dW, f.dA, f.N, Np);
         g_launches++;
     } else {
-        IBO_CUDA_TRY(cudaEventRecord(m->evStep, s2));
-        IBO_CUDA_TRY(cudaStreamWaitEvent(st, m->evStep, 0));
-        IBO_CUDA_TRY(cudaEventRecord(m->evFar, s4));
-        IBO_CUDA_TRY(cudaStreamWaitEvent(st, m->evFar, 0));
+        IBO_CUDA_TRY(cudaEventRecord(ln.evStep, s2));
+        IBO_CUDA_TRY(cudaStreamWaitEvent(st, ln.evStep, 0));
+        IBO_CUDA_TRY(cudaEventRecord(ln.evFar, s4));
+        IBO_CUDA_TRY(cudaStreamWaitEvent(st, ln.evFar, 0));
     }
-    if (pack) { pack_w_kernel<<<dim3(nb * KB_PER_BLOCK, nb), 256, 0, st>>>(m->dW, m->dWpack, Np, nb); g_launches++; }
-    tri_matvec_kernel<<<(Np + 7) / 8, 256, 0, st>>>(m->dW, m->dY, m->dBetaY, Np);
+    if (pack) { pack_w_kernel<<<dim3(nb * KB_PER_BLOCK, nb), 256, 0, st>>>(f.dW, f.dWpack, Np, nb); g_launches++; }
+    tri_matvec_kernel<<<(Np + 7) / 8, 256, 0, st>>>(f.dW, f.dY, f.dBetaY, Np);
     g_launches++;
     IBO_CUDA_TRY(cudaGetLastError());
     return IBO_OK;
@@ -1147,7 +1133,7 @@ static int create_common(int device, int kind, const double* hyper, int nhyper, 
                 pref_build_C_kernel<<<(Np + 127) / 128, 128, 0, st>>>(m->dA, N, Np, pref->P, dPairs, dPairs + pref->P, dWts, pref->cdiag);
             }
             g_launches++;
-            rc = launch_factorize(m, false, false, true);
+            rc = launch_factorize(*m, *m, false, false, true);
             int cinfo = 0;
             if (!rc) {
                 TRYM(cudaMemcpyAsync(&cinfo, m->dInfo, sizeof(int), cudaMemcpyDeviceToHost, st));
@@ -1174,7 +1160,7 @@ static int create_common(int device, int kind, const double* hyper, int nhyper, 
         TRYM(pool_malloc((void**)&m->dAorig, sizeof(double) * (size_t)Np * Np));
         TRYM(cudaMemcpyAsync(m->dAorig, m->dA, sizeof(double) * (size_t)Np * Np, cudaMemcpyDeviceToDevice, st));
     }
-    rc = launch_factorize(m, invR != nullptr, true, true);
+    rc = launch_factorize(*m, *m, invR != nullptr, true, true);
     if (rc) { if (dTmp) pool_free(dTmp); return fail(rc); }
     // beta1 = W 1 (prior-mean correction term)
     TRYM(cudaMemcpyAsync(m->dBeta1, ones.data(), sizeof(double) * Np, cudaMemcpyHostToDevice, st));

@@ -6,18 +6,36 @@
 #include <utility>
 #include <vector>
 
-namespace ibo { struct CandWork; }
+namespace ibo {
+struct CandWork;
 
-struct ibo_model {
-    int device = 0;
+// the streams and events launch_factorize runs on: the model's own, whatever it factorises
+struct Lanes {
     cudaStream_t stream = nullptr;
     cudaStream_t stream2 = nullptr;   // inversion pipeline of the model build; K1 of the next chunk on the INT8 path
     cudaStream_t stream3 = nullptr;   // bulk trailing updates of the look-ahead Cholesky
     cudaStream_t stream4 = nullptr;   // bulk row updates of the inversion that follows it
     cudaEvent_t evStep = nullptr, evRest = nullptr, evScale = nullptr, evFar = nullptr;
-    int N = 0, d = 0, kind = 0;
-    int nb = 0;          // 128-row blocks
-    int Np = 0;          // nb * 128 (identity padded)
+};
+
+// the matrices launch_factorize reads and writes: the model's, or a scratch factor of the candidate workspace
+struct Factor {
+    int N = 0;
+    int Np = 0;                 // nb * 128 (identity padded)
+    int nb = 0;                 // 128-row blocks
+    double* dA = nullptr;       // [Np][Np] row-major: A (the model's R (+Cinv)), overwritten by L (lower)
+    double* dD = nullptr;       // [nb][128][128] inverses of the diagonal blocks of L
+    double* dW = nullptr;       // [Np][Np] row-major: W = inv(L), exact zeros above the diagonal
+    double* dWpack = nullptr;   // packed blobs, wpack_base(nb) * BLOB doubles
+    double* dY = nullptr;       // [Np]
+    double* dBetaY = nullptr;   // [Np]  W Y
+    int* dInfo = nullptr;       // 0, or the pivot at which A is not positive definite
+};
+}  // namespace ibo
+
+struct ibo_model : ibo::Lanes, ibo::Factor {
+    int device = 0;
+    int d = 0, kind = 0;
     double noise = 0, sf2 = 1;
     bool cpp_prior = false;
     bool has_cinv = false;            // A = R + inv(C): no rank-1 append
@@ -28,15 +46,8 @@ struct ibo_model {
     double* dXt = nullptr;      // scaled training inputs x/theta, [Np][d], rows >= N are zero
     double* dInvTheta = nullptr;// [d]
     double* dCenter = nullptr;  // [d] mean of the scaled training inputs (dXt is stored centred)
-    double* dA = nullptr;       // [Np][Np] row-major: A = R (+Cinv), overwritten by L (lower)
     double* dAorig = nullptr;   // optional copy of A (kept for get_matrix(0)); N<=4096 only
-    double* dW = nullptr;       // [Np][Np] row-major: W = inv(L), exact zeros above the diagonal
-    double* dD = nullptr;       // [nb][128][128] inverses of the diagonal blocks of L
-    double* dWpack = nullptr;   // packed blobs, wpack_base(nb) * BLOB doubles
-    double* dBetaY = nullptr;   // [Np]  W Y
     double* dBeta1 = nullptr;   // [Np]  W 1
-    double* dY = nullptr;       // [Np]
-    int* dInfo = nullptr;
     bool from_inverse = false;        // built from a caller-supplied inverse (legacy acqmaxGP): sigma^2 >= noise is not guaranteed
     // INT8 path of wide batches (score_i8.cuh), built on first use: the seven base-256 digits of W packed for shared memory
     // (dWi8s), per-row scales ([Np] slicing scale, [Np] 2 scale sf2, [Np] shift constant), alpha = W^T W Y and W^T W 1
@@ -78,25 +89,25 @@ struct ibo_model {
 };
 
 namespace ibo {
-// Workspace of the candidate-side entry points (joint.cu, grad.cu, qei.cu, mes.cu), kept with the model that owns the call and grown
-// on demand.  One call at a time runs on a model, so the four share one set of buffers, one per role; g is the variance model when
-// one is attached and the model otherwise.  Within a call no two live roles share a buffer: Z overwrites K* and y overwrites V
+// Workspace of the candidate-side entry points (joint.cu, grad.cu, qei.cu, mes.cu), of sample-path creation (paths.cu) and of the
+// Laplace fit (laplace.cu), kept with the model that owns the call and grown on demand.  One call at a time runs on a model, so they
+// share one set of buffers, one per role; g is the variance model when one is attached and the model otherwise.  Within a call no two live roles share a buffer: Z overwrites K* and y overwrites V
 // once K* and V are dead.  A call grows every buffer it uses before it takes a pointer into the workspace.
 struct CandWork {
     double* dRaw = nullptr;     size_t rawCap = 0;     // candidates as given [M][d]
     double* dScaled = nullptr;  size_t scaledCap = 0;  // candidates (of the chunk) scaled and centred like g's training inputs [Mcp][d]
     double* dScaledM = nullptr; size_t scaledMCap = 0; // the same scaled like the model's (variance model attached) [Mcp][d]
-    double* dKc = nullptr;      size_t kcCap = 0;      // K* = R(X_g, X*), then Z = W_g^T V [Np][Mcp]
-    double* dV = nullptr;       size_t vCap = 0;       // V = W_g K*, then y (q-EI) [Np][Mcp]
+    double* dKc = nullptr;      size_t kcCap = 0;      // K* = R(X_g, X*), then Z = W_g^T V [Np][Mcp]; T = W_g V (paths) [Np][Sp]
+    double* dV = nullptr;       size_t vCap = 0;       // V = W_g K*, then y (q-EI) [Np][Mcp]; Phi_g w + E e, then c (paths) [Np][Sp]
     double* dAB = nullptr;      size_t abCap = 0;      // a | b [2][Np]
     double* dKb = nullptr;      size_t kbCap = 0;      // k^T b [M] (prior only)
     double* dG = nullptr;       size_t gCap = 0;       // three [M][d] gradient planes
-    double* dNormals = nullptr; size_t normalsCap = 0; // standard normals: [Mp][Sp] zero padded (samples), [q][S] (q-EI)
+    double* dNormals = nullptr; size_t normalsCap = 0; // standard normals: [Mp][Sp] zero padded (samples), [q][S] (q-EI), e [Ng][S] (paths)
     double* dPost = nullptr;    size_t postCap = 0;    // [score | mu | s2] of the scoring path, 3 M + 2 (joint, gradients; MES values in
                                                        // the score plane, best value and index at 3 M); mu [M] (q-EI)
-    // joint posterior only
-    ibo_model chol;                                    // Sigma in chol.dA (Mp x Mp), factorised in place; its streams and events are the owner's
-                                                       // (q-NEI: Sigma of the baseline, with W = inv(L) in chol.dW)
+    // scratch factor of the joint posterior, q-NEI, the Laplace fit and the noise factor of sample paths, on the owner's lanes
+    Factor chol;                                       // Sigma in chol.dA (Mp x Mp), factorised in place (q-NEI: Sigma of the baseline,
+                                                       // with W = inv(L) in chol.dW; Laplace fit: B = I + G G^T and its inverse factor)
     size_t cholACap = 0, cholDCap = 0;                 // chol.dA, chol.dD
     size_t cholWCap = 0, cholYCap = 0;                 // chol.dW; chol.dY (zeros) | chol.dBetaY [2][Mp], when inverted
     double* dF = nullptr;       size_t fCap = 0;       // samples [Mp][Sp]
@@ -144,8 +155,9 @@ void pool_free(void* p);
 cudaError_t pinned_get(double** p);
 void pinned_put(double* p);
 // launches (all on m->stream)
+// f.dA = L L^T in place on the streams and events of `ln` (the model build passes the model as both: launch_factorize(*m, *m, ..)).
 // invert = false: the Cholesky factor only (no W = inv(L), no beta = W Y); dW, dWpack and the beta vectors are not touched
-int launch_factorize(ibo_model* m, bool from_inverse_reversed, bool pack, bool invert);
+int launch_factorize(const Lanes& ln, Factor& f, bool from_inverse_reversed, bool pack, bool invert);
 void launch_tri_matvec(const double* T, const double* v, double* out, int Np, cudaStream_t st);              // out = T v, T lower [Np][Np]
 void launch_tri_matvec_t(const double* T, const double* v, double* out, int n, int Np, cudaStream_t st);     // out = T^T v over the leading n x n
 int launch_syrk_identity(double* C, const double* G, int Np, int K, cudaStream_t st);                        // C = I + G G^T (lower tiles)
@@ -168,13 +180,13 @@ void launch_scale_cands(double* Cs, const double* X, const ibo_model* g, long M,
 void launch_cross_cov(double* Kc, const ibo_model* g, const double* Cs, int M, int Mp, cudaStream_t st);
 void launch_w_gemm_v(double* V, const ibo_model* g, const double* Kc, int Mp, cudaStream_t st);
 void launch_w_gemm_z(double* Z, const ibo_model* g, const double* V, int Mp, cudaStream_t st);
-// joint.cu: the workspace's Cholesky model (chol) shaped for an M x M matrix, with the owner's streams and events; invert: also
-// chol.dW and the vectors launch_factorize(.., invert = true) reads and writes
+// joint.cu: the workspace's scratch factor (chol) sized for an M x M matrix; it is factorised on the model's lanes
+// (launch_factorize(*m, w->chol, ..)); invert: also chol.dW and the vectors launch_factorize(.., invert = true) reads and writes
 int chol_setup(ibo_model* m, long M, bool invert);
-// joint.cu, on st: chol.dA (lower tiles) = R(X*, X*) with `diag` on the diagonal, kernel of g elsewhere, - V^T V (K = g->Np) + jitter I
-void launch_joint_sigma(ibo_model* c, const double* Cs, const double* V, const ibo_model* g, double diag, double jitter, cudaStream_t st);
-// joint.cu, on st: zeros above the diagonal inside the diagonal blocks of a factorised chol.dA
-void launch_clear_diag_upper(ibo_model* c, cudaStream_t st);
+// joint.cu, on st: c.dA (lower tiles) = R(X*, X*) with `diag` on the diagonal, kernel of g elsewhere, - V^T V (K = g->Np) + jitter I
+void launch_joint_sigma(Factor& c, const double* Cs, const double* V, const ibo_model* g, double diag, double jitter, cudaStream_t st);
+// joint.cu, on st: zeros above the diagonal inside the diagonal blocks of a factorised c.dA
+void launch_clear_diag_upper(Factor& c, cudaStream_t st);
 // joint.cu, on st: per column s < S of F ([M][ldf]) the argmax (lowest index wins, NaN never wins) and, when best is non-null, the max
 void launch_sample_max(const double* F, int ldf, int M, int S, long long* arg, double* best, cudaStream_t st);
 // joint.cu, on st: Kc[i][j] = k(xa_i, x*_j) with g's kernel for the Na points Xa scaled like g, exact zeros in the padding ([Nap][Mp])

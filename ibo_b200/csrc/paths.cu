@@ -352,19 +352,11 @@ struct ibo_paths {
 namespace ibo {
 namespace {
 
-int grow_dev(double** p, size_t* cap, size_t need) {
-    if (need <= *cap) return IBO_OK;
-    if (*p) cudaFree(*p);
-    *p = nullptr; *cap = 0;
-    IBO_CUDA_TRY(cudaMalloc(p, sizeof(double) * need));
-    *cap = need;
-    return IBO_OK;
-}
-
 void free_paths(ibo_paths* p) {
     if (!p) return;
     cudaSetDevice(p->device);
-    for (double* q : {p->dRows, p->dPhase, p->dCoef, p->dScale, p->dPrior, p->dWork}) if (q) cudaFree(q);
+    if (p->stream) cudaStreamSynchronize(p->stream);   // blocks go back to the pool: nothing may still be using them
+    for (double* q : {p->dRows, p->dPhase, p->dCoef, p->dScale, p->dPrior, p->dWork}) pool_free(q);
     if (p->stream) cudaStreamDestroy(p->stream);
     delete p;
 }
@@ -438,10 +430,10 @@ extern "C" int ibo_paths_create(ibo_model* m, int F, int S, const double* omega,
     const int ldc = (int)round_to(S + 1, PC);
     cudaStream_t st = m->stream;     // create reads the model: it runs on the model's stream and ends in a synchronisation
     size_t cap = 0;
-    if ((rc = grow_dev(&p->dRows, &cap, (size_t)R * d))) return fail(rc);
-    cap = 0; if ((rc = grow_dev(&p->dPhase, &cap, (size_t)R))) return fail(rc);
-    cap = 0; if ((rc = grow_dev(&p->dCoef, &cap, (size_t)R * ldc))) return fail(rc);
-    cap = 0; if ((rc = grow_dev(&p->dScale, &cap, (size_t)4 * d))) return fail(rc);
+    if ((rc = grow(&p->dRows, &cap, (size_t)R * d))) return fail(rc);
+    cap = 0; if ((rc = grow(&p->dPhase, &cap, (size_t)R))) return fail(rc);
+    cap = 0; if ((rc = grow(&p->dCoef, &cap, (size_t)R * ldc))) return fail(rc);
+    cap = 0; if ((rc = grow(&p->dScale, &cap, (size_t)4 * d))) return fail(rc);
     if (cudaMemsetAsync(p->dRows, 0, sizeof(double) * (size_t)R * d, st) || cudaMemsetAsync(p->dPhase, 0, sizeof(double) * R, st) ||
         cudaMemsetAsync(p->dCoef, 0, sizeof(double) * (size_t)R * ldc, st)) { set_error("cudaMemsetAsync failed"); return fail(IBO_E_CUDA); }
     auto d2d = [&](double* dst, const double* src, size_t nd) { return cudaMemcpyAsync(dst, src, sizeof(double) * nd, cudaMemcpyDeviceToDevice, st); };
@@ -466,7 +458,7 @@ extern "C" int ibo_paths_create(ibo_model* m, int F, int S, const double* omega,
     TRYP(d2d(p->dScale + 3 * d, g->dCenter, d));
     if (prior) {
         const int nb = m->npb;
-        cap = 0; if ((rc = grow_dev(&p->dPrior, &cap, (size_t)nb * d + nb + 2 * d))) return fail(rc);
+        cap = 0; if ((rc = grow(&p->dPrior, &cap, (size_t)nb * d + nb + 2 * d))) return fail(rc);
         TRYP(d2d(p->dPrior, m->dPmeans, (size_t)nb * d));
         TRYP(d2d(p->dPrior + (size_t)nb * d, m->dPbeta, nb));
         TRYP(d2d(p->dPrior + (size_t)nb * d + nb, m->dPlb, d));
@@ -478,16 +470,15 @@ extern "C" int ibo_paths_create(ibo_model* m, int F, int S, const double* omega,
     PathsDev& P = p->P;
     P.rows = p->dRows; P.phase = p->dPhase; P.coef = p->dCoef; P.ldc = ldc; P.d = d;
     P.kindm = m->kind; P.kindg = g->kind; P.sf2m = m->sf2; P.sf2g = g->sf2; P.amp = std::sqrt(2.0 * g->sf2 / F);
-    // Phi_g w: the eval kernel over the feature segment alone, with g's training points as the candidates
+    // Phi_g w: the eval kernel over the feature segment alone, with g's training points as the candidates.  The intermediates live in
+    // the model's workspace: V (Phi_g w + E e, then c), T = W_g V, the normals e and a | b
     const int Sp = (int)round128(S), Npg = g->Np;
-    double *dV = nullptr, *dT = nullptr, *dE = nullptr, *dAB = nullptr, *dWk = nullptr;
-    auto cleanup = [&]() { for (double* q : {dV, dT, dE, dAB, dWk}) if (q) cudaFree(q); };
-    auto failc = [&](int r) { cudaStreamSynchronize(st); cleanup(); return fail(r); };
-    if (cudaMalloc(&dV, sizeof(double) * (size_t)Npg * Sp) || cudaMalloc(&dT, sizeof(double) * (size_t)Npg * Sp) ||
-        cudaMalloc(&dE, sizeof(double) * (size_t)Ng * S) || cudaMalloc(&dAB, sizeof(double) * 2 * (size_t)m->Np) ||
-        cudaMalloc(&dWk, sizeof(double) * (size_t)Ng * d)) {
-        set_error("out of device memory"); return failc(IBO_E_NOMEM);
-    }
+    CandWork* cw = cand_work(m);
+    auto failc = [&](int r) { cudaStreamSynchronize(st); return fail(r); };
+    if ((rc = grow(&cw->dV, &cw->vCap, (size_t)Npg * Sp)) || (rc = grow(&cw->dKc, &cw->kcCap, (size_t)Npg * Sp)) ||
+        (rc = grow(&cw->dNormals, &cw->normalsCap, (size_t)Ng * S)) || (rc = grow(&cw->dAB, &cw->abCap, 2 * (size_t)m->Np)))
+        return failc(rc);
+    double *dV = cw->dV, *dT = cw->dKc, *dE = cw->dNormals, *dAB = cw->dAB;
     if (cudaMemsetAsync(dV, 0, sizeof(double) * (size_t)Npg * Sp, st) || cudaMemsetAsync(dAB, 0, sizeof(double) * 2 * (size_t)m->Np, st) ||
         h2d(dE, e, (size_t)Ng * S)) { set_error("copy failed"); return failc(IBO_E_CUDA); }
     {
@@ -501,41 +492,29 @@ extern "C" int ibo_paths_create(ibo_model* m, int F, int S, const double* omega,
         g_launches++;
     }
     // + E e: sqrt(1 + noise - sf2) e for a plain, legacy or appended model; chol(inv(C) + (1 + noise - sf2) I) e with a Laplace term,
-    // factorised on the device in a scratch model (as joint.cu factorises Sigma); then c = W_g^T W_g (.)
+    // factorised on the device in the model's scratch factor (as joint.cu factorises Sigma); then c = W_g^T W_g (.)
     if (!g->has_cinv) {
         const double escale = std::sqrt(std::max(0.0, 1.0 + g->noise - g->sf2));
         add_scaled_kernel<<<(unsigned)(((long)Ng * S + 255) / 256), 256, 0, st>>>(dV, Sp, dE, Ng, S, escale);
         g_launches++;
     } else {
-        ibo_model sc;
-        sc.device = m->device;
-        sc.stream = m->stream; sc.stream2 = m->stream2; sc.stream3 = m->stream3; sc.stream4 = m->stream4;
-        sc.evStep = m->evStep; sc.evRest = m->evRest; sc.evScale = m->evScale; sc.evFar = m->evFar;
-        sc.N = Ng; sc.Np = Npg; sc.nb = Npg / 128; sc.d = d;
-        auto freesc = [&]() { for (void* q : {(void*)sc.dA, (void*)sc.dD, (void*)sc.dInfo}) if (q) cudaFree(q); };
-        if (cudaMalloc(&sc.dA, sizeof(double) * (size_t)Npg * Npg) || cudaMalloc(&sc.dD, sizeof(double) * (size_t)sc.nb * 128 * 128) ||
-            cudaMalloc(&sc.dInfo, sizeof(int)) || cudaMemsetAsync(sc.dInfo, 0, sizeof(int), st)) {
-            freesc(); set_error("out of device memory"); return failc(IBO_E_NOMEM);
-        }
+        if ((rc = chol_setup(m, Ng, false))) return failc(rc);
+        Factor& sc = cw->chol;
         const bool fromA = g->dCinv == nullptr;
         noise_matrix_kernel<<<dim3((Npg + 255) / 256, Npg), 256, 0, st>>>(sc.dA, Npg, fromA ? g->dAorig : g->dCinv, fromA ? 1 : 0, g->dXt, Ng, d,
                                                                           g->kind, g->sf2, 1.0 + g->noise - g->sf2);
         g_launches++;
         int hinfo = 0;
-        if ((rc = launch_factorize(&sc, false, false, false)) ||
-            (rc = cudaMemcpyAsync(&hinfo, sc.dInfo, sizeof(int), cudaMemcpyDeviceToHost, st) || cudaStreamSynchronize(st) ? IBO_E_CUDA : 0)) {
-            cudaStreamSynchronize(st); freesc(); return failc(rc);
-        }
+        if ((rc = launch_factorize(*m, sc, false, false, false)) ||
+            (rc = cudaMemcpyAsync(&hinfo, sc.dInfo, sizeof(int), cudaMemcpyDeviceToHost, st) || cudaStreamSynchronize(st) ? IBO_E_CUDA : 0))
+            return failc(rc);
         if (hinfo != 0) {
-            freesc();
             if (info) *info = hinfo;
             set_error("inv(C) + (1 + noise - sf2) I is not positive definite (pivot " + std::to_string(hinfo) + ")");
             return failc(IBO_E_NOTSPD);
         }
         tri_noise_kernel<<<dim3((S + 255) / 256, Ng), 256, 0, st>>>(dV, Sp, sc.dA, Npg, dE, S);
         g_launches++;
-        cudaStreamSynchronize(st);
-        freesc();
     }
     launch_w_gemm_v(dT, g, dV, Sp, st);
     launch_w_gemm_z(dV, g, dT, Sp, st);
@@ -543,7 +522,6 @@ extern "C" int ibo_paths_create(ibo_model* m, int F, int S, const double* omega,
     build_coef_kernel<<<dim3((ldc + 255) / 256, std::max(Nm, Ng)), 256, 0, st>>>(p->dCoef, ldc, Nm, Ng, r1, dAB, dB, dV, Sp, S, merged ? 1 : 0);
     g_launches++;
     if (cudaStreamSynchronize(st) != cudaSuccess || cudaGetLastError() != cudaSuccess) { set_error("paths create failed"); return failc(IBO_E_CUDA); }
-    cleanup();
     P.nseg = 0;
     P.segEnd[P.nseg] = r1; P.segKind[P.nseg++] = SEG_KM;
     if (!merged) { P.segEnd[P.nseg] = r2; P.segKind[P.nseg++] = SEG_KG; }
@@ -559,7 +537,7 @@ extern "C" int ibo_paths_eval(ibo_paths* p, const double* Xs, long M, double* va
     const long chunk = std::min<long>(round_to(M, PT), eval_chunk(d, S));
     const size_t raw = (size_t)chunk * d, vals = (size_t)chunk * S, res = 2 * (size_t)S;
     int rc;
-    if ((rc = grow_dev(&p->dWork, &p->workCap, raw + vals + res + eval_work(d, S, chunk)))) return rc;
+    if ((rc = grow(&p->dWork, &p->workCap, raw + vals + res + eval_work(d, S, chunk)))) return rc;
     double* dX = p->dWork;
     double* dVals = dX + raw;
     double* dBest = dVals + vals;
@@ -596,7 +574,7 @@ extern "C" int ibo_paths_grad(ibo_paths* p, const double* Xs, long M, const int*
     const int d = p->d;
     const size_t n = (size_t)M;
     int rc;
-    if ((rc = grow_dev(&p->dWork, &p->workCap, n * (4 * d + 1) + (n + 1) / 2))) return rc;
+    if ((rc = grow(&p->dWork, &p->workCap, n * (4 * d + 1) + (n + 1) / 2))) return rc;
     double* dX = p->dWork;
     double* Cm = dX + n * d;
     double* Cg = Cm + n * d;

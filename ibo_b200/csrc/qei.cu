@@ -444,7 +444,7 @@ int qnei_device(ibo_model* m, const double* Xs, long B, int q, const double* Xba
         if (prior && (rc = grow(&w->dKb, &w->kbCap, (size_t)M))) return rc;
     }
     if ((rc = chol_setup(m, P, true))) return rc;
-    ibo_model* const c = &w->chol;
+    Factor& c = w->chol;
     double* const baseRaw = w->dBase;
     double* const baseS = baseRaw + (size_t)P * d;
     double* const mub = baseS + (size_t)Pp * d;
@@ -467,9 +467,9 @@ int qnei_device(ibo_model* m, const double* Xs, long B, int q, const double* Xba
     launch_w_gemm_v(w->dVb, g, w->dKc, Pp, st);
     if (wantGrad) launch_w_gemm_z(w->dZbase, g, w->dVb, Pp, st);                                 // R_g^-1 K(X_g, X_b)
     launch_joint_sigma(c, baseS, w->dVb, g, g->sf2, jitter, st);
-    if ((rc = launch_factorize(c, false, false, true))) return rc;
+    if ((rc = launch_factorize(*m, c, false, false, true))) return rc;
     int hinfo = 0;
-    IBO_CUDA_TRY(cudaMemcpyAsync(&hinfo, c->dInfo, sizeof(int), cudaMemcpyDeviceToHost, st));
+    IBO_CUDA_TRY(cudaMemcpyAsync(&hinfo, c.dInfo, sizeof(int), cudaMemcpyDeviceToHost, st));
     IBO_CUDA_TRY(cudaStreamSynchronize(st));
     if (hinfo != 0) {
         if (info) *info = hinfo;
@@ -477,7 +477,7 @@ int qnei_device(ibo_model* m, const double* Xs, long B, int q, const double* Xba
         return IBO_E_NOTSPD;
     }
     launch_clear_diag_upper(c, st);
-    launch_trimm(w->dFb, Sp, c->dA, Pp, w->dZb, Sp, nbP, Sp, mub, Pi, st);
+    launch_trimm(w->dFb, Sp, c.dA, Pp, w->dZb, Sp, nbP, Sp, mub, Pi, st);
     launch_sample_max(w->dFb, Sp, Pi, S, reinterpret_cast<long long*>(w->dArg), mmax, st);
     const size_t plane = (size_t)M * d;
     for (long b0 = 0; b0 < B; b0 += Bc) {
@@ -495,7 +495,7 @@ int qnei_device(ibo_model* m, const double* Xs, long B, int q, const double* Xba
         launch_w_gemm_v(w->dV, g, w->dKc, Mcp, st);
         launch_cross_cov_pts(w->dCT, baseS, Pi, Pp, g, w->dScaled, Mc, Mcp, st);                  // C = K(X_b, X_q) - V_b^T V_q
         launch_gemm(w->dCT, Mcp, w->dVb, Pp, true, w->dV, Mcp, Pp, Mcp, Np, -1.0, true, st);
-        launch_trimm(T, Mcp, c->dW, Pp, w->dCT, Mcp, nbP, Mcp, nullptr, 0, st);                   // T = W_bb C
+        launch_trimm(T, Mcp, c.dW, Pp, w->dCT, Mcp, nbP, Mcp, nullptr, 0, st);                    // T = W_bb C
         launch_gemm(w->dH, Mcp, w->dZb, Sp, true, T, Mcp, Sp, Mcp, Pp, 1.0, false, st);           // H = Z_b^T T
         // Schur complements Sigma_qq - T^T T: the rows of [V_q; T] (V_q's padding rows are zero)
         qei_sigma_kernel<<<nbt, 256, 0, st>>>(w->dSig, w->dV, Mcp, w->dScaled, Np + Pi, q, d, g->kind, g->sf2, g->sf2);
@@ -512,7 +512,7 @@ int qnei_device(ibo_model* m, const double* Xs, long B, int q, const double* Xba
         launch_gemm(w->dCT, Mcp, w->dZb, Sp, false, w->dH, Mcp, Pp, Mcp, Sp, 1.0, false, st);     // Tbar = Z_b E - 2 T Gbar
         qei_y_kernel<true><<<dim3((Mc + 255) / 256, Pi), 256, 0, st>>>(w->dCT, T, Mcp, w->dGbar, Mc, q);
         g_launches++;
-        launch_trimm_t(T, Mcp, c->dW, Pp, w->dCT, Mcp, nbP, Mcp, st);                             // Cbar = W_bb^T Tbar
+        launch_trimm_t(T, Mcp, c.dW, Pp, w->dCT, Mcp, nbP, Mcp, st);                              // Cbar = W_bb^T Tbar
         launch_w_gemm_z(w->dKc, g, w->dV, Mcp, st);                                               // y = Z_q Gbar + Z_b Cbar / 2
         qei_y_kernel<<<dim3((Mc + 255) / 256, g->N), 256, 0, st>>>(w->dV, w->dKc, Mcp, w->dGbar, Mc, q);
         g_launches++;

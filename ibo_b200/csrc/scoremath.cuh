@@ -1,11 +1,14 @@
-// Device math shared by the scoring kernels (score.cu: K1-K3, tiny.cu: the fused small-model kernel): covariance from the
-// scaled squared distance, the kernels' own exp, the reference's two erf / EI / PI / UCB arithmetics, the RBF prior mean.
+// Device math shared by the scoring kernels (score.cu: K1-K3, tiny.cu: the fused small-model kernel) and the other kernels that
+// need the same arithmetic: covariance from the scaled squared distance, the kernels' own exp, the reference's two erf / EI / PI /
+// UCB arithmetics, the RBF prior mean.
 #pragma once
 #include "common.cuh"
 #include "../../include/ibo_b200.h"
 
 namespace ibo {
 
+// covariance from the scaled squared distance r2 = sum_j ((x_j - y_j) / theta_j)^2: the model build, the scoring path and the
+// marginal likelihood all evaluate it here (ego/gaussianprocess/kernel.py:87-89,147-149,207-210,246-248; cpp/optimizeGP.cpp:70-112)
 __device__ __forceinline__ double cov_r2(int kind, double sf2, double r2) {
     if (kind <= IBO_KERNEL_SE_ISO) return sf2 * exp(-0.5 * r2);
     double r = sqrt(r2);

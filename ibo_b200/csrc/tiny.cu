@@ -256,28 +256,6 @@ __global__ void __launch_bounds__(128) tiny_fused_kernel(const __grid_constant__
     }
 }
 
-__global__ void __launch_bounds__(256) tiny_argmax_kernel(const double* __restrict__ blkBest, const long long* __restrict__ blkIdx,
-                                                          int nblk, double* __restrict__ best, long long* __restrict__ bestIdx) {
-    __shared__ double ws[256];
-    __shared__ long long wi[256];
-    double sc = -INFINITY;
-    long long idx = 0x7fffffffffffffffLL;
-    for (int b = threadIdx.x; b < nblk; b += 256) {
-        const double os = blkBest[b]; const long long oi = blkIdx[b];
-        if (os > sc || (os == sc && oi < idx)) { sc = os; idx = oi; }
-    }
-    ws[threadIdx.x] = sc; wi[threadIdx.x] = idx;
-    __syncthreads();
-    for (int o = 128; o > 0; o >>= 1) {
-        if ((int)threadIdx.x < o) {
-            const double os = ws[threadIdx.x + o]; const long long oi = wi[threadIdx.x + o];
-            if (os > ws[threadIdx.x] || (os == ws[threadIdx.x] && oi < wi[threadIdx.x])) { ws[threadIdx.x] = os; wi[threadIdx.x] = oi; }
-        }
-        __syncthreads();
-    }
-    if (threadIdx.x == 0) { *best = ws[0]; *bestIdx = wi[0]; }
-}
-
 cudaError_t set_tiny_attrs() {
     const int maxsm = 200 * 1024;
     cudaError_t e = cudaFuncSetAttribute(tiny_fused_kernel<0, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, maxsm);
@@ -359,12 +337,12 @@ int score_tiny(ibo_model* m, const double* cand, long M, const ScoreReq& rq, dou
     if (m->kind <= IBO_KERNEL_SE_ISO) tiny_fused_kernel<0, false><<<grid, 128, smem, st>>>(P, *Ip, nullptr, nullptr);
     else if (m->kind == IBO_KERNEL_MATERN3) tiny_fused_kernel<1, false><<<grid, 128, smem, st>>>(P, *Ip, nullptr, nullptr);
     else tiny_fused_kernel<2, false><<<grid, 128, smem, st>>>(P, *Ip, nullptr, nullptr);
+    g_launches++;
     long nlaunch = 1;
     if (P.want_argmax) {
-        tiny_argmax_kernel<<<1, 256, 0, st>>>(m->dBlkBest, m->dBlkIdx, grid, out + 3 * M, reinterpret_cast<long long*>(out + 3 * M + 1));
+        launch_argmax_final(m->dBlkBest, m->dBlkIdx, grid, out + 3 * M, reinterpret_cast<long long*>(out + 3 * M + 1), st);
         nlaunch++;
     }
-    g_launches += nlaunch;
     if (prof) {
         IBO_CUDA_TRY(cudaEventRecord(m->ev[5], st));
         IBO_CUDA_TRY(cudaEventSynchronize(m->ev[5]));

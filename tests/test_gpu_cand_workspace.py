@@ -1,6 +1,8 @@
-"""GPU tests of the workspace that the joint posterior, the candidate gradients and q-EI share on a model handle: the three entry
-points interleaved on one handle, with sizes that grow and shrink so that buffers grown by one are reused smaller by another, give
-byte for byte what the same call gives on a freshly built handle (empty workspace; model builds are bit-reproducible)."""
+"""GPU tests of the workspace that the candidate-side entry points share on a model handle: the joint posterior, the candidate
+gradients and q-EI, and the entry points that factorise in the workspace's scratch factor (samples, q-NEI, the Laplace fit, sample
+paths of a Laplace model), interleaved on one handle with sizes that grow and shrink so that buffers grown by one are reused smaller
+by another, give byte for byte what the same call gives on a freshly built handle (empty workspace; model builds are
+bit-reproducible)."""
 import ctypes
 
 import numpy as np
@@ -68,6 +70,20 @@ def _pref(N, seed):
     return make, Y.max()
 
 
+def _laplace(N, seed):
+    """a Laplace model with a host-supplied inv(C): N <= 4096 keeps A = R + inv(C), from which sample paths form their noise factor"""
+    rs = np.random.RandomState(seed)
+    X = rs.rand(N, D)
+    Y = 0.5 * rs.randn(N)
+    A = rs.randn(N, N) * 0.05
+    Cinv = np.linalg.inv(np.eye(N) * 5 + A.dot(A.T))
+
+    def make():
+        L = _lib()
+        return L.Model(orc.K_SE_ARD, THETA, X, Y, 0.1, Cinv=Cinv), []
+    return make, Y.max()
+
+
 def _steps(N, ymax, seed):
     """(name, call) in order: sizes grow and shrink across the three entry points, with rejected calls in between"""
     L = _lib()
@@ -111,17 +127,60 @@ def _steps(N, ymax, seed):
     ]
 
 
+def _factor_steps(N, ymax, seed, pref):
+    """(name, call) in order over the entry points that factorise in the scratch factor: the factor grows and shrinks from one to
+    the next (M = 2500, N, P = 300, N, M = 100, P = 50), and sample paths resize V, K*, the normals and a | b; the Laplace fit only
+    on a plain model (pref)"""
+    from ibo_b200.gaussianprocess import path_draws
+    rs = np.random.RandomState(seed)
+    gen = np.random.default_rng(seed)
+    Xs1 = rs.rand(2500, D)
+    Z1 = gen.standard_normal((2500, 16))
+    Xb2, Xbase2 = rs.rand(20, 3, D), rs.rand(300, D)
+    Z2 = gen.standard_normal((303, 64))
+    dr3, Xs3 = path_draws(orc.K_SE_ARD, D, 1024, 80, N, seed), rs.rand(700, D)
+    Xs4 = rs.rand(100, D)
+    Z4 = gen.standard_normal((100, 40))
+    Xb5, Xbase5 = rs.rand(5, 2, D), rs.rand(50, D)
+    Z5 = gen.standard_normal((52, 33))
+    dr6, Xs6 = path_draws(orc.K_SE_ARD, D, 300, 7, N, seed + 1), rs.rand(64, D)
+    v, u = rs.randint(0, N, 400), rs.randint(0, N - 1, 400)
+    u += u >= v                                        # distinct pairs
+    deg = (rs.rand(400) < 0.2).astype(float)
+    start = np.where(np.isin(np.arange(N), v), 0.5, -0.5)
+
+    def paths(dr, Xs):
+        def call(m):
+            p = m.sample_paths(*dr)
+            out = p.eval(Xs)
+            p.close()
+            return out
+        return call
+
+    fit = [("pref_fit", lambda m: m.pref_fit(v, u, deg, start))] if pref else []
+    return [("sample M=2500", lambda m: m.posterior_sample(Xs1, Z1, jitter=1e-9))] + fit + [
+        ("qnei P=300", lambda m: m.qnei(Xb2, Xbase2, Z2, jitter=1e-6)),
+        ("paths S=80", paths(dr3, Xs3)),
+        ("sample M=100", lambda m: m.posterior_sample(Xs4, Z4)),
+    ] + fit + [
+        ("qnei P=50", lambda m: m.qnei(Xb5, Xbase5, Z5, jitter=1e-6, want_grad=False)),
+        ("paths S=7", paths(dr6, Xs6)),
+    ] + fit
+
+
 def _bytes(out):
     if not isinstance(out, tuple):
         out = (out,)
     return [None if a is None else np.asarray(a).tobytes() for a in out]
 
 
-@pytest.mark.parametrize("case,N", [("plain", 8192), ("prior", 2048), ("pref", 300)])
+@pytest.mark.parametrize("case,N", [("plain", 8192), ("prior", 2048), ("pref", 300), ("plain_factor", 600), ("laplace_factor", 700)])
 def test_interleaved_calls_on_one_handle_equal_fresh_handles(case, N):
-    make, ymax = {"plain": _plain, "prior": _prior, "pref": _pref}[case](N, 40)
+    build = {"plain": _plain, "prior": _prior, "pref": _pref, "plain_factor": _plain, "laplace_factor": _laplace}[case]
+    make, ymax = build(N, 40)
+    steps = _factor_steps(N, ymax, 41, case == "plain_factor") if case.endswith("_factor") else _steps(N, ymax, 41)
     shared, keep = make()
-    for name, call in _steps(N, ymax, 41):
+    for name, call in steps:
         got = _bytes(call(shared))
         fresh, keep_f = make()
         want = _bytes(call(fresh))
@@ -129,4 +188,28 @@ def test_interleaved_calls_on_one_handle_equal_fresh_handles(case, N):
             h.close()
         assert got == want, name
     for h in [shared] + keep:
+        h.close()
+
+
+def test_pref_fit_after_a_failed_sample_on_the_same_handle():
+    """a failed ibo_posterior_sample leaves its pivot in the scratch factor's status word; a Laplace fit on the same handle from a
+    start that already meets gtol (no Newton step, so no factorisation clears it) still succeeds, with a fresh handle's bytes"""
+    L = _lib()
+    X = np.array([[3.0 * i, 0.0] for i in range(6)])
+    hyper = [0.3, 2.0]                                 # Matern-3/2, sf2 = 4 > 1 + noise: a repeated candidate is indefinite
+
+    def make():
+        return L.Model(orc.K_MATERN3, hyper, X, np.zeros(6), 0.1)
+    Xs = np.array([[100., 100.], [100., 100.], [50., 50.]])
+    Z = np.random.default_rng(0).standard_normal((3, 4))
+    v, u, deg, start = [0, 2, 4], [1, 3, 5], [0.0, 1.0, 0.0], np.array([.5, -.5, .5, -.5, .5, -.5])
+    m = make()
+    with pytest.raises(L.NotPositiveDefinite) as ei:
+        m.posterior_sample(Xs, Z)
+    assert ei.value.pivot == 2
+    got = m.pref_fit(v, u, deg, start, gtol=1e6)
+    assert got[3] == 0
+    fresh = make()
+    assert _bytes(got) == _bytes(fresh.pref_fit(v, u, deg, start, gtol=1e6))
+    for h in (m, fresh):
         h.close()
