@@ -31,7 +31,7 @@
 
 namespace ibo {
 void set_error(const std::string& s);
-int eval_neg_acq(ibo_model* m, const double* Xs, long n, int acq, double ymax, double parm, int flags, double* y);
+int eval_neg_acq(ibo_model* m, const double* Xs, long n, int acq, double ymax, double parm, int flags, ScoreForce force, double* y);
 int batch_uses_i8(ibo_model* m, long n, int flags);
 bool tiny_server_fits(const ibo_model* m, long n);
 int tiny_server_eval(ibo_model* m, const double* X, long n, int acq, double ymax, double parm, int flags, double* y);
@@ -596,8 +596,10 @@ void gpu_batch(void* user, long n, int ndim, const double* X, double* y) {
         int rcLocal = IBO_OK;
         // INT8 or FP64 kernels: decided from the size of the whole batch, exactly as the unsharded query decides it, so that every
         // candidate gets the same bits on whatever rank and in whatever slice it is evaluated
-        const int sliceFlags = g->flags | (batch_uses_i8(g->m, n, g->flags) ? 0x20000000 : IBO_FLAG_FP64);
-        if (hi > lo) rcLocal = eval_neg_acq(g->m, X + (size_t)lo * ndim, hi - lo, g->acq, g->ymax, g->parm, sliceFlags, g->mine.data());
+        const bool i8 = batch_uses_i8(g->m, n, g->flags) != 0;
+        const int sliceFlags = i8 ? g->flags : g->flags | IBO_FLAG_FP64;
+        const ScoreForce force = i8 ? ScoreForce::I8 : ScoreForce::None;
+        if (hi > lo) rcLocal = eval_neg_acq(g->m, X + (size_t)lo * ndim, hi - lo, g->acq, g->ymax, g->parm, sliceFlags, force, g->mine.data());
         g->mine[(size_t)per] = rcLocal == IBO_OK ? 0.0 : 1.0;
         int rc2 = ibo_comm_allgather(g->mine.data(), per + 1, g->all.data());
         g->rc = rcLocal != IBO_OK ? rcLocal : rc2;
@@ -615,7 +617,7 @@ void gpu_batch(void* user, long n, int ndim, const double* X, double* y) {
         g->rc = tiny_server_eval(g->m, X, n, g->acq, g->ymax, g->parm, g->flags, y);
     } else {
         if (g->server) tiny_server_stop(g->m);      // the resident kernel owns the model's stream: it leaves before anything else is launched
-        g->rc = eval_neg_acq(g->m, X, n, g->acq, g->ymax, g->parm, g->flags, y);
+        g->rc = eval_neg_acq(g->m, X, n, g->acq, g->ymax, g->parm, g->flags, ScoreForce::None, y);
     }
     g->t_eval += std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
     g->batches++; g->points += n;

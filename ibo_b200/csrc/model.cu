@@ -103,6 +103,17 @@ int grow(double** p, size_t* cap, size_t need) {
     return IBO_OK;
 }
 
+int grow_blk(ibo_model* m, size_t need, size_t cap) {
+    if (m->blkCap >= need) return IBO_OK;
+    if (m->dBlkBest) cudaFree(m->dBlkBest);
+    if (m->dBlkIdx) cudaFree(m->dBlkIdx);
+    m->dBlkBest = nullptr; m->dBlkIdx = nullptr; m->blkCap = 0;
+    IBO_CUDA_TRY(cudaMalloc(&m->dBlkBest, sizeof(double) * cap));
+    IBO_CUDA_TRY(cudaMalloc(&m->dBlkIdx, sizeof(long long) * cap));
+    m->blkCap = cap;
+    return IBO_OK;
+}
+
 // A[i][j] = k(x_i, x_j) (i != j), `diag` (1 + noise for the GP's R) on the diagonal, + Cinv; identity in the padding.
 __global__ void build_A_kernel(double* __restrict__ A, const double* __restrict__ Xt, const double* __restrict__ Cinv,
                                int N, int Np, int d, int kind, double sf2, double diag) {

@@ -144,7 +144,9 @@ namespace ibo {
 struct ScoreReq;
 // fused single-launch path for models of one row-block (tiny.cu)
 bool tiny_eligible(const ibo_model* m, long M);
-int score_tiny(ibo_model* m, const double* cand, long M, const ScoreReq& rq, double* out, const double* host_cand);
+int score_tiny(ibo_model* m, const double* cand, long M, const ScoreReq& rq, double* out, const CandInline* inl);
+// the scoring path's block-argmax pair (dBlkBest, dBlkIdx) holds at least `need` blocks; a smaller pair is freed and `cap` blocks allocated
+int grow_blk(ibo_model* m, size_t need, size_t cap);
 // batch server for one DIRECT query on such a model: y[i] = -acq(X[i]); the first call starts the resident kernel, stop ends it
 bool tiny_server_fits(const ibo_model* m, long n);
 int tiny_server_eval(ibo_model* m, const double* X, long n, int acq, double ymax, double parm, int flags, double* y);

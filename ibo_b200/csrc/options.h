@@ -1,4 +1,5 @@
-// Tuning / debugging switches of libibo_b200 (host-only header: shared by the CUDA sources and the host DIRECT driver).
+// Tuning / debugging switches of libibo_b200 and the scoring paths a caller can force (host-only header: shared by the CUDA
+// sources and the host DIRECT driver).
 #pragma once
 
 namespace ibo {
@@ -26,5 +27,9 @@ enum {
     OPT_COUNT
 };
 long get_option(int id);
+
+// A scoring path a caller imposes on a batch whatever its size (score.cu, plan_score): the guard pass re-scores its candidates with
+// K2's throughput shape, and a sharded DIRECT slice takes the INT8 path when the whole batch does.
+enum class ScoreForce { None, Fp64Wide, I8 };
 
 }  // namespace ibo

@@ -679,8 +679,6 @@ static long chunk_tiles_default(int sms) {
     return v > 0 ? v : 2L * sms;
 }
 
-static long narrow_threshold() { return get_option(OPT_NARROW_MAX); }
-
 // ---------------------------------------------------------------------------------------------
 // K2 launch plans.  A plan fixes the CTA shape (MT), the number G of CTAs that share one candidate tile, and the table
 // that deals the (row-block, sub-block) units of a tile to those G CTAs.
@@ -905,10 +903,6 @@ static void launch_kstar(const ibo_model* m, const double* dCand, double* slab, 
 #include "score_i8.cuh"
 namespace ibo {
 
-constexpr int FLAG_FORCE_WIDE = 0x40000000;     // internal: K2's throughput shape (and no fused small-model kernel) whatever the batch size
-constexpr int FLAG_I8_ANY_SIZE = 0x20000000;    // internal (sharded DIRECT): the INT8 path whatever the size of this slice -- the
-                                                // arithmetic of a candidate is chosen from the size of the FULL batch on every rank
-
 static cudaError_t set_i8_attrs() {
     return cudaFuncSetAttribute(trigemm_i8_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, I8_SMEM);
 }
@@ -920,105 +914,121 @@ static bool i8_eligible(const ibo_model* m, int flags) {
     if (m->var_model || m->d > 32 || m->Np > 16384 || (flags & IBO_FLAG_FP64)) return false;
     return (flags & IBO_FLAG_INT8) || get_option(OPT_INT8) != 0;
 }
-// Mid-size batches (DIRECT's, up to narrow_max candidates) on a model of more than one row-block: the FP64 latency shapes need
-// N^2 flops per candidate at 37 TF/s, the INT8 kernels finish a large enough batch several times sooner.  Where "large enough"
-// starts was measured (tools/i8_crossover.py, host candidates in, scores out, d = 6 and 20): the INT8 call costs ~50 us + N / 60 us
-// up to ~256 candidates, the FP64 call ~40 us + 3.5e-8 us x M N^2; they cross at M = 735 / 300 / 133 / 62 for N = 1024 / 2048 /
-// 4096 / 8192.  Option i8_min_batch: -1 this rule, 0 never, > 0 a fixed batch size.
-static bool i8_for_small_batch(const ibo_model* m, long M, int flags) {
-    if (!i8_eligible(m, flags) || m->nb < 2) return false;
-    if (flags & FLAG_I8_ANY_SIZE) return true;
+
+// The kernels that score a batch: the fused small-model kernel (tiny.cu), K2's latency shapes, its throughput shape, or the INT8 path.
+// A forced INT8 path (a sharded DIRECT slice) takes the arithmetic the whole batch was given whatever the size of the slice.
+enum class ScorePath { Tiny, Fp64Latency, Fp64Wide, I8 };
+
+static ScorePath score_path(const ibo_model* m, long M, int flags, ScoreForce force) {
+    if (force == ScoreForce::None && tiny_eligible(m, M)) return ScorePath::Tiny;      // N <= 128, small batch: one fused launch
+    if (force == ScoreForce::Fp64Wide) return ScorePath::Fp64Wide;
+    const bool i8 = i8_eligible(m, flags);
+    if (force == ScoreForce::I8 && i8) return ScorePath::I8;
+    if (M > get_option(OPT_NARROW_MAX)) return i8 ? ScorePath::I8 : ScorePath::Fp64Wide;
+    // Mid-size batches (DIRECT's, up to narrow_max candidates) on a model of more than one row-block: the FP64 latency shapes need
+    // N^2 flops per candidate at 37 TF/s, the INT8 kernels finish a large enough batch several times sooner.  Where "large enough"
+    // starts was measured (tools/i8_crossover.py, host candidates in, scores out, d = 6 and 20): the INT8 call costs ~50 us + N / 60 us
+    // up to ~256 candidates, the FP64 call ~40 us + 3.5e-8 us x M N^2; they cross at M = 735 / 300 / 133 / 62 for N = 1024 / 2048 /
+    // 4096 / 8192.  Option i8_min_batch: -1 this rule, 0 never, > 0 a fixed batch size.
     const long lo = get_option(OPT_I8_MIN_BATCH);
-    if (lo >= 0) return lo > 0 && M >= lo;
     const double n = (double)m->Np;
-    return (double)M * 3.5e-8 * n * n >= 10.0 + n / 60.0;
+    const bool mid = lo >= 0 ? lo > 0 && M >= lo : (double)M * 3.5e-8 * n * n >= 10.0 + n / 60.0;
+    return (i8 && m->nb >= 2 && mid) ? ScorePath::I8 : ScorePath::Fp64Latency;
 }
 
-// Runs K1..K4 for M candidates resident at dCand; results land in m->dOut ([score|mu|s2][M]) and
-// the (best score, best index) pair at m->dOut[3M], [3M+1].  Everything is enqueued on m->stream; the only host
-// synchronisation is the 4-byte read of the guard count on the INT8 path of a small-noise model.
+// Everything score_device launches for a batch, decided before anything is launched.  Nothing is allocated here but a K2 latency
+// plan the model has not cached yet.
+struct ScorePlan {
+    ScorePath path;
+    bool inlineCand;            // a batch in host memory rides in the parameter buffer of K1 or of the fused kernel
+    long tilesTotal, chunkTiles, Mpad;     // 128-candidate tiles of the batch and of a chunk; columns of a chunk's partial planes
+    K2Plan k2, k2Var;           // FP64 K2 of the model and of its variance model (a shorter last chunk of the wide shape regroups)
+    bool guard;                 // INT8 path: candidates with a small sigma^2 are re-scored by the DMMA kernels
+    bool i8pipe;                // INT8 path: K1 of chunk c+1 on stream2 under K2 of chunk c
+};
+
+static ScorePlan plan_score(ibo_model* m, long M, int flags, ScoreForce force) {
+    ScorePlan p{};
+    p.path = score_path(m, M, flags, force);
+    ibo_model* vm = m->var_model;
+    const bool i8 = p.path == ScorePath::I8, narrow = p.path == ScorePath::Fp64Latency;
+    // the fused kernel and the FP64 K1 in its expansion form read the parameter buffer (K3 reads candidates only for a prior mean)
+    p.inlineCand = (size_t)M * m->d <= (size_t)CAND_INLINE &&
+                   (p.path == ScorePath::Tiny || (!i8 && m->npb == 0 && kstar_uses_mma(m) && (!vm || kstar_uses_mma(vm))));
+    if (p.path == ScorePath::Tiny) return p;
+    const int sms = dev_info(m->device).sms;
+    p.tilesTotal = (M + TN - 1) / TN;
+    p.chunkTiles = std::min<long>(p.tilesTotal, chunk_tiles_default(sms));
+    // keep the slab below ~6 GiB (FP64: 8 N bytes per candidate; INT8: 7 N bytes, double buffered)
+    while (p.chunkTiles > 1 && (double)p.chunkTiles * m->nb * KB_PER_BLOCK * BLOB * (i8 ? 14.0 : 8.0) > 6.0e9) p.chunkTiles = (p.chunkTiles + 1) / 2;
+    p.Mpad = p.chunkTiles * TN;
+    const long ctaTiles = narrow ? (std::min<long>(M, p.Mpad) + 31) / 32 : p.chunkTiles;      // K2 CTAs along the candidate axis
+    p.k2 = narrow ? plan_narrow_cached(m, ctaTiles) : K2Plan{8, pick_groups_wide(m->nb, p.chunkTiles, sms)};
+    if (vm) p.k2Var = narrow ? plan_narrow_cached(vm, ctaTiles) : K2Plan{8, pick_groups_wide(vm->nb, p.chunkTiles, sms)};
+    // a guard pass only for a model whose sigma^2 can get below the threshold (sigma^2 >= noise for a model built from R)
+    p.guard = i8 && get_option(OPT_I8_GUARD) != 0 && (m->noise < I8_GUARD_S2 || m->from_inverse);
+    // a single chunk has nothing to overlap; with IBO_FLAG_PROFILE the chunks run back to back so that K1 / K2 can be timed
+    p.i8pipe = i8 && !(flags & IBO_FLAG_PROFILE) && get_option(OPT_I8_PIPE) != 0 && p.tilesTotal > p.chunkTiles;
+    return p;
+}
+
+static int guard_pass(ibo_model* m, const double* dCand, long M, const ScoreReq& rq, unsigned char* dFlag, double* out, int* guarded);
+
+// Runs the kernels of `plan` for M candidates resident at dCand: K1..K3 per chunk, K4, and the guard pass of the INT8 path.  Results
+// land in m->dOut ([score|mu|s2][M]) and the (best score, best index) pair at m->dOut[3M], [3M+1].  Everything is enqueued on
+// m->stream; the only host synchronisation is the 4-byte read of the guard count on the INT8 path of a small-noise model.
+// `inl`: a batch from host memory that the plan puts in the parameter buffer (dCand is then null).
 // `hostWide`: the candidates are still in host memory (all M of them, destined for dCand): every chunk is copied on a separate
 // stream two chunks ahead of the kernels that read it, so that a call from host buffers pays for the first chunk's copy only.
-static int score_device(ibo_model* m, const double* dCand, long M, const ScoreReq& rq, double* outBase = nullptr,
-                        const double* hostCand = nullptr, const double* hostWide = nullptr) {
+static int score_device(ibo_model* m, const ScorePlan& plan, const double* dCand, long M, const ScoreReq& rq, double* outBase = nullptr,
+                        const CandInline* inl = nullptr, const double* hostWide = nullptr) {
     cudaError_t ae = ensure_attrs(m->device, ATTR_SCORE, set_score_attrs);
     if (ae != cudaSuccess) { set_error(std::string("cudaFuncSetAttribute: ") + cudaGetErrorString(ae)); return IBO_E_CUDA; }
     if (m->d > 64) { set_error("d > 64 not supported"); return IBO_E_BADARG; }
-    const bool forceWide = (rq.flags & FLAG_FORCE_WIDE) != 0;
-    if (!forceWide && tiny_eligible(m, M)) {       // N <= 128, small batch: one fused launch (tiny.cu)
-        int rc0;
-        if (!outBase && (rc0 = grow(&m->dOut, &m->outCap, (size_t)3 * M + 2))) return rc0;
+    int rc;
+    if (plan.path == ScorePath::Tiny) {
+        if (!outBase && (rc = grow(&m->dOut, &m->outCap, (size_t)3 * M + 2))) return rc;
         if (hostWide) IBO_CUDA_TRY(cudaMemcpyAsync(const_cast<double*>(dCand), hostWide, sizeof(double) * (size_t)M * m->d, cudaMemcpyHostToDevice, m->stream));
-        return score_tiny(m, dCand, M, rq, outBase ? outBase : m->dOut, hostCand);
+        return score_tiny(m, dCand, M, rq, outBase ? outBase : m->dOut, inl);
     }
     cudaStream_t st = m->stream;
     const int sms = dev_info(m->device).sms;
     const bool prof = (rq.flags & IBO_FLAG_PROFILE) != 0;
     ibo_model* vm = m->var_model;
     const int nb = m->nb;
-    // hostCand given and dCand null: the batch is small enough to ride in K1's parameter buffer (score_host decided)
-    CandInline inlBuf;
-    const CandInline* inl = nullptr;
-    if (hostCand && !dCand) {
-        std::memcpy(inlBuf.x, hostCand, sizeof(double) * (size_t)M * m->d);
-        inl = &inlBuf;
-    }
-    const long tilesTotal = (M + TN - 1) / TN;
-    long chunkTiles = std::min<long>(tilesTotal, chunk_tiles_default(sms));
-    const bool i8small = !forceWide && M <= narrow_threshold() && i8_for_small_batch(m, M, rq.flags);
-    const bool narrow = !forceWide && !i8small && M <= narrow_threshold();
-    const bool i8 = !narrow && i8_eligible(m, rq.flags);
-    // keep the slab below ~6 GiB (FP64: 8 N bytes per candidate; INT8: 7 N bytes, double buffered)
-    while (chunkTiles > 1 && (double)chunkTiles * nb * KB_PER_BLOCK * BLOB * (i8 ? 14.0 : 8.0) > 6.0e9) chunkTiles = (chunkTiles + 1) / 2;
-    const long Mpad = chunkTiles * TN;
-    int rc;
-    const long ctaTilesAll = narrow ? (std::min<long>(M, Mpad) + 31) / 32 : chunkTiles;      // K2 CTAs along the candidate axis
-    const K2Plan plan = narrow ? plan_narrow_cached(m, ctaTilesAll) : K2Plan{8, pick_groups_wide(nb, chunkTiles, sms)};
-    const int subs = 8 / plan.MT;
+    const bool i8 = plan.path == ScorePath::I8, narrow = plan.path == ScorePath::Fp64Latency;
+    const long tilesTotal = plan.tilesTotal, chunkTiles = plan.chunkTiles, Mpad = plan.Mpad;
+    const int subs = 8 / plan.k2.MT;
     if (i8) {
         ae = ensure_attrs(m->device, ATTR_I8, set_i8_attrs);
         if (ae != cudaSuccess) { set_error(std::string("cudaFuncSetAttribute: ") + cudaGetErrorString(ae)); return IBO_E_CUDA; }
         if ((rc = ensure_i8(m))) return rc;
     }
     // int8 path: K1 of chunk c+1 (FP64 / integer pipes, low-priority stream2) runs under K2 of chunk c (tensor pipe, main stream);
-    // slab and partial-sum planes are double buffered.  With IBO_FLAG_PROFILE the chunks run back to back so that K1 / K2 can be timed.
-    const bool i8pipe = i8 && !prof && get_option(OPT_I8_PIPE) != 0 && tilesTotal > chunkTiles;     // a single chunk has nothing to overlap
+    // slab and partial-sum planes are double buffered
     const size_t i8SlabBytes = (size_t)chunkTiles * 2 * nb * 4 * I8_B_STAGE, i8PartDbl = (size_t)3 * nb * Mpad;
-    // guard pass: only a model whose sigma^2 can get below the threshold needs it (sigma^2 >= noise for a model built from R)
-    const bool guard = i8 && get_option(OPT_I8_GUARD) != 0 && (m->noise < I8_GUARD_S2 || m->from_inverse);
     if (i8) {
         if ((rc = grow(&m->dSlab, &m->slabCap, 2 * ((i8SlabBytes + 7) / 8)))) return rc;
         if ((rc = grow(&m->dPart, &m->partCap, 2 * i8PartDbl))) return rc;
-        if (guard && (rc = grow(&m->dGuard, &m->guardCap, (size_t)(M + 7) / 8 + (size_t)(M + 1023) / 1024 / 2 + 4))) return rc;
-        if (i8pipe) {
+        if (plan.guard && (rc = grow(&m->dGuard, &m->guardCap, (size_t)(M + 7) / 8 + (size_t)(M + 1023) / 1024 / 2 + 4))) return rc;
+        if (plan.i8pipe) {
             IBO_CUDA_TRY(cudaEventRecord(m->evI8[4], st));
             IBO_CUDA_TRY(cudaStreamWaitEvent(m->stream2, m->evI8[4], 0));
         }
     } else {
         if ((rc = grow(&m->dSlab, &m->slabCap, (size_t)chunkTiles * nb * KB_PER_BLOCK * BLOB))) return rc;
     }
-    unsigned char* const dFlag = guard ? reinterpret_cast<unsigned char*>(m->dGuard) : nullptr;
+    unsigned char* const dFlag = plan.guard ? reinterpret_cast<unsigned char*>(m->dGuard) : nullptr;
     long ci = 0;
     if ((rc = grow(&m->dPart, &m->partCap, (size_t)3 * nb * subs * Mpad))) return rc;
     if ((rc = grow(&m->dOut, &m->outCap, (size_t)3 * M + 2))) return rc;
     double* const out = outBase ? outBase : m->dOut;     // outBase: device-visible pinned host memory (zero-copy results)
     if (vm) {
         if ((rc = grow(&vm->dSlab, &vm->slabCap, (size_t)chunkTiles * vm->nb * KB_PER_BLOCK * BLOB))) return rc;
-    }
-    K2Plan planV{8, 1};
-    if (vm) {
-        planV = narrow ? plan_narrow_cached(vm, ctaTilesAll) : K2Plan{8, pick_groups_wide(vm->nb, chunkTiles, sms)};
-        if ((rc = grow(&vm->dPart, &vm->partCap, (size_t)3 * vm->nb * (8 / planV.MT) * Mpad))) return rc;
+        if ((rc = grow(&vm->dPart, &vm->partCap, (size_t)3 * vm->nb * (8 / plan.k2Var.MT) * Mpad))) return rc;
     }
     const long nblkTotal = (M + 7) / 8 + tilesTotal;       // generous upper bound (chunk boundaries, 8-candidate blocks of small batches)
-    if (m->blkCap < (size_t)nblkTotal) {
-        if (m->dBlkBest) cudaFree(m->dBlkBest);
-        if (m->dBlkIdx) cudaFree(m->dBlkIdx);
-        m->dBlkBest = nullptr; m->dBlkIdx = nullptr; m->blkCap = 0;
-        IBO_CUDA_TRY(cudaMalloc(&m->dBlkBest, sizeof(double) * nblkTotal));
-        IBO_CUDA_TRY(cudaMalloc(&m->dBlkIdx, sizeof(long long) * nblkTotal));
-        m->blkCap = nblkTotal;
-    }
+    if ((rc = grow_blk(m, (size_t)nblkTotal, (size_t)nblkTotal))) return rc;
     double tK1 = 0, tK2 = 0, tK3 = 0;
     long nlaunch = 0, nK2 = 0;
     if (prof) IBO_CUDA_TRY(cudaEventRecord(m->ev[0], st));
@@ -1044,16 +1054,16 @@ static int score_device(ibo_model* m, const double* dCand, long M, const ScoreRe
             }
             // slot ci & 3 is re-recorded for chunk ci + 4 only two iterations from now, after these waits have been enqueued
             IBO_CUDA_TRY(cudaStreamWaitEvent(st, m->evCopy[ci & 3], 0));
-            if (i8pipe) IBO_CUDA_TRY(cudaStreamWaitEvent(m->stream2, m->evCopy[ci & 3], 0));
+            if (plan.i8pipe) IBO_CUDA_TRY(cudaStreamWaitEvent(m->stream2, m->evCopy[ci & 3], 0));
         }
         const long ctaTiles = narrow ? (chunkM + 31) / 32 : tiles;      // K2 CTAs along the candidate axis
-        K2Plan pl = plan;
+        K2Plan pl = plan.k2;
         if (!narrow && tiles != chunkTiles) pl.G = pick_groups_wide(nb, tiles, sms);      // last, shorter chunk
         if (prof) IBO_CUDA_TRY(cudaEventRecord(m->ev[1], st));
         const int buf = (int)(ci & 1);
         uint8_t* const i8Slab = reinterpret_cast<uint8_t*>(m->dSlab) + (size_t)buf * (((i8SlabBytes + 7) / 8) * 8);
         double* const chunkPart = i8 ? m->dPart + (size_t)buf * i8PartDbl : m->dPart;
-        if (i8pipe) {
+        if (plan.i8pipe) {
             if (ci >= 2) IBO_CUDA_TRY(cudaStreamWaitEvent(m->stream2, m->evI8[2 + buf], 0));     // chunk ci-2 is done with this buffer
             launch_kstar_i8(m, dCand, tiles, M, m0, Mpad, i8Slab, chunkPart, m->stream2);
             IBO_CUDA_TRY(cudaEventRecord(m->evI8[buf], m->stream2));
@@ -1071,7 +1081,7 @@ static int score_device(ibo_model* m, const double* dCand, long M, const ScoreRe
         else if ((rc = launch_trigemm(m, narrow, pl, m->npb > 0, ctaTiles, Mpad, chunkM, st))) return rc;
         nlaunch++; nK2++;
         if (vm) {
-            K2Plan plv = planV;
+            K2Plan plv = plan.k2Var;
             if (!narrow && tiles != chunkTiles) plv.G = pick_groups_wide(vm->nb, tiles, sms);
             if ((rc = launch_trigemm(vm, narrow, plv, false, ctaTiles, Mpad, chunkM, st))) return rc;
             nlaunch++; nK2++;
@@ -1082,7 +1092,7 @@ static int score_device(ibo_model* m, const double* dCand, long M, const ScoreRe
         P.npb = m->npb; P.want_p1 = m->npb > 0;
         P.M = M; P.m0 = m0; P.chunkM = chunkM; P.Mpad = Mpad;
         P.noise = m->noise; P.ymax = rq.ymax; P.parm = rq.parm; P.ptheta = m->ptheta;
-        P.part = chunkPart; P.partVar = vm ? vm->dPart : nullptr; P.nbVarPart = vm ? vm->nb * (8 / planV.MT) : 0; P.MpadVar = Mpad;
+        P.part = chunkPart; P.partVar = vm ? vm->dPart : nullptr; P.nbVarPart = vm ? vm->nb * (8 / plan.k2Var.MT) : 0; P.MpadVar = Mpad;
         P.cand = dCand; P.pmeans = m->dPmeans; P.pbeta = m->dPbeta; P.plb = m->dPlb; P.pwidth = m->dPwidth;
         P.score = rq.want_score ? out : nullptr;
         P.mu = rq.want_mu ? out + M : nullptr;
@@ -1096,7 +1106,7 @@ static int score_device(ibo_model* m, const double* dCand, long M, const ScoreRe
         launch_ex(epilogue_kernel, dim3(nblk), dim3(256), 0, st, narrow && pdl_enabled() && !prof, P);
         nlaunch++;
         blk0 += nblk;
-        if (i8pipe) IBO_CUDA_TRY(cudaEventRecord(m->evI8[2 + buf], st));
+        if (plan.i8pipe) IBO_CUDA_TRY(cudaEventRecord(m->evI8[2 + buf], st));
         ci++;
         if (prof) {
             IBO_CUDA_TRY(cudaEventRecord(m->ev[4], st));
@@ -1114,34 +1124,7 @@ static int score_device(ibo_model* m, const double* dCand, long M, const ScoreRe
     }
     g_launches += nlaunch;
     int guarded = 0;
-    if (guard) {
-        // ---- guard pass: the flagged candidates (ascending index) are re-scored by the DMMA kernels and merged ----
-        const int nblkG = (int)((M + 1023) / 1024);
-        int* blkCnt = reinterpret_cast<int*>(dFlag + (((size_t)M + 7) / 8) * 8);
-        int* dCount = blkCnt + nblkG;
-        guard_count_kernel<<<nblkG, 256, 0, st>>>(dFlag, M, blkCnt);
-        guard_scan_kernel<<<1, 256, 0, st>>>(blkCnt, nblkG, dCount);
-        int count = 0;
-        IBO_CUDA_TRY(cudaMemcpyAsync(&count, dCount, sizeof(int), cudaMemcpyDeviceToHost, st));
-        IBO_CUDA_TRY(cudaStreamSynchronize(st));
-        g_launches += 2;
-        guarded = count;
-        if (count > 0) {
-            if ((rc = grow(&m->dGuardList, &m->guardListCap, (size_t)count * (1 + m->d) + 3 * (size_t)count + 2))) return rc;
-            long long* list = reinterpret_cast<long long*>(m->dGuardList);
-            double* gcand = m->dGuardList + count;
-            double* gout = gcand + (size_t)count * m->d;
-            guard_gather_kernel<<<nblkG, 256, 0, st>>>(dFlag, M, blkCnt, dCand, m->d, list, gcand);
-            ScoreReq r2 = rq;
-            // the throughput shape whatever the count: a guarded candidate then gets exactly the value the FP64 path gives it in any
-            // wide batch -- its score stays a function of (model, x) only
-            r2.flags = (rq.flags | IBO_FLAG_FP64 | FLAG_FORCE_WIDE) & ~(IBO_FLAG_INT8 | IBO_FLAG_PROFILE);
-            if ((rc = score_device(m, gcand, count, r2, gout))) return rc;
-            guard_scatter_kernel<<<(count + 255) / 256, 256, 0, st>>>(list, count, gout, out, M, rq.want_score ? 1 : 0, rq.want_mu ? 1 : 0,
-                                                                       rq.want_s2 ? 1 : 0, (rq.acq >= 0 && rq.want_argmax) ? 1 : 0);
-            g_launches += 2;
-        }
-    }
+    if (plan.guard && (rc = guard_pass(m, dCand, M, rq, dFlag, out, &guarded))) return rc;
     m->lastGuarded = guarded;
     if (prof) {
         IBO_CUDA_TRY(cudaEventRecord(m->ev[5], st));
@@ -1153,6 +1136,38 @@ static int score_device(ibo_model* m, const double* dCand, long M, const ScoreRe
     return IBO_OK;
 }
 
+// Guard pass of the INT8 path: the candidates K3 flagged (ascending index) are re-scored and merged into out; *guarded = their count.
+// They take K2's throughput shape whatever the count: a guarded candidate then gets exactly the value the FP64 path gives it in any
+// wide batch -- its score stays a function of (model, x) only.
+static int guard_pass(ibo_model* m, const double* dCand, long M, const ScoreReq& rq, unsigned char* dFlag, double* out, int* guarded) {
+    cudaStream_t st = m->stream;
+    const int nblkG = (int)((M + 1023) / 1024);
+    int* blkCnt = reinterpret_cast<int*>(dFlag + (((size_t)M + 7) / 8) * 8);
+    int* dCount = blkCnt + nblkG;
+    guard_count_kernel<<<nblkG, 256, 0, st>>>(dFlag, M, blkCnt);
+    guard_scan_kernel<<<1, 256, 0, st>>>(blkCnt, nblkG, dCount);
+    int count = 0;
+    IBO_CUDA_TRY(cudaMemcpyAsync(&count, dCount, sizeof(int), cudaMemcpyDeviceToHost, st));
+    IBO_CUDA_TRY(cudaStreamSynchronize(st));
+    g_launches += 2;
+    *guarded = count;
+    if (count == 0) return IBO_OK;
+    int rc;
+    if ((rc = grow(&m->dGuardList, &m->guardListCap, (size_t)count * (1 + m->d) + 3 * (size_t)count + 2))) return rc;
+    long long* list = reinterpret_cast<long long*>(m->dGuardList);
+    double* gcand = m->dGuardList + count;
+    double* gout = gcand + (size_t)count * m->d;
+    guard_gather_kernel<<<nblkG, 256, 0, st>>>(dFlag, M, blkCnt, dCand, m->d, list, gcand);
+    ScoreReq r2 = rq;
+    r2.flags = rq.flags & ~IBO_FLAG_PROFILE;
+    r2.force = ScoreForce::Fp64Wide;
+    if ((rc = score_device(m, plan_score(m, count, r2.flags, r2.force), gcand, count, r2, gout))) return rc;
+    guard_scatter_kernel<<<(count + 255) / 256, 256, 0, st>>>(list, count, gout, out, M, rq.want_score ? 1 : 0, rq.want_mu ? 1 : 0,
+                                                               rq.want_s2 ? 1 : 0, (rq.acq >= 0 && rq.want_argmax) ? 1 : 0);
+    g_launches += 2;
+    return IBO_OK;
+}
+
 static int score_host(ibo_model* m, const double* Xs, long M, const ScoreReq& rq, double* scores, double* mu, double* s2,
                       double* best_score, long* best_idx) {
     if (!m || !Xs || M < 0) { set_error("bad argument"); return IBO_E_BADARG; }
@@ -1160,6 +1175,7 @@ static int score_host(ibo_model* m, const double* Xs, long M, const ScoreReq& rq
     IBO_CUDA_TRY(cudaSetDevice(m->device));
     int rc;
     if ((rc = grow(&m->dCand, &m->candCap, (size_t)M * m->d))) return rc;
+    const ScorePlan plan = plan_score(m, M, rq.flags, rq.force);
     cudaStream_t st = m->stream;
     // Small batches (DIRECT, gallery) are latency bound: stage through one pinned buffer so that the H2D and the
     // single D2H are plain DMA transfers instead of pageable copies (each of which costs a staging round trip).
@@ -1178,21 +1194,19 @@ static int score_host(ibo_model* m, const double* Xs, long M, const ScoreReq& rq
         // candidates go to device memory with one small DMA (K1 reading them over PCIe costs ~15 us of dependent round trips);
         // the fused small-model kernel stages its tile with one parallel load and reads the mapped buffer directly
         const double* cand = m->dCand;
-        const ibo_model* vmh = m->var_model;
-        if (tiny_eligible(m, M)) cand = m->hPinned;
-        else if (nin <= (size_t)CAND_INLINE && m->npb == 0 && kstar_uses_mma(m) && (!vmh || kstar_uses_mma(vmh)) &&
-                 !i8_for_small_batch(m, M, rq.flags))
-            cand = nullptr;          // the FP64 K1 takes the batch from its parameter buffer (K3 reads candidates only for a prior mean)
+        CandInline inl;
+        if (plan.inlineCand) { std::memcpy(inl.x, Xs, sizeof(double) * nin); cand = nullptr; }
+        else if (plan.path == ScorePath::Tiny) cand = m->hPinned;
         else IBO_CUDA_TRY(cudaMemcpyAsync(m->dCand, m->hPinned, sizeof(double) * nin, cudaMemcpyHostToDevice, st));
         double* ho = m->hPinned + nin;
-        if ((rc = score_device(m, cand, M, rq, ho, m->hPinned))) return rc;
+        if ((rc = score_device(m, plan, cand, M, rq, ho, plan.inlineCand ? &inl : nullptr))) return rc;
         IBO_CUDA_TRY(cudaStreamSynchronize(st));
         if (scores) std::memcpy(scores, ho, sizeof(double) * M);
         if (mu) std::memcpy(mu, ho + M, sizeof(double) * M);
         if (s2) std::memcpy(s2, ho + 2 * M, sizeof(double) * M);
         if (rq.acq >= 0 && rq.want_argmax) { hb = ho[3 * M]; std::memcpy(&hi, &ho[3 * M + 1], 8); }
     } else {
-        if ((rc = score_device(m, m->dCand, M, rq, nullptr, nullptr, Xs))) return rc;
+        if ((rc = score_device(m, plan, m->dCand, M, rq, nullptr, nullptr, Xs))) return rc;
         if (scores) IBO_CUDA_TRY(cudaMemcpyAsync(scores, m->dOut, sizeof(double) * M, cudaMemcpyDeviceToHost, st));
         if (mu) IBO_CUDA_TRY(cudaMemcpyAsync(mu, m->dOut + M, sizeof(double) * M, cudaMemcpyDeviceToHost, st));
         if (s2) IBO_CUDA_TRY(cudaMemcpyAsync(s2, m->dOut + 2 * M, sizeof(double) * M, cudaMemcpyDeviceToHost, st));
@@ -1212,24 +1226,24 @@ __global__ void debug_exp_kernel(const double* __restrict__ x, long n, double* _
     if (i < n) { fast[i] = exp_nonpos(x[i]); ref[i] = exp(x[i]); }
 }
 
-// used by the DIRECT objective (direct.cpp): negated acquisition for n points
-// the arithmetic a DIRECT batch of n points gets (sharded DIRECT asks with the size of the full batch and forces the answer on
-// every rank's slice): 1 = INT8 path, 0 = FP64 kernels
+// sharded DIRECT (direct.cpp): whether a batch of n points is scored on the INT8 path; every rank's slice of it is then scored with
+// ScoreForce::I8 or with IBO_FLAG_FP64, so that a candidate gets the arithmetic of the whole batch
 int batch_uses_i8(ibo_model* m, long n, int flags) {
-    if (n > narrow_threshold()) return i8_eligible(m, flags) ? 1 : 0;
-    return i8_for_small_batch(m, n, flags) ? 1 : 0;
+    return score_path(m, n, flags, ScoreForce::None) == ScorePath::I8 ? 1 : 0;
 }
 // values of the joint posterior (joint.cu) and of the candidate gradients (grad.cu): the scoring path's own kernels, so that they
 // are ibo_score_batch's / ibo_posterior_batch's bit for bit
 int posterior_score_device(ibo_model* m, const double* dCand, long M, int acq, double ymax, double parm, int flags, double* out) {
     ScoreReq rq{acq, ymax, parm, flags, acq >= 0, true, true};
     rq.want_argmax = false;
-    return score_device(m, dCand, M, rq, out);
+    return score_device(m, plan_score(m, M, flags, ScoreForce::None), dCand, M, rq, out);
 }
 
-int eval_neg_acq(ibo_model* m, const double* Xs, long n, int acq, double ymax, double parm, int flags, double* y) {
+// used by the DIRECT objective (direct.cpp): negated acquisition for n points
+int eval_neg_acq(ibo_model* m, const double* Xs, long n, int acq, double ymax, double parm, int flags, ScoreForce force, double* y) {
     ScoreReq rq{acq, ymax, parm, flags, true, false, false};
     rq.want_argmax = false;      // DIRECT consumes every value; the argmax kernels would be wasted launches
+    rq.force = force;
     int rc = score_host(m, Xs, n, rq, y, nullptr, nullptr, nullptr, nullptr);
     if (rc) return rc;
     for (long i = 0; i < n; i++) y[i] = -y[i];
@@ -1280,7 +1294,7 @@ extern "C" int ibo_score_resident(ibo_model* m, ibo_cands* c, int acq, double ym
     cudaStream_t st = m->stream;
     ScoreReq rq{acq, ymax, parm, flags, true, false, false};
     IBO_CUDA_TRY(cudaEventRecord(m->ev[6], st));
-    int rc = score_device(m, c->dX, c->M, rq);
+    int rc = score_device(m, plan_score(m, c->M, flags, ScoreForce::None), c->dX, c->M, rq);
     if (rc) return rc;
     IBO_CUDA_TRY(cudaEventRecord(m->ev[7], st));
     double hb = 0; long long hi = -1;

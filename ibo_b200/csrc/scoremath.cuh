@@ -184,6 +184,7 @@ struct ScoreReq {
     int flags;
     bool want_score, want_mu, want_s2;
     bool want_argmax = true;
+    ScoreForce force = ScoreForce::None;
 };
 
 }  // namespace ibo

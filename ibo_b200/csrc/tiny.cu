@@ -291,8 +291,8 @@ bool tiny_eligible(const ibo_model* m, long M) {
 
 // Scores M candidates at `cand` (device memory, or mapped pinned host memory) into out = [score | mu | s2][M] (+ the argmax
 // pair at out[3M], out[3M+1]); everything is enqueued on m->stream.
-// `host_cand`: the same candidates in host memory when the caller has them there (small batches ride in the parameter buffer)
-int score_tiny(ibo_model* m, const double* cand, long M, const ScoreReq& rq, double* out, const double* host_cand) {
+// `inl`: the batch in the parameter buffer (the caller's plan put it there; cand is then null)
+int score_tiny(ibo_model* m, const double* cand, long M, const ScoreReq& rq, double* out, const CandInline* inl) {
     const cudaError_t ae = ensure_attrs(m->device, ATTR_TINY, set_tiny_attrs);
     if (ae != cudaSuccess) { set_error(std::string("cudaFuncSetAttribute: ") + cudaGetErrorString(ae)); return IBO_E_CUDA; }
     const int g_tiny_sms = dev_info(m->device).sms;
@@ -304,15 +304,8 @@ int score_tiny(ibo_model* m, const double* cand, long M, const ScoreReq& rq, dou
     const size_t smem = tiny_smem(m->N, vm ? vm->N : 0, m->d);
     const int perSM = (int)std::max<size_t>(1, std::min<size_t>(8, (200 * 1024) / smem));
     const int grid = (int)std::min<long>(ntile, (long)g_tiny_sms * perSM);
-    if (m->blkCap < (size_t)grid) {
-        if (m->dBlkBest) cudaFree(m->dBlkBest);
-        if (m->dBlkIdx) cudaFree(m->dBlkIdx);
-        m->dBlkBest = nullptr; m->dBlkIdx = nullptr; m->blkCap = 0;
-        const size_t cap = (size_t)g_tiny_sms * 8;
-        IBO_CUDA_TRY(cudaMalloc(&m->dBlkBest, sizeof(double) * cap));
-        IBO_CUDA_TRY(cudaMalloc(&m->dBlkIdx, sizeof(long long) * cap));
-        m->blkCap = cap;
-    }
+    int rc;
+    if ((rc = grow_blk(m, (size_t)grid, (size_t)g_tiny_sms * 8))) return rc;
     TinyParams P;
     P.side[0] = TinySide{m->dW, m->dXt, m->dCenter, m->N};
     P.side[1] = vm ? TinySide{vm->dW, vm->dXt, vm->dCenter, vm->N} : TinySide{nullptr, nullptr, nullptr, 0};
@@ -325,14 +318,8 @@ int score_tiny(ibo_model* m, const double* cand, long M, const ScoreReq& rq, dou
     P.M = M; P.d = m->d; P.acq = rq.acq; P.mode_py = (rq.flags & IBO_FLAG_MODE_PY) ? 1 : 0; P.npb = m->npb;
     P.want_argmax = (rq.acq >= 0 && rq.want_argmax) ? 1 : 0;
     P.sf2 = m->sf2; P.noise = m->noise; P.ymax = rq.ymax; P.parm = rq.parm; P.ptheta = m->ptheta;
-    static CandInline I;        // launches copy the parameter buffer synchronously; one host thread per model (INTEGRATION.md)
-    CandInline Ilocal;
-    CandInline* Ip = &I;
-    if (host_cand && (size_t)M * m->d <= (size_t)CAND_INLINE) {
-        std::memcpy(Ilocal.x, host_cand, sizeof(double) * (size_t)M * m->d);
-        P.cand = nullptr;
-        Ip = &Ilocal;
-    }
+    static CandInline none;
+    const CandInline* Ip = inl ? inl : &none;
     if (prof) IBO_CUDA_TRY(cudaEventRecord(m->ev[0], st));
     if (m->kind <= IBO_KERNEL_SE_ISO) tiny_fused_kernel<0, false><<<grid, 128, smem, st>>>(P, *Ip, nullptr, nullptr);
     else if (m->kind == IBO_KERNEL_MATERN3) tiny_fused_kernel<1, false><<<grid, 128, smem, st>>>(P, *Ip, nullptr, nullptr);

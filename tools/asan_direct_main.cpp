@@ -1,10 +1,11 @@
 #include "../include/ibo_b200.h"
+#include "../ibo_b200/csrc/options.h"
 #include <cstdio>
 #include <cmath>
 #include <string>
 #include <vector>
 #include <random>
-namespace ibo { void set_error(const std::string&) {} int eval_neg_acq(ibo_model*, const double*, long, int, double, double, int, double*) { return -2; } }
+namespace ibo { void set_error(const std::string&) {} int eval_neg_acq(ibo_model*, const double*, long, int, double, double, int, ScoreForce, double*) { return -2; } }
 extern "C" int ibo_comm_size(void) { return 1; }
 extern "C" int ibo_comm_rank(void) { return 0; }
 extern "C" int ibo_comm_allgather(const double*, long, double*) { return -5; }
